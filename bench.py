@@ -3,6 +3,8 @@
 
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torchrun, one rank per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W   (the reference's own CPU path)
+    python bench.py --gpus N ... --dump-outputs DIR    also write what the last timed step computed as DIR/<name>.npy
+                                                     (N > 1: DIR/<name>_rank<r>.npy, one set per rank)
 
 A "step" is one pass of the hot path over one batch of synthetic input: BLOCKS_PER_STEP independent 32 MiB blocks
 of order-2 Markov text per GPU (BASELINE.json config 5 at one GPU's share), transformed through the batched
@@ -298,6 +300,27 @@ def measure_workload(bw, torch, dev, local_rank, kind, nbytes, nblocks, depth, r
             "launches_per_step": launches, "sum_block_gpu_ms": gms}
 
 
+DUMP_SAMPLES_PER_BLOCK = 1 << 19
+
+
+def dump_outputs(directory, suffix, dev_out, LF, nLF, freqs):
+    """What the last timed step handed its caller for this rank's blocks, as float arrays: the transformed bytes at a
+    fixed sample of distinct positions (seed 0, float32, 32 MiB per rank), and the LFpowers and freqs (float64: exact
+    for the u32 values).  The inputs are seeded too, so two builds given the same arguments can be compared file by
+    file."""
+    import torch
+
+    os.makedirs(directory, exist_ok=True)
+    n = dev_out[0].numel()
+    pos = np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLES_PER_BLOCK, replace=False))
+    idx = torch.from_numpy(pos).to(dev_out[0].device)
+    sample = torch.stack([t[idx] for t in dev_out]).float().cpu().numpy()
+    np.save(os.path.join(directory, "bwt_sample%s.npy" % suffix), sample)
+    np.save(os.path.join(directory, "lfpowers%s.npy" % suffix),
+            np.stack([LF[i, : nLF[i]] for i in range(len(dev_out))]).astype(np.float64))
+    np.save(os.path.join(directory, "freqs%s.npy" % suffix), np.asarray(freqs, np.float64))
+
+
 def main_gpu(args):
     import torch
     import torch.distributed as dist
@@ -361,6 +384,8 @@ def main_gpu(args):
     barrier()
     wall = time.perf_counter() - t0
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "_rank%d" % rank if world > 1 else "", dev_out, LF, nLF, freqs)
 
     # ---- e2e: host (pinned) buffers through the same C-ABI call, H2D + D2H inside the timed region
     for _ in range(max(1, args.warmup // 2)):
@@ -589,6 +614,9 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true")
     ap.add_argument("--no-compress", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the last timed step's outputs (sampled BWT bytes, LFpowers, freqs) as DIR/<name>.npy, "
+                         "or DIR/<name>_rank<r>.npy for each rank with several GPUs; GPU path only")
     ap.add_argument("--leg", default="")
     ap.add_argument("--leg-device", type=int, default=0)
     ap.add_argument("--leg-blocks", type=int, default=32)
@@ -601,6 +629,8 @@ def main():
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the GPU path's outputs; --impl reference has none to write")
         return main_reference(args)
     return main_gpu(args)
 

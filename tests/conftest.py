@@ -4,6 +4,8 @@ Only tests/ (plus __graft_entry__.smoke() and bench.py's cpu_baseline / --impl r
 oracle/liboracle.so or oracle/_ref/libbwtc_ref.so — they are checkers, never the product path.
 """
 import ctypes
+import hashlib
+import json
 import os
 import subprocess
 import sys
@@ -123,9 +125,36 @@ class Reference:
         return int(self.lib.ref_uncompress(src.encode(), dst.encode()))
 
 
+def digest(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+class OracleRecord:
+    """The C oracle's forward transform of the GPU tests' full-size generated blocks, recorded in
+    tests/golden/oracle_bwt_digests.json by tests/golden/make_oracle_digests.py: digests of the transformed bytes and
+    freqs, and the LFpowers, keyed by the digest of the input."""
+
+    def __init__(self):
+        with open(os.path.join(ROOT, "tests", "golden", "oracle_bwt_digests.json")) as f:
+            self.rec = json.load(f)
+
+    def check(self, x, starts, out, LF, fr=None):
+        key = f"{digest(x)}:{starts}"
+        e = self.rec.get(key)
+        assert e is not None, f"no recorded oracle output for this input ({key}): run tests/golden/make_oracle_digests.py"
+        assert [int(v) for v in LF] == e["LF"], (LF, e["LF"])
+        assert fr is None or digest(fr) == e["freqs"], "freqs differ from the oracle's"
+        assert digest(out) == e["bwt"], "BWT bytes differ from the oracle's"
+
+
 @pytest.fixture(scope="session")
 def oracle():
     return Oracle()
+
+
+@pytest.fixture(scope="session")
+def oracle_record():
+    return OracleRecord()
 
 
 @pytest.fixture(scope="session")

@@ -1,7 +1,7 @@
 """GPU parity of the INVERSE transform (SURVEY.md §8f row f4; bwtc_cuda_inverse_block / _raw, kernels in
-bwtc_b200/csrc/ibwt_kernels.cuh): bit-exact against the oracle's restatement and the reference's own
-InverseBWTransform (MtlSaInverseBWT), on the outputs of the REFERENCE forward transform — the inverse must not merely
-undo this repo's forward path — and at BASELINE block sizes."""
+bwtc_b200/csrc/ibwt_kernels.cuh): bit-exact against the oracle's restatement, on the outputs of the oracle's forward
+transform — the inverse must not merely undo this repo's forward path — and at BASELINE block sizes.  The reference's
+own inverse (MtlSaInverseBWT) pins the oracle's in tests/test_oracle.py where the reference is built."""
 import numpy as np
 import pytest
 
@@ -43,11 +43,13 @@ def test_inverse_of_oracle_forward_small_and_structured(ctx, oracle):
 
 
 @pytest.mark.parametrize("kind", ["markov", "dna", "repetitive", "random"])
-def test_inverse_of_reference_forward_matches_reference_inverse(ctx, reference, kind):
+def test_inverse_of_reference_forward_matches_reference_inverse(ctx, oracle, kind):
+    """The forward output of the oracle (the restatement of the reference's forward transform): the GPU's inverse equals
+    the oracle's inverse (the restatement of the reference's) and restores x."""
     x = bw.generate(kind, (1 << 20) + 13, seed=71)
-    b, LF, fr = reference.block(x, 8)
+    b, LF, fr = oracle.block(x, 8)
     back = _gpu_inverse(ctx, b, LF)
-    assert np.array_equal(back, reference.inverse_block(b, LF))
+    assert np.array_equal(back, oracle.inverse_block(b, LF[0]))
     assert np.array_equal(back, x)
 
 
@@ -82,9 +84,9 @@ def test_forward_then_inverse_on_the_device_in_place():
 
 
 @pytest.mark.parametrize("kind,mib", [("markov", 32), ("dna", 64), ("repetitive", 16), ("random", 128)])
-def test_inverse_full_size_blocks(reference, kind, mib):
+def test_inverse_full_size_blocks(oracle_record, kind, mib):
     """BASELINE block sizes: GPU forward (bit-exact to the reference, tests/test_gpu_fullsize.py) then GPU inverse restores
-    the block; the 32 MiB case is also checked against the reference's inverse of the same bytes."""
+    the block; up to 32 MiB the forward output that was inverted is also checked against the oracle's recorded one."""
     n = mib << 20
     x = bw.generate(kind, n, seed=73)
     ctx = bw.CudaContext(n)
@@ -99,7 +101,7 @@ def test_inverse_full_size_blocks(reference, kind, mib):
         ctx.close()
     assert np.array_equal(b, x), kind
     if mib <= 32:
-        assert np.array_equal(reference.inverse_block(fwd, LF), x)
+        oracle_record.check(x, 8, fwd, LF)
     print(f"inverse {kind} {mib} MiB: gpu_ms={st['gpu_ms']:.3f} = {n / 1e6 / (st['gpu_ms'] / 1e3):.0f} MB/s, {st['kernel_launches']} launches")
 
 
