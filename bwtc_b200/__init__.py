@@ -117,6 +117,7 @@ C_ABI = [
     ("bwtc_cuda_inverse_block", ctypes.c_int64, [_vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32]),
     ("bwtc_cuda_inverse_block_device", ctypes.c_int64, [_vp, _vp, _vp, ctypes.c_uint32, ctypes.c_uint32]),
     ("bwtc_cuda_inverse_raw", ctypes.c_int64, [_vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32]),
+    ("bwtc_cuda_inverse_blocks", ctypes.c_int, [_vp, _vp, _vp, _vp, ctypes.c_uint32, ctypes.c_int, _vp, _vp]),
     ("bwtc_cuda_bwt_blocks", ctypes.c_int,
      [_vp, _vp, _vp, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_int, _vp, _vp, _vp]),
     ("bwtc_cuda_num_starting_points", ctypes.c_uint32, [ctypes.c_uint32, ctypes.c_uint32]),
@@ -130,6 +131,8 @@ C_ABI = [
     ("bwtc_cuda_pipeline_submit", ctypes.c_int,
      [_vp, _vp, _vp, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_int, _vp, _vp, _vp, _vp, ctypes.POINTER(ctypes.c_uint64)]),
     ("bwtc_cuda_pipeline_wait", ctypes.c_int, [_vp, ctypes.c_uint64]),
+    ("bwtc_cuda_pipeline_submit_inverse", ctypes.c_int,
+     [_vp, _vp, _vp, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_int, _vp, ctypes.POINTER(ctypes.c_uint64)]),
     ("bwtc_cuda_pipeline_submit_runs", ctypes.c_int,
      [_vp, _vp, _vp, ctypes.c_uint32, ctypes.c_uint32, _vp, _vp, _vp, _vp, ctypes.POINTER(ctypes.c_uint64)]),
     ("bwtc_cuda_pipeline_timing_begin", ctypes.c_int, [_vp]),
@@ -256,6 +259,28 @@ class CudaContext:
         assert bwt.dtype == np.uint8 and LFpowers.dtype == np.uint32
         return self._check(self._lib.bwtc_cuda_inverse_raw(self._h, bwt.ctypes.data, bwt.size, LFpowers.ctypes.data, LFpowers.size))
 
+    def inverse_blocks(self, blocks, LF, on_device: bool = False, out=None) -> None:
+        """bwtc_cuda_inverse_blocks: restore the given blocks (uint8 arrays, or CUDA tensors / (pointer, size) pairs when
+        on_device) IN PLACE, or into `out` (same kinds, same sizes).  LF: per block its LFpowers row (e.g. what bwt_blocks
+        returned) or just its end-of-block row; only LF[k][0] is used.  Equal-sized runs are inverted as one device-side
+        problem; stats() then describes the last run."""
+        count = len(blocks)
+        ptrs, sizes = zip(*[_block_ptr(b, on_device) for b in blocks]) if count else ((), ())
+        a_in = (ctypes.c_void_p * count)(*ptrs)
+        a_out = None
+        if out is not None:
+            assert len(out) == count
+            optrs, osizes = zip(*[_block_ptr(b, on_device) for b in out]) if count else ((), ())
+            assert tuple(osizes) == tuple(sizes), "out[k] must have the size of blocks[k]"
+            a_out = (ctypes.c_void_p * count)(*optrs)
+        a_sz = np.asarray(sizes, dtype=np.uint32)
+        eob = np.asarray(LF, dtype=np.uint32)
+        eob = eob.reshape(count, -1)[:, 0] if eob.size else eob
+        rows = np.zeros((count, 256), dtype=np.uint32)
+        rows[:, 0] = eob
+        self._check(self._lib.bwtc_cuda_inverse_blocks(self._h, a_in, a_out, a_sz.ctypes.data, count, 1 if on_device else 0,
+                                                       rows.ctypes.data, None))
+
     def bwt_blocks(self, blocks, starts: int, want_freqs: bool = True):
         """bwtc_cuda_bwt_blocks: transform the given uint8 arrays IN PLACE (equal-sized runs are batched into one
         device-side sort).  Returns (LFpowers[count, 256], nLF[count], freqs[count, 256] or None)."""
@@ -273,6 +298,16 @@ class CudaContext:
                          freqs: Optional[np.ndarray]) -> int:
         return self._check(self._lib.bwtc_cuda_bwt_block_device(self._h, d_in, d_out, n, LFpowers.ctypes.data,
                                                                  LFpowers.size, _ptr(freqs)))
+
+
+def _block_ptr(b, on_device: bool):
+    """(address, bytes) of a block argument: a uint8 numpy array (host), a CUDA tensor, or a (pointer, size) pair."""
+    if isinstance(b, tuple):
+        return int(b[0]), int(b[1])
+    if on_device:
+        return int(b.data_ptr()), int(b.numel() * b.element_size())
+    assert isinstance(b, np.ndarray) and b.dtype == np.uint8
+    return b.ctypes.data, b.size
 
 
 class BWTBlock:
@@ -447,16 +482,51 @@ class Pipeline:
             raise BwtcCudaError(rc, self._lib.bwtc_cuda_pipeline_error(self._h).decode())
         return h
 
+    def submit_inverse(self, block: np.ndarray, LF):
+        """Streaming inverse (bwtc_cuda_pipeline_submit_inverse): queues one host block (the output of a forward block
+        transform) to be restored in place and returns a handle; wait(handle) returns the block.  LF: the block's
+        LFpowers (only LF[0] is used) or its end-of-block row.  The block must stay alive until then."""
+        assert block.dtype == np.uint8
+        eob = int(np.asarray(LF, dtype=np.uint32).reshape(-1)[0])
+        h = {"kind": "inverse", "block": block, "ticket": ctypes.c_uint64(0)}
+        rc = self._lib.bwtc_cuda_pipeline_submit_inverse(self._h, block.ctypes.data, block.ctypes.data, block.size, eob, 0,
+                                                         None, ctypes.byref(h["ticket"]))
+        if rc < 0:
+            raise BwtcCudaError(rc, self._lib.bwtc_cuda_pipeline_error(self._h).decode())
+        return h
+
     def wait(self, h):
+        """Waits for a handle of submit (returns (LFpowers, freqs)) or of submit_inverse (returns the restored block)."""
         rc = self._lib.bwtc_cuda_pipeline_wait(self._h, h["ticket"])
         if rc < 0:
             raise BwtcCudaError(rc, self._lib.bwtc_cuda_pipeline_error(self._h).decode())
+        if h.get("kind") == "inverse":
+            return h["block"]
         return h["LF"][: h["nLF"].value].copy(), h["freqs"]
 
     def run(self, blocks: Sequence[np.ndarray], starts: int = 8):
         """Transforms host blocks in place."""
         ptrs = [b.ctypes.data for b in blocks]
         return self.run_ptrs(ptrs, ptrs, [b.size for b in blocks], starts, on_device=False)
+
+    def run_inverse(self, blocks: Sequence[np.ndarray], LF) -> None:
+        """Restores host blocks in place: submit_inverse for all, then wait for all (LF[k][0] = block k's end-of-block
+        row).  Raises the first error after every block has been waited for."""
+        LF = np.asarray(LF, dtype=np.uint32).reshape(len(blocks), -1)
+        handles, first = [], None
+        for k, b in enumerate(blocks):
+            try:
+                handles.append(self.submit_inverse(b, LF[k]))
+            except BwtcCudaError as e:  # (the blocks already queued are still waited for)
+                first = e
+                break
+        for h in handles:
+            try:
+                self.wait(h)
+            except BwtcCudaError as e:
+                first = first or e
+        if first is not None:
+            raise first
 
     def timing_begin(self):
         rc = self._lib.bwtc_cuda_pipeline_timing_begin(self._h)

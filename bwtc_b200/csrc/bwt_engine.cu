@@ -1430,6 +1430,63 @@ int64_t run_transform(bwtc_cuda_ctx* ctx, bool block_mode, const uint8_t* h_in, 
 // bwtc_cuda_bwt_block produced (hole at eob filled with L[N-1]), result n bytes of the original block — the contract of
 // InverseBWTransform::doTransform(BWTBlock&) (InverseBWT.cpp:47-51).  raw: N = n_in bytes L[0..N) with L[eob] ignored,
 // result N-1 bytes — the virtual doTransform(byte*, uint32, LFpow) (InverseBWT.hpp:49-50).
+// The device part of an inversion (one block, or a batch of them, ibwt_kernels.cuh InvShape): ev_begin, the keys and C
+// tables, the 2 digit passes, walk1, pointer jumping, walk2 into d_dst.  Adds its launches and algorithmic bytes to
+// ctx->stats; nothing is waited for.  A batch (bhist != nullptr) counts per-block histograms and gets per-block C tables.
+int enqueue_inverse(bwtc_cuda_ctx* ctx, const InvShape& sh, bool block_mode, const uint8_t* d_src, uint8_t* d_dst,
+                    uint32_t* rounds_out, uint32_t* passes_out) {
+  cudaStream_t st = ctx->stream;
+  bwtc_cuda_stats& S = ctx->stats;
+  PassTimer pt{ctx};
+  const uint32_t B = sh.nblocks, N = inv_rows(sh);
+  uint32_t* bhist = B > 1 ? ctx->d_bhist : nullptr;
+  CK(ctx, cudaEventRecord(ctx->ev_begin, st));
+  CK(ctx, cudaMemsetAsync(ctx->d_zero, 0, (size_t)CTR_STICKY * 4, st));
+  if (zero_round_state(ctx, N, N, RS_TILE32, 3u)) return BWTC_CUDA_ECUDA;
+  if (bhist) CK(ctx, cudaMemsetAsync(bhist, 0, (size_t)B * 256 * 4, st));
+  uint32_t* keys0 = static_cast<uint32_t*>(ctx->d_keys[0]);
+  uint32_t* C = ctx->d_ktab;  // B x 258 words (the lazy-rank prefix table is idle outside a forward transform)
+  const dim3 kgrid(std::max<uint32_t>(1u, div_up((uint32_t)ctx->sm_count * 8u, B)), B);
+  k_inv_keys<<<kgrid, 256, 0, st>>>(d_src, sh, block_mode ? 1 : 0, keys0, ctx->d_hist(), bhist);
+  k_inv_ctable<<<B, 32, 0, st>>>(ctx->d_hist(), bhist, sh, C);
+  CK(ctx, cudaGetLastError());
+  S.kernel_launches += 2;
+  S.algorithmic_bytes += (uint64_t)N * 5;
+  int cur = 0;
+  uint32_t pdone = 0;
+  const int rc = run_sort<uint32_t, RS_IPT32>(ctx, N, 3u, true, N - 1, &cur, &pt, &pdone);
+  if (rc) return rc;
+  const uint32_t* vals = ctx->d_idx[cur];
+  const uint32_t Sn = inv_splitters(sh);  // <= N / INV_K + B
+  uint32_t* nxtA = ctx->d_scat;
+  uint32_t* distA = nxtA + Sn;
+  uint32_t* nxtB = distA + Sn;
+  uint32_t* distB = nxtB + Sn;
+  uint32_t* len = distB + Sn;  // 5 * ceil(N / INV_K) words fit d_scat (N + 16 words) unless N is tiny
+  if ((uint64_t)5 * Sn > (uint64_t)N + 16) {  // tiny N: use the (idle) second id / key buffers as well (Sn <= N / 2)
+    nxtA = ctx->d_idx[cur ^ 1]; distA = nxtA + Sn; nxtB = ctx->d_scat; distB = nxtB + Sn; len = static_cast<uint32_t*>(ctx->d_keys[1]);
+  }
+  const dim3 wgrid(div_up(sh.S0, 256), B);
+  k_inv_walk1<<<wgrid, 256, 0, st>>>(vals, sh, nxtA, len, ctx->d_ctrl());
+  CK(ctx, cudaMemcpyAsync(distA, len, (size_t)Sn * 4, cudaMemcpyDeviceToDevice, st));
+  uint32_t* nin = nxtA; uint32_t* din = distA; uint32_t* nout = nxtB; uint32_t* dout = distB;
+  uint32_t rounds = 0;
+  for (uint64_t span = 1; span < (uint64_t)sh.S0; span <<= 1) {  // a chain never leaves its block: ceil(log2 S0) rounds
+    k_inv_jump<<<div_up(Sn, 256), 256, 0, st>>>(nin, din, Sn, nout, dout);
+    std::swap(nin, nout);
+    std::swap(din, dout);
+    ++rounds;
+  }
+  k_inv_walk2<<<wgrid, 256, 0, st>>>(vals, len, din, C, sh, d_dst, ctx->d_ctrl());
+  CK(ctx, cudaGetLastError());
+  S.kernel_launches += 2 + rounds;
+  S.algorithmic_bytes += (uint64_t)N * (4 + 4 + 1) + (uint64_t)Sn * 16 * (rounds + 1);
+  CK(ctx, cudaEventRecord(ctx->ev_end, st));
+  *rounds_out = rounds;
+  *passes_out = pdone;
+  return 0;
+}
+
 int64_t run_inverse(bwtc_cuda_ctx* ctx, bool block_mode, const uint8_t* h_in, uint8_t* h_out, const uint8_t* in_dev, uint8_t* out_dev,
                     uint32_t n_in, uint32_t eob) {
   ctx->err[0] = 0;
@@ -1451,53 +1508,20 @@ int64_t run_inverse(bwtc_cuda_ctx* ctx, bool block_mode, const uint8_t* h_in, ui
   memset(&S, 0, sizeof(S));
   S.n_suffixes = N;
   S.batch_blocks = 1;
-  PassTimer pt{ctx};
   const uint8_t* d_src = in_dev;
   if (!in_dev) {
     if (upload(ctx, ctx->d_in, h_in, n_in)) return BWTC_CUDA_ECUDA;
     d_src = ctx->d_in;
   }
   uint8_t* d_dst = out_dev ? out_dev : ctx->d_out;
-  CK(ctx, cudaEventRecord(ctx->ev_begin, st));
-  CK(ctx, cudaMemsetAsync(ctx->d_zero, 0, (size_t)CTR_STICKY * 4, st));
-  if (zero_round_state(ctx, N, N, RS_TILE32, 3u)) return BWTC_CUDA_ECUDA;
-  uint32_t* keys0 = static_cast<uint32_t*>(ctx->d_keys[0]);
-  uint32_t* C = ctx->d_bhist;  // 258 words
-  k_inv_keys<<<ctx->sm_count * 8, 256, 0, st>>>(d_src, N, eob, block_mode ? 1 : 0, keys0, ctx->d_hist());
-  k_inv_ctable<<<1, 32, 0, st>>>(ctx->d_hist(), N, C);
-  CK(ctx, cudaGetLastError());
-  S.kernel_launches += 2;
-  S.algorithmic_bytes += (uint64_t)N * 5;
-  int cur = 0;
-  uint32_t pdone = 0;
-  const int rc = run_sort<uint32_t, RS_IPT32>(ctx, N, 3u, true, N - 1, &cur, &pt, &pdone);
-  if (rc) return rc;
-  const uint32_t* vals = ctx->d_idx[cur];
-  const uint32_t Sn = div_up(N, INV_K);
-  uint32_t* nxtA = ctx->d_scat;
-  uint32_t* distA = nxtA + Sn;
-  uint32_t* nxtB = distA + Sn;
-  uint32_t* distB = nxtB + Sn;
-  uint32_t* len = distB + Sn;  // 5 * ceil(N / INV_K) words fit d_scat (N + 16 words) unless N is tiny
-  if ((uint64_t)5 * Sn > (uint64_t)N + 16) {  // tiny N: use the (idle) second id / key buffers as well
-    nxtA = ctx->d_idx[cur ^ 1]; distA = nxtA + Sn; nxtB = ctx->d_scat; distB = nxtB + Sn; len = static_cast<uint32_t*>(ctx->d_keys[1]);
-  }
-  const uint32_t sgrid = div_up(Sn, 256);
-  k_inv_walk1<<<sgrid, 256, 0, st>>>(vals, N, Sn, nxtA, len, ctx->d_ctrl());
-  CK(ctx, cudaMemcpyAsync(distA, len, (size_t)Sn * 4, cudaMemcpyDeviceToDevice, st));
-  uint32_t* nin = nxtA; uint32_t* din = distA; uint32_t* nout = nxtB; uint32_t* dout = distB;
-  uint32_t rounds = 0;
-  for (uint64_t span = 1; span < (uint64_t)Sn; span <<= 1) {
-    k_inv_jump<<<sgrid, 256, 0, st>>>(nin, din, Sn, nout, dout);
-    std::swap(nin, nout);
-    std::swap(din, dout);
-    ++rounds;
-  }
-  k_inv_walk2<<<sgrid, 256, 0, st>>>(vals, len, din, C, N, Sn, d_dst, ctx->d_ctrl());
-  CK(ctx, cudaGetLastError());
-  S.kernel_launches += 2 + rounds;
-  S.algorithmic_bytes += (uint64_t)N * (4 + 4 + 1) + (uint64_t)Sn * 16 * (rounds + 1);
-  CK(ctx, cudaEventRecord(ctx->ev_end, st));
+  InvShape sh;
+  sh.nblocks = 1;
+  sh.R = sh.N_last = N;
+  sh.n0 = n;
+  sh.S0 = sh.S_last = div_up(N, INV_K);
+  sh.eob[0] = eob;
+  uint32_t rounds = 0, pdone = 0;
+  if (const int rc = enqueue_inverse(ctx, sh, block_mode, d_src, d_dst, &rounds, &pdone)) return rc;
   CK(ctx, cudaMemcpyAsync(ctx->h_ctrl(), ctx->d_ctrl(), CTR_STICKY * 4, cudaMemcpyDeviceToHost, st));
   if (!out_dev && is_pinned_host(h_out)) CK(ctx, cudaMemcpyAsync(h_out, ctx->d_out, n, cudaMemcpyDeviceToHost, st));
   if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
@@ -1574,6 +1598,109 @@ int transform_batch(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out,
     ctx->stats.batch_blocks = 1;
     if (stats) stats[k] = ctx->stats;
     if (rc < 0) return (int)rc;
+  }
+  return 0;
+}
+
+// 2..MAX_BATCH blocks (block contract) that batchable() accepts, inverted as ONE device-side problem (DESIGN.md §3.7).  The
+// caller has checked the arguments.  The blocks are staged in d_in (stride n0) and restored into d_out; the caller's
+// buffers are written only after the host has read CTR_ERR.  After a look-back watchdog the device part is repeated with
+// ticket tile ids from the staged input — never from the caller's buffers, which may alias the outputs.
+int run_inverse_batch(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out, const uint32_t* sizes, uint32_t count,
+                      bool on_device, const uint32_t* eobs) {
+  ctx->err[0] = 0;
+  if (cudaSetDevice(ctx->device) != cudaSuccess) {
+    set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device);
+    return BWTC_CUDA_ECUDA;
+  }
+  static_assert(INV_MAX_BLOCKS == MAX_BATCH, "InvShape holds one end-of-block row per block of a batch");
+  cudaStream_t st = ctx->stream;
+  InvShape sh;
+  sh.nblocks = count;
+  sh.n0 = sizes[0];
+  sh.R = sizes[0] + 1u;
+  sh.N_last = sizes[count - 1] + 1u;
+  sh.S0 = div_up(sh.R, INV_K);
+  sh.S_last = div_up(sh.N_last, INV_K);
+  for (uint32_t k = 0; k < count; ++k) sh.eob[k] = eobs[k];
+  for (uint32_t k = 0; k < count; ++k) {
+    uint8_t* d = ctx->d_in + (size_t)k * sh.n0;
+    if (on_device) CK(ctx, cudaMemcpyAsync(d, in[k], sizes[k], cudaMemcpyDeviceToDevice, st));
+    else if (upload(ctx, d, static_cast<const uint8_t*>(in[k]), sizes[k])) return BWTC_CUDA_ECUDA;
+  }
+  bwtc_cuda_stats& S = ctx->stats;
+  uint32_t rounds = 0, pdone = 0;
+  for (;;) {
+    memset(&S, 0, sizeof(S));
+    if (const int rc = enqueue_inverse(ctx, sh, true, ctx->d_in, ctx->d_out, &rounds, &pdone)) return rc;
+    CK(ctx, cudaMemcpyAsync(ctx->h_ctrl(), ctx->d_ctrl(), CTR_STICKY * 4, cudaMemcpyDeviceToHost, st));
+    if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
+    if (!ctx->h_ctrl()[CTR_ERR] && !(ctx->debug_fake_watchdog && ctx->static_tiles)) break;
+    if (!ctx->static_tiles) {
+      set_err(ctx->err, "inverse: look-back watchdog fired");
+      return BWTC_CUDA_EINTERNAL;
+    }
+    ctx->static_tiles = 0;  // the two digit passes again with ticket tile ids (cannot fire twice)
+  }
+  bool pending = false;
+  for (uint32_t k = 0; k < count; ++k) {
+    const uint8_t* d = ctx->d_out + (size_t)k * sh.n0;
+    uint8_t* o = static_cast<uint8_t*>(out[k]);
+    if (on_device) {
+      CK(ctx, cudaMemcpyAsync(o, d, sizes[k], cudaMemcpyDeviceToDevice, st));
+      pending = true;
+    } else if (is_pinned_host(o)) {
+      CK(ctx, cudaMemcpyAsync(o, d, sizes[k], cudaMemcpyDeviceToHost, st));
+      pending = true;
+    } else if (download_staged(ctx, o, d, sizes[k])) {
+      return BWTC_CUDA_ECUDA;
+    }
+  }
+  if (pending && host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
+  float ms = 0;
+  CK(ctx, cudaEventElapsedTime(&ms, ctx->ev_begin, ctx->ev_end));
+  S.n_suffixes = inv_rows(sh);
+  S.batch_blocks = count;
+  S.gpu_ms = ms;
+  S.rounds = rounds;
+  S.passes[0] = pdone;
+  S.live[0] = S.n_suffixes;
+  S.flags = 2u | (ctx->static_tiles ? 0u : 1u);
+  return 0;
+}
+
+// count blocks (block contract) through one context, each restored as run_inverse would: runs are formed greedily as in
+// bwtc_cuda_bwt_blocks, a run that batchable() accepts is inverted as one problem, any other block on its own.  Every
+// argument is checked before any work, so a bad block leaves all caller buffers untouched.  stats: count records (the
+// blocks of a batch share one) or nullptr.
+int inverse_blocks(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out, const uint32_t* sizes, uint32_t count,
+                   bool on_device, const uint32_t* eobs, bwtc_cuda_stats* stats) {
+  for (uint32_t k = 0; k < count; ++k) {
+    if (!in[k] || !out[k] || sizes[k] == 0) { set_err(ctx->err, "inverse: null or empty block %u", k); return BWTC_CUDA_EARG; }
+    if (sizes[k] > ctx->cap) {
+      set_err(ctx->err, "inverse: block %u of %u bytes exceeds context capacity %u", k, sizes[k], ctx->cap);
+      return BWTC_CUDA_ETOOBIG;
+    }
+    if (eobs[k] > sizes[k]) {
+      set_err(ctx->err, "inverse: end-of-block position %u of block %u outside [0, %u)", eobs[k], k, sizes[k] + 1u);
+      return BWTC_CUDA_EARG;
+    }
+  }
+  for (uint32_t k0 = 0; k0 < count;) {
+    uint32_t k1 = std::min<uint32_t>(count, k0 + MAX_BATCH);
+    while (k1 > k0 + 1 && !batchable(ctx, sizes + k0, k1 - k0)) --k1;
+    int64_t rc;
+    if (k1 - k0 >= 2)
+      rc = run_inverse_batch(ctx, in + k0, out + k0, sizes + k0, k1 - k0, on_device, eobs + k0);
+    else if (on_device)
+      rc = run_inverse(ctx, true, nullptr, nullptr, static_cast<const uint8_t*>(in[k0]), static_cast<uint8_t*>(out[k0]), sizes[k0],
+                       eobs[k0]);
+    else
+      rc = run_inverse(ctx, true, static_cast<const uint8_t*>(in[k0]), static_cast<uint8_t*>(out[k0]), nullptr, nullptr, sizes[k0],
+                       eobs[k0]);
+    if (rc < 0) return (int)rc;
+    if (stats) for (uint32_t k = k0; k < k1; ++k) stats[k] = ctx->stats;
+    k0 = k1;
   }
   return 0;
 }
@@ -1904,6 +2031,15 @@ int64_t bwtc_cuda_inverse_block_device(bwtc_cuda_ctx* ctx, const void* d_in, voi
   return run_inverse(ctx, true, nullptr, nullptr, static_cast<const uint8_t*>(d_in), static_cast<uint8_t*>(d_out), n, eob);
 }
 
+int bwtc_cuda_inverse_blocks(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out, const uint32_t* sizes, uint32_t count,
+                             int on_device, const uint32_t* LFpowers, bwtc_cuda_stats* stats) {
+  if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
+  if (!in || !sizes || !LFpowers || count == 0) { set_err(ctx->err, "bad arguments"); return BWTC_CUDA_EARG; }
+  std::vector<uint32_t> eobs(count);
+  for (uint32_t k = 0; k < count; ++k) eobs[k] = LFpowers[(size_t)k * 256];
+  return inverse_blocks(ctx, in, out ? out : const_cast<void* const*>(in), sizes, count, on_device != 0, eobs.data(), stats);
+}
+
 int64_t bwtc_cuda_inverse_raw(bwtc_cuda_ctx* ctx, uint8_t* bwt, uint32_t N, const uint32_t* LFpowers, uint32_t nLFpowers) {
   if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
   if (!bwt || N < 2 || !LFpowers || nLFpowers < 1) { set_err(ctx->err, "null / too short input or no starting point"); return BWTC_CUDA_EARG; }
@@ -1925,10 +2061,13 @@ uint32_t bwtc_cuda_num_starting_points(uint32_t block_bytes, uint32_t starts) {
 // events while the GPU works: an idle or waiting pipeline costs no host core.
 // =====================================================================================================
 namespace {
+enum PipeKind : int { PIPE_FORWARD = 0, PIPE_INVERSE = 1 };
 struct PipeItem {
+  int kind = PIPE_FORWARD;
   const void* in = nullptr;
   void* out = nullptr;
   uint32_t n = 0, starts = 0;
+  uint32_t eob = 0;         // inverse: the end-of-block row (LFpowers[0] of the forward transform)
   bool on_device = false;
   uint32_t* LF = nullptr;   // 256 words
   uint32_t* nLF = nullptr;
@@ -1967,7 +2106,7 @@ void pipeline_worker(bwtc_cuda_pipeline* p, bwtc_cuda_ctx* c) {
   std::vector<std::shared_ptr<PipeItem>> grp;
   std::vector<const void*> in;
   std::vector<void*> out;
-  std::vector<uint32_t> sizes, nLF, LF, freqs;
+  std::vector<uint32_t> sizes, nLF, LF, freqs, eobs;
   std::vector<bwtc_cuda_stats> stats;
   for (;;) {
     grp.clear();
@@ -1977,13 +2116,15 @@ void pipeline_worker(bwtc_cuda_pipeline* p, bwtc_cuda_ctx* c) {
       if (p->queue.empty()) return;  // stopping
       grp.push_back(p->queue.front());
       p->queue.pop_front();
-      // consecutive small blocks of equal size (same contract parameters) go to ONE device-side sort
+      // consecutive small blocks of equal size (same kind and contract parameters) go to ONE device-side sort / inversion
       if (grp[0]->n <= p->batch_max_block && !grp[0]->runs) {
         sizes.assign(1, grp[0]->n);
         const uint32_t lim = std::min<uint32_t>(MAX_BATCH, p->batch_blocks);
         while (!p->queue.empty() && grp.size() < lim) {
           const PipeItem& nx = *p->queue.front();
-          if (nx.starts != grp[0]->starts || nx.on_device != grp[0]->on_device || (nx.freqs == nullptr) != (grp[0]->freqs == nullptr) || nx.runs) break;
+          if (nx.kind != grp[0]->kind || nx.on_device != grp[0]->on_device) break;
+          if (nx.kind == PIPE_FORWARD &&
+              (nx.starts != grp[0]->starts || (nx.freqs == nullptr) != (grp[0]->freqs == nullptr) || nx.runs)) break;
           sizes.push_back(nx.n);
           if (!batchable(c, sizes.data(), (uint32_t)sizes.size())) { sizes.pop_back(); break; }
           grp.push_back(p->queue.front());
@@ -1993,7 +2134,14 @@ void pipeline_worker(bwtc_cuda_pipeline* p, bwtc_cuda_ctx* c) {
     }
     const uint32_t cnt = (uint32_t)grp.size();
     int rc;
-    if (cnt == 1) {
+    if (grp[0]->kind == PIPE_INVERSE) {
+      in.resize(cnt); out.resize(cnt); sizes.resize(cnt); eobs.resize(cnt); stats.resize(cnt);
+      for (uint32_t k = 0; k < cnt; ++k) { in[k] = grp[k]->in; out[k] = grp[k]->out; sizes[k] = grp[k]->n; eobs[k] = grp[k]->eob; }
+      rc = inverse_blocks(c, in.data(), out.data(), sizes.data(), cnt, grp[0]->on_device, eobs.data(), stats.data());
+      if (rc >= 0)
+        for (uint32_t k = 0; k < cnt; ++k)
+          if (grp[k]->stats) *grp[k]->stats = stats[k];
+    } else if (cnt == 1) {
       PipeItem& it = *grp[0];
       const void* i1 = it.in;
       void* o1 = it.out;
@@ -2026,8 +2174,10 @@ void pipeline_worker(bwtc_cuda_pipeline* p, bwtc_cuda_ctx* c) {
 }
 
 uint64_t pipeline_enqueue_locked(bwtc_cuda_pipeline* p, const void* in, void* out, uint32_t n, uint32_t starts, bool on_device,
-                                 uint32_t* LF, uint32_t* nLF, uint32_t* freqs, bwtc_cuda_stats* stats, bwtc_cuda_runs* runs = nullptr) {
+                                 uint32_t* LF, uint32_t* nLF, uint32_t* freqs, bwtc_cuda_stats* stats, bwtc_cuda_runs* runs = nullptr,
+                                 int kind = PIPE_FORWARD, uint32_t eob = 0) {
   auto it = std::make_shared<PipeItem>();
+  it->kind = kind; it->eob = eob;
   it->in = in; it->out = out; it->n = n; it->starts = starts; it->on_device = on_device;
   it->LF = LF; it->nLF = nLF; it->freqs = freqs; it->stats = stats; it->runs = runs;
   it->ticket = p->next_ticket++;
@@ -2144,6 +2294,19 @@ int bwtc_cuda_pipeline_submit_runs(bwtc_cuda_pipeline* p, const uint8_t* in, uin
   {
     std::lock_guard<std::mutex> lk(p->mu);
     *ticket = pipeline_enqueue_locked(p, in, out, n, starts, false, LFpowers, nLF, freqs, nullptr, runs);
+  }
+  p->cv_work.notify_one();
+  return 0;
+}
+
+int bwtc_cuda_pipeline_submit_inverse(bwtc_cuda_pipeline* p, const uint8_t* in, uint8_t* out, uint32_t n, uint32_t eob,
+                                      int on_device, bwtc_cuda_stats* stats, uint64_t* ticket) {
+  if (!p) { set_err(g_err, "null pipeline"); return BWTC_CUDA_EARG; }
+  if (!in || !out || !ticket || n == 0) { set_err(p->err, "bad arguments"); return BWTC_CUDA_EARG; }
+  if (eob > n) { set_err(p->err, "inverse: end-of-block position %u outside [0, %u)", eob, n + 1u); return BWTC_CUDA_EARG; }
+  {
+    std::lock_guard<std::mutex> lk(p->mu);
+    *ticket = pipeline_enqueue_locked(p, in, out, n, 0, on_device != 0, nullptr, nullptr, nullptr, stats, nullptr, PIPE_INVERSE, eob);
   }
   p->cv_work.notify_one();
   return 0;

@@ -17,6 +17,9 @@
  *                                              bwtransforms/BWTManager.cpp:60-64, BWTBlock.cpp:104-108
  *   bwtc_cuda_inverse_block / _raw         <-  InverseBWTransform::doTransform(BWTBlock&) / (byte*, uint32, LFpow)
  *                                              bwtransforms/InverseBWT.cpp:47-51, InverseBWT.hpp:49-50 (MtlSaInverseBWT.cpp)
+ *   bwtc_cuda_inverse_blocks /             <-  the per-slice InverseBWTransform::doTransform calls of
+ *   bwtc_cuda_pipeline_submit_inverse          Decompressor::decompress (Decompressor.cpp:58-94, InverseBWT.cpp:47-51):
+ *                                              equal-sized slices inverted as one device-side problem, or streamed
  *   bwtc_cuda_pipeline_*                   <-  the per-slice loop of Compressor::compress
  *                                              Compressor.cpp:100-109 (independent BWT blocks), batched
  *                                              with look-ahead over several in-flight blocks per GPU
@@ -167,6 +170,17 @@ int64_t bwtc_cuda_inverse_block_device(bwtc_cuda_ctx* ctx, const void* d_in, voi
 /* Raw virtual doTransform(byte* bwt, uint32 N, LFpow) (InverseBWT.hpp:49-50): bwt[0..N) = L with bwt[LFpowers[0]] ignored;
  * on return bwt[0..N-1) is the original block (bwt[N-1] is left as it was).  Returns N-1. */
 int64_t bwtc_cuda_inverse_raw(bwtc_cuda_ctx* ctx, uint8_t* bwt, uint32_t N, const uint32_t* LFpowers, uint32_t nLFpowers);
+/* Several blocks through one context, each restored exactly as bwtc_cuda_inverse_block would: in[k] holds the sizes[k]
+ * bytes a forward block transform produced, the original bytes land in out[k] (out may be NULL: in place; out[k] may alias
+ * in[k]).  Host pointers, or device pointers when on_device != 0.  LFpowers: count x 256 words in the layout
+ * bwtc_cuda_bwt_blocks / bwtc_cuda_pipeline_run produce; only LFpowers[k*256] (block k's end-of-block row) is read.  Runs
+ * that qualify as for bwtc_cuda_bwt_blocks (2..BWTC_CUDA_MAX_BATCH blocks of equal size, the last may be shorter, together
+ * within the context's capacity) are inverted as ONE device-side problem — whatever byte values the blocks contain —
+ * others one after the other.  The byte after each block is never touched.  Every argument is checked before any work.
+ * stats: count records (the blocks of a batch share one, batch_blocks = its size, flags bit 1 set) or NULL.
+ * Returns 0 or a negative error. */
+int bwtc_cuda_inverse_blocks(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out, const uint32_t* sizes,
+                             uint32_t count, int on_device, const uint32_t* LFpowers, bwtc_cuda_stats* stats);
 /* BWTManager::setStartingPoints clamp + BWTBlock::prepareLFpowers sizing. */
 uint32_t bwtc_cuda_num_starting_points(uint32_t block_bytes, uint32_t starts);
 
@@ -196,6 +210,13 @@ int  bwtc_cuda_pipeline_submit(bwtc_cuda_pipeline* p, const uint8_t* in, uint8_t
                                int on_device, uint32_t* LFpowers, uint32_t* nLF, uint32_t* freqs,
                                bwtc_cuda_stats* stats, uint64_t* ticket);
 int  bwtc_cuda_pipeline_wait(bwtc_cuda_pipeline* p, uint64_t ticket);
+/* Streaming inverse: queue ONE block (block contract of bwtc_cuda_inverse_block: in holds the n transformed bytes, the
+ * original n bytes land in out, which may alias in; device memory when on_device != 0; eob = LFpowers[0] of the forward
+ * transform; stats may be NULL) and return at once with a ticket of the same sequence as bwtc_cuda_pipeline_submit's; wait
+ * for it with bwtc_cuda_pipeline_wait.  Queued inverse blocks of equal size are inverted as one device-side problem;
+ * forward and inverse blocks are never grouped together. */
+int  bwtc_cuda_pipeline_submit_inverse(bwtc_cuda_pipeline* p, const uint8_t* in, uint8_t* out, uint32_t n, uint32_t eob,
+                                       int on_device, bwtc_cuda_stats* stats, uint64_t* ticket);
 /* submit + run statistics (filled when the block completes; such a block is transformed on its own, not in a batch). */
 int  bwtc_cuda_pipeline_submit_runs(bwtc_cuda_pipeline* p, const uint8_t* in, uint8_t* out, uint32_t n, uint32_t starts,
                                     uint32_t* LFpowers, uint32_t* nLF, uint32_t* freqs, bwtc_cuda_runs* runs, uint64_t* ticket);
