@@ -281,17 +281,19 @@ class CudaContext:
         self._check(self._lib.bwtc_cuda_inverse_blocks(self._h, a_in, a_out, a_sz.ctypes.data, count, 1 if on_device else 0,
                                                        rows.ctypes.data, None))
 
-    def bwt_blocks(self, blocks, starts: int, want_freqs: bool = True):
-        """bwtc_cuda_bwt_blocks: transform the given uint8 arrays IN PLACE (equal-sized runs are batched into one
-        device-side sort).  Returns (LFpowers[count, 256], nLF[count], freqs[count, 256] or None)."""
+    def bwt_blocks(self, blocks, starts: int, want_freqs: bool = True, on_device: bool = False):
+        """bwtc_cuda_bwt_blocks: transform the given blocks (uint8 arrays, or CUDA tensors / (pointer, size) pairs when
+        on_device) IN PLACE (equal-sized runs are batched into one device-side sort).  Returns (LFpowers[count, 256],
+        nLF[count], freqs[count, 256] or None)."""
         count = len(blocks)
-        ptrs = (ctypes.c_void_p * count)(*[b.ctypes.data for b in blocks])
-        sizes = np.array([b.size for b in blocks], dtype=np.uint32)
+        ptrs, sizes = zip(*[_block_ptr(b, on_device) for b in blocks]) if count else ((), ())
+        a_ptrs = (ctypes.c_void_p * count)(*ptrs)
+        a_sz = np.asarray(sizes, dtype=np.uint32)
         LF = np.zeros((count, 256), dtype=np.uint32)
         nLF = np.zeros(count, dtype=np.uint32)
         fr = np.zeros((count, 256), dtype=np.uint32) if want_freqs else None
-        self._check(self._lib.bwtc_cuda_bwt_blocks(self._h, ptrs, sizes.ctypes.data, count, starts, 0, LF.ctypes.data,
-                                                   nLF.ctypes.data, _ptr(fr)))
+        self._check(self._lib.bwtc_cuda_bwt_blocks(self._h, a_ptrs, a_sz.ctypes.data, count, starts, 1 if on_device else 0,
+                                                   LF.ctypes.data, nLF.ctypes.data, _ptr(fr)))
         return LF, nLF, fr
 
     def bwt_block_device(self, d_in: int, d_out: int, n: int, LFpowers: np.ndarray,

@@ -183,12 +183,7 @@ def test_forward_then_inverse_on_the_same_device_tensors(ctx):
 
     xs = [bw.generate(KINDS[k % 4], 1 << 16, seed=800 + k) for k in range(12)] + [bw.generate("dna", 999, seed=1)]
     dev = [torch.from_numpy(x.copy()).cuda() for x in xs]
-    ptrs = (ctypes.c_void_p * len(xs))(*[t.data_ptr() for t in dev])
-    sizes = np.array([x.size for x in xs], np.uint32)
-    LF = np.zeros((len(xs), 256), np.uint32)
-    nLF = np.zeros(len(xs), np.uint32)
-    ctx._check(ctx._lib.bwtc_cuda_bwt_blocks(ctx._h, ptrs, sizes.ctypes.data, len(xs), 8, 1, LF.ctypes.data,
-                                             nLF.ctypes.data, None))
+    LF, nLF, _ = ctx.bwt_blocks(dev, 8, want_freqs=False, on_device=True)
     torch.cuda.synchronize()
     assert not np.array_equal(dev[0].cpu().numpy(), xs[0])
     ctx.inverse_blocks(dev, LF, on_device=True)

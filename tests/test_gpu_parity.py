@@ -294,8 +294,9 @@ def test_batched_small_blocks_equal_single_blocks(oracle):
         mixed = [bw.generate("dna", n, seed=n) for n in (40000, 40000, 40000, 1000, 50000, 50000, 1, 2, 2)]
         _check_batch(ctx, oracle, mixed, 256)
         # repetitive blocks: many doubling rounds inside a batch
-        rep = [bw.generate("repetitive", 1 << 17, seed=7 + k) for k in range(4)]
-        _check_batch(ctx, oracle, rep, 8)
+        rep = [np.minimum(bw.generate("repetitive", 1 << 17, seed=7 + k), 254) for k in range(4)]  # 255 byte values
+        st = _check_batch(ctx, oracle, rep, 8)
+        assert st["batch_blocks"] == 4 and st["rounds"] >= 3
     finally:
         ctx.close()
 
@@ -354,16 +355,29 @@ ENGINE_KNOBS = [
 ]
 
 
+_ORACLE_BLOCKS = {}
+
+
+def _oracle_generated(oracle, kind, seed, size, x):
+    """oracle.block(x, 8) of a generated input x, computed once per (kind, seed, size) for the whole module."""
+    key = (kind, seed, size)
+    if key not in _ORACLE_BLOCKS:
+        _ORACLE_BLOCKS[key] = oracle.block(x, 8)
+    return _ORACLE_BLOCKS[key]
+
+
 @pytest.mark.parametrize("knobs", ENGINE_KNOBS, ids=lambda k: ",".join(f"{a[5:]}={b}" for a, b in k.items()) or "default")
 def test_every_engine_path_is_bit_exact(oracle, monkeypatch, knobs):
     """The engine picks between code paths by block size (L2 windows of the rank scatter, packed predecessor
     characters, segmented vs global rounds).  The tuning knobs are read when a context is created, so every path can
-    be forced at sizes the oracle handles: all of them must produce the oracle's bytes."""
+    be forced at sizes the oracle handles: all of them must produce the oracle's bytes.  Batches of small blocks
+    (DESIGN.md §3.6) run through the same context and the same paths."""
     for k, v in knobs.items():
         monkeypatch.setenv(k, v)
     n = (2 << 20) + 4097
     ctx = bw.CudaContext(n)
     rng = np.random.default_rng(77)
+    tickets = knobs.get("BWTC_STATIC_TILES") == "0" or knobs.get("BWTC_DEBUG_FAKE_WATCHDOG") == "1"
     # (the repetitive block keeps ~all suffixes live through its global doubling rounds: with n suffixes their rank scatter
     # is windowed / bucketed exactly like round 0's)
     cases = [("markov", n), ("dna", n), ("repetitive", 1 << 20), ("repetitive", n - 5), ("random", n - 4099)]
@@ -372,7 +386,7 @@ def test_every_engine_path_is_bit_exact(oracle, monkeypatch, knobs):
             x = bw.generate(kind, sz, seed=41)
             if kind == "random":
                 x[rng.integers(0, sz, 1000)] = 0  # zeros inside the block: the sentinel shares a code with data
-            want = oracle.block(x, 8)
+            want = _oracle_generated(oracle, kind + "+zeros" if kind == "random" else kind, 41, sz, x)
             got = _gpu_block(ctx, x, 8)
             assert (got[0] == want[0]).all(), (kind, knobs)
             assert (got[1] == want[1]).all(), (kind, knobs)
@@ -380,10 +394,27 @@ def test_every_engine_path_is_bit_exact(oracle, monkeypatch, knobs):
         flags = ctx.stats()["flags"]
         if knobs.get("BWTC_LAZY") == "2":
             assert flags & 16, "lazy ranks should have been used for the last block"
-        if knobs.get("BWTC_STATIC_TILES") == "0" or knobs.get("BWTC_DEBUG_FAKE_WATCHDOG") == "1":
+        if tickets:
             assert flags & 1, "the look-back kernels should have run with ticket counters"
         else:
             assert not (flags & 1), "unexpected watchdog fallback"
+        # batches: 8 x 256 KiB and a short last block fill the context (sum of n_k + 1 <= n + 1); 4 repetitive blocks keep
+        # most suffixes live through global rounds
+        for kind, sizes in (("markov", [1 << 18] * 8 + [4000]), ("dna", [1 << 18] * 8 + [4000]), ("repetitive", [1 << 18] * 4)):
+            xs = [np.minimum(bw.generate(kind, sz, seed=60 + k), 254) for k, sz in enumerate(sizes)]  # 255 values at most
+            bufs = [np.append(x, np.uint8(0xAB)) for x in xs]
+            views = [b[:-1] for b in bufs]
+            LF, nLF, fr = ctx.bwt_blocks(views, 8)
+            st = ctx.stats()
+            for k, x in enumerate(xs):
+                want = _oracle_generated(oracle, kind, 60 + k, x.size, x)
+                assert bufs[k][-1] == 0xAB, (kind, k, "byte after the block was written")
+                assert (views[k] == want[0]).all(), (kind, k, knobs)
+                assert nLF[k] == want[1].size and (LF[k, : nLF[k]] == want[1]).all(), (kind, k, knobs)
+                assert (fr[k] == want[2]).all(), (kind, k, knobs)
+            assert st["flags"] & 2 and st["batch_blocks"] == len(xs), (kind, st["flags"], st["batch_blocks"])
+            assert not st["flags"] & (8 | 16), "a batch carries no aux payload and uses no lazy ranks"
+            assert bool(st["flags"] & 1) == tickets, (kind, st["flags"])
     finally:
         ctx.close()
 
