@@ -28,6 +28,10 @@ MAX_ROUNDS = 40
 MAX_BLOCK = 0x7FFFFFFD            # BWTC_CUDA_MAX_BLOCK
 SCRATCH_BYTES_PER_SUFFIX = 40     # BWTC_CUDA_SCRATCH_BYTES_PER_SUFFIX
 SCRATCH_FIXED_BYTES = 8 << 20     # BWTC_CUDA_SCRATCH_FIXED_BYTES
+ECORRUPT = -6                     # BWTC_CUDA_ECORRUPT: an inverse input that is not the BWT of any text
+EVERIFY = -7                      # BWTC_CUDA_EVERIFY: a verified forward output did not restore its input
+FLAG_VERIFIED = 1 << 6            # stats flags bit 6: the forward output was verified on the device
+FLAG_CORRUPT = 1 << 7             # stats flags bit 7: this inverse block is corrupt
 
 
 class BwtcCudaUnavailable(RuntimeError):
@@ -35,9 +39,10 @@ class BwtcCudaUnavailable(RuntimeError):
 
 
 class BwtcCudaError(RuntimeError):
-    def __init__(self, code: int, msg: str):
+    def __init__(self, code: int, msg: str, blocks: Optional[List[int]] = None):
         super().__init__(f"bwtc_cuda error {code}: {msg}")
         self.code = code
+        self.blocks = blocks  # ECORRUPT from inverse_blocks: the indices of the corrupt blocks
 
 
 class Stats(ctypes.Structure):
@@ -107,6 +112,7 @@ C_ABI = [
     ("bwtc_cuda_get_stats", ctypes.c_int, [_vp, ctypes.POINTER(Stats)]),
     ("bwtc_cuda_ctx_set_round0", ctypes.c_int, [_vp, ctypes.c_uint32, ctypes.c_uint32]),
     ("bwtc_cuda_ctx_set_timing", ctypes.c_int, [_vp, ctypes.c_int]),
+    ("bwtc_cuda_ctx_set_verify", ctypes.c_int, [_vp, ctypes.c_int]),
     ("bwtc_cuda_ctx_set_debug", ctypes.c_int, [_vp, ctypes.c_uint32]),
     ("bwtc_cuda_debug_read", ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_uint64, _vp, ctypes.c_uint64]),
     ("bwtc_cuda_divbwtf", ctypes.c_int64, [_vp, _vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp]),
@@ -126,6 +132,7 @@ C_ABI = [
     ("bwtc_cuda_pipeline_error", ctypes.c_char_p, [_vp]),
     ("bwtc_cuda_pipeline_set_round0", ctypes.c_int, [_vp, ctypes.c_uint32, ctypes.c_uint32]),
     ("bwtc_cuda_pipeline_set_timing", ctypes.c_int, [_vp, ctypes.c_int]),
+    ("bwtc_cuda_pipeline_set_verify", ctypes.c_int, [_vp, ctypes.c_int]),
     ("bwtc_cuda_pipeline_run", ctypes.c_int,
      [_vp, _vp, _vp, _vp, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_int, _vp, _vp, _vp, _vp]),
     ("bwtc_cuda_pipeline_submit", ctypes.c_int,
@@ -211,6 +218,11 @@ class CudaContext:
     def set_debug(self, max_rounds: int):
         self._check(self._lib.bwtc_cuda_ctx_set_debug(self._h, max_rounds))
 
+    def set_verify(self, on: bool):
+        """bwtc_cuda_ctx_set_verify: every block-contract forward call inverts its output on the device and compares it with
+        the input before it returns; a mismatch raises BwtcCudaError with code EVERIFY and leaves the input in place."""
+        self._check(self._lib.bwtc_cuda_ctx_set_verify(self._h, 1 if on else 0))
+
     def debug_read(self, which: int, dtype, count: int, offset_bytes: int = 0) -> np.ndarray:
         out = np.empty(count, dtype=dtype)
         self._check(self._lib.bwtc_cuda_debug_read(self._h, which, offset_bytes, out.ctypes.data, out.nbytes))
@@ -263,7 +275,9 @@ class CudaContext:
         """bwtc_cuda_inverse_blocks: restore the given blocks (uint8 arrays, or CUDA tensors / (pointer, size) pairs when
         on_device) IN PLACE, or into `out` (same kinds, same sizes).  LF: per block its LFpowers row (e.g. what bwt_blocks
         returned) or just its end-of-block row; only LF[k][0] is used.  Equal-sized runs are inverted as one device-side
-        problem; stats() then describes the last run."""
+        problem; stats() then describes the last run.  Corrupt blocks (not the BWT of any text with their end-of-block row)
+        raise BwtcCudaError with code ECORRUPT and .blocks = their indices, after every valid block has been restored; a
+        corrupt block's buffer is left as it was."""
         count = len(blocks)
         ptrs, sizes = zip(*[_block_ptr(b, on_device) for b in blocks]) if count else ((), ())
         a_in = (ctypes.c_void_p * count)(*ptrs)
@@ -278,8 +292,13 @@ class CudaContext:
         eob = eob.reshape(count, -1)[:, 0] if eob.size else eob
         rows = np.zeros((count, 256), dtype=np.uint32)
         rows[:, 0] = eob
-        self._check(self._lib.bwtc_cuda_inverse_blocks(self._h, a_in, a_out, a_sz.ctypes.data, count, 1 if on_device else 0,
-                                                       rows.ctypes.data, None))
+        stats = (Stats * max(count, 1))()
+        rc = self._lib.bwtc_cuda_inverse_blocks(self._h, a_in, a_out, a_sz.ctypes.data, count, 1 if on_device else 0,
+                                                rows.ctypes.data, ctypes.addressof(stats))
+        if rc == ECORRUPT:
+            raise BwtcCudaError(rc, self._lib.bwtc_cuda_last_error(self._h).decode(),
+                                [k for k in range(count) if stats[k].flags & FLAG_CORRUPT])
+        self._check(rc)
 
     def bwt_blocks(self, blocks, starts: int, want_freqs: bool = True, on_device: bool = False):
         """bwtc_cuda_bwt_blocks: transform the given blocks (uint8 arrays, or CUDA tensors / (pointer, size) pairs when
@@ -455,6 +474,12 @@ class Pipeline:
     def set_timing(self, detail: int):
         self._lib.bwtc_cuda_pipeline_set_timing(self._h, detail)
 
+    def set_verify(self, on: bool):
+        """bwtc_cuda_pipeline_set_verify: forward blocks are verified on the device (see CudaContext.set_verify)."""
+        rc = self._lib.bwtc_cuda_pipeline_set_verify(self._h, 1 if on else 0)
+        if rc < 0:
+            raise BwtcCudaError(rc, self._lib.bwtc_cuda_pipeline_error(self._h).decode())
+
     def run_ptrs(self, in_ptrs: Sequence[int], out_ptrs: Sequence[int], sizes: Sequence[int], starts: int,
                  on_device: bool, want_freqs: bool = True, want_stats: bool = True):
         nb = len(sizes)
@@ -498,7 +523,8 @@ class Pipeline:
         return h
 
     def wait(self, h):
-        """Waits for a handle of submit (returns (LFpowers, freqs)) or of submit_inverse (returns the restored block)."""
+        """Waits for a handle of submit (returns (LFpowers, freqs)) or of submit_inverse (returns the restored block).  Raises
+        for a failed handle only: a corrupt inverse block (code ECORRUPT) does not fail the other blocks of its group."""
         rc = self._lib.bwtc_cuda_pipeline_wait(self._h, h["ticket"])
         if rc < 0:
             raise BwtcCudaError(rc, self._lib.bwtc_cuda_pipeline_error(self._h).decode())

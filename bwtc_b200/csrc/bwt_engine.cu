@@ -122,6 +122,8 @@ struct bwtc_cuda_ctx {
   int lb_watchdog = 0;            // the last transform failed on the look-back watchdog
   int debug_fake_watchdog = 0;    // test hook: pretend the watchdog fired while static tile ids are in use
   int debug_reverse_tiles = 0;    // test hook: static tile ids in REVERSE dispatch order (a real violation)
+  int verify = 0;                 // block-contract forward outputs are inverted on the device and compared (DESIGN.md §3.10)
+  int debug_corrupt_out = 0;      // test hook: one byte of the forward output is changed before it is verified
   int d2h_kernel = 0;             // BWTC_D2H_KERNEL=1: result copies to pinned host buffers by a copying kernel (k_copy_out)
                                   // instead of the copy engine — measured no better (profiles/r02_experiments.md), kept as a knob
   int d2h_ctas = 16;
@@ -826,6 +828,8 @@ int64_t phase_input(bwtc_cuda_ctx* ctx, Job& J) {
   return 0;
 }
 
+int verify_forward(bwtc_cuda_ctx* ctx, const Job& J);
+
 // ---- phase B: round 0, the device-controlled ladder of sort-free rounds, host-driven global radix rounds where
 // groups are large, final extraction, result copies.  Works from ctx->d_text only, so it can be repeated (with ticket
 // tile ids) after a look-back watchdog without the caller's input.
@@ -1075,6 +1079,8 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
   // the end if the block was not finished by then.
   const bool direct_out = bs ? (bs->on_device || is_pinned_host(bs->out[0]))
                              : (J.out_dev != nullptr || (J.block_mode && J.h_out && is_pinned_host(J.h_out)));
+  // verification (DESIGN.md §3.10): the caller's host and batch outputs are written only after the check word is read
+  const bool verify = ctx->verify && J.block_mode && !ctx->debug_max_rounds;
   uint32_t* h_bLF = reinterpret_cast<uint32_t*>(ctx->h_batch + MAX_BATCH * sizeof(void*)) + MAX_BATCH * 256;
   auto enqueue_direct_out = [&]() -> int {
     if (bs) {
@@ -1165,7 +1171,7 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
     CK(ctx, cudaMemcpyAsync(ctx->h_state, ctx->d_state, sizeof(LadderState), cudaMemcpyDeviceToHost, st));
     if (bs) CK(ctx, cudaMemcpyAsync(h_bLF, ctx->d_LF, (size_t)bs->nblocks * 256 * 4, cudaMemcpyDeviceToHost, st));
     else CK(ctx, cudaMemcpyAsync(ctx->h_LF(), ctx->d_LF, J.nLF * 4, cudaMemcpyDeviceToHost, st));
-    if (first_chunk && direct_out && !dbg) {
+    if (first_chunk && direct_out && !dbg && !verify) {
       if (enqueue_direct_out()) return BWTC_CUDA_ECUDA;
       out_enqueued = true;
     }
@@ -1321,6 +1327,22 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
     lists_pending = true;
   }
 
+  // ---- run statistics first: the verification below reuses d_scat
+  if (finished && J.runs && !bs && J.block_mode) {
+    const uint32_t cnt = ctx->h_state->nruns;
+    if (cnt <= J.runs->capacity && cnt <= n && J.runs->symbol && J.runs->start) {
+      if (download_staged(ctx, J.runs->symbol, ctx->d_aux[0], cnt)) return BWTC_CUDA_ECUDA;
+      if (download_staged(ctx, reinterpret_cast<uint8_t*>(J.runs->start), reinterpret_cast<const uint8_t*>(ctx->d_scat), (size_t)cnt * 4))
+        return BWTC_CUDA_ECUDA;
+      J.runs->count = cnt;
+    } else {
+      J.runs->count = BWTC_CUDA_RUNS_OVERFLOW;
+    }
+  }
+  if (finished && verify) {
+    rc = verify_forward(ctx, J);
+    if (rc) return rc;
+  }
   // ---- result copies that could not be enqueued speculatively
   if (finished) {
     if (bs) {
@@ -1353,17 +1375,6 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
           return BWTC_CUDA_ECUDA;
         }
       }
-    }
-  }
-  if (finished && J.runs && !bs && J.block_mode) {
-    const uint32_t cnt = ctx->h_state->nruns;
-    if (cnt <= J.runs->capacity && cnt <= n && J.runs->symbol && J.runs->start) {
-      if (download_staged(ctx, J.runs->symbol, ctx->d_aux[0], cnt)) return BWTC_CUDA_ECUDA;
-      if (download_staged(ctx, reinterpret_cast<uint8_t*>(J.runs->start), reinterpret_cast<const uint8_t*>(ctx->d_scat), (size_t)cnt * 4))
-        return BWTC_CUDA_ECUDA;
-      J.runs->count = cnt;
-    } else {
-      J.runs->count = BWTC_CUDA_RUNS_OVERFLOW;
     }
   }
   // ---- results for the caller: LFpowers, freqs (incremented only now that the block has succeeded)
@@ -1433,14 +1444,16 @@ int64_t run_transform(bwtc_cuda_ctx* ctx, bool block_mode, const uint8_t* h_in, 
 // The device part of an inversion (one block, or a batch of them, ibwt_kernels.cuh InvShape): ev_begin, the keys and C
 // tables, the 2 digit passes, walk1, pointer jumping, walk2 into d_dst.  Adds its launches and algorithmic bytes to
 // ctx->stats; nothing is waited for.  A batch (bhist != nullptr) counts per-block histograms and gets per-block C tables.
+// Bit k of ctrl[CTR_INV_BAD..] ends up set for each block k that is not the BWT of any text.  timed = false: ev_begin /
+// ev_end are left to the caller (the verification of a forward transform).
 int enqueue_inverse(bwtc_cuda_ctx* ctx, const InvShape& sh, bool block_mode, const uint8_t* d_src, uint8_t* d_dst,
-                    uint32_t* rounds_out, uint32_t* passes_out) {
+                    uint32_t* rounds_out, uint32_t* passes_out, bool timed = true) {
   cudaStream_t st = ctx->stream;
   bwtc_cuda_stats& S = ctx->stats;
   PassTimer pt{ctx};
   const uint32_t B = sh.nblocks, N = inv_rows(sh);
   uint32_t* bhist = B > 1 ? ctx->d_bhist : nullptr;
-  CK(ctx, cudaEventRecord(ctx->ev_begin, st));
+  if (timed) CK(ctx, cudaEventRecord(ctx->ev_begin, st));
   CK(ctx, cudaMemsetAsync(ctx->d_zero, 0, (size_t)CTR_STICKY * 4, st));
   if (zero_round_state(ctx, N, N, RS_TILE32, 3u)) return BWTC_CUDA_ECUDA;
   if (bhist) CK(ctx, cudaMemsetAsync(bhist, 0, (size_t)B * 256 * 4, st));
@@ -1477,18 +1490,22 @@ int enqueue_inverse(bwtc_cuda_ctx* ctx, const InvShape& sh, bool block_mode, con
     std::swap(din, dout);
     ++rounds;
   }
-  k_inv_walk2<<<wgrid, 256, 0, st>>>(vals, len, din, C, sh, d_dst, ctx->d_ctrl());
+  // single-cycle check: per-block length sums and CTA counters in the gram histogram words (zeroed above, idle here)
+  k_inv_walk2<<<wgrid, 256, 0, st>>>(vals, len, din, nin, C, sh, d_dst, ctx->d_ctrl(), ctx->d_hist() + GRAM_OFF);
   CK(ctx, cudaGetLastError());
   S.kernel_launches += 2 + rounds;
-  S.algorithmic_bytes += (uint64_t)N * (4 + 4 + 1) + (uint64_t)Sn * 16 * (rounds + 1);
-  CK(ctx, cudaEventRecord(ctx->ev_end, st));
+  S.algorithmic_bytes += (uint64_t)N * (4 + 4 + 1) + (uint64_t)Sn * (16 * (rounds + 1) + 4);
+  if (timed) CK(ctx, cudaEventRecord(ctx->ev_end, st));
   *rounds_out = rounds;
   *passes_out = pdone;
   return 0;
 }
 
+// spec (the single-block entry points): pinned host and device outputs are written without waiting for the check, so a
+// valid block costs one host wait; a corrupt one leaves them unspecified.  !spec (a block of bwtc_cuda_inverse_blocks):
+// restored into d_out, copied to the caller only if valid.
 int64_t run_inverse(bwtc_cuda_ctx* ctx, bool block_mode, const uint8_t* h_in, uint8_t* h_out, const uint8_t* in_dev, uint8_t* out_dev,
-                    uint32_t n_in, uint32_t eob) {
+                    uint32_t n_in, uint32_t eob, bool spec = true) {
   ctx->err[0] = 0;
   if (cudaSetDevice(ctx->device) != cudaSuccess) {
     set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device);
@@ -1513,36 +1530,105 @@ int64_t run_inverse(bwtc_cuda_ctx* ctx, bool block_mode, const uint8_t* h_in, ui
     if (upload(ctx, ctx->d_in, h_in, n_in)) return BWTC_CUDA_ECUDA;
     d_src = ctx->d_in;
   }
-  uint8_t* d_dst = out_dev ? out_dev : ctx->d_out;
+  uint8_t* d_dst = (out_dev && spec) ? out_dev : ctx->d_out;
+  const bool pinned_out = !out_dev && is_pinned_host(h_out);
   InvShape sh;
   sh.nblocks = 1;
   sh.R = sh.N_last = N;
-  sh.n0 = n;
+  sh.n0 = sh.istride = n;
   sh.S0 = sh.S_last = div_up(N, INV_K);
   sh.eob[0] = eob;
+  sh.d_eob = nullptr;
   uint32_t rounds = 0, pdone = 0;
   if (const int rc = enqueue_inverse(ctx, sh, block_mode, d_src, d_dst, &rounds, &pdone)) return rc;
   CK(ctx, cudaMemcpyAsync(ctx->h_ctrl(), ctx->d_ctrl(), CTR_STICKY * 4, cudaMemcpyDeviceToHost, st));
-  if (!out_dev && is_pinned_host(h_out)) CK(ctx, cudaMemcpyAsync(h_out, ctx->d_out, n, cudaMemcpyDeviceToHost, st));
+  if (pinned_out && spec) CK(ctx, cudaMemcpyAsync(h_out, ctx->d_out, n, cudaMemcpyDeviceToHost, st));
   if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
   if (ctx->h_ctrl()[CTR_ERR]) {
     // the only look-back kernels here are the two digit passes; repeat with tickets (cannot happen twice)
     if (ctx->static_tiles) {
       ctx->static_tiles = 0;
-      return run_inverse(ctx, block_mode, h_in, h_out, in_dev ? in_dev : nullptr, out_dev, n_in, eob);
+      return run_inverse(ctx, block_mode, h_in, h_out, in_dev ? in_dev : nullptr, out_dev, n_in, eob, spec);
     }
     set_err(ctx->err, "inverse: look-back watchdog fired");
     return BWTC_CUDA_EINTERNAL;
   }
-  if (!out_dev && !is_pinned_host(h_out) && download_staged(ctx, h_out, ctx->d_out, n)) return BWTC_CUDA_ECUDA;
+  const bool corrupt = (ctx->h_ctrl()[CTR_INV_BAD] & 1u) != 0u;
+  if (!corrupt) {
+    if (!spec && (out_dev || pinned_out)) {
+      CK(ctx, cudaMemcpyAsync(out_dev ? out_dev : h_out, ctx->d_out, n, out_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, st));
+      if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
+    } else if (!out_dev && !pinned_out && download_staged(ctx, h_out, ctx->d_out, n)) {
+      return BWTC_CUDA_ECUDA;
+    }
+  }
   float ms = 0;
   CK(ctx, cudaEventElapsedTime(&ms, ctx->ev_begin, ctx->ev_end));
   S.gpu_ms = ms;
   S.rounds = rounds;
   S.passes[0] = pdone;
   S.live[0] = N;
-  S.flags = ctx->static_tiles ? 0u : 1u;
+  S.flags = (ctx->static_tiles ? 0u : 1u) | (corrupt ? 128u : 0u);
+  if (corrupt) {
+    set_err(ctx->err, "inverse: block 0 is not the BWT of any text (with end-of-block row %u)", eob);
+    return BWTC_CUDA_ECORRUPT;
+  }
   return (int64_t)n;
+}
+
+// Verification of a finished block-contract forward transform (DESIGN.md §3.10): its device-resident output (J.d_dst, a
+// batch at stride n0 + 1) is inverted into d_aux[1] — end-of-block rows read from d_LF on the device — and compared with
+// the input, which d_text still holds reversed.  One host wait.  On failure an in-place device block is rewritten from
+// d_text and BWTC_CUDA_EVERIFY is returned; nothing else of the caller's has been written yet.
+int verify_forward(bwtc_cuda_ctx* ctx, const Job& J) {
+  cudaStream_t st = ctx->stream;
+  bwtc_cuda_stats& S = ctx->stats;
+  const BatchSpec* bs = J.bs;
+  InvShape sh;
+  sh.nblocks = bs ? bs->nblocks : 1u;
+  sh.n0 = bs ? bs->n0 : J.n;
+  sh.istride = bs ? J.bstride : J.n;
+  sh.R = bs ? J.bstride : J.N;
+  sh.N_last = bs ? bs->n_last + 1u : J.N;
+  sh.S0 = div_up(sh.R, INV_K);
+  sh.S_last = div_up(sh.N_last, INV_K);
+  sh.d_eob = ctx->d_LF;
+  if (ctx->debug_corrupt_out) {
+    k_debug_flip_byte<<<1, 1, 0, st>>>(J.d_dst + sh.n0 / 2);
+    CK(ctx, cudaGetLastError());
+    S.kernel_launches++;
+  }
+  for (;;) {
+    uint32_t rounds = 0, pdone = 0;
+    if (const int rc = enqueue_inverse(ctx, sh, true, J.d_dst, ctx->d_aux[1], &rounds, &pdone, false)) return rc;
+    const dim3 vgrid(std::max<uint32_t>(1u, div_up((uint32_t)ctx->sm_count * 8u, sh.nblocks)), sh.nblocks);
+    k_inv_verify<<<vgrid, 256, 0, st>>>(ctx->d_aux[1], J.d_text, sh, ctx->d_ctrl());
+    CK(ctx, cudaGetLastError());
+    S.kernel_launches++;
+    S.algorithmic_bytes += 2ull * J.n;
+    CK(ctx, cudaEventRecord(ctx->ev_end, st));
+    CK(ctx, cudaMemcpyAsync(ctx->h_ctrl(), ctx->d_ctrl(), CTR_STICKY * 4, cudaMemcpyDeviceToHost, st));
+    if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
+    if (!ctx->h_ctrl()[CTR_ERR]) break;
+    if (!ctx->static_tiles) {
+      set_err(ctx->err, "verification: look-back watchdog fired in the inverse");
+      return BWTC_CUDA_EINTERNAL;
+    }
+    ctx->static_tiles = 0;  // the inverse's two digit passes again with ticket tile ids (cannot fire twice)
+  }
+  S.flags |= 64u;
+  const uint64_t mask = (uint64_t)ctx->h_ctrl()[CTR_INV_BAD] | ((uint64_t)ctx->h_ctrl()[CTR_INV_BAD + 1] << 32);
+  if (!mask) return 0;
+  if (!bs && J.out_dev && J.out_dev == J.in_dev) {
+    k_text_unreverse<<<ctx->sm_count * 4, 256, 0, st>>>(J.d_text, J.n, J.out_dev);
+    CK(ctx, cudaGetLastError());
+    S.kernel_launches++;
+    if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
+  }
+  uint32_t first = 0;
+  while (!((mask >> first) & 1u)) ++first;
+  set_err(ctx->err, "verification failed: the forward output of block %u of %u does not restore its input", first, sh.nblocks);
+  return BWTC_CUDA_EVERIFY;
 }
 
 // count blocks (block contract) through one context: as ONE batch when they qualify — 2..MAX_BATCH blocks, all of
@@ -1606,8 +1692,10 @@ int transform_batch(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out,
 // caller has checked the arguments.  The blocks are staged in d_in (stride n0) and restored into d_out; the caller's
 // buffers are written only after the host has read CTR_ERR.  After a look-back watchdog the device part is repeated with
 // ticket tile ids from the staged input — never from the caller's buffers, which may alias the outputs.
+// *bad: bit k set = block k is corrupt; its buffer is not written, and the call returns BWTC_CUDA_ECORRUPT.
 int run_inverse_batch(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out, const uint32_t* sizes, uint32_t count,
-                      bool on_device, const uint32_t* eobs) {
+                      bool on_device, const uint32_t* eobs, uint64_t* bad) {
+  *bad = 0;
   ctx->err[0] = 0;
   if (cudaSetDevice(ctx->device) != cudaSuccess) {
     set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device);
@@ -1617,8 +1705,9 @@ int run_inverse_batch(bwtc_cuda_ctx* ctx, const void* const* in, void* const* ou
   cudaStream_t st = ctx->stream;
   InvShape sh;
   sh.nblocks = count;
-  sh.n0 = sizes[0];
+  sh.n0 = sh.istride = sizes[0];
   sh.R = sizes[0] + 1u;
+  sh.d_eob = nullptr;
   sh.N_last = sizes[count - 1] + 1u;
   sh.S0 = div_up(sh.R, INV_K);
   sh.S_last = div_up(sh.N_last, INV_K);
@@ -1642,8 +1731,10 @@ int run_inverse_batch(bwtc_cuda_ctx* ctx, const void* const* in, void* const* ou
     }
     ctx->static_tiles = 0;  // the two digit passes again with ticket tile ids (cannot fire twice)
   }
+  const uint64_t mask = (uint64_t)ctx->h_ctrl()[CTR_INV_BAD] | ((uint64_t)ctx->h_ctrl()[CTR_INV_BAD + 1] << 32);
   bool pending = false;
   for (uint32_t k = 0; k < count; ++k) {
+    if ((mask >> k) & 1u) continue;  // a corrupt block's buffer stays as it was
     const uint8_t* d = ctx->d_out + (size_t)k * sh.n0;
     uint8_t* o = static_cast<uint8_t*>(out[k]);
     if (on_device) {
@@ -1666,7 +1757,8 @@ int run_inverse_batch(bwtc_cuda_ctx* ctx, const void* const* in, void* const* ou
   S.passes[0] = pdone;
   S.live[0] = S.n_suffixes;
   S.flags = 2u | (ctx->static_tiles ? 0u : 1u);
-  return 0;
+  *bad = mask;
+  return mask ? BWTC_CUDA_ECORRUPT : 0;
 }
 
 // count blocks (block contract) through one context, each restored as run_inverse would: runs are formed greedily as in
@@ -1686,21 +1778,36 @@ int inverse_blocks(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out, 
       return BWTC_CUDA_EARG;
     }
   }
+  uint32_t ncorrupt = 0, first_corrupt = 0;
   for (uint32_t k0 = 0; k0 < count;) {
     uint32_t k1 = std::min<uint32_t>(count, k0 + MAX_BATCH);
     while (k1 > k0 + 1 && !batchable(ctx, sizes + k0, k1 - k0)) --k1;
     int64_t rc;
+    uint64_t bad = 0;
     if (k1 - k0 >= 2)
-      rc = run_inverse_batch(ctx, in + k0, out + k0, sizes + k0, k1 - k0, on_device, eobs + k0);
+      rc = run_inverse_batch(ctx, in + k0, out + k0, sizes + k0, k1 - k0, on_device, eobs + k0, &bad);
     else if (on_device)
       rc = run_inverse(ctx, true, nullptr, nullptr, static_cast<const uint8_t*>(in[k0]), static_cast<uint8_t*>(out[k0]), sizes[k0],
-                       eobs[k0]);
+                       eobs[k0], false);
     else
       rc = run_inverse(ctx, true, static_cast<const uint8_t*>(in[k0]), static_cast<uint8_t*>(out[k0]), nullptr, nullptr, sizes[k0],
-                       eobs[k0]);
-    if (rc < 0) return (int)rc;
-    if (stats) for (uint32_t k = k0; k < k1; ++k) stats[k] = ctx->stats;
+                       eobs[k0], false);
+    if (rc == BWTC_CUDA_ECORRUPT && k1 - k0 == 1) bad = 1u;
+    else if (rc < 0 && rc != BWTC_CUDA_ECORRUPT) return (int)rc;
+    for (uint32_t k = k0; k < k1; ++k) {
+      const bool b = (bad >> (k - k0)) & 1u;
+      if (b && !ncorrupt++) first_corrupt = k;
+      if (stats) {
+        stats[k] = ctx->stats;
+        stats[k].flags = (ctx->stats.flags & ~128u) | (b ? 128u : 0u);
+      }
+    }
     k0 = k1;
+  }
+  if (ncorrupt) {
+    set_err(ctx->err, "inverse: block %u (%u of %u blocks corrupt) is not the BWT of any text (with end-of-block row %u)",
+            first_corrupt, ncorrupt, count, eobs[first_corrupt]);
+    return BWTC_CUDA_ECORRUPT;
   }
   return 0;
 }
@@ -1746,6 +1853,7 @@ int bwtc_cuda_ctx_create(bwtc_cuda_ctx** out, int device, uint32_t max_block_byt
   if (const char* e = getenv("BWTC_STATIC_TILES")) c->static_tiles = atoi(e);
   if (const char* e = getenv("BWTC_DEBUG_FAKE_WATCHDOG")) c->debug_fake_watchdog = atoi(e);
   if (const char* e = getenv("BWTC_DEBUG_REVERSE_TILES")) c->debug_reverse_tiles = atoi(e);
+  if (const char* e = getenv("BWTC_DEBUG_CORRUPT_OUT")) c->debug_corrupt_out = atoi(e);
   if (const char* e = getenv("BWTC_DEBUG_SKIP_COPIES")) c->debug_skip_copies = atoi(e);
   if (const char* e = getenv("BWTC_D2H_KERNEL")) c->d2h_kernel = atoi(e);
   if (const char* e = getenv("BWTC_D2H_CTAS")) c->d2h_ctas = std::max(1, atoi(e));
@@ -1927,6 +2035,12 @@ int bwtc_cuda_ctx_set_timing(bwtc_cuda_ctx* ctx, int detail) {
       if (cudaEventCreate(&ev) != cudaSuccess) { set_err(ctx->err, "cudaEventCreate failed"); return BWTC_CUDA_ECUDA; }
   }
   ctx->timing_detail = detail;
+  return 0;
+}
+
+int bwtc_cuda_ctx_set_verify(bwtc_cuda_ctx* ctx, int on) {
+  if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
+  ctx->verify = on ? 1 : 0;
   return 0;
 }
 
@@ -2138,7 +2252,7 @@ void pipeline_worker(bwtc_cuda_pipeline* p, bwtc_cuda_ctx* c) {
       in.resize(cnt); out.resize(cnt); sizes.resize(cnt); eobs.resize(cnt); stats.resize(cnt);
       for (uint32_t k = 0; k < cnt; ++k) { in[k] = grp[k]->in; out[k] = grp[k]->out; sizes[k] = grp[k]->n; eobs[k] = grp[k]->eob; }
       rc = inverse_blocks(c, in.data(), out.data(), sizes.data(), cnt, grp[0]->on_device, eobs.data(), stats.data());
-      if (rc >= 0)
+      if (rc >= 0 || rc == BWTC_CUDA_ECORRUPT)
         for (uint32_t k = 0; k < cnt; ++k)
           if (grp[k]->stats) *grp[k]->stats = stats[k];
     } else if (cnt == 1) {
@@ -2166,8 +2280,20 @@ void pipeline_worker(bwtc_cuda_pipeline* p, bwtc_cuda_ctx* c) {
     }
     {
       std::lock_guard<std::mutex> lk(p->mu);
-      if (rc < 0 && !p->err[0]) set_err(p->err, "block ticket %llu (+%u): %s", (unsigned long long)grp[0]->ticket, cnt - 1, c->err);
-      for (auto& it : grp) { it->rc = rc < 0 ? rc : 0; it->done = true; }
+      if (rc == BWTC_CUDA_ECORRUPT && grp[0]->kind == PIPE_INVERSE) {
+        // only the tickets of the corrupt blocks fail; the rest of the group was restored (DESIGN.md §5.2)
+        for (uint32_t k = 0; k < cnt; ++k) {
+          PipeItem& it = *grp[k];
+          it.rc = (stats[k].flags & 128u) ? BWTC_CUDA_ECORRUPT : 0;
+          if (it.rc && !p->err[0])
+            set_err(p->err, "block ticket %llu: inverse: not the BWT of any text (with end-of-block row %u)",
+                    (unsigned long long)it.ticket, it.eob);
+          it.done = true;
+        }
+      } else {
+        if (rc < 0 && !p->err[0]) set_err(p->err, "block ticket %llu (+%u): %s", (unsigned long long)grp[0]->ticket, cnt - 1, c->err);
+        for (auto& it : grp) { it->rc = rc < 0 ? rc : 0; it->done = true; }
+      }
     }
     p->cv_done.notify_all();
   }
@@ -2273,6 +2399,12 @@ int bwtc_cuda_pipeline_set_timing(bwtc_cuda_pipeline* p, int detail) {
     int rc = bwtc_cuda_ctx_set_timing(c, detail);
     if (rc) return rc;
   }
+  return 0;
+}
+
+int bwtc_cuda_pipeline_set_verify(bwtc_cuda_pipeline* p, int on) {
+  if (!p) { set_err(g_err, "null pipeline"); return BWTC_CUDA_EARG; }
+  for (bwtc_cuda_ctx* c : p->ctxs) c->verify = on ? 1 : 0;
   return 0;
 }
 

@@ -15,7 +15,8 @@
 //   4. k_inv_walk1    every K-th rank (K = 32) is a SPLITTER; each splitter follows Psi to the next splitter: (next, length)
 //   5. k_inv_jump     x ceil(log2 S): pointer jumping over the S = N/K splitters -> distance of each to the end of the
 //                     cycle opened at rank 0 (suffix N-1), i.e. its text position
-//   6. k_inv_walk2    each splitter walks its stretch again and writes X[n-1-q] = F[rank(q)] for its text positions q
+//   6. k_inv_walk2    each splitter walks its stretch again and writes X[n-1-q] = F[rank(q)] for its text positions q;
+//                     it also decides whether L is the BWT of any text at all (Psi one cycle, DESIGN.md §3.7)
 // Two passes of N dependent-per-chain but mutually independent random reads with ~N/K chains in flight: bound by the
 // L2/DRAM random-access rate, not by latency.  LFpowers[1..] are not needed (the device makes far denser samples).
 #pragma once
@@ -31,6 +32,10 @@ constexpr uint32_t INV_K = BWTC_INV_K;   // splitter spacing in rank space = ave
                                          // block): 128 -> 2.63 ms, 64 -> 2.29 ms, 32 -> 2.00 ms: shorter chains even out the
                                          // geometric spread of chain lengths that leaves lanes idle (profiles/r02_summary.md)
 constexpr uint32_t INV_NIL = 0xFFFFFFFFu;
+// ctrl[2..3]: bit k set = block k of the inversion is corrupt (its Psi is not one cycle: not the BWT of any text with that
+// end-of-block row) or, when a forward transform is verified, does not restore its text.  Zeroed with the sticky words.
+constexpr int CTR_INV_BAD = 2;
+__device__ __forceinline__ void inv_mark_bad(uint32_t* ctrl, uint32_t k) { atomicOr(&ctrl[CTR_INV_BAD + (k >> 5)], 1u << (k & 31u)); }
 
 // Batch of blocks inverted as ONE problem (DESIGN.md §3.7), the layout of the forward batch (§3.6): B blocks of n0 bytes,
 // the last one n_last <= n0 bytes; block k has N_k = n_k + 1 rows and owns rows [k R, k R + N_k) with R = n0 + 1, its
@@ -42,12 +47,15 @@ constexpr uint32_t INV_MAX_BLOCKS = 64;  // = BWTC_CUDA_MAX_BATCH
 struct InvShape {
   uint32_t nblocks;  // B
   uint32_t R;        // row stride (B = 1: N)
-  uint32_t n0;       // byte stride of the input / output blocks (B = 1: unused)
+  uint32_t n0;       // byte stride of the output blocks (B = 1: unused)
+  uint32_t istride;  // byte stride of the input blocks: n0, or R for the output of a forward batch (B = 1: unused)
   uint32_t N_last;   // rows of the last block
   uint32_t S0;       // splitters of a full block (ceil(R / INV_K)) ...
   uint32_t S_last;   // ... and of the last block
-  uint32_t eob[INV_MAX_BLOCKS];  // per block: the end-of-block row (LFpowers[0])
+  uint32_t eob[INV_MAX_BLOCKS];  // per block: the end-of-block row (LFpowers[0]) ...
+  const uint32_t* d_eob;         // ... or, if not null, read on the device from d_eob[256 k] (a forward transform's LFpowers rows)
 };
+__device__ __forceinline__ uint32_t inv_eob(const InvShape& sh, uint32_t k) { return sh.d_eob ? sh.d_eob[256u * k] : sh.eob[k]; }
 __host__ __device__ __forceinline__ uint32_t inv_rows(const InvShape& sh) { return (sh.nblocks - 1u) * sh.R + sh.N_last; }
 __host__ __device__ __forceinline__ uint32_t inv_splitters(const InvShape& sh) { return (sh.nblocks - 1u) * sh.S0 + sh.S_last; }
 
@@ -65,8 +73,8 @@ __global__ void __launch_bounds__(256) k_inv_keys(const uint8_t* __restrict__ in
   if (threadIdx.x == 0) s_hi = 0;
   __syncthreads();
   const uint32_t k = blockIdx.y;
-  const uint32_t N = (k + 1u == sh.nblocks) ? sh.N_last : sh.R, eob = sh.eob[k];
-  const uint8_t* __restrict__ ink = in + (size_t)k * sh.n0;
+  const uint32_t N = (k + 1u == sh.nblocks) ? sh.N_last : sh.R, eob = inv_eob(sh, k);
+  const uint8_t* __restrict__ ink = in + (size_t)k * sh.istride;
   uint32_t* __restrict__ kk = keys + (size_t)k * sh.R;
   const uint32_t top = k << 9;
   for (uint32_t r = blockIdx.x * blockDim.x + threadIdx.x; r < N; r += gridDim.x * blockDim.x) {
@@ -158,23 +166,49 @@ __global__ void __launch_bounds__(256) k_inv_jump(const uint32_t* __restrict__ n
 // dist[s] = D(s) = steps from splitter s to the end of its block's opened cycle (back at rank 0), so the text position of
 // splitter s is q0 = (2N_k - 1 - D(s)) mod N_k (splitter 0 = rank 0 = suffix N_k - 1).  Walk len[s] steps: the row at
 // step t is the suffix at text position q = q0 + t; its first character F[g] is X_k[n_k-1-q] (q = N_k-1: the sentinel).
+// Single-cycle check (DESIGN.md §3.7): L with this eob is the BWT of a text exactly when Psi is one cycle, i.e. when
+//   (a) the walk-1 lengths of the block's splitters sum to N_k (every cycle holds a splitter: walk 1 ends on the splitter's
+//       own cycle, so the sum counts exactly the rows of cycles that have one), and
+//   (b) after the ceil(log2 S0) jump rounds every splitter has nxt == INV_NIL (it lies on the cycle through row 0; on any
+//       other cycle a chain never reaches NIL).
+// Each CTA adds its part of the sum to chk[k] (chk: [2B] zeroed words; chk[B + k] counts the CTAs of block k that are done)
+// and the last CTA of the block compares; a failed test sets bit k of ctrl[CTR_INV_BAD..].  The output is written anyway.
 __global__ void __launch_bounds__(256) k_inv_walk2(const uint32_t* __restrict__ vals, const uint32_t* __restrict__ len,
-                                                   const uint32_t* __restrict__ dist, const uint32_t* __restrict__ C,
-                                                   const InvShape sh, uint8_t* __restrict__ out,
-                                                   const uint32_t* __restrict__ ctrl) {
+                                                   const uint32_t* __restrict__ dist, const uint32_t* __restrict__ nxt,
+                                                   const uint32_t* __restrict__ C, const InvShape sh, uint8_t* __restrict__ out,
+                                                   uint32_t* __restrict__ ctrl, uint32_t* __restrict__ chk) {
   __shared__ uint32_t s_C[258];
-  if (ctrl[0]) return;  // (the caller's buffer — possibly the in-place input — stays untouched)
+  __shared__ uint32_t s_sum, s_open;
+  if (ctrl[CTR_ERR]) return;  // (the caller's buffer — possibly the in-place input — stays untouched)
   const uint32_t k = blockIdx.y;
   for (int i = threadIdx.x; i < 258; i += blockDim.x) s_C[i] = C[(size_t)k * 258 + i];
+  if (threadIdx.x == 0) { s_sum = 0; s_open = 0; }
   __syncthreads();
   const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
   const bool last = k + 1u == sh.nblocks;
-  if (j >= (last ? sh.S_last : sh.S0)) return;
+  const bool active = j < (last ? sh.S_last : sh.S0);
   const uint32_t N = last ? sh.N_last : sh.R, n = N - 1u, top = inv_rows(sh) - 1u;
   const uint32_t s = k * sh.S0 + j;
+  const uint32_t L = active ? len[s] : 0u;  // (a cycle's splitters split it: the sum never exceeds N_k)
+  const uint32_t wsum = __reduce_add_sync(0xFFFFFFFFu, L);
+  const bool wopen = __any_sync(0xFFFFFFFFu, active && nxt[s] != INV_NIL);
+  if ((threadIdx.x & 31u) == 0u) {
+    if (wsum) atomicAdd(&s_sum, wsum);
+    if (wopen) s_open = 1u;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    atomicAdd(&chk[k], s_sum);
+    if (s_open) inv_mark_bad(ctrl, k);
+    __threadfence();
+    if (atomicAdd(&chk[sh.nblocks + k], 1u) == gridDim.x - 1u) {  // the last CTA of block k: every part is in chk[k]
+      __threadfence();
+      if (atomicAdd(&chk[k], 0u) != N) inv_mark_bad(ctrl, k);
+    }
+  }
+  if (!active) return;
   uint8_t* __restrict__ outk = out + (size_t)k * sh.n0;
   uint32_t g = k * sh.R + j * INV_K;
-  const uint32_t L = len[s];
   uint32_t q = (uint32_t)((2ull * N - 1ull - (unsigned long long)dist[s]) % N);
   for (uint32_t t = 0; t < L; ++t) {
     if (q < n) {
@@ -190,6 +224,29 @@ __global__ void __launch_bounds__(256) k_inv_walk2(const uint32_t* __restrict__ 
     q = (q + 1u == N) ? 0u : q + 1u;
   }
 }
+
+// ---- verification of a forward transform (DESIGN.md §3.10).  Grid (x, B).  Block k restored into rest + k n0 must equal
+// X_k, which the forward's text still holds reversed: T'_k = text + k R, X_k[i] = T'_k[n_k - 1 - i].  A difference sets bit k
+// of ctrl[CTR_INV_BAD..], like a corrupt block.
+__global__ void __launch_bounds__(256) k_inv_verify(const uint8_t* __restrict__ rest, const uint8_t* __restrict__ text,
+                                                    const InvShape sh, uint32_t* __restrict__ ctrl) {
+  if (ctrl[CTR_ERR]) return;
+  const uint32_t k = blockIdx.y;
+  const uint32_t n = ((k + 1u == sh.nblocks) ? sh.N_last : sh.R) - 1u;
+  const uint8_t* __restrict__ rk = rest + (size_t)k * sh.n0;
+  const uint8_t* __restrict__ tk = text + (size_t)k * sh.R;
+  bool diff = false;
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) diff |= rk[i] != tk[n - 1u - i];
+  if (__any_sync(0xFFFFFFFFu, diff) && (threadIdx.x & 31u) == 0u) inv_mark_bad(ctrl, k);
+}
+
+// out[i] = text[n - 1 - i]: puts the input of a failed in-place forward transform back from its reversed text.
+__global__ void __launch_bounds__(256) k_text_unreverse(const uint8_t* __restrict__ text, uint32_t n, uint8_t* __restrict__ out) {
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) out[i] = text[n - 1u - i];
+}
+
+// Test hook BWTC_DEBUG_CORRUPT_OUT: one byte of the forward output changed before it is verified.
+__global__ void k_debug_flip_byte(uint8_t* p) { *p ^= 1u; }
 
 // =====================================================================================================
 // Run statistics of the transformed block (SURVEY.md §8f row f3; the reference's own TODO at HuffmanCoders.cpp:54:

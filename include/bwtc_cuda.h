@@ -39,6 +39,10 @@ extern "C" {
 #define BWTC_CUDA_ECUDA     (-3)  /* a CUDA runtime call or kernel failed */
 #define BWTC_CUDA_EINTERNAL (-4)  /* internal consistency check failed (e.g. look-back watchdog) */
 #define BWTC_CUDA_ETOOBIG   (-5)  /* block larger than the context capacity / engine limit */
+#define BWTC_CUDA_ECORRUPT  (-6)  /* inverse: the input is not the BWT of any text (with this end-of-block row); the message
+                                   * names the block */
+#define BWTC_CUDA_EVERIFY   (-7)  /* forward with verification on: the output did not restore the input (see
+                                   * bwtc_cuda_ctx_set_verify); every caller buffer still holds its input */
 
 /* Largest block (bytes, excluding the sentinel slot) the engine accepts: the reference's own limit — blocks below
  * 2^31 - 2 bytes (Compressor.cpp:78-79, PrecompressorBlock.cpp:126; N = n + 1 suffixes must index with 31 bits because
@@ -77,9 +81,12 @@ typedef struct bwtc_cuda_stats {
   float    sort0_ms;                        /* device time inside the round-0 passes (detailed timing on) */
   uint32_t flags;            /* bit 0: look-back kernels ran with ticket counters (watchdog fallback or BWTC_STATIC_TILES=0);
                               * bit 1: the blocks of a batch were sorted as one text; bit 2: predecessor codes packed above the ids;
-                              * bit 3: ... carried as a one-byte payload array */
+                              * bit 3: ... carried as a one-byte payload array; bit 6: the forward output was verified by a
+                              * device-side inversion (bwtc_cuda_ctx_set_verify); bit 7: inverse only, this block is corrupt
+                              * (BWTC_CUDA_ECORRUPT) */
   uint32_t batch_blocks;     /* blocks this record describes: 1, or the size of the batch that was sorted as one text (every
-                              * block of the batch then carries the SAME record — count it once) */
+                              * block of the batch then carries the SAME record — count it once; flags bit 7 is the one field
+                              * in which the records of one inverse batch may differ) */
 } bwtc_cuda_stats;
 
 /* ---- library / device ------------------------------------------------------------------------ */
@@ -102,6 +109,16 @@ int         bwtc_cuda_ctx_set_round0(bwtc_cuda_ctx* ctx, uint32_t chars, uint32_
 /* detail != 0: bracket every radix digit pass with CUDA events on the context's stream so that
  * stats.sort_ms / sort_bytes / sort_launches give the dominant kernel's average launch duration. */
 int         bwtc_cuda_ctx_set_timing(bwtc_cuda_ctx* ctx, int detail);
+/* on != 0: every block-contract forward call (bwtc_cuda_bwt_block, _device, _runs, bwtc_cuda_bwt_blocks) is verified before
+ * it returns: the device inverts its device-resident output (end-of-block rows from the device-side LFpowers, a batch as one
+ * batched inversion) and compares the result with the input, which the device still holds reversed.  On a mismatch the call
+ * returns BWTC_CUDA_EVERIFY and every caller buffer holds its input: host outputs, LFpowers and freqs are written only after
+ * the host has read the check word, and an in-place device block is rewritten from the device copy (a device output that
+ * does not alias its input, and the run arrays of bwtc_cuda_bwt_block_runs, are then unspecified).  Costs about one inverse
+ * transform and one host wait per call; stats.flags bit 6 marks a verified block, stats.gpu_ms includes the check.  The
+ * raw contract (bwtc_cuda_divbwt / divbwtf) is never verified.  Off (0) by default; off, every call runs exactly the
+ * kernels it runs without this switch.  The context stays usable after BWTC_CUDA_EVERIFY. */
+int         bwtc_cuda_ctx_set_verify(bwtc_cuda_ctx* ctx, int on);
 /* Debug / test hooks: max_rounds != 0 stops the refinement after that many sort rounds (the output is
  * then deliberately incomplete); bwtc_cuda_debug_read copies an engine buffer to the host
  * (which: 0 text, 1 rank[], 2/3 sorted keys/ids of the last round, 4/5 the other sort buffer,
@@ -164,7 +181,10 @@ int64_t bwtc_cuda_bwt_block_runs(bwtc_cuda_ctx* ctx, uint8_t* block, uint32_t n,
 /* ---- inverse transform (SURVEY.md §8f, row f4): InverseBWTransform::doTransform (InverseBWT.hpp:45-55) ---------------- */
 /* Block level (InverseBWT.cpp:47-51): block holds the n bytes a forward block transform produced, LFpowers its starting
  * points (only LFpowers[0], the end-of-block position, is needed: the device makes its own, far denser samples).  The
- * original n bytes are restored IN PLACE; the byte after the block is never touched.  Returns n. */
+ * original n bytes are restored IN PLACE; the byte after the block is never touched.  Returns n.
+ * Every inverse entry point checks that its input is the BWT of some text with that end-of-block row (exactly: the
+ * permutation it defines is one cycle) and returns BWTC_CUDA_ECORRUPT if not.  A pageable host block is then untouched; a
+ * pinned host or device output (written speculatively, so that a valid block costs no extra wait) holds unspecified bytes. */
 int64_t bwtc_cuda_inverse_block(bwtc_cuda_ctx* ctx, uint8_t* block, uint32_t n, const uint32_t* LFpowers, uint32_t nLFpowers);
 int64_t bwtc_cuda_inverse_block_device(bwtc_cuda_ctx* ctx, const void* d_in, void* d_out, uint32_t n, uint32_t eob);
 /* Raw virtual doTransform(byte* bwt, uint32 N, LFpow) (InverseBWT.hpp:49-50): bwt[0..N) = L with bwt[LFpowers[0]] ignored;
@@ -178,6 +198,8 @@ int64_t bwtc_cuda_inverse_raw(bwtc_cuda_ctx* ctx, uint8_t* bwt, uint32_t N, cons
  * within the context's capacity) are inverted as ONE device-side problem — whatever byte values the blocks contain —
  * others one after the other.  The byte after each block is never touched.  Every argument is checked before any work.
  * stats: count records (the blocks of a batch share one, batch_blocks = its size, flags bit 1 set) or NULL.
+ * Corrupt blocks do not stop the call: every valid block is restored, the buffer of each corrupt block is left untouched
+ * (whatever its kind), its record gets flags bit 7, and the call returns BWTC_CUDA_ECORRUPT naming the first one.
  * Returns 0 or a negative error. */
 int bwtc_cuda_inverse_blocks(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out, const uint32_t* sizes,
                              uint32_t count, int on_device, const uint32_t* LFpowers, bwtc_cuda_stats* stats);
@@ -192,6 +214,8 @@ void bwtc_cuda_pipeline_destroy(bwtc_cuda_pipeline* p);
 const char* bwtc_cuda_pipeline_error(const bwtc_cuda_pipeline* p);
 int  bwtc_cuda_pipeline_set_round0(bwtc_cuda_pipeline* p, uint32_t chars, uint32_t key_bytes);
 int  bwtc_cuda_pipeline_set_timing(bwtc_cuda_pipeline* p, int detail);
+/* bwtc_cuda_ctx_set_verify on every context of the pipeline: forward blocks (run, submit, submit_runs) are verified. */
+int  bwtc_cuda_pipeline_set_verify(bwtc_cuda_pipeline* p, int on);
 /* Transforms nblocks blocks.  in[i]/out[i]: sizes[i] bytes each (may alias; host memory, or device
  * memory when on_device != 0).  LFpowers: nblocks x 256 uint32 (row i gets nLF[i] entries, where
  * nLF[i] = bwtc_cuda_num_starting_points(sizes[i], starts) is written by the call); freqs: nblocks x 256
@@ -214,7 +238,9 @@ int  bwtc_cuda_pipeline_wait(bwtc_cuda_pipeline* p, uint64_t ticket);
  * original n bytes land in out, which may alias in; device memory when on_device != 0; eob = LFpowers[0] of the forward
  * transform; stats may be NULL) and return at once with a ticket of the same sequence as bwtc_cuda_pipeline_submit's; wait
  * for it with bwtc_cuda_pipeline_wait.  Queued inverse blocks of equal size are inverted as one device-side problem;
- * forward and inverse blocks are never grouped together. */
+ * forward and inverse blocks are never grouped together.  An error is reported through every ticket of the group it
+ * happened in, except BWTC_CUDA_ECORRUPT: only the ticket of a corrupt block returns it (its out buffer is untouched), the
+ * other blocks of its group complete normally. */
 int  bwtc_cuda_pipeline_submit_inverse(bwtc_cuda_pipeline* p, const uint8_t* in, uint8_t* out, uint32_t n, uint32_t eob,
                                        int on_device, bwtc_cuda_stats* stats, uint64_t* ticket);
 /* submit + run statistics (filled when the block completes; such a block is transformed on its own, not in a batch). */
