@@ -703,8 +703,9 @@ int64_t phase_input(bwtc_cuda_ctx* ctx, Job& J) {
   const uint32_t n = J.n;
   const uint32_t N = J.block_mode ? n + 1 : n;
   J.N = N;
-  if (n > ctx->cap) {
-    set_err(ctx->err, "block of %u bytes exceeds context capacity %u", n, ctx->cap);
+  // a context holds N = cap + 1 suffixes: a block of cap bytes plus its sentinel, or a raw text of cap + 1 bytes
+  if (n > (J.block_mode ? (uint64_t)ctx->cap : (uint64_t)ctx->cap + 1)) {
+    set_err(ctx->err, "%s of %u bytes exceeds context capacity %u", J.block_mode ? "block" : "raw text", n, ctx->cap);
     return BWTC_CUDA_ETOOBIG;
   }
   if (J.nLF < 1 || J.nLF > 256 || J.nLF > N || !J.LF) {

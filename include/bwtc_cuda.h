@@ -98,7 +98,8 @@ const char* bwtc_cuda_global_error(void);
 
 /* ---- context ------------------------------------------------------------------------------------ */
 /* Allocates streams, device scratch (BWTC_CUDA_SCRATCH_BYTES_PER_SUFFIX bytes per suffix) and small pinned buffers for
- * blocks up to max_block_bytes on `device`.  Replaces the per-call malloc of divbwtf (divsufsort.c:491-493). */
+ * blocks up to max_block_bytes on `device` (raw texts up to max_block_bytes + 1: the same max_block_bytes + 1 suffixes).
+ * Replaces the per-call malloc of divbwtf (divsufsort.c:491-493). */
 int         bwtc_cuda_ctx_create(bwtc_cuda_ctx** out, int device, uint32_t max_block_bytes);
 uint64_t    bwtc_cuda_scratch_bytes(uint32_t max_block_bytes);  /* device bytes such a context allocates */
 void        bwtc_cuda_ctx_destroy(bwtc_cuda_ctx* ctx);

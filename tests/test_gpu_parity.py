@@ -462,3 +462,39 @@ def test_maximum_block_size_properties(n):
     assert (LF <= n).all() and len(set(LF.tolist())) == 8
     with pytest.raises(bw.BwtcCudaError):  # one byte above the limit is refused loudly (no silent truncation, no fallback)
         bw.CudaContext(0x7FFFFFFE)
+
+
+def test_maximum_raw_text_size_properties():
+    """The reference's largest block (2^31 - 3 bytes) reaches the raw contract (integration options A and B) as
+    T = reverse(X)·0x00 of 2^31 - 2 bytes; a context of the largest capacity holds exactly that many suffixes.  The
+    size-independent checks of test_maximum_block_size_properties: freqs = byte histogram of T[:-1], U keeps it (plus the
+    untouched U[pidx] = T[pidx]), and the sampled suffixes' ranks order them as their first 64 bytes do."""
+    N = bw.MAX_BLOCK + 1
+    try:
+        ctx = bw.CudaContext(bw.MAX_BLOCK)
+    except bw.BwtcCudaError as e:
+        pytest.skip(f"cannot allocate scratch for a {N >> 20} MiB text: {e}")
+    T = np.empty(N, np.uint8)
+    bw.generate("random", N - 1, seed=34, out=T)
+    T[12345:12345 + 4096] = T[777:777 + 4096]
+    T[-1] = 0
+    hist = _hist_chunked(T[:-1])
+    U = T.copy()
+    LF = np.zeros(8, np.uint32)
+    fr = np.zeros(256, np.uint32)
+    try:
+        pidx = ctx.divbwtf(U, U, LF, fr)
+        st = ctx.stats()
+    finally:
+        ctx.close()
+    assert st["n_suffixes"] == N and pidx == LF[0] and st["rounds"] >= 2
+    assert U[pidx] == T[pidx]
+    onehot = np.zeros(256, np.int64)
+    onehot[T[pidx]] = 1
+    assert (fr == hist).all() and (_hist_chunked(U) == hist + onehot).all()
+    del U
+    xs = N // 8
+    pos = [0] + [N - j * xs for j in range(1, 8)]
+    keys = [bytes(T[p:p + 64]) for p in pos]  # (a proper prefix sorts first, as bytes compare)
+    assert list(np.argsort(LF)) == sorted(range(8), key=lambda i: keys[i])
+    assert (LF < N).all() and len(set(LF.tolist())) == 8
