@@ -1470,6 +1470,10 @@ int enqueue_inverse(bwtc_cuda_ctx* ctx, const InvShape& sh, bool block_mode, con
   uint32_t pdone = 0;
   const int rc = run_sort<uint32_t, RS_IPT32>(ctx, N, 3u, true, N - 1, &cur, &pt, &pdone);
   if (rc) return rc;
+  if (ctx->debug_fake_watchdog && ctx->static_tiles) {
+    // test hook: the state a look-back watchdog in the digit passes leaves (every later kernel returns at entry)
+    CK(ctx, cudaMemsetAsync(ctx->d_ctrl() + CTR_ERR, 0xFF, 4, st));
+  }
   const uint32_t* vals = ctx->d_idx[cur];
   const uint32_t Sn = inv_splitters(sh);  // <= N / INV_K + B
   uint32_t* nxtA = ctx->d_scat;
@@ -1486,7 +1490,7 @@ int enqueue_inverse(bwtc_cuda_ctx* ctx, const InvShape& sh, bool block_mode, con
   uint32_t* nin = nxtA; uint32_t* din = distA; uint32_t* nout = nxtB; uint32_t* dout = distB;
   uint32_t rounds = 0;
   for (uint64_t span = 1; span < (uint64_t)sh.S0; span <<= 1) {  // a chain never leaves its block: ceil(log2 S0) rounds
-    k_inv_jump<<<div_up(Sn, 256), 256, 0, st>>>(nin, din, Sn, nout, dout);
+    k_inv_jump<<<div_up(Sn, 256), 256, 0, st>>>(nin, din, Sn, nout, dout, ctx->d_ctrl());
     std::swap(nin, nout);
     std::swap(din, dout);
     ++rounds;
@@ -1504,7 +1508,9 @@ int enqueue_inverse(bwtc_cuda_ctx* ctx, const InvShape& sh, bool block_mode, con
 
 // spec (the single-block entry points): pinned host and device outputs are written without waiting for the check, so a
 // valid block costs one host wait; a corrupt one leaves them unspecified.  !spec (a block of bwtc_cuda_inverse_blocks):
-// restored into d_out, copied to the caller only if valid.
+// restored into d_out, copied to the caller only if valid.  After a look-back watchdog the device part is repeated with
+// ticket tile ids from the device copy of the input (d_in, or in_dev, which walk2 left untouched) — never from h_in, which
+// the speculative copy may already have overwritten with stale bytes when it aliases a pinned h_out.
 int64_t run_inverse(bwtc_cuda_ctx* ctx, bool block_mode, const uint8_t* h_in, uint8_t* h_out, const uint8_t* in_dev, uint8_t* out_dev,
                     uint32_t n_in, uint32_t eob, bool spec = true) {
   ctx->err[0] = 0;
@@ -1523,9 +1529,6 @@ int64_t run_inverse(bwtc_cuda_ctx* ctx, bool block_mode, const uint8_t* h_in, ui
   }
   cudaStream_t st = ctx->stream;
   bwtc_cuda_stats& S = ctx->stats;
-  memset(&S, 0, sizeof(S));
-  S.n_suffixes = N;
-  S.batch_blocks = 1;
   const uint8_t* d_src = in_dev;
   if (!in_dev) {
     if (upload(ctx, ctx->d_in, h_in, n_in)) return BWTC_CUDA_ECUDA;
@@ -1541,18 +1544,21 @@ int64_t run_inverse(bwtc_cuda_ctx* ctx, bool block_mode, const uint8_t* h_in, ui
   sh.eob[0] = eob;
   sh.d_eob = nullptr;
   uint32_t rounds = 0, pdone = 0;
-  if (const int rc = enqueue_inverse(ctx, sh, block_mode, d_src, d_dst, &rounds, &pdone)) return rc;
-  CK(ctx, cudaMemcpyAsync(ctx->h_ctrl(), ctx->d_ctrl(), CTR_STICKY * 4, cudaMemcpyDeviceToHost, st));
-  if (pinned_out && spec) CK(ctx, cudaMemcpyAsync(h_out, ctx->d_out, n, cudaMemcpyDeviceToHost, st));
-  if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
-  if (ctx->h_ctrl()[CTR_ERR]) {
+  for (;;) {
+    memset(&S, 0, sizeof(S));
+    S.n_suffixes = N;
+    S.batch_blocks = 1;
+    if (const int rc = enqueue_inverse(ctx, sh, block_mode, d_src, d_dst, &rounds, &pdone)) return rc;
+    CK(ctx, cudaMemcpyAsync(ctx->h_ctrl(), ctx->d_ctrl(), CTR_STICKY * 4, cudaMemcpyDeviceToHost, st));
+    if (pinned_out && spec) CK(ctx, cudaMemcpyAsync(h_out, ctx->d_out, n, cudaMemcpyDeviceToHost, st));
+    if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
+    if (!ctx->h_ctrl()[CTR_ERR]) break;
     // the only look-back kernels here are the two digit passes; repeat with tickets (cannot happen twice)
-    if (ctx->static_tiles) {
-      ctx->static_tiles = 0;
-      return run_inverse(ctx, block_mode, h_in, h_out, in_dev ? in_dev : nullptr, out_dev, n_in, eob, spec);
+    if (!ctx->static_tiles) {
+      set_err(ctx->err, "inverse: look-back watchdog fired");
+      return BWTC_CUDA_EINTERNAL;
     }
-    set_err(ctx->err, "inverse: look-back watchdog fired");
-    return BWTC_CUDA_EINTERNAL;
+    ctx->static_tiles = 0;
   }
   const bool corrupt = (ctx->h_ctrl()[CTR_INV_BAD] & 1u) != 0u;
   if (!corrupt) {
@@ -1725,7 +1731,7 @@ int run_inverse_batch(bwtc_cuda_ctx* ctx, const void* const* in, void* const* ou
     if (const int rc = enqueue_inverse(ctx, sh, true, ctx->d_in, ctx->d_out, &rounds, &pdone)) return rc;
     CK(ctx, cudaMemcpyAsync(ctx->h_ctrl(), ctx->d_ctrl(), CTR_STICKY * 4, cudaMemcpyDeviceToHost, st));
     if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
-    if (!ctx->h_ctrl()[CTR_ERR] && !(ctx->debug_fake_watchdog && ctx->static_tiles)) break;
+    if (!ctx->h_ctrl()[CTR_ERR]) break;
     if (!ctx->static_tiles) {
       set_err(ctx->err, "inverse: look-back watchdog fired");
       return BWTC_CUDA_EINTERNAL;

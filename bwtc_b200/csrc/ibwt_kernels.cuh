@@ -149,9 +149,10 @@ __global__ void __launch_bounds__(256) k_inv_walk1(const uint32_t* __restrict__ 
 
 // One pointer-jumping round: dist_out[s] = dist_in[s] + dist_in[nxt_in[s]], nxt_out[s] = nxt_in[nxt_in[s]].
 __global__ void __launch_bounds__(256) k_inv_jump(const uint32_t* __restrict__ nxt_in, const uint32_t* __restrict__ dist_in,
-                                                  uint32_t S, uint32_t* __restrict__ nxt_out, uint32_t* __restrict__ dist_out) {
+                                                  uint32_t S, uint32_t* __restrict__ nxt_out, uint32_t* __restrict__ dist_out,
+                                                  const uint32_t* __restrict__ ctrl) {
   const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
-  if (s >= S) return;
+  if (s >= S || ctrl[CTR_ERR]) return;  // sticky error: walk1 did not run, nxt_in holds stale indices
   const uint32_t nx = nxt_in[s];
   uint32_t d = dist_in[s], n2 = INV_NIL;
   if (nx != INV_NIL) {
