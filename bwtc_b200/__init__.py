@@ -219,8 +219,10 @@ class CudaContext:
         self._check(self._lib.bwtc_cuda_ctx_set_debug(self._h, max_rounds))
 
     def set_verify(self, on: bool):
-        """bwtc_cuda_ctx_set_verify: every block-contract forward call inverts its output on the device and compares it with
-        the input before it returns; a mismatch raises BwtcCudaError with code EVERIFY and leaves the input in place."""
+        """bwtc_cuda_ctx_set_verify: every forward call, block contract and raw (divbwtf), inverts its output on the device
+        and compares it with the input, and checks every LFpowers entry against the inversion, before it returns; a
+        mismatch raises BwtcCudaError with code EVERIFY and leaves the input, LFpowers and freqs in place.  The initial
+        value comes from BWTC_VERIFY (read when the context is created, default off); this call overrides it."""
         self._check(self._lib.bwtc_cuda_ctx_set_verify(self._h, 1 if on else 0))
 
     def debug_read(self, which: int, dtype, count: int, offset_bytes: int = 0) -> np.ndarray:
@@ -475,7 +477,8 @@ class Pipeline:
         self._lib.bwtc_cuda_pipeline_set_timing(self._h, detail)
 
     def set_verify(self, on: bool):
-        """bwtc_cuda_pipeline_set_verify: forward blocks are verified on the device (see CudaContext.set_verify)."""
+        """bwtc_cuda_pipeline_set_verify: forward blocks and their LFpowers are verified on the device (see
+        CudaContext.set_verify); overrides BWTC_VERIFY for every context of the pipeline."""
         rc = self._lib.bwtc_cuda_pipeline_set_verify(self._h, 1 if on else 0)
         if rc < 0:
             raise BwtcCudaError(rc, self._lib.bwtc_cuda_pipeline_error(self._h).decode())

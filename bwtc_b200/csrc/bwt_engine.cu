@@ -122,8 +122,9 @@ struct bwtc_cuda_ctx {
   int lb_watchdog = 0;            // the last transform failed on the look-back watchdog
   int debug_fake_watchdog = 0;    // test hook: pretend the watchdog fired while static tile ids are in use
   int debug_reverse_tiles = 0;    // test hook: static tile ids in REVERSE dispatch order (a real violation)
-  int verify = 0;                 // block-contract forward outputs are inverted on the device and compared (DESIGN.md §3.10)
+  int verify = 0;                 // forward outputs are inverted on the device and compared (DESIGN.md §3.10); BWTC_VERIFY
   int debug_corrupt_out = 0;      // test hook: one byte of the forward output is changed before it is verified
+  uint32_t debug_corrupt_lf = 0;  // test hook (j >= 1): LFpowers[j] is changed on the device before it is verified
   int d2h_kernel = 0;             // BWTC_D2H_KERNEL=1: result copies to pinned host buffers by a copying kernel (k_copy_out)
                                   // instead of the copy engine — measured no better (profiles/r02_experiments.md), kept as a knob
   int d2h_ctas = 16;
@@ -551,6 +552,7 @@ struct Job {
   // ---- phase A
   uint32_t N = 0, bstride = 0, blk_bits = 0;
   bool sentinel_outside_alphabet = false;
+  uint8_t last = 0;                // raw: T[N-1], the byte of the end-of-text row
   bool present[256];
   Round0Plan pl;
   const uint8_t* d_text = nullptr;
@@ -806,6 +808,7 @@ int64_t phase_input(bwtc_cuda_ctx* ctx, Job& J) {
     if (!J.present[0]) J.sentinel_outside_alphabet = true;
   } else {
     const uint8_t last = J.h_in[N - 1];
+    J.last = last;
     J.present[last] = true;
     count[last] += 1;
   }
@@ -1081,7 +1084,7 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
   const bool direct_out = bs ? (bs->on_device || is_pinned_host(bs->out[0]))
                              : (J.out_dev != nullptr || (J.block_mode && J.h_out && is_pinned_host(J.h_out)));
   // verification (DESIGN.md §3.10): the caller's host and batch outputs are written only after the check word is read
-  const bool verify = ctx->verify && J.block_mode && !ctx->debug_max_rounds;
+  const bool verify = ctx->verify && !ctx->debug_max_rounds;
   uint32_t* h_bLF = reinterpret_cast<uint32_t*>(ctx->h_batch + MAX_BATCH * sizeof(void*)) + MAX_BATCH * 256;
   auto enqueue_direct_out = [&]() -> int {
     if (bs) {
@@ -1445,10 +1448,12 @@ int64_t run_transform(bwtc_cuda_ctx* ctx, bool block_mode, const uint8_t* h_in, 
 // The device part of an inversion (one block, or a batch of them, ibwt_kernels.cuh InvShape): ev_begin, the keys and C
 // tables, the 2 digit passes, walk1, pointer jumping, walk2 into d_dst.  Adds its launches and algorithmic bytes to
 // ctx->stats; nothing is waited for.  A batch (bhist != nullptr) counts per-block histograms and gets per-block C tables.
-// Bit k of ctrl[CTR_INV_BAD..] ends up set for each block k that is not the BWT of any text.  timed = false: ev_begin /
-// ev_end are left to the caller (the verification of a forward transform).
+// Bit k of ctrl[CTR_INV_BAD..] ends up set for each block k that is not the BWT of any text.  verify (the verification of
+// a forward transform): the walk kernels' VERIFY variants, which also check the LFpowers rows at sh.d_eob and honour
+// sh.eot; ev_begin / ev_end are then left to the caller.
 int enqueue_inverse(bwtc_cuda_ctx* ctx, const InvShape& sh, bool block_mode, const uint8_t* d_src, uint8_t* d_dst,
-                    uint32_t* rounds_out, uint32_t* passes_out, bool timed = true) {
+                    uint32_t* rounds_out, uint32_t* passes_out, bool verify = false) {
+  const bool timed = !verify;
   cudaStream_t st = ctx->stream;
   bwtc_cuda_stats& S = ctx->stats;
   PassTimer pt{ctx};
@@ -1485,7 +1490,8 @@ int enqueue_inverse(bwtc_cuda_ctx* ctx, const InvShape& sh, bool block_mode, con
     nxtA = ctx->d_idx[cur ^ 1]; distA = nxtA + Sn; nxtB = ctx->d_scat; distB = nxtB + Sn; len = static_cast<uint32_t*>(ctx->d_keys[1]);
   }
   const dim3 wgrid(div_up(sh.S0, 256), B);
-  k_inv_walk1<<<wgrid, 256, 0, st>>>(vals, sh, nxtA, len, ctx->d_ctrl());
+  if (verify) k_inv_walk1<true><<<wgrid, 256, 0, st>>>(vals, sh, C, nxtA, len, ctx->d_ctrl());
+  else k_inv_walk1<false><<<wgrid, 256, 0, st>>>(vals, sh, C, nxtA, len, ctx->d_ctrl());
   CK(ctx, cudaMemcpyAsync(distA, len, (size_t)Sn * 4, cudaMemcpyDeviceToDevice, st));
   uint32_t* nin = nxtA; uint32_t* din = distA; uint32_t* nout = nxtB; uint32_t* dout = distB;
   uint32_t rounds = 0;
@@ -1496,7 +1502,8 @@ int enqueue_inverse(bwtc_cuda_ctx* ctx, const InvShape& sh, bool block_mode, con
     ++rounds;
   }
   // single-cycle check: per-block length sums and CTA counters in the gram histogram words (zeroed above, idle here)
-  k_inv_walk2<<<wgrid, 256, 0, st>>>(vals, len, din, nin, C, sh, d_dst, ctx->d_ctrl(), ctx->d_hist() + GRAM_OFF);
+  if (verify) k_inv_walk2<true><<<wgrid, 256, 0, st>>>(vals, len, din, nin, C, sh, d_dst, ctx->d_ctrl(), ctx->d_hist() + GRAM_OFF);
+  else k_inv_walk2<false><<<wgrid, 256, 0, st>>>(vals, len, din, nin, C, sh, d_dst, ctx->d_ctrl(), ctx->d_hist() + GRAM_OFF);
   CK(ctx, cudaGetLastError());
   S.kernel_launches += 2 + rounds;
   S.algorithmic_bytes += (uint64_t)N * (4 + 4 + 1) + (uint64_t)Sn * (16 * (rounds + 1) + 4);
@@ -1583,9 +1590,11 @@ int64_t run_inverse(bwtc_cuda_ctx* ctx, bool block_mode, const uint8_t* h_in, ui
   return (int64_t)n;
 }
 
-// Verification of a finished block-contract forward transform (DESIGN.md §3.10): its device-resident output (J.d_dst, a
-// batch at stride n0 + 1) is inverted into d_aux[1] — end-of-block rows read from d_LF on the device — and compared with
-// the input, which d_text still holds reversed.  One host wait.  On failure an in-place device block is rewritten from
+// Verification of a finished forward transform (DESIGN.md §3.10): its device-resident output (J.d_dst, a batch at stride
+// n0 + 1) is inverted into d_aux[1] — end-of-block rows read from d_LF on the device, every LFpowers entry checked against
+// the rows the walk visits — and compared with the input, which d_text still holds reversed (block contract) or as it is
+// (raw: T itself, whose restored N-1 bytes walk 2 writes reversed).  A raw text is one block whose end-of-text row has the
+// key c = T[N-1] (ibwt_kernels.cuh k_inv_keys).  One host wait.  On failure an in-place device block is rewritten from
 // d_text and BWTC_CUDA_EVERIFY is returned; nothing else of the caller's has been written yet.
 int verify_forward(bwtc_cuda_ctx* ctx, const Job& J) {
   cudaStream_t st = ctx->stream;
@@ -1600,14 +1609,23 @@ int verify_forward(bwtc_cuda_ctx* ctx, const Job& J) {
   sh.S0 = div_up(sh.R, INV_K);
   sh.S_last = div_up(sh.N_last, INV_K);
   sh.d_eob = ctx->d_LF;
+  sh.eot[0] = J.block_mode ? 0 : J.last;
+  sh.nLF = J.nLF;
+  sh.nLF_last = bs ? bs->nLF_last : J.nLF;
   if (ctx->debug_corrupt_out) {
-    k_debug_flip_byte<<<1, 1, 0, st>>>(J.d_dst + sh.n0 / 2);
+    if (J.block_mode) k_debug_flip_byte<<<1, 1, 0, st>>>(J.d_dst + sh.n0 / 2);
+    else k_debug_flip_raw<<<1, 1, 0, st>>>(J.d_dst, J.N / 2, J.N, ctx->d_LF);
+    CK(ctx, cudaGetLastError());
+    S.kernel_launches++;
+  }
+  if (ctx->debug_corrupt_lf) {
+    k_debug_corrupt_lf<<<1, MAX_BATCH, 0, st>>>(ctx->d_LF, ctx->debug_corrupt_lf, sh.nblocks, sh.nLF, sh.nLF_last);
     CK(ctx, cudaGetLastError());
     S.kernel_launches++;
   }
   for (;;) {
     uint32_t rounds = 0, pdone = 0;
-    if (const int rc = enqueue_inverse(ctx, sh, true, J.d_dst, ctx->d_aux[1], &rounds, &pdone, false)) return rc;
+    if (const int rc = enqueue_inverse(ctx, sh, J.block_mode, J.d_dst, ctx->d_aux[1], &rounds, &pdone, true)) return rc;
     const dim3 vgrid(std::max<uint32_t>(1u, div_up((uint32_t)ctx->sm_count * 8u, sh.nblocks)), sh.nblocks);
     k_inv_verify<<<vgrid, 256, 0, st>>>(ctx->d_aux[1], J.d_text, sh, ctx->d_ctrl());
     CK(ctx, cudaGetLastError());
@@ -1626,7 +1644,7 @@ int verify_forward(bwtc_cuda_ctx* ctx, const Job& J) {
   S.flags |= 64u;
   const uint64_t mask = (uint64_t)ctx->h_ctrl()[CTR_INV_BAD] | ((uint64_t)ctx->h_ctrl()[CTR_INV_BAD + 1] << 32);
   if (!mask) return 0;
-  if (!bs && J.out_dev && J.out_dev == J.in_dev) {
+  if (!bs && J.block_mode && J.out_dev && J.out_dev == J.in_dev) {
     k_text_unreverse<<<ctx->sm_count * 4, 256, 0, st>>>(J.d_text, J.n, J.out_dev);
     CK(ctx, cudaGetLastError());
     S.kernel_launches++;
@@ -1860,7 +1878,9 @@ int bwtc_cuda_ctx_create(bwtc_cuda_ctx** out, int device, uint32_t max_block_byt
   if (const char* e = getenv("BWTC_STATIC_TILES")) c->static_tiles = atoi(e);
   if (const char* e = getenv("BWTC_DEBUG_FAKE_WATCHDOG")) c->debug_fake_watchdog = atoi(e);
   if (const char* e = getenv("BWTC_DEBUG_REVERSE_TILES")) c->debug_reverse_tiles = atoi(e);
+  if (const char* e = getenv("BWTC_VERIFY")) c->verify = atoi(e) ? 1 : 0;
   if (const char* e = getenv("BWTC_DEBUG_CORRUPT_OUT")) c->debug_corrupt_out = atoi(e);
+  if (const char* e = getenv("BWTC_DEBUG_CORRUPT_LF")) c->debug_corrupt_lf = (uint32_t)std::max(0, atoi(e));
   if (const char* e = getenv("BWTC_DEBUG_SKIP_COPIES")) c->debug_skip_copies = atoi(e);
   if (const char* e = getenv("BWTC_D2H_KERNEL")) c->d2h_kernel = atoi(e);
   if (const char* e = getenv("BWTC_D2H_CTAS")) c->d2h_ctas = std::max(1, atoi(e));

@@ -7,8 +7,8 @@
 // (FastInverseBWTransform, InverseBWT.cpp:58-115) — one dependent random access per byte, inherently serial; its MTL-SA
 // variant runs a handful of such chains (the LFpowers starting points) on CPU threads.  A GPU needs ~10^5 independent
 // chains, so the starting points are made on the device instead:
-//   1. k_inv_keys     key[r] = L[r] + 1 (0 for the sentinel row), 9 significant bits (+ the block number of a batch
-//                     above them), + both digit histograms
+//   1. k_inv_keys     key[r] = L[r] + 1 (0 for the sentinel row; a raw text's last byte c in general, see below),
+//                     9 significant bits (+ the block number of a batch above them), + both digit histograms
 //   2. k_radix_pass   x 2 (the forward path's one-sweep LSD pass, stable): Psi[g] = the L-row of F-row g, i.e. the
 //                     rank of the suffix that starts one position LATER in T' — walking Psi walks T' forwards
 //   3. k_inv_ctable   C[c] = number of key values < c (F[g] is recovered by a search in C, no F array in memory)
@@ -18,7 +18,8 @@
 //   6. k_inv_walk2    each splitter walks its stretch again and writes X[n-1-q] = F[rank(q)] for its text positions q;
 //                     it also decides whether L is the BWT of any text at all (Psi one cycle, DESIGN.md §3.7)
 // Two passes of N dependent-per-chain but mutually independent random reads with ~N/K chains in flight: bound by the
-// L2/DRAM random-access rate, not by latency.  LFpowers[1..] are not needed (the device makes far denser samples).
+// L2/DRAM random-access rate, not by latency.  LFpowers[1..] are not needed (the device makes far denser samples); the
+// verification of a forward transform (walk kernels with VERIFY) checks them against the rows the walk visits.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -54,12 +55,17 @@ struct InvShape {
   uint32_t S_last;   // ... and of the last block
   uint32_t eob[INV_MAX_BLOCKS];  // per block: the end-of-block row (LFpowers[0]) ...
   const uint32_t* d_eob;         // ... or, if not null, read on the device from d_eob[256 k] (a forward transform's LFpowers rows)
+  uint8_t eot[INV_MAX_BLOCKS] = {};  // per block: the byte c of its end-of-text row (0 except when a raw forward is verified)
+  uint32_t nLF = 1, nLF_last = 1;    // verification only: LFpowers per full block / in the last block, in the d_eob rows
 };
 __device__ __forceinline__ uint32_t inv_eob(const InvShape& sh, uint32_t k) { return sh.d_eob ? sh.d_eob[256u * k] : sh.eob[k]; }
 __host__ __device__ __forceinline__ uint32_t inv_rows(const InvShape& sh) { return (sh.nblocks - 1u) * sh.R + sh.N_last; }
 __host__ __device__ __forceinline__ uint32_t inv_splitters(const InvShape& sh) { return (sh.nblocks - 1u) * sh.S0 + sh.S_last; }
 
-// key[r] = L[r] + 1, 0 at the sentinel row, block number k (= blockIdx.y) above bit 9.  Row N_k-1 holds, in the block
+// key[r] = L[r] + [L[r] >= c], c at the end-of-text row eob, block number k (= blockIdx.y) above bit 9; c = sh.eot[k] is
+// the text's last byte, 0 for a sentinel-terminated text (key = L + 1, 0 at eob).  The value c belongs to the eob row alone,
+// rows with L < c keep their bucket, rows with L >= c move up by the one F entry of the last suffix: the stable sort puts
+// every row at its F-row, the eob row at C[c], the row of suffix N_k - 1 (DESIGN.md §3.10).  Row N_k-1 holds, in the block
 // contract, the byte the forward transform moved into the hole (out[eob] = L[N-1], BWTransform.cpp:60); in the raw
 // contract (single block only) in[N-1] itself.
 // hist[0..255] = histogram of key & 0xFF (all blocks), hist[256 + 2k + 1] = keys of block k with value 256 (byte 0xFF);
@@ -76,12 +82,15 @@ __global__ void __launch_bounds__(256) k_inv_keys(const uint8_t* __restrict__ in
   const uint32_t N = (k + 1u == sh.nblocks) ? sh.N_last : sh.R, eob = inv_eob(sh, k);
   const uint8_t* __restrict__ ink = in + (size_t)k * sh.istride;
   uint32_t* __restrict__ kk = keys + (size_t)k * sh.R;
-  const uint32_t top = k << 9;
+  const uint32_t top = k << 9, c = sh.eot[k];
   for (uint32_t r = blockIdx.x * blockDim.x + threadIdx.x; r < N; r += gridDim.x * blockDim.x) {
     uint32_t key;
-    if (r == eob) key = 0;
-    else if (r == N - 1u && block_mode) key = (uint32_t)ink[eob] + 1u;
-    else key = (uint32_t)ink[r] + 1u;
+    if (r == eob) {
+      key = c;
+    } else {
+      key = (r == N - 1u && block_mode) ? (uint32_t)ink[eob] : (uint32_t)ink[r];
+      key += key >= c ? 1u : 0u;
+    }
     kk[r] = top | key;
     atomicAdd(&s_lo[key & 0xFFu], 1u);
     if (key >> 8) atomicAdd(&s_hi, 1u);
@@ -126,22 +135,37 @@ __device__ __forceinline__ uint32_t inv_psi(const uint32_t* __restrict__ vals, u
   return iota_top - vals[g];
 }
 
-// Grid (ceil(S0 / 256), B).  Splitter j of block k = local row j*K, global index k S0 + j.  Follow Psi until the next
-// splitter of the block: nxt = its index, len = steps taken (>= 1).  The splitter whose successor is the block's splitter 0
-// gets nxt = INV_NIL: each block's cycle is opened at its own rank 0 (= suffix N_k - 1).
+// Splitter rows are counted from the block's anchor a, the F-row of suffix N_k - 1: local row (a + j K) mod N_k is splitter
+// j.  The plain inverse has a = 0 (c = 0: the eob row sorts first); a verified forward (VERIFY) reads a = C[k][c] - k R.
+template <bool VERIFY>
+__device__ __forceinline__ uint32_t inv_anchor(const uint32_t* C, const InvShape& sh, uint32_t k) {
+  return VERIFY ? C[(size_t)k * 258 + sh.eot[k]] - k * sh.R : 0u;
+}
+// local row x -> its distance from the anchor (mod N)
+template <bool VERIFY>
+__device__ __forceinline__ uint32_t inv_from_anchor(uint32_t x, uint32_t a, uint32_t N) {
+  return VERIFY ? (x >= a ? x - a : x + N - a) : x;
+}
+
+// Grid (ceil(S0 / 256), B).  Splitter j of block k = local row (a + j K) mod N_k, global index k S0 + j.  Follow Psi until
+// the next splitter of the block: nxt = its index, len = steps taken (>= 1).  The splitter whose successor is the block's
+// splitter 0 gets nxt = INV_NIL: each block's cycle is opened at its anchor (= suffix N_k - 1).
+template <bool VERIFY>
 __global__ void __launch_bounds__(256) k_inv_walk1(const uint32_t* __restrict__ vals, const InvShape sh,
-                                                   uint32_t* __restrict__ nxt, uint32_t* __restrict__ len,
-                                                   const uint32_t* __restrict__ ctrl) {
+                                                   const uint32_t* __restrict__ C, uint32_t* __restrict__ nxt,
+                                                   uint32_t* __restrict__ len, const uint32_t* __restrict__ ctrl) {
   const uint32_t k = blockIdx.y, j = blockIdx.x * blockDim.x + threadIdx.x;
   const bool last = k + 1u == sh.nblocks;
   if (j >= (last ? sh.S_last : sh.S0) || ctrl[0]) return;  // ctrl[CTR_ERR]: a digit pass failed, Psi is not trustworthy
   const uint32_t N = last ? sh.N_last : sh.R, base = k * sh.R, top = inv_rows(sh) - 1u;
-  uint32_t g = base + j * INV_K, t = 0;
+  const uint32_t a = inv_anchor<VERIFY>(C, sh, k);
+  uint32_t g = base + (VERIFY ? (a + j * INV_K) % N : j * INV_K), t = 0, x;
   do {
     g = inv_psi(vals, top, g);
     ++t;
-  } while ((g - base) % INV_K != 0u && t < N);
-  const uint32_t to = (g - base) / INV_K;
+    x = inv_from_anchor<VERIFY>(g - base, a, N);
+  } while (x % INV_K != 0u && t < N);
+  const uint32_t to = x / INV_K;
   const uint32_t s = k * sh.S0 + j;
   nxt[s] = (to == 0u) ? INV_NIL : k * sh.S0 + to;
   len[s] = t;
@@ -174,6 +198,10 @@ __global__ void __launch_bounds__(256) k_inv_jump(const uint32_t* __restrict__ n
 //       other cycle a chain never reaches NIL).
 // Each CTA adds its part of the sum to chk[k] (chk: [2B] zeroed words; chk[B + k] counts the CTAs of block k that are done)
 // and the last CTA of the block compares; a failed test sets bit k of ctrl[CTR_INV_BAD..].  The output is written anyway.
+// VERIFY (a forward transform's output): splitters counted from the anchor, F recovered as byte(v) = v - [v > c], and the
+// starting points checked — at text position q = N_k - j x (x = floor(N_k / nLF_k), 1 <= j < nLF_k) the row must be
+// LFpowers_k[j] (d_eob[256 k + j]); a difference sets bit k like a corrupt block.
+template <bool VERIFY>
 __global__ void __launch_bounds__(256) k_inv_walk2(const uint32_t* __restrict__ vals, const uint32_t* __restrict__ len,
                                                    const uint32_t* __restrict__ dist, const uint32_t* __restrict__ nxt,
                                                    const uint32_t* __restrict__ C, const InvShape sh, uint8_t* __restrict__ out,
@@ -209,9 +237,18 @@ __global__ void __launch_bounds__(256) k_inv_walk2(const uint32_t* __restrict__ 
   }
   if (!active) return;
   uint8_t* __restrict__ outk = out + (size_t)k * sh.n0;
-  uint32_t g = k * sh.R + j * INV_K;
+  const uint32_t base = k * sh.R;
+  uint32_t g = base + (VERIFY ? (s_C[sh.eot[k]] - base + j * INV_K) % N : j * INV_K);  // (s_C: block k's C table)
   uint32_t q = (uint32_t)((2ull * N - 1ull - (unsigned long long)dist[s]) % N);
+  // VERIFY: the next sampled position is where d = N - q reaches a multiple of x; jj = d / x, rem = d % x, kept per step
+  const uint32_t c = VERIFY ? sh.eot[k] : 0u;
+  const uint32_t nl = VERIFY ? (last ? sh.nLF_last : sh.nLF) : 1u, x = VERIFY ? N / nl : 1u;
+  const uint32_t* __restrict__ LFk = VERIFY ? sh.d_eob + 256u * k : nullptr;
+  uint32_t jj = 0, rem = 0;
+  bool lf_bad = false;
+  if (VERIFY) { jj = (N - q) / x; rem = (N - q) % x; }
   for (uint32_t t = 0; t < L; ++t) {
+    if (VERIFY && rem == 0u && jj >= 1u && jj < nl) lf_bad |= g - base != LFk[jj];
     if (q < n) {
       // F[g]: the largest key value v with C[v] <= g (binary search over the 257 bucket starts)
       uint32_t lo = 0, hi = 256;
@@ -219,11 +256,17 @@ __global__ void __launch_bounds__(256) k_inv_walk2(const uint32_t* __restrict__ 
         const uint32_t mid = (lo + hi + 1u) >> 1;
         if (s_C[mid] <= g) lo = mid; else hi = mid - 1u;
       }
-      outk[n - 1u - q] = (uint8_t)(lo - 1u);
+      outk[n - 1u - q] = (uint8_t)(VERIFY ? lo - (lo > c ? 1u : 0u) : lo - 1u);
     }
     g = inv_psi(vals, top, g);
     q = (q + 1u == N) ? 0u : q + 1u;
+    if (VERIFY) {
+      if (q == 0u) { jj = N / x; rem = N % x; }
+      else if (rem == 0u) { --jj; rem = x - 1u; }
+      else --rem;
+    }
   }
+  if (VERIFY && lf_bad) inv_mark_bad(ctrl, k);
 }
 
 // ---- verification of a forward transform (DESIGN.md §3.10).  Grid (x, B).  Block k restored into rest + k n0 must equal
@@ -248,6 +291,16 @@ __global__ void __launch_bounds__(256) k_text_unreverse(const uint8_t* __restric
 
 // Test hook BWTC_DEBUG_CORRUPT_OUT: one byte of the forward output changed before it is verified.
 __global__ void k_debug_flip_byte(uint8_t* p) { *p ^= 1u; }
+// ... of a raw output: row i, or the next row if i is pidx (= LF[0]; the inverse ignores U[pidx], a change there is no error)
+__global__ void k_debug_flip_raw(uint8_t* out, uint32_t i, uint32_t N, const uint32_t* __restrict__ LF) {
+  if (LF[0] == i) i = (i + 1u) % N;
+  out[i] ^= 1u;
+}
+// Test hook BWTC_DEBUG_CORRUPT_LF=j: LFpowers[j] of every block that has one changed before the forward output is verified.
+__global__ void k_debug_corrupt_lf(uint32_t* LF, uint32_t j, uint32_t nblocks, uint32_t nLF, uint32_t nLF_last) {
+  const uint32_t k = threadIdx.x;
+  if (k < nblocks && j >= 1u && j < (k + 1u == nblocks ? nLF_last : nLF)) LF[256u * k + j] ^= 1u;
+}
 
 // =====================================================================================================
 // Run statistics of the transformed block (SURVEY.md §8f row f3; the reference's own TODO at HuffmanCoders.cpp:54:

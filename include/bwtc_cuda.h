@@ -81,8 +81,9 @@ typedef struct bwtc_cuda_stats {
   float    sort0_ms;                        /* device time inside the round-0 passes (detailed timing on) */
   uint32_t flags;            /* bit 0: look-back kernels ran with ticket counters (watchdog fallback or BWTC_STATIC_TILES=0);
                               * bit 1: the blocks of a batch were sorted as one text; bit 2: predecessor codes packed above the ids;
-                              * bit 3: ... carried as a one-byte payload array; bit 6: the forward output was verified by a
-                              * device-side inversion (bwtc_cuda_ctx_set_verify); bit 7: inverse only, this block is corrupt
+                              * bit 3: ... carried as a one-byte payload array; bit 6: the forward output (block or raw
+                              * contract) and its LFpowers were verified by a device-side inversion (bwtc_cuda_ctx_set_verify,
+                              * BWTC_VERIFY); bit 7: inverse only, this block is corrupt
                               * (BWTC_CUDA_ECORRUPT) */
   uint32_t batch_blocks;     /* blocks this record describes: 1, or the size of the batch that was sorted as one text (every
                               * block of the batch then carries the SAME record — count it once; flags bit 7 is the one field
@@ -110,15 +111,19 @@ int         bwtc_cuda_ctx_set_round0(bwtc_cuda_ctx* ctx, uint32_t chars, uint32_
 /* detail != 0: bracket every radix digit pass with CUDA events on the context's stream so that
  * stats.sort_ms / sort_bytes / sort_launches give the dominant kernel's average launch duration. */
 int         bwtc_cuda_ctx_set_timing(bwtc_cuda_ctx* ctx, int detail);
-/* on != 0: every block-contract forward call (bwtc_cuda_bwt_block, _device, _runs, bwtc_cuda_bwt_blocks) is verified before
- * it returns: the device inverts its device-resident output (end-of-block rows from the device-side LFpowers, a batch as one
- * batched inversion) and compares the result with the input, which the device still holds reversed.  On a mismatch the call
- * returns BWTC_CUDA_EVERIFY and every caller buffer holds its input: host outputs, LFpowers and freqs are written only after
- * the host has read the check word, and an in-place device block is rewritten from the device copy (a device output that
- * does not alias its input, and the run arrays of bwtc_cuda_bwt_block_runs, are then unspecified).  Costs about one inverse
- * transform and one host wait per call; stats.flags bit 6 marks a verified block, stats.gpu_ms includes the check.  The
- * raw contract (bwtc_cuda_divbwt / divbwtf) is never verified.  Off (0) by default; off, every call runs exactly the
- * kernels it runs without this switch.  The context stays usable after BWTC_CUDA_EVERIFY. */
+/* on != 0: every forward call (bwtc_cuda_bwt_block, _device, _runs, bwtc_cuda_bwt_blocks, and the raw bwtc_cuda_divbwt /
+ * divbwtf) is verified before it returns: the device inverts its device-resident output (end-of-block rows from the
+ * device-side LFpowers, a batch as one batched inversion, a raw text with its own last byte as the key of its end-of-text
+ * row) and compares the result with the input, which the device still holds; every LFpowers entry (LFpowers[j],
+ * 1 <= j < nLFpowers, of every block) is checked against the row the inversion visits at its text position.  On a mismatch
+ * the call returns BWTC_CUDA_EVERIFY and every caller buffer holds its input: host outputs (a raw U, aliasing T or not),
+ * LFpowers and freqs are written only after the host has read the check word, and an in-place device block is rewritten
+ * from the device copy (a device output that does not alias its input, and the run arrays of bwtc_cuda_bwt_block_runs,
+ * are then unspecified).  Costs about one inverse transform and one host wait per call; stats.flags bit 6 marks a verified
+ * block, stats.gpu_ms includes the check.  Raw texts of n <= 1 bytes return early, unverified.  Off (0) by default; the
+ * environment variable BWTC_VERIFY=1, read when a context is created, makes on the initial value of every context (and
+ * so of every pipeline and host-side class), which this call still overrides per context.  Off, every call runs exactly
+ * the kernels it runs without this switch.  The context stays usable after BWTC_CUDA_EVERIFY. */
 int         bwtc_cuda_ctx_set_verify(bwtc_cuda_ctx* ctx, int on);
 /* Debug / test hooks: max_rounds != 0 stops the refinement after that many sort rounds (the output is
  * then deliberately incomplete); bwtc_cuda_debug_read copies an engine buffer to the host
@@ -215,7 +220,8 @@ void bwtc_cuda_pipeline_destroy(bwtc_cuda_pipeline* p);
 const char* bwtc_cuda_pipeline_error(const bwtc_cuda_pipeline* p);
 int  bwtc_cuda_pipeline_set_round0(bwtc_cuda_pipeline* p, uint32_t chars, uint32_t key_bytes);
 int  bwtc_cuda_pipeline_set_timing(bwtc_cuda_pipeline* p, int detail);
-/* bwtc_cuda_ctx_set_verify on every context of the pipeline: forward blocks (run, submit, submit_runs) are verified. */
+/* bwtc_cuda_ctx_set_verify on every context of the pipeline: forward blocks (run, submit, submit_runs) are verified.
+ * Its contexts start from BWTC_VERIFY like any other. */
 int  bwtc_cuda_pipeline_set_verify(bwtc_cuda_pipeline* p, int on);
 /* Transforms nblocks blocks.  in[i]/out[i]: sizes[i] bytes each (may alias; host memory, or device
  * memory when on_device != 0).  LFpowers: nblocks x 256 uint32 (row i gets nLF[i] entries, where
