@@ -32,6 +32,7 @@ ECORRUPT = -6                     # BWTC_CUDA_ECORRUPT: an inverse input that is
 EVERIFY = -7                      # BWTC_CUDA_EVERIFY: a verified forward output did not restore its input
 FLAG_VERIFIED = 1 << 6            # stats flags bit 6: the forward output was verified on the device
 FLAG_CORRUPT = 1 << 7             # stats flags bit 7: this inverse block is corrupt
+FLAG_SA = 1 << 8                  # stats flags bit 8: this call produced a suffix array (divsufsort)
 
 
 class BwtcCudaUnavailable(RuntimeError):
@@ -117,6 +118,9 @@ C_ABI = [
     ("bwtc_cuda_debug_read", ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_uint64, _vp, ctypes.c_uint64]),
     ("bwtc_cuda_divbwtf", ctypes.c_int64, [_vp, _vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp]),
     ("bwtc_cuda_divbwt", ctypes.c_int64, [_vp, _vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32]),
+    ("bwtc_cuda_divsufsort", ctypes.c_int, [_vp, _vp, _vp, ctypes.c_uint32]),
+    ("bwtc_cuda_divsufsort_device", ctypes.c_int, [_vp, _vp, _vp, ctypes.c_uint32]),
+    ("bwtc_cuda_sufcheck", ctypes.c_int, [_vp, _vp, _vp, ctypes.c_uint32]),
     ("bwtc_cuda_bwt_block", ctypes.c_int64, [_vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp]),
     ("bwtc_cuda_bwt_block_device", ctypes.c_int64, [_vp, _vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp]),
     ("bwtc_cuda_bwt_block_runs", ctypes.c_int64, [_vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp, _vp]),
@@ -240,6 +244,35 @@ class CudaContext:
         assert T.dtype == np.uint8 and U.dtype == np.uint8 and LFpowers.dtype == np.uint32
         return self._check(self._lib.bwtc_cuda_divbwtf(self._h, T.ctypes.data, U.ctypes.data, T.size,
                                                         LFpowers.ctypes.data, LFpowers.size, _ptr(freqs)))
+
+    def last_error(self) -> str:
+        return self._lib.bwtc_cuda_last_error(self._h).decode()
+
+    # suffix array of a raw text: libdivsufsort's divsufsort(T, SA, n) / sufcheck(T, SA, n, verbose)
+    def divsufsort(self, T: np.ndarray, SA: Optional[np.ndarray] = None) -> np.ndarray:
+        """The suffix array of T (uint8) under the raw contract's order: int32[T.size], or written into SA (int32,
+        pageable or pinned) when given.  Raises BwtcCudaError on failure (EVERIFY with verification on: SA untouched)."""
+        assert T.dtype == np.uint8 and T.flags.c_contiguous
+        if SA is None:
+            SA = np.empty(T.size, dtype=np.int32)
+        assert SA.dtype == np.int32 and SA.size >= T.size and SA.flags.c_contiguous
+        self._check(self._lib.bwtc_cuda_divsufsort(self._h, T.ctypes.data, SA.ctypes.data, T.size))
+        return SA
+
+    def divsufsort_device(self, d_T: int, d_SA: int, n: int) -> None:
+        """divsufsort with T (n bytes) and SA (n int32, 4-byte aligned) in device memory (e.g. torch data_ptr())."""
+        self._check(self._lib.bwtc_cuda_divsufsort_device(self._h, d_T, d_SA, n))
+
+    def sufcheck(self, T: np.ndarray, SA: np.ndarray) -> bool:
+        """True if SA (int32) is the suffix array of T (uint8); False if not (last_error() names the first offending row).
+        Other failures raise BwtcCudaError."""
+        assert T.dtype == np.uint8 and SA.dtype == np.int32 and SA.size == T.size
+        assert T.flags.c_contiguous and SA.flags.c_contiguous
+        rc = self._lib.bwtc_cuda_sufcheck(self._h, T.ctypes.data, SA.ctypes.data, T.size)
+        if rc == ECORRUPT:
+            return False
+        self._check(rc)
+        return True
 
     # block contract: BWTransform::doTransform(BWTBlock&, freqs) — BWTransform.cpp:52-64
     def bwt_block(self, block: np.ndarray, LFpowers: np.ndarray, freqs: Optional[np.ndarray]) -> int:

@@ -108,6 +108,8 @@ struct bwtc_cuda_ctx {
   unsigned long long* d_wtab = nullptr;  // window-sample table: WS_SLOTS keys, WS_SLOTS counters, 2 doubles
   uint32_t* d_bhist = nullptr;    // [MAX_BATCH][256] per-block byte histograms of a batch
   const uint8_t** d_bptr = nullptr;  // [MAX_BATCH] device pointers to the blocks of a batch
+  int32_t* d_sa = nullptr;        // suffix array of bwtc_cuda_divsufsort (host variant): 4 (cap + 1) bytes, allocated by its
+                                  // first call, not counted by bwtc_cuda_scratch_bytes
   // ---- pinned host memory
   uint32_t* h_small = nullptr;    // [ctrl CTR_WORDS][hist HIST_WORDS][LF 256 + pair statistics]
   uint8_t* h_batch = nullptr;     // [MAX_BATCH] pointers, [MAX_BATCH][256] histograms, [MAX_BATCH][256] LFpowers
@@ -125,6 +127,7 @@ struct bwtc_cuda_ctx {
   int verify = 0;                 // forward outputs are inverted on the device and compared (DESIGN.md §3.10); BWTC_VERIFY
   int debug_corrupt_out = 0;      // test hook: one byte of the forward output is changed before it is verified
   uint32_t debug_corrupt_lf = 0;  // test hook (j >= 1): LFpowers[j] is changed on the device before it is verified
+  int64_t debug_corrupt_sa = -1;  // test hook (r >= 0): SA[r] and SA[r+1] are swapped on the device before they are verified
   int d2h_kernel = 0;             // BWTC_D2H_KERNEL=1: result copies to pinned host buffers by a copying kernel (k_copy_out)
                                   // instead of the copy engine — measured no better (profiles/r02_experiments.md), kept as a knob
   int d2h_ctas = 16;
@@ -195,7 +198,7 @@ void ctx_free(bwtc_cuda_ctx* c) {
   cudaFree(c->d_keys[0]); cudaFree(c->d_keys[1]); cudaFree(c->d_idx[0]); cudaFree(c->d_idx[1]);
   cudaFree(c->d_zero); cudaFree(c->d_status); cudaFree(c->d_LF); cudaFree(c->d_wtab); cudaFree(c->d_tilecnt); cudaFree(c->d_scat);
   cudaFree(c->d_bhist); cudaFree(c->d_bptr); cudaFree(c->d_aux[0]); cudaFree(c->d_aux[1]);
-  cudaFree(c->d_state); cudaFree(c->d_livebits); cudaFree(c->d_ktab); cudaFree(c->d_lookup);
+  cudaFree(c->d_state); cudaFree(c->d_livebits); cudaFree(c->d_ktab); cudaFree(c->d_lookup); cudaFree(c->d_sa);
   if (c->h_lookup) cudaFreeHost(c->h_lookup);
   if (c->h_batch) cudaFreeHost(c->h_batch);
   if (c->h_small) cudaFreeHost(c->h_small);
@@ -461,6 +464,16 @@ int launch_rerank(bwtc_cuda_ctx* ctx, int cur, uint32_t m, uint32_t N, RerankPar
   const uint32_t nwin = single_window ? 1u : rerank_windows(ctx, N, m);
   const KeyT* keys = static_cast<const KeyT*>(ctx->d_keys[cur]);
   uint32_t* woff = ctx->d_tilecnt + 2 * ctx->max_aux_tiles;
+  // (ep.sa: the instantiation that also writes the suffix array)
+  auto rerank = [&](unsigned long long* tstate, const StageParams& sp) {
+    if (ROUND0 && rp.lazy) {
+      if (ep.sa) k_rerank<KeyT, ROUND0, ROUND0, true><<<tiles, 256, 0, st>>>(keys, ctx->d_idx[cur], ctx->d_rank, rp, tstate, ctx->d_ctrl(), ep, sp);
+      else k_rerank<KeyT, ROUND0, ROUND0><<<tiles, 256, 0, st>>>(keys, ctx->d_idx[cur], ctx->d_rank, rp, tstate, ctx->d_ctrl(), ep, sp);
+    } else {
+      if (ep.sa) k_rerank<KeyT, ROUND0, false, true><<<tiles, 256, 0, st>>>(keys, ctx->d_idx[cur], ctx->d_rank, rp, tstate, ctx->d_ctrl(), ep, sp);
+      else k_rerank<KeyT, ROUND0><<<tiles, 256, 0, st>>>(keys, ctx->d_idx[cur], ctx->d_rank, rp, tstate, ctx->d_ctrl(), ep, sp);
+    }
+  };
   const bool hybrid2 = ctx->hybrid2 && nwin == 2u && !(ROUND0 && rp.lazy);
   if ((ctx->bucket_min_windows && nwin >= (uint32_t)ctx->bucket_min_windows) || hybrid2) {
     const uint32_t win_ids = div_up(N, nwin);
@@ -474,10 +487,7 @@ int launch_rerank(bwtc_cuda_ctx* ctx, int cur, uint32_t m, uint32_t N, RerankPar
     rp.direct0 = hybrid2 ? 1u : 0u;
     rp.bucket_magic = (uint32_t)(((1ull << 32) + win_ids - 1) / win_ids);
     StageParams sp{stage_nr, stage_id, ctx->d_tilecnt, no_stage ? 0 : 1, ctx->d_idx[cur ^ 1], ctx->d_scat, woff};
-    if (ROUND0 && rp.lazy)
-      k_rerank<KeyT, ROUND0, ROUND0><<<tiles, 256, 0, st>>>(keys, ctx->d_idx[cur], ctx->d_rank, rp, ctx->d_tstate(), ctx->d_ctrl(), ep, sp);
-    else
-      k_rerank<KeyT, ROUND0><<<tiles, 256, 0, st>>>(keys, ctx->d_idx[cur], ctx->d_rank, rp, ctx->d_tstate(), ctx->d_ctrl(), ep, sp);
+    rerank(ctx->d_tstate(), sp);
     const uint32_t grid = std::min<uint32_t>(div_up(tiles, 8), (uint32_t)ctx->sm_count * 8u);
     for (uint32_t b = hybrid2 ? 1u : 0u; b < nwin; ++b)
       k_scatter_bucket<<<grid, 256, 0, st>>>(ctx->d_idx[cur ^ 1], ctx->d_scat, woff, tiles, nwin, b, AUX_TILE, ctx->d_rank, ctx->d_ctrl());
@@ -511,12 +521,7 @@ int launch_rerank(bwtc_cuda_ctx* ctx, int cur, uint32_t m, uint32_t N, RerankPar
     rp.direct0 = 0;
     rp.bucket_magic = 0;
     StageParams sp{stage_nr, stage_id, ctx->d_tilecnt, (w == 0 && !no_stage) ? 1 : 0, nullptr, nullptr, nullptr};
-    if (ROUND0 && rp.lazy)
-      k_rerank<KeyT, ROUND0, ROUND0><<<tiles, 256, 0, st>>>(keys, ctx->d_idx[cur], ctx->d_rank, rp,
-                                                            ctx->d_tstate() + (size_t)w * ctx->max_aux_tiles, ctx->d_ctrl(), ep, sp);
-    else
-      k_rerank<KeyT, ROUND0><<<tiles, 256, 0, st>>>(keys, ctx->d_idx[cur], ctx->d_rank, rp,
-                                                     ctx->d_tstate() + (size_t)w * ctx->max_aux_tiles, ctx->d_ctrl(), ep, sp);
+    rerank(ctx->d_tstate() + (size_t)w * ctx->max_aux_tiles, sp);
     CK(ctx, cudaGetLastError());
     ctx->stats.kernel_launches++;
   }
@@ -549,6 +554,8 @@ struct Job {
   uint32_t* freqs = nullptr;
   const BatchSpec* bs = nullptr;   // batch of blocks (block contract): the fields above come from *bs
   bwtc_cuda_runs* runs = nullptr;  // run statistics wanted (single block, block contract)
+  int32_t* sa = nullptr;           // raw contract: the suffix array is emitted here (device; bwtc_cuda_divsufsort) ...
+  int32_t* h_sa = nullptr;         // ... and copied to this host array once the block is finished (and verified)
   // ---- phase A
   uint32_t N = 0, bstride = 0, blk_bits = 0;
   bool sentinel_outside_alphabet = false;
@@ -784,6 +791,8 @@ int64_t phase_input(bwtc_cuda_ctx* ctx, Job& J) {
   }
   if (bs) CK(ctx, cudaMemcpyAsync(h_bhist, ctx->d_bhist, (size_t)bs->nblocks * 256 * 4, cudaMemcpyDeviceToHost, st));
   else CK(ctx, cudaMemcpyAsync(ctx->h_hist(), ctx->d_hist(), 256 * 4, cudaMemcpyDeviceToHost, st));
+  uint8_t* h_last = reinterpret_cast<uint8_t*>(ctx->h_LF() + 260);  // (behind the 16 bytes of pair statistics)
+  if (!J.block_mode && !J.h_in) CK(ctx, cudaMemcpyAsync(h_last, d_src + (N - 1), 1, cudaMemcpyDeviceToHost, st));
   if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
 
   uint64_t count[256];
@@ -807,7 +816,7 @@ int64_t phase_input(bwtc_cuda_ctx* ctx, Job& J) {
   } else if (J.block_mode) {
     if (!J.present[0]) J.sentinel_outside_alphabet = true;
   } else {
-    const uint8_t last = J.h_in[N - 1];
+    const uint8_t last = J.h_in ? J.h_in[N - 1] : *h_last;
     J.last = last;
     J.present[last] = true;
     count[last] += 1;
@@ -823,6 +832,7 @@ int64_t phase_input(bwtc_cuda_ctx* ctx, Job& J) {
   J.ep.lastch = ctx->d_LF + LF_PARK;
   J.ep.N = N;
   J.ep.block_mode = J.block_mode ? 1 : 0;
+  J.ep.sa = J.sa;
   S.sigma = J.pl.sigma;
   S.bits_per_char = J.pl.bits;
   S.chars_round0 = J.pl.chars;
@@ -833,6 +843,7 @@ int64_t phase_input(bwtc_cuda_ctx* ctx, Job& J) {
 }
 
 int verify_forward(bwtc_cuda_ctx* ctx, const Job& J);
+int verify_sa(bwtc_cuda_ctx* ctx, const Job& J);
 
 // ---- phase B: round 0, the device-controlled ladder of sort-free rounds, host-driven global radix rounds where
 // groups are large, final extraction, result copies.  Works from ctx->d_text only, so it can be repeated (with ticket
@@ -1018,7 +1029,8 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
       memcpy(L.lut, pl.pp.lut, 256);
       CK(ctx, cudaMemcpyAsync(ctx->d_lookup, ctx->h_lookup, sizeof(LookupParams), cudaMemcpyHostToDevice, st));
     }
-    S.flags = (ctx->static_tiles ? 0u : 1u) | (bs ? 2u : 0u) | (pack_pred ? 4u : 0u) | (aux_pred ? 8u : 0u) | (lazy ? 16u : 0u);
+    S.flags = (ctx->static_tiles ? 0u : 1u) | (bs ? 2u : 0u) | (pack_pred ? 4u : 0u) | (aux_pred ? 8u : 0u) | (lazy ? 16u : 0u) |
+              (J.sa ? 256u : 0u);
     rp.packed = pack_pred ? 1u : (aux_pred ? 2u : 0u);
     rp.pred_aux = ctx->d_aux[cur];
     rp.id_bits = pack_pred ? id_bits : 31u;
@@ -1135,14 +1147,20 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
         // persistent grid; the first round behind a sort is the big one, later (often skipped) ones get a leaner grid
         const uint32_t per_sm = (k == 0) ? 12u : 4u;
         const uint32_t seg_grid = std::max<uint32_t>(1u, std::min<uint32_t>(div_up(m_bound, SEG_T), (uint32_t)ctx->sm_count * per_sm));
-        if (lkp) k_seg_round<true><<<seg_grid, 256, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), lkp);
-        else k_seg_round<false><<<seg_grid, 256, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), nullptr);
+        if (ep.sa) {
+          if (lkp) k_seg_round<true, true><<<seg_grid, 256, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), lkp);
+          else k_seg_round<false, true><<<seg_grid, 256, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), nullptr);
+        } else {
+          if (lkp) k_seg_round<true><<<seg_grid, 256, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), lkp);
+          else k_seg_round<false><<<seg_grid, 256, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), nullptr);
+        }
         k_apply_ranks<<<ctx->sm_count * 8, 256, 0, st>>>(ctx->d_state, pool, ctx->d_ctrl(), ctx->d_rank);
         k_commit_seg<<<1, 1, 0, st>>>(ctx->d_state, ctx->d_ctrl());
         S.kernel_launches += 3;
       }
       if (!dbg) {
-        k_small_rounds<<<1, 1024, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), lkp);
+        if (ep.sa) k_small_rounds<true><<<1, 1024, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), lkp);
+        else k_small_rounds<<<1, 1024, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), lkp);
         S.kernel_launches++;
       }
       CK(ctx, cudaGetLastError());
@@ -1344,12 +1362,20 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
     }
   }
   if (finished && verify) {
-    rc = verify_forward(ctx, J);
+    rc = J.sa ? verify_sa(ctx, J) : verify_forward(ctx, J);
     if (rc) return rc;
   }
   // ---- result copies that could not be enqueued speculatively
   if (finished) {
-    if (bs) {
+    if (J.sa) {
+      // the suffix array (its BWT bytes stay on the device): 4 bytes per suffix, direct from pinned memory, else staged
+      if (J.h_sa && is_pinned_host(J.h_sa)) {
+        CK(ctx, cudaMemcpyAsync(J.h_sa, J.sa, (size_t)N * 4, cudaMemcpyDeviceToHost, st));
+        if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
+      } else if (J.h_sa && download_staged(ctx, reinterpret_cast<uint8_t*>(J.h_sa), reinterpret_cast<const uint8_t*>(J.sa), (size_t)N * 4)) {
+        return BWTC_CUDA_ECUDA;
+      }
+    } else if (bs) {
       if (!out_enqueued || !direct_out) {
         if (direct_out) {
           if (enqueue_direct_out() || host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
@@ -1415,6 +1441,17 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
 // Phase A, phase B, and the fallback of the static tile ids (see k_radix_pass): if the look-back watchdog fired, the
 // context switches to ticket counters for good and repeats phase B.  The reversed, sentinel-terminated text is still
 // intact on the device, so this works for in-place device buffers too; nothing was written to LFpowers / freqs.
+int64_t run_job(bwtc_cuda_ctx* ctx, Job& J) {
+  int64_t rc = phase_input(ctx, J);
+  if (rc < 0) return rc;
+  rc = phase_sort(ctx, J);
+  if (rc == BWTC_CUDA_EINTERNAL && ctx->lb_watchdog && ctx->static_tiles) {
+    ctx->static_tiles = 0;
+    rc = phase_sort(ctx, J);
+  }
+  return rc;
+}
+
 int64_t run_transform(bwtc_cuda_ctx* ctx, bool block_mode, const uint8_t* h_in, uint8_t* h_out, const uint8_t* in_dev,
                       uint8_t* out_dev, uint32_t n, uint32_t* LF, uint32_t nLF, uint32_t* freqs,
                       const BatchSpec* bs = nullptr, bwtc_cuda_runs* runs = nullptr) {
@@ -1431,14 +1468,7 @@ int64_t run_transform(bwtc_cuda_ctx* ctx, bool block_mode, const uint8_t* h_in, 
   J.nLF = nLF;
   J.freqs = freqs;
   J.bs = bs;
-  int64_t rc = phase_input(ctx, J);
-  if (rc < 0) return rc;
-  rc = phase_sort(ctx, J);
-  if (rc == BWTC_CUDA_EINTERNAL && ctx->lb_watchdog && ctx->static_tiles) {
-    ctx->static_tiles = 0;
-    rc = phase_sort(ctx, J);
-  }
-  return rc;
+  return run_job(ctx, J);
 }
 
 // ---- inverse transform (SURVEY.md §8f row f4; kernels in ibwt_kernels.cuh).  block_mode: the n bytes a forward
@@ -1654,6 +1684,69 @@ int verify_forward(bwtc_cuda_ctx* ctx, const Job& J) {
   while (!((mask >> first) & 1u)) ++first;
   set_err(ctx->err, "verification failed: the forward output of block %u of %u does not restore its input", first, sh.nblocks);
   return BWTC_CUDA_EVERIFY;
+}
+
+// sufcheck on the device (bwt_kernels.cuh k_sa_perm / k_sa_order): ISA in d_keys[0], idle outside a transform.  Enqueues
+// the check and the read-back of the control words into h_ctrl; the caller waits.
+int enqueue_sufcheck(bwtc_cuda_ctx* ctx, const uint8_t* d_text, const int32_t* d_sa, uint32_t n) {
+  cudaStream_t st = ctx->stream;
+  uint32_t* isa = static_cast<uint32_t*>(ctx->d_keys[0]);
+  CK(ctx, cudaMemsetAsync(ctx->d_ctrl() + CTR_SA_BAD, 0, 8, st));
+  CK(ctx, cudaMemsetAsync(isa, 0xFF, (size_t)n * 4, st));
+  const uint32_t grid = std::max<uint32_t>(1u, std::min<uint32_t>(div_up(n, 256), (uint32_t)ctx->sm_count * 8u));
+  k_sa_perm<<<grid, 256, 0, st>>>(d_sa, n, isa, ctx->d_ctrl());
+  k_sa_order<<<grid, 256, 0, st>>>(d_text, d_sa, n, isa, ctx->d_ctrl());
+  CK(ctx, cudaGetLastError());
+  CK(ctx, cudaMemcpyAsync(ctx->h_ctrl(), ctx->d_ctrl(), CTR_STICKY * 4, cudaMemcpyDeviceToHost, st));
+  ctx->stats.kernel_launches += 2;
+  ctx->stats.algorithmic_bytes += (uint64_t)n * 4 * 4 + (uint64_t)n * 13;  // ISA fill + SA twice + ISA min; 3 ISA / 1 T gathers
+  return 0;
+}
+
+// After the wait: 0 if the check passed, else 1 with the first failing row and its reason in ctx->err.
+int sufcheck_failed(bwtc_cuda_ctx* ctx, uint32_t n, const char* what) {
+  const uint64_t w = (uint64_t)ctx->h_ctrl()[CTR_SA_BAD] | ((uint64_t)ctx->h_ctrl()[CTR_SA_BAD + 1] << 32);
+  if (!w) return 0;
+  const uint64_t key = ~w;
+  const uint32_t row = (uint32_t)((key >> 2) & 0xFFFFFFFFull), reason = (uint32_t)(key & 3u);
+  set_err(ctx->err, "%s: row %u of %u: %s", what, row, n,
+          reason == SA_BAD_RANGE ? "value out of range" :
+          reason == SA_BAD_DUP ? "duplicate (an earlier row holds the same value)" :
+          "out of order (its suffix does not sort after the one of the row before)");
+  return 1;
+}
+
+// Verification of a suffix array (bwtc_cuda_divsufsort with verification on, DESIGN.md §3.11): sufcheck on the device
+// against the text it was sorted from, before anything is copied to the caller.  One host wait.
+int verify_sa(bwtc_cuda_ctx* ctx, const Job& J) {
+  cudaStream_t st = ctx->stream;
+  bwtc_cuda_stats& S = ctx->stats;
+  if (ctx->debug_corrupt_sa >= 0 && (uint64_t)ctx->debug_corrupt_sa + 1 < J.N) {
+    k_debug_swap_sa<<<1, 1, 0, st>>>(J.sa, (uint32_t)ctx->debug_corrupt_sa);
+    CK(ctx, cudaGetLastError());
+    S.kernel_launches++;
+  }
+  if (enqueue_sufcheck(ctx, J.d_text, J.sa, J.N)) return BWTC_CUDA_ECUDA;
+  CK(ctx, cudaEventRecord(ctx->ev_end, st));
+  if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
+  S.flags |= 64u;
+  return sufcheck_failed(ctx, J.N, "verification failed: the suffix array") ? BWTC_CUDA_EVERIFY : 0;
+}
+
+// bwtc_cuda_divsufsort(_device): the raw transform with SA emission into d_sa; h_sa receives a copy.
+int run_divsufsort(bwtc_cuda_ctx* ctx, const uint8_t* h_T, const uint8_t* d_T, int32_t* h_SA, int32_t* d_SA, uint32_t n) {
+  uint32_t pidx = 0;
+  Job J;
+  J.block_mode = false;
+  J.h_in = h_T;
+  J.in_dev = d_T;
+  J.n = n;
+  J.LF = &pidx;
+  J.nLF = 1;
+  J.sa = d_SA;
+  J.h_sa = h_SA;
+  const int64_t rc = run_job(ctx, J);
+  return rc < 0 ? (int)rc : 0;
 }
 
 // count blocks (block contract) through one context: as ONE batch when they qualify — 2..MAX_BATCH blocks, all of
@@ -1881,6 +1974,7 @@ int bwtc_cuda_ctx_create(bwtc_cuda_ctx** out, int device, uint32_t max_block_byt
   if (const char* e = getenv("BWTC_VERIFY")) c->verify = atoi(e) ? 1 : 0;
   if (const char* e = getenv("BWTC_DEBUG_CORRUPT_OUT")) c->debug_corrupt_out = atoi(e);
   if (const char* e = getenv("BWTC_DEBUG_CORRUPT_LF")) c->debug_corrupt_lf = (uint32_t)std::max(0, atoi(e));
+  if (const char* e = getenv("BWTC_DEBUG_CORRUPT_SA")) c->debug_corrupt_sa = std::max(-1L, atol(e));
   if (const char* e = getenv("BWTC_DEBUG_SKIP_COPIES")) c->debug_skip_copies = atoi(e);
   if (const char* e = getenv("BWTC_D2H_KERNEL")) c->d2h_kernel = atoi(e);
   if (const char* e = getenv("BWTC_D2H_CTAS")) c->d2h_ctas = std::max(1, atoi(e));
@@ -2120,6 +2214,77 @@ int64_t bwtc_cuda_divbwtf(bwtc_cuda_ctx* ctx, const uint8_t* T, uint8_t* U, uint
 int64_t bwtc_cuda_divbwt(bwtc_cuda_ctx* ctx, const uint8_t* T, uint8_t* U, uint32_t n, uint32_t* LFpowers,
                          uint32_t nLFpowers) {
   return bwtc_cuda_divbwtf(ctx, T, U, n, LFpowers, nLFpowers, nullptr);
+}
+
+int bwtc_cuda_divsufsort(bwtc_cuda_ctx* ctx, const uint8_t* T, int32_t* SA, uint32_t n) {
+  if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
+  ctx->err[0] = 0;
+  if (!T || !SA) { set_err(ctx->err, "null T or SA"); return BWTC_CUDA_EARG; }  // divsufsort.c: (T == NULL) || (SA == NULL)
+  if (n <= 1) {
+    if (n == 1) SA[0] = 0;
+    return 0;
+  }
+  if ((uint64_t)n > (uint64_t)ctx->cap + 1) {
+    set_err(ctx->err, "raw text of %u bytes exceeds context capacity %u", n, ctx->cap);
+    return BWTC_CUDA_ETOOBIG;
+  }
+  if (!ctx->d_sa) {
+    if (cudaSetDevice(ctx->device) != cudaSuccess) { set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device); return BWTC_CUDA_ECUDA; }
+    const size_t bytes = ((size_t)ctx->cap + 1) * 4;
+    const cudaError_t e = cudaMalloc((void**)&ctx->d_sa, bytes);
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      ctx->d_sa = nullptr;
+      set_err(ctx->err, "cudaMalloc(%zu bytes) for the suffix array: %s", bytes, cudaGetErrorString(e));
+      return BWTC_CUDA_EALLOC;
+    }
+  }
+  return run_divsufsort(ctx, T, nullptr, SA, ctx->d_sa, n);
+}
+
+int bwtc_cuda_divsufsort_device(bwtc_cuda_ctx* ctx, const void* d_T, void* d_SA, uint32_t n) {
+  if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
+  ctx->err[0] = 0;
+  if (!d_T || !d_SA || (reinterpret_cast<uintptr_t>(d_SA) & 3u)) { set_err(ctx->err, "null d_T / d_SA, or d_SA not 4-byte aligned"); return BWTC_CUDA_EARG; }
+  if (n == 0) return 0;
+  if (n == 1) {
+    if (cudaSetDevice(ctx->device) != cudaSuccess) { set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device); return BWTC_CUDA_ECUDA; }
+    CK(ctx, cudaMemsetAsync(d_SA, 0, 4, ctx->stream));
+    return host_wait(ctx, ctx->stream) ? BWTC_CUDA_ECUDA : 0;
+  }
+  return run_divsufsort(ctx, nullptr, static_cast<const uint8_t*>(d_T), nullptr, static_cast<int32_t*>(d_SA), n);
+}
+
+int bwtc_cuda_sufcheck(bwtc_cuda_ctx* ctx, const uint8_t* T, const int32_t* SA, uint32_t n) {
+  if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
+  ctx->err[0] = 0;
+  if (!T || !SA) { set_err(ctx->err, "null T or SA"); return BWTC_CUDA_EARG; }
+  if (n == 0) return 0;
+  if ((uint64_t)n > (uint64_t)ctx->cap + 1) {
+    set_err(ctx->err, "raw text of %u bytes exceeds context capacity %u", n, ctx->cap);
+    return BWTC_CUDA_ETOOBIG;
+  }
+  if (n == 1) {
+    if (SA[0] == 0) return 0;
+    set_err(ctx->err, "sufcheck: row 0 of 1: value out of range");
+    return BWTC_CUDA_ECORRUPT;
+  }
+  if (cudaSetDevice(ctx->device) != cudaSuccess) { set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device); return BWTC_CUDA_ECUDA; }
+  cudaStream_t st = ctx->stream;
+  bwtc_cuda_stats& S = ctx->stats;
+  memset(&S, 0, sizeof(S));
+  S.n_suffixes = n;
+  int32_t* d_SA = static_cast<int32_t*>(ctx->d_keys[1]);  // (8 bytes per suffix; the ISA goes to d_keys[0])
+  if (upload(ctx, ctx->d_in, T, n)) return BWTC_CUDA_ECUDA;
+  if (upload(ctx, reinterpret_cast<uint8_t*>(d_SA), reinterpret_cast<const uint8_t*>(SA), (size_t)n * 4)) return BWTC_CUDA_ECUDA;
+  CK(ctx, cudaEventRecord(ctx->ev_begin, st));
+  if (enqueue_sufcheck(ctx, ctx->d_in, d_SA, n)) return BWTC_CUDA_ECUDA;
+  CK(ctx, cudaEventRecord(ctx->ev_end, st));
+  if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
+  float ms = 0;
+  CK(ctx, cudaEventElapsedTime(&ms, ctx->ev_begin, ctx->ev_end));
+  S.gpu_ms = ms;
+  return sufcheck_failed(ctx, n, "sufcheck") ? BWTC_CUDA_ECORRUPT : 0;
 }
 
 int64_t bwtc_cuda_bwt_block(bwtc_cuda_ctx* ctx, uint8_t* block, uint32_t n, uint32_t* LFpowers, uint32_t nLFpowers,

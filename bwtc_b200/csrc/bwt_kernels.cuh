@@ -1358,6 +1358,10 @@ struct EmitParams {
   // ranks [k*stride, k*stride + N_k) — the block number is the most significant part of every sort key.
   uint32_t nblocks;
   uint32_t stride;
+  // Suffix array of a raw text (bwtc_cuda_divsufsort, DESIGN.md §3.11): sa[rank] = id for EVERY singleton, suffix 0
+  // included.  Only the SA = true instantiations of k_rerank / k_seg_round / k_small_rounds read it (null otherwise), so
+  // the kernels of every other call are the ones they were without it.
+  int32_t* sa;
 };
 
 // Suffix 0 of a block owns the hole at pidx: it has no preceding character to emit.
@@ -1378,7 +1382,7 @@ __device__ __forceinline__ void emit_bwt(const EmitParams& ep, uint32_t nr, uint
   else ep.out[nr] = ch;
 }
 
-template <typename KeyT, bool ROUND0, bool LAZY = false>
+template <typename KeyT, bool ROUND0, bool LAZY = false, bool SA = false>
 __global__ void __launch_bounds__(256, (ROUND0 && !LAZY) ? 5 : 4) k_rerank(const KeyT* __restrict__ keys, const uint32_t* __restrict__ idx,
                                                 uint32_t* __restrict__ rank, RerankParams rp,
                                                 unsigned long long* __restrict__ tstate,
@@ -1634,6 +1638,7 @@ __global__ void __launch_bounds__(256, (ROUND0 && !LAZY) ? 5 : 4) k_rerank(const
   uint32_t wrmask = 0, bpos[IPT];
   uint32_t anymask = 0;  // records whose rank word changed or became final (whatever their id window)
   uint32_t embits = 0, ew0 = 0, ew1 = 0;  // ROUND0: the BWT bytes of my eight (consecutive) sorted positions
+  uint32_t sabits = 0;                    // SA && ROUND0: which of them are final (their SA entries leave as whole words)
 #pragma unroll
   for (int k = 0; k < IPT; ++k) {
     const uint32_t j = j0 + k;
@@ -1666,6 +1671,11 @@ __global__ void __launch_bounds__(256, (ROUND0 && !LAZY) ? 5 : 4) k_rerank(const
         } else {
           emit_bwt(ep, nr, ch);
         }
+      }
+      // SA[nr] = id, under the same "emitted by this launch" rule as the BWT byte, but for suffix 0 too
+      if (SA && single && emit_here && !(LAZY && rp.lazy == 2u)) {
+        if (ROUND0) sabits |= 1u << k;
+        else ep.sa[nr] = (int32_t)id[k];
       }
       if (single) nr |= RANK_DONE;
       else if (sp.enable) { ++live; livemask |= 1u << k; gmax = max(gmax, j - HF + 1u); }
@@ -1730,6 +1740,24 @@ __global__ void __launch_bounds__(256, (ROUND0 && !LAZY) ? 5 : 4) k_rerank(const
         for (int k = 4; k < 8; ++k)
           if ((embits >> k) & 1u) emit_bwt(ep, j0 + k, (uint8_t)(ew1 >> (8 * (k - 4))));
       }
+    }
+  }
+  if (SA && ROUND0 && sabits) {  // the same eight positions: SA[j0 + k] = id[k], one 16-byte store per four final records
+    int32_t* ps = ep.sa + j0;
+    const bool al = (reinterpret_cast<uintptr_t>(ep.sa) & 15u) == 0u;  // (j0 % 8 == 0)
+    if (al && (sabits & 0xFu) == 0xFu) {
+      *reinterpret_cast<int4*>(ps) = make_int4((int)id[0], (int)id[1], (int)id[2], (int)id[3]);
+    } else {
+#pragma unroll
+      for (int k = 0; k < 4; ++k)
+        if ((sabits >> k) & 1u) ps[k] = (int32_t)id[k];
+    }
+    if (al && (sabits & 0xF0u) == 0xF0u) {
+      *reinterpret_cast<int4*>(ps + 4) = make_int4((int)id[4], (int)id[5], (int)id[6], (int)id[7]);
+    } else {
+#pragma unroll
+      for (int k = 4; k < 8; ++k)
+        if ((sabits >> k) & 1u) ps[k] = (int32_t)id[k];
     }
   }
   if (rp.nr_out) {
@@ -2052,7 +2080,7 @@ __global__ void __launch_bounds__(256) k_build_from_list(const uint32_t* __restr
 #ifndef BWTC_SEG_MINB_LAZY
 #define BWTC_SEG_MINB_LAZY 4  // (3 CTAs/SM with 80 registers measured the same)
 #endif
-template <bool LAZY>
+template <bool LAZY, bool SA = false>
 __global__ void __launch_bounds__(256, LAZY ? BWTC_SEG_MINB_LAZY : BWTC_SEG_MINB) k_seg_round(const LadderState* __restrict__ st, PoolPtrs pool,
                                                    const uint32_t* __restrict__ rank, uint32_t N, EmitParams ep,
                                                    uint32_t* __restrict__ ctrl, const LookupParams* __restrict__ lkp) {
@@ -2245,6 +2273,7 @@ __global__ void __launch_bounds__(256, LAZY ? BWTC_SEG_MINB_LAZY : BWTC_SEG_MINB
       const bool single = ((hfmask >> k) & 1u) && (j + 1 >= L || nk != key[k]);
       uint32_t nr = (uint32_t)(key[k] >> 32) + (HF - HH);
       if (single && !owns_hole(ep, myid[k])) emit_bwt(ep, nr, ep.text[myid[k] - 1]);
+      if (SA && single) ep.sa[nr] = (int32_t)myid[k];
       if (single) nr |= RANK_DONE; else { keep |= 1u << k; gmax = max(gmax, j - HF + 1u); }
       newnr[k] = nr;
       if (single || HF != HH) updm |= 1u << k;
@@ -2339,6 +2368,7 @@ __global__ void __launch_bounds__(256) k_apply_ranks(const LadderState* __restri
 // without returning to the host, instead of ~10 launch-latency-bound kernels per round.
 // Replaces the tail of trsort's loop (trsort.c:563-585), where only a few groups are left.
 // =====================================================================================================
+template <bool SA = false>
 __global__ void __launch_bounds__(1024) k_small_rounds(LadderState* st, PoolPtrs pool, uint32_t* rank,
                                                        uint32_t N, EmitParams ep, uint32_t* __restrict__ ctrl,
                                                        const LookupParams* __restrict__ lkp) {
@@ -2438,6 +2468,7 @@ __global__ void __launch_bounds__(1024) k_small_rounds(LadderState* st, PoolPtrs
         const bool single = hf2[q] && (j + 1 >= m || nk != key2[q]);
         uint32_t nr = (uint32_t)(key2[q] >> 32) + (HF - HH);
         if (single && !owns_hole(ep, id2[q])) emit_bwt(ep, nr, ep.text[id2[q] - 1]);
+        if (SA && single) ep.sa[nr] = (int32_t)id2[q];
         if (single) nr |= RANK_DONE; else keep |= 1u << q;
         if (single || HF != HH) rank[id2[q]] = nr;
       }
@@ -2560,6 +2591,74 @@ __global__ void __launch_bounds__(256) k_finish_batch(const uint32_t* __restrict
     const uint32_t lc = lastch[k];
     if (lc & 0x100u) out[start + pidx] = (uint8_t)(lc & 0xFFu);
   }
+}
+
+// =====================================================================================================
+// sufcheck on the device (bwtc_cuda_sufcheck, and the verification of bwtc_cuda_divsufsort; DESIGN.md §3.11).
+// SA[0..n) is the suffix array of T exactly when
+//   (1) it is a permutation of [0, n): every value in range, none twice, and
+//   (2) for every r >= 1: (T[SA[r-1]], ISA'[SA[r-1]+1]) < (T[SA[r]], ISA'[SA[r]+1]), ISA' = the inverse of SA with
+//       ISA'[n] = -1 standing for the empty suffix
+// (neighbours ordered by first byte, then by the rank of their successor, are ordered lexicographically: induction
+// on the suffix length).  k_sa_perm scatters ISA[SA[r]] = min r (atomicMin over an all-ones ISA), so a value held twice
+// keeps its FIRST row and k_sa_order finds every later one as isa[v] != r.  Failures meet in one 64-bit control word as
+// the maximum of ~((phase << 62) | (row << 2) | reason): the host reads the smallest (phase, row) — range and duplicate
+// failures (phase 0) before order failures (phase 1, whose ISA is only meaningful for a permutation).
+// =====================================================================================================
+constexpr int CTR_SA_BAD = 2;  // [2..3] (the words of the inverse's corrupt mask, read back the same way, CTR_INV_BAD)
+enum : uint32_t { SA_BAD_RANGE = 1, SA_BAD_DUP = 2, SA_BAD_ORDER = 3 };
+
+__device__ __forceinline__ void sa_fail(uint32_t* ctrl, uint32_t phase, uint32_t row, uint32_t reason) {
+  const unsigned long long key = ((unsigned long long)phase << 62) | ((unsigned long long)row << 2) | reason;
+  atomicMax(reinterpret_cast<unsigned long long*>(ctrl + CTR_SA_BAD), ~key);
+}
+
+// (1a) ranges, and ISA[v] = the first row holding v.  isa[0..n) must hold 0xFFFFFFFF.
+__global__ void __launch_bounds__(256) k_sa_perm(const int32_t* __restrict__ sa, uint32_t n, uint32_t* __restrict__ isa,
+                                                 uint32_t* __restrict__ ctrl) {
+  const uint32_t stride = gridDim.x * blockDim.x;
+  for (uint32_t r = blockIdx.x * blockDim.x + threadIdx.x; r < n; r += stride) {
+    const uint32_t v = (uint32_t)sa[r];  // (a negative value is >= n here)
+    if (v >= n) sa_fail(ctrl, 0, r, SA_BAD_RANGE);
+    else atomicMin(&isa[v], r);
+  }
+}
+
+// (1b) duplicates and (2) order.  A warp owns 32 consecutive rows: row r's key (T[SA[r]], ISA'[SA[r]+1] + 1) is
+// compared with the key of row r-1, which lane r-1 holds (lane 0 loads it).
+__global__ void __launch_bounds__(256) k_sa_order(const uint8_t* __restrict__ text, const int32_t* __restrict__ sa, uint32_t n,
+                                                  const uint32_t* __restrict__ isa, uint32_t* __restrict__ ctrl) {
+  const uint32_t lane = threadIdx.x & 31u;
+  const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = (gridDim.x * blockDim.x) >> 5;
+  auto key_of = [&](uint32_t v) -> unsigned long long {  // v < n
+    const uint32_t succ = (v + 1u < n) ? isa[v + 1u] + 1u : 0u;  // the empty suffix ranks below every other
+    return ((unsigned long long)text[v] << 32) | succ;
+  };
+  for (uint32_t base = warp * 32u; base < n; base += nwarps * 32u) {
+    const uint32_t r = base + lane;
+    const uint32_t v = (r < n) ? (uint32_t)sa[r] : 0xFFFFFFFFu;
+    const bool valid = v < n;
+    unsigned long long key = 0;
+    if (valid) {
+      if (isa[v] != r) sa_fail(ctrl, 0, r, SA_BAD_DUP);
+      key = key_of(v);
+    }
+    unsigned long long pkey = __shfl_up_sync(0xFFFFFFFFu, key, 1);
+    bool pvalid = __shfl_up_sync(0xFFFFFFFFu, valid ? 1u : 0u, 1) != 0u;
+    if (lane == 0) {
+      const uint32_t u = (r > 0u && r < n) ? (uint32_t)sa[r - 1u] : 0xFFFFFFFFu;
+      pvalid = u < n;
+      pkey = pvalid ? key_of(u) : 0ull;
+    }
+    if (valid && pvalid && r > 0u && !(pkey < key)) sa_fail(ctrl, 1, r, SA_BAD_ORDER);
+  }
+}
+
+// Test hook (BWTC_DEBUG_CORRUPT_SA=r): swap SA[r] and SA[r+1] before the verification checks them.
+__global__ void k_debug_swap_sa(int32_t* sa, uint32_t r) {
+  const int32_t a = sa[r];
+  sa[r] = sa[r + 1u];
+  sa[r + 1u] = a;
 }
 
 }  // namespace bwtc_b200

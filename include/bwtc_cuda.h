@@ -10,6 +10,9 @@
  *   bwtc_cuda_divbwt / bwtc_cuda_divbwtf   <-  divbwt / divbwtf          bwtransforms/divsufsort.h:86-94,
  *                                              bwtransforms/divsufsort.c:440-522 (as called by
  *                                              Divsufsorter::doTransform, bwtransforms/Divsufsorter.hpp:54-65)
+ *   bwtc_cuda_divsufsort / _device /       <-  divsufsort / sufcheck                  bwtransforms/divsufsort.h (the
+ *   bwtc_cuda_sufcheck                         library's suffix-array entry point and its checker, beside the BWT
+ *                                              entry points above)
  *   bwtc_cuda_bwt_block                    <-  BWTransform::doTransform(BWTBlock&, uint32 freqs[256])
  *                                              bwtransforms/BWTransform.cpp:39-64 (reverse / sentinel /
  *                                              hole-fill fused on the device)
@@ -83,8 +86,9 @@ typedef struct bwtc_cuda_stats {
                               * bit 1: the blocks of a batch were sorted as one text; bit 2: predecessor codes packed above the ids;
                               * bit 3: ... carried as a one-byte payload array; bit 6: the forward output (block or raw
                               * contract) and its LFpowers were verified by a device-side inversion (bwtc_cuda_ctx_set_verify,
-                              * BWTC_VERIFY); bit 7: inverse only, this block is corrupt
-                              * (BWTC_CUDA_ECORRUPT) */
+                              * BWTC_VERIFY; for bwtc_cuda_divsufsort: its suffix array passed the device-side sufcheck); bit 7:
+                              * inverse only, this block is corrupt (BWTC_CUDA_ECORRUPT); bit 8: this call produced a suffix
+                              * array (bwtc_cuda_divsufsort, _device) */
   uint32_t batch_blocks;     /* blocks this record describes: 1, or the size of the batch that was sorted as one text (every
                               * block of the batch then carries the SAME record — count it once; flags bit 7 is the one field
                               * in which the records of one inverse batch may differ) */
@@ -143,6 +147,28 @@ int64_t bwtc_cuda_divbwtf(bwtc_cuda_ctx* ctx, const uint8_t* T, uint8_t* U, uint
                           uint32_t* LFpowers, uint32_t nLFpowers, uint32_t* freqs);
 int64_t bwtc_cuda_divbwt(bwtc_cuda_ctx* ctx, const uint8_t* T, uint8_t* U, uint32_t n,
                          uint32_t* LFpowers, uint32_t nLFpowers);
+
+/* ---- suffix array of a raw text: libdivsufsort's divsufsort / sufcheck (divsufsort.h) ------------- */
+/* divsufsort(T, SA, n): SA[0..n) = the suffix array of T under the raw contract's order (implicit end sentinel, a suffix
+ * that is a prefix of another sorts first) -- the order bwtc_cuda_divbwtf's output is defined by (U[r] = T[SA[r]-1],
+ * pidx = the row of suffix 0).  Returns 0 or a negative error (-1 / -2 keep divsufsort's meaning).  n == 0: nothing;
+ * n == 1: SA[0] = 0 (the host variant does not touch the device).  n <= max_block_bytes + 1 (else BWTC_CUDA_ETOOBIG).
+ * T and SA may be pageable or pinned host memory: pinned SA is copied directly, pageable SA through the context's pinned
+ * staging ring.  The SA is written on the device where each suffix becomes unique, beside its BWT byte.  Memory: the host
+ * variant allocates a 4 (max_block_bytes + 1)-byte device array on its first call (BWTC_CUDA_EALLOC if that fails, the
+ * context stays usable), freed by bwtc_cuda_ctx_destroy -- on top of bwtc_cuda_scratch_bytes; _device emits straight into
+ * d_SA (n int32 entries, 4-byte aligned, else BWTC_CUDA_EARG) and allocates nothing.  With verification on
+ * (bwtc_cuda_ctx_set_verify, BWTC_VERIFY) the device runs the sufcheck below on the SA before anything reaches the caller:
+ * on a failure the call returns BWTC_CUDA_EVERIFY, a host SA is untouched, a d_SA holds unspecified values.
+ * stats.flags bit 8 is set (bit 6 too when verified); no other entry point sets bit 8. */
+int bwtc_cuda_divsufsort(bwtc_cuda_ctx* ctx, const uint8_t* T, int32_t* SA, uint32_t n);
+int bwtc_cuda_divsufsort_device(bwtc_cuda_ctx* ctx, const void* d_T, void* d_SA, uint32_t n);  /* d_SA 4-byte aligned */
+/* sufcheck(T, SA, n): 0 if SA (host, pageable or pinned) is the suffix array of T, BWTC_CUDA_ECORRUPT if not -- the message
+ * names the first offending row and why: out of range / duplicate (of an earlier row) / out of order; range and duplicate
+ * failures are reported before order failures.  Other negatives as usual (BWTC_CUDA_ETOOBIG above max_block_bytes + 1).
+ * Unlike libdivsufsort's sequential sufcheck, which returns -2 / -3 / -4 for the three kinds of failure, one code is used:
+ * those values are BWTC_CUDA_EALLOC / ECUDA / EINTERNAL here.  Runs in the context's scratch (stats: gpu_ms = the check). */
+int bwtc_cuda_sufcheck(bwtc_cuda_ctx* ctx, const uint8_t* T, const int32_t* SA, uint32_t n);
 
 /* ---- block contract: BWTransform::doTransform(BWTBlock&, freqs) (BWTransform.cpp:52-64) ---------- */
 /* block: n bytes (host), transformed IN PLACE; unlike the reference wrapper the byte after the block
