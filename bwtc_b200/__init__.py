@@ -545,6 +545,26 @@ class Pipeline:
             raise BwtcCudaError(rc, self._lib.bwtc_cuda_pipeline_error(self._h).decode())
         return h
 
+    def submit_runs(self, block: np.ndarray, capacity: int, starts: int = 8, out: Optional[np.ndarray] = None):
+        """Streaming transform with run statistics (bwtc_cuda_pipeline_submit_runs): queues one host block, transformed in
+        place or into `out` (same size; `block` is then left as it is), and returns a handle; wait(handle) returns
+        (LFpowers, freqs, runs) with runs = (symbol[], start[]) of the output's maximal runs, or None when there are more
+        than `capacity`.  Such a block is never batched with others.  The buffers must stay alive until then."""
+        assert block.dtype == np.uint8
+        dst = block if out is None else out
+        assert dst.dtype == np.uint8 and dst.size == block.size
+        sym = np.zeros(max(capacity, 1), np.uint8)
+        start = np.zeros(max(capacity, 1), np.uint32)
+        h = {"kind": "runs", "block": block, "out": dst, "LF": np.zeros(256, np.uint32), "nLF": ctypes.c_uint32(0),
+             "freqs": np.zeros(256, np.uint32), "sym": sym, "start": start,
+             "runs": Runs(capacity, 0, sym.ctypes.data, start.ctypes.data), "ticket": ctypes.c_uint64(0)}
+        rc = self._lib.bwtc_cuda_pipeline_submit_runs(self._h, block.ctypes.data, dst.ctypes.data, block.size, starts,
+                                                      h["LF"].ctypes.data, ctypes.addressof(h["nLF"]), h["freqs"].ctypes.data,
+                                                      ctypes.addressof(h["runs"]), ctypes.byref(h["ticket"]))
+        if rc < 0:
+            raise BwtcCudaError(rc, self._lib.bwtc_cuda_pipeline_error(self._h).decode())
+        return h
+
     def submit_inverse(self, block: np.ndarray, LF):
         """Streaming inverse (bwtc_cuda_pipeline_submit_inverse): queues one host block (the output of a forward block
         transform) to be restored in place and returns a handle; wait(handle) returns the block.  LF: the block's
@@ -559,13 +579,18 @@ class Pipeline:
         return h
 
     def wait(self, h):
-        """Waits for a handle of submit (returns (LFpowers, freqs)) or of submit_inverse (returns the restored block).  Raises
-        for a failed handle only: a corrupt inverse block (code ECORRUPT) does not fail the other blocks of its group."""
+        """Waits for a handle of submit (returns (LFpowers, freqs)), of submit_runs (returns (LFpowers, freqs, runs or None))
+        or of submit_inverse (returns the restored block).  Raises for a failed handle only: a corrupt inverse block (code
+        ECORRUPT) does not fail the other blocks of its group."""
         rc = self._lib.bwtc_cuda_pipeline_wait(self._h, h["ticket"])
         if rc < 0:
             raise BwtcCudaError(rc, self._lib.bwtc_cuda_pipeline_error(self._h).decode())
         if h.get("kind") == "inverse":
             return h["block"]
+        if h.get("kind") == "runs":
+            cnt = h["runs"].count
+            runs = None if cnt == RUNS_OVERFLOW else (h["sym"][:cnt].copy(), h["start"][:cnt].copy())
+            return h["LF"][: h["nLF"].value].copy(), h["freqs"], runs
         return h["LF"][: h["nLF"].value].copy(), h["freqs"]
 
     def run(self, blocks: Sequence[np.ndarray], starts: int = 8):

@@ -1186,8 +1186,7 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
       k_run_emit<<<rtiles, 256, 0, st>>>(J.d_dst, n, rcnt, rexcl, rtiles, cap_dev, ctx->d_aux[0], ctx->d_scat, &ctx->d_state->nruns,
                                          ctx->d_state);
       CK(ctx, cudaGetLastError());
-      S.kernel_launches += 3;
-      S.algorithmic_bytes += 2ull * n;
+      S.kernel_launches += 3;  // (queued in every chunk; they return at once in all but the one that finishes the block)
     }
     CK(ctx, cudaEventRecord(ctx->ev_end, st));
     CK(ctx, cudaMemcpyAsync(ctx->h_state, ctx->d_state, sizeof(LadderState), cudaMemcpyDeviceToHost, st));
@@ -1351,6 +1350,7 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
 
   // ---- run statistics first: the verification below reuses d_scat
   if (finished && J.runs && !bs && J.block_mode) {
+    S.algorithmic_bytes += 2ull * n;  // the run kernels read the output twice, once per block whatever the chunk count
     const uint32_t cnt = ctx->h_state->nruns;
     if (cnt <= J.runs->capacity && cnt <= n && J.runs->symbol && J.runs->start) {
       if (download_staged(ctx, J.runs->symbol, ctx->d_aux[0], cnt)) return BWTC_CUDA_ECUDA;
@@ -1468,7 +1468,10 @@ int64_t run_transform(bwtc_cuda_ctx* ctx, bool block_mode, const uint8_t* h_in, 
   J.nLF = nLF;
   J.freqs = freqs;
   J.bs = bs;
-  return run_job(ctx, J);
+  const int64_t rc = run_job(ctx, J);
+  // a failure after the runs were downloaded (EVERIFY, or an error in a later copy) must not leave a valid-looking count
+  if (rc < 0 && runs) runs->count = BWTC_CUDA_RUNS_OVERFLOW;
+  return rc;
 }
 
 // ---- inverse transform (SURVEY.md §8f row f4; kernels in ibwt_kernels.cuh).  block_mode: the n bytes a forward
@@ -2296,6 +2299,7 @@ int64_t bwtc_cuda_bwt_block(bwtc_cuda_ctx* ctx, uint8_t* block, uint32_t n, uint
 
 int64_t bwtc_cuda_bwt_block_runs(bwtc_cuda_ctx* ctx, uint8_t* block, uint32_t n, uint32_t* LFpowers, uint32_t nLFpowers,
                                  uint32_t* freqs, bwtc_cuda_runs* runs) {
+  if (runs) runs->count = BWTC_CUDA_RUNS_OVERFLOW;  // (every negative return leaves it so)
   if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
   if (!block || n == 0) { set_err(ctx->err, "null or empty block"); return BWTC_CUDA_EARG; }
   return run_transform(ctx, true, block, block, nullptr, nullptr, n, LFpowers, nLFpowers, freqs, nullptr, runs);
@@ -2614,6 +2618,7 @@ int bwtc_cuda_pipeline_submit(bwtc_cuda_pipeline* p, const uint8_t* in, uint8_t*
 
 int bwtc_cuda_pipeline_submit_runs(bwtc_cuda_pipeline* p, const uint8_t* in, uint8_t* out, uint32_t n, uint32_t starts,
                                    uint32_t* LFpowers, uint32_t* nLF, uint32_t* freqs, bwtc_cuda_runs* runs, uint64_t* ticket) {
+  if (runs) runs->count = BWTC_CUDA_RUNS_OVERFLOW;  // (stays so unless the block succeeds)
   if (!p || !in || !out || !LFpowers || !nLF || !ticket || n == 0) { if (p) set_err(p->err, "bad arguments"); return BWTC_CUDA_EARG; }
   {
     std::lock_guard<std::mutex> lk(p->mu);

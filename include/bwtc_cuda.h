@@ -198,7 +198,11 @@ int bwtc_cuda_bwt_blocks(bwtc_cuda_ctx* ctx, void* const* blocks, const uint32_t
  * during BWT", HuffmanCoders.cpp:54); the host slices the runs at its section boundaries.  The caller provides the two
  * arrays and their capacity; if the block has more runs than that, count = BWTC_CUDA_RUNS_OVERFLOW and the arrays are
  * left alone (text-like blocks have ~0.75 runs per byte: scanning on the host is then cheaper than 5 bytes per run over
- * PCIe — pass a capacity of n/8 or so and fall back to the scan on overflow). */
+ * PCIe — pass a capacity of n/8 or so and fall back to the scan on overflow).  A NULL symbol or start array counts as
+ * overflow.  Every negative return (arguments, capacity, BWTC_CUDA_EVERIFY, ...) also leaves count =
+ * BWTC_CUDA_RUNS_OVERFLOW, so a caller that only looks at count never takes the runs of a failed block; the arrays are
+ * then untouched, except after BWTC_CUDA_EVERIFY, which leaves them unspecified.  On success the entries from index count
+ * on are untouched. */
 #define BWTC_CUDA_RUNS_OVERFLOW 0xFFFFFFFFu
 typedef struct bwtc_cuda_runs {
   uint32_t  capacity;  /* in : runs the arrays can hold */
@@ -276,7 +280,9 @@ int  bwtc_cuda_pipeline_wait(bwtc_cuda_pipeline* p, uint64_t ticket);
  * other blocks of its group complete normally. */
 int  bwtc_cuda_pipeline_submit_inverse(bwtc_cuda_pipeline* p, const uint8_t* in, uint8_t* out, uint32_t n, uint32_t eob,
                                        int on_device, bwtc_cuda_stats* stats, uint64_t* ticket);
-/* submit + run statistics (filled when the block completes; such a block is transformed on its own, not in a batch). */
+/* submit + run statistics (filled when the block completes; such a block is transformed on its own, not in a batch).
+ * in and out may differ (out-of-place host block).  runs->count is BWTC_CUDA_RUNS_OVERFLOW from this call on, and stays so
+ * unless the block succeeds with at most runs->capacity runs. */
 int  bwtc_cuda_pipeline_submit_runs(bwtc_cuda_pipeline* p, const uint8_t* in, uint8_t* out, uint32_t n, uint32_t starts,
                                     uint32_t* LFpowers, uint32_t* nLF, uint32_t* freqs, bwtc_cuda_runs* runs, uint64_t* ticket);
 /* Device-side timing of whatever the pipeline's streams execute between the two calls: begin records

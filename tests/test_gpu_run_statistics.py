@@ -68,3 +68,24 @@ def test_pipelined_compress_with_gpu_run_statistics_is_byte_identical(tmp_path, 
         assert served > 0, "the GPU's runs should have replaced the coder's scans"
     else:
         assert served == 0
+
+
+def test_pipelined_compress_mixed_blocks_with_and_without_run_statistics(tmp_path, monkeypatch):
+    """One file, three kinds of block (16 MiB blocks): repetitive (few runs: the GPU's runs are served to the coder),
+    Markov (over the size/8 capacity: the coder scans), and a last block below 8 MiB (no runs asked for).  Byte-identical
+    to the reference, and again with BWTC_RUN_STATS=0."""
+    need_libs()
+    x = np.concatenate([bw.generate("repetitive", 16 << 20, seed=83), bw.generate("markov", 16 << 20, seed=84),
+                        bw.generate("random", (3 << 20) + 77, seed=85)])
+    src = tmp_path / "in.bin"
+    x.tofile(src)
+    mem = 90687655  # 16 MiB blocks
+    run_tool("compress", "cpu", src, tmp_path / "ref.bwtc", mem, "H", 8, tool=REFTOOL)
+    ref = (tmp_path / "ref.bwtc").read_bytes()
+    out = json.loads(run_tool("pipe_compress", src, tmp_path / "pipe.bwtc", mem, "H", "c", 8, 4, 0, "0", 2))
+    assert (tmp_path / "pipe.bwtc").read_bytes() == ref
+    assert out.get("run_statistics_served", 0) > 0, "the repetitive block's runs should have been served"
+    monkeypatch.setenv("BWTC_RUN_STATS", "0")
+    out = json.loads(run_tool("pipe_compress", src, tmp_path / "off.bwtc", mem, "H", "c", 8, 4, 0, "0", 2))
+    assert (tmp_path / "off.bwtc").read_bytes() == ref
+    assert out.get("run_statistics_served", 0) == 0
