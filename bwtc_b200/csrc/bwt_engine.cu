@@ -149,8 +149,10 @@ struct bwtc_cuda_ctx {
   int use_lazy = 1;               // lazy ranks after round 0 (DESIGN.md §3.9): 0 never, 1 when the key-shape policy predicts
                                   // that few suffixes stay in groups, 2 always (tests)
   uint32_t lazy_min_suffixes = 4u << 20;
-  double lazy_max_live = 0.065;   // measured break-even with the sector look-ups: -15..-19% at 3%, -10..-12% at 4.6%, -4% at 6%,
-                                  // +-1% at 9% predicted live (DNA / random bytes, 128..384 MiB)
+  double lazy_max_live = 0.09;    // i.i.d.-like blocks: at most this predicted live fraction after round 0.  Measured with the
+                                  // look-up-free segmented rounds: random bytes 256 / 384 MiB (6.1% / 8.9%) -8% / -5%
+  double lazy_max_repeats = 32.0; // blocks with memory: at most this many other positions share a position's 8-gram (Markov
+                                  // 16 / 32 / 64 MiB: 1.3 / 3.0 / 5.2; repetitive 16 MiB: ~3800, source text ~1.5e5)
   int use_seg = 1;                // segmented (sort-free) doubling rounds when every group is small
   int use_batch = 1;              // small equal-sized blocks of one call are sorted as one text
   int use_pack_pred = 1;          // carry code(T[id-1]) above the id through the round-0 sort when it fits
@@ -224,6 +226,7 @@ struct Round0Plan {
   PackParams pp;
   bool has_memory;    // the 8-gram sample says the source is not i.i.d.-like (text, repeats)
   double live_pred;   // i.i.d.-like sources: predicted fraction of suffixes still tied after round 0, L(chars)
+  double repeats;     // mean number of other text positions sharing a position's 8-gram (N x sampled pair collision rate)
 };
 
 // Dense alphabet + round-0 key shape (DESIGN.md §3.2).  present[c] != 0 for every byte of the text.
@@ -289,14 +292,17 @@ void plan_round0(const bwtc_cuda_ctx* ctx, const uint64_t* count, const bool* pr
   }
   pl->has_memory = true;
   pl->live_pred = 1.0;
+  pl->repeats = HUGE_VAL;
   if (!(ctx->force_chars || ctx->force_keybytes)) {
     double q2 = 0.0;
     for (int c = 0; c < 256; ++c)
       if (present[c] && count[c]) { const double q = (double)count[c] / total; q2 += q * q; }
     const double samples = pair_stats[1];
-    const double expected = samples * (samples - 1.0) * 0.5 * std::pow(q2, 8.0);
+    const double all_pairs = samples * (samples - 1.0) * 0.5;
+    const double expected = all_pairs * std::pow(q2, 8.0);
     pl->has_memory = (H0 < 1e-3) || samples < 64.0 || (pair_stats[0] > 8.0 * expected + 16.0);
     if (!pl->has_memory) pl->live_pred = 1.0 - std::exp(-(double)N * std::exp2(-H0 * (double)chars));
+    if (samples >= 64.0) pl->repeats = pair_stats[0] / all_pairs * (double)N;
   }
   pl->sigma = sigma;
   pl->bits = b;
@@ -983,18 +989,26 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
   S.rounds = 1;
   // ---- lazy ranks? (DESIGN.md §3.9)  The rank scatter of round 0 — a random 4-byte write per suffix — is 20-35% of a block,
   // but after round 0 only the ranks of suffixes that are still in a group are ever refined, and a singleton's rank is simply
-  // its position in the sorted key array.  If a sample of the sorted keys says few suffixes stay in groups, rank[] is
-  // written for those only and the others are looked up in the retained sorted keys when needed (rank_lookup).
+  // its position in the sorted key array.  If few suffixes will stay in groups, rank[] is written for those only; the
+  // segmented rounds order group members by cmp (round-0 key, then rank where it is stored) and need no integer rank, the
+  // tail (k_small_rounds, k_finish) looks the few ranks it needs up in the retained sorted keys (rank_lookup).
   bool lazy = false;
   const uint32_t keybits0 = pl.chars * pl.bits + pl.rbits;
   if (ctx->use_lazy && !bs && !dbg_any(ctx) && N >= 64 && keybits0 >= 1) {
-    // The decision needs no measurement: for an i.i.d.-like source (DNA, random bytes) the key-shape policy has already
-    // predicted the fraction of suffixes still tied after round 0, L(c) = 1 - exp(-N 2^(-H0 c)) — it matches the measured
-    // live fractions to three digits (DNA 64 MiB: 0.0156 / 0.0155; random 256 MiB: 0.0606 / 0.0606).  Lazy ranks pay a
-    // search per looked-up rank (~0.1 us each), so they win only when few ranks are looked up: measured -15% on the DNA
-    // 64 MiB block (1.5% live), break-even at ~8% (Markov text), a loss at 6% on 256 MiB blocks whose sorted keys are far
-    // larger than L2 (profiles/r02_experiments.md).  A wrong prediction only costs time: the fallback below is exact.
-    lazy = ctx->use_lazy >= 2 || (!pl.has_memory && pl.live_pred <= ctx->lazy_max_live && N >= ctx->lazy_min_suffixes);
+    // The decision needs no extra measurement.  For an i.i.d.-like source (DNA, random bytes) the key-shape policy has
+    // already predicted the fraction of suffixes still tied after round 0, L(c) = 1 - exp(-N 2^(-H0 c)) — it matches the
+    // measured live fractions to three digits (DNA 64 MiB: 0.0156 / 0.0155; random 256 MiB: 0.0606 / 0.0606).  For a source
+    // with memory the 8-gram sample tells text (a few other positions share a position's 8-gram: Markov 32 MiB 3.0, 3% live
+    // after its 10.7-character keys) from repeats (thousands: the 4 KiB-seed block keeps ~all suffixes tied through global
+    // radix rounds and would only pay the materialising fallback).  The 8-gram sample says nothing about how much a key
+    // longer than 8 characters separates, so a block with memory also needs keys of at least LAZY_MIN_CHARS characters
+    // (codes of <= 6 bits): the same Markov text as a 65-symbol raw text (7-bit codes, 9-character keys) left more or
+    // larger groups after round 0 than the segmented rounds take and fell back.  Segmented rounds are what makes lazy ranks cheap, so a block with memory
+    // goes lazy only where they run.  A wrong prediction only costs time: the fallback below is exact.
+    constexpr uint32_t LAZY_MIN_CHARS = 10;
+    const bool memory_ok = ctx->use_seg && pl.chars >= LAZY_MIN_CHARS && pl.repeats <= ctx->lazy_max_repeats;
+    lazy = ctx->use_lazy >= 2 ||
+           (N >= ctx->lazy_min_suffixes && (pl.has_memory ? memory_ok : pl.live_pred <= ctx->lazy_max_live));
   }
   const uint32_t tbits = std::min<uint32_t>(KTAB_BITS, keybits0);
   const uint32_t lazy_cap = N / 6;  // the lists of lazy mode live in six slices of d_scat
@@ -1997,6 +2011,7 @@ int bwtc_cuda_ctx_create(bwtc_cuda_ctx** out, int device, uint32_t max_block_byt
   c->status_row_words = status_row_words_for(c->use_radix9);
   if (const char* e = getenv("BWTC_LAZY_MIN_MIB")) c->lazy_min_suffixes = (uint32_t)std::max(0L, atol(e)) << 20;
   if (const char* e = getenv("BWTC_LAZY_MAX_LIVE")) c->lazy_max_live = atof(e);
+  if (const char* e = getenv("BWTC_LAZY_MAX_REPEATS")) c->lazy_max_repeats = atof(e);
   if (const char* e = getenv("BWTC_SEG")) c->use_seg = atoi(e);
   if (const char* e = getenv("BWTC_BATCH")) c->use_batch = atoi(e);
   if (const char* e = getenv("BWTC_PACK_PRED")) c->use_pack_pred = atoi(e);

@@ -1174,7 +1174,8 @@ struct LookupParams {
 // Lower bound of `key` in sorted[lo, hi) reading whole 32-byte sectors: the first probe is INTERPOLATED from the key bits
 // below the table prefix (inside one table bucket they are close to uniform), then the search walks to the neighbouring
 // sector twice before it falls back to bisection.  A bucket of ~32 keys costs 1-2 DRAM sectors instead of the ~3 distinct
-// ones of a plain binary search (the look-ups are bound by random DRAM sectors).  The key array is padded to a sector.
+// ones of a plain binary search.  The key array is padded to a sector.  Only the tail of a lazy block searches (k_small_rounds:
+// <= 2048 look-ups per round in one CTA, k_finish: <= 257), so what counts is the chain of dependent DRAM round trips.
 template <typename KeyT>
 __device__ __forceinline__ uint32_t sector_lower_bound(const KeyT* __restrict__ sk, KeyT key, uint32_t lo, uint32_t hi,
                                                        uint32_t frac16) {
@@ -1212,10 +1213,9 @@ __device__ __forceinline__ uint32_t sector_lower_bound(const KeyT* __restrict__ 
   return lo;
 }
 
-// rank of suffix j (without the DONE flag).
-__device__ __forceinline__ uint32_t rank_lookup(const LookupParams& lk, const uint32_t* __restrict__ rank, uint32_t j) {
-  if (!lk.enabled || ((lk.livebits[j >> 5] >> (j & 31u)) & 1u)) return rank[j] & RANK_MASK;
-  unsigned long long key = 0;  // the round-0 key of suffix j, as k_pack_round0 builds it
+// The round-0 key of suffix j, as k_pack_round0 builds it (windows past the end of the text padded with code 0).
+__device__ __forceinline__ unsigned long long round0_key(const LookupParams& lk, uint32_t j) {
+  unsigned long long key = 0;
   for (uint32_t c = 0; c < lk.chars; ++c) {
     const uint32_t g = j + c;
     key = (key << lk.bits) | (unsigned long long)((g < lk.N) ? lk.lut[lk.text[g]] : 0u);
@@ -1224,32 +1224,21 @@ __device__ __forceinline__ uint32_t rank_lookup(const LookupParams& lk, const ui
     const uint32_t g = j + lk.chars;
     key = (key << lk.rbits) | (unsigned long long)(((g < lk.N) ? (uint32_t)lk.lut[lk.text[g]] : 0u) >> (lk.bits - lk.rbits));
   }
+  return key;
+}
+
+// rank of suffix j (without the DONE flag).
+__device__ __forceinline__ uint32_t rank_lookup(const LookupParams& lk, const uint32_t* __restrict__ rank, uint32_t j) {
+  if (!lk.enabled || ((lk.livebits[j >> 5] >> (j & 31u)) & 1u)) return rank[j] & RANK_MASK;
+  const unsigned long long key = round0_key(lk, j);
   const uint32_t p = (uint32_t)(key >> lk.tshift);
   uint32_t lo = lk.ktab[p], hi = lk.ktab[p + 1u];
-#ifndef BWTC_LAZY_BINSEARCH
   // the 16 key bits below the table prefix, as a fraction of the bucket
   const uint32_t frac16 = lk.tshift >= 16u ? (uint32_t)(key >> (lk.tshift - 16u)) & 0xFFFFu
                                            : ((uint32_t)key << (16u - lk.tshift)) & 0xFFFFu;
   if (lk.keybytes == 8u)
     return sector_lower_bound<unsigned long long>(static_cast<const unsigned long long*>(lk.sorted_keys), key, lo, hi, frac16);
   return sector_lower_bound<uint32_t>(static_cast<const uint32_t*>(lk.sorted_keys), (uint32_t)key, lo, hi, frac16);
-#else
-  if (lk.keybytes == 8u) {
-    const unsigned long long* sk = static_cast<const unsigned long long*>(lk.sorted_keys);
-    while (lo < hi) {  // lower bound: the key is unique (singleton), so this is its position
-      const uint32_t mid = lo + ((hi - lo) >> 1);
-      if (sk[mid] < key) lo = mid + 1u; else hi = mid;
-    }
-  } else {
-    const uint32_t* sk = static_cast<const uint32_t*>(lk.sorted_keys);
-    const uint32_t k32 = (uint32_t)key;
-    while (lo < hi) {
-      const uint32_t mid = lo + ((hi - lo) >> 1);
-      if (sk[mid] < k32) lo = mid + 1u; else hi = mid;
-    }
-  }
-  return lo;
-#endif
 }
 
 // ktab holds the first sorted position of every key prefix that occurs (k_rerank, lazy) and 0xFFFFFFFF elsewhere; fill the
@@ -2087,6 +2076,7 @@ __global__ void __launch_bounds__(256, LAZY ? BWTC_SEG_MINB_LAZY : BWTC_SEG_MINB
   constexpr int IPT = SEG_CAP / 256;
   __shared__ unsigned long long s_key[SEG_CAP];
   __shared__ uint32_t s_id[SEG_CAP];
+  __shared__ unsigned long long s_k0[LAZY ? SEG_CAP : 1];  // lazy: round-0 key of suffix i+h (first part of cmp(i+h))
   __shared__ uint32_t s_wa[8], s_wb[8];
   __shared__ uint32_t s_start, s_end, s_base;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -2158,28 +2148,40 @@ __global__ void __launch_bounds__(256, LAZY ? BWTC_SEG_MINB_LAZY : BWTC_SEG_MINB
   uint32_t woff = 0, L = 0;
 #pragma unroll
   for (int w = 0; w < 8; ++w) { const uint32_t t = s_wa[w]; if (w < warp) woff += t; L += t; }
-  {
+  if constexpr (!LAZY) {
     uint32_t lo[IPT];
-    if (!LAZY) {
 #pragma unroll
-      for (int k = 0; k < IPT; ++k) {  // independent gathers first (all in flight together), shared-memory writes after
-        lo[k] = 0;
-        if (((livemask >> k) & 1u) && h < N - myid[k]) lo[k] = (rank[myid[k] + h] & RANK_MASK) + 1u;
-      }
-    } else {  // lazy ranks: a singleton's rank is found in the sorted round-0 keys (LookupParams live in global memory)
-      // (one search after the other: running the IPT searches of a thread in lockstep, IPT independent loads per step, was
-      // measured SLOWER — the look-ups are bound by random DRAM sectors, not by the dependent chain: r02_experiments.md)
-#pragma unroll
-      for (int k = 0; k < IPT; ++k) {
-        lo[k] = 0;
-        if (((livemask >> k) & 1u) && h < N - myid[k]) lo[k] = rank_lookup(*lkp, rank, myid[k] + h) + 1u;
-      }
+    for (int k = 0; k < IPT; ++k) {  // independent gathers first (all in flight together), shared-memory writes after
+      lo[k] = 0;
+      if (((livemask >> k) & 1u) && h < N - myid[k]) lo[k] = (rank[myid[k] + h] & RANK_MASK) + 1u;
     }
     uint32_t pos = woff + inc - cnt;
 #pragma unroll
     for (int k = 0; k < IPT; ++k) {
       if ((livemask >> k) & 1u) {
         s_key[pos] = ((unsigned long long)mynr[k] << 32) | lo[k];
+        s_id[pos] = myid[k];
+        ++pos;
+      }
+    }
+  } else {
+    // Lazy ranks (DESIGN.md §3.9): the integer rank of i+h is not needed, only the order and equality of the members of a
+    // group, and cmp(j) = (round-0 key of j, livebits(j) ? rank[j] + 1 : 0xFFFFFFFF) gives both — no search.  A suffix
+    // with i+h >= N gets (0, 0), below every real cmp (those have a second part >= 1), as the 0 of the full path.
+    uint32_t pos = woff + inc - cnt;
+#pragma unroll
+    for (int k = 0; k < IPT; ++k) {
+      if ((livemask >> k) & 1u) {
+        unsigned long long k0 = 0;
+        uint32_t lo = 0;
+        if (h < N - myid[k]) {
+          const uint32_t j = myid[k] + h;
+          const uint32_t lw = lkp->livebits[j >> 5];  // (issued before the key's text loads)
+          k0 = round0_key(*lkp, j);
+          lo = ((lw >> (j & 31u)) & 1u) ? (rank[j] & RANK_MASK) + 1u : 0xFFFFFFFFu;
+        }
+        s_key[pos] = ((unsigned long long)mynr[k] << 32) | lo;
+        s_k0[pos] = k0;
         s_id[pos] = myid[k];
         ++pos;
       }
@@ -2205,16 +2207,42 @@ __global__ void __launch_bounds__(256, LAZY ? BWTC_SEG_MINB_LAZY : BWTC_SEG_MINB
         ireg[k] = s_id[j];
         const uint32_t g = (uint32_t)(kreg[k] >> 32);
         uint32_t cntb = 0, gs = j;
-        for (uint32_t q = j; q-- > 0;) {
-          const unsigned long long kq = s_key[q];
-          if ((uint32_t)(kq >> 32) != g) break;
-          cntb += (kq <= kreg[k]) ? 1u : 0u;
-          gs = q;
-        }
-        for (uint32_t q = j + 1; q < L; ++q) {
-          const unsigned long long kq = s_key[q];
-          if ((uint32_t)(kq >> 32) != g) break;
-          cntb += (kq < kreg[k]) ? 1u : 0u;
+        if constexpr (!LAZY) {
+          for (uint32_t q = j; q-- > 0;) {
+            const unsigned long long kq = s_key[q];
+            if ((uint32_t)(kq >> 32) != g) break;
+            cntb += (kq <= kreg[k]) ? 1u : 0u;
+            gs = q;
+          }
+          for (uint32_t q = j + 1; q < L; ++q) {
+            const unsigned long long kq = s_key[q];
+            if ((uint32_t)(kq >> 32) != g) break;
+            cntb += (kq < kreg[k]) ? 1u : 0u;
+          }
+        } else {
+          // order by cmp = (s_k0, low word of s_key).  My key for the re-rank below becomes (old rank, number of group
+          // members with a smaller cmp): it orders and ties exactly as cmp does
+          const unsigned long long k0 = s_k0[j];
+          const uint32_t lo = (uint32_t)kreg[k];
+          uint32_t nlt = 0;
+          for (uint32_t q = j; q-- > 0;) {
+            const unsigned long long kq = s_key[q];
+            if ((uint32_t)(kq >> 32) != g) break;
+            const unsigned long long k0q = s_k0[q];
+            const bool lt = k0q < k0 || (k0q == k0 && (uint32_t)kq < lo);
+            nlt += lt ? 1u : 0u;
+            cntb += (lt || (k0q == k0 && (uint32_t)kq == lo)) ? 1u : 0u;
+            gs = q;
+          }
+          for (uint32_t q = j + 1; q < L; ++q) {
+            const unsigned long long kq = s_key[q];
+            if ((uint32_t)(kq >> 32) != g) break;
+            const unsigned long long k0q = s_k0[q];
+            const bool lt = k0q < k0 || (k0q == k0 && (uint32_t)kq < lo);
+            nlt += lt ? 1u : 0u;
+            cntb += lt ? 1u : 0u;
+          }
+          kreg[k] = ((unsigned long long)g << 32) | nlt;
         }
         npos[k] = gs + cntb;
       }
