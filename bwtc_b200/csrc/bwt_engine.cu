@@ -33,11 +33,8 @@ constexpr uint32_t RS_TILE64 = RS_BLOCK * RS_IPT64;
 constexpr uint32_t RS_TILE32 = RS_BLOCK * RS_IPT32;
 constexpr uint32_t AUX_TILE = 2048;  // k_pack_round0 / k_build_keys / k_rerank tile
 constexpr int MAX_PASSES = 8;
-constexpr uint32_t GRAM_OFF = MAX_PASSES * 512;    // the gram histogram of k_pack_round0 sits behind the digit histograms
-constexpr uint32_t HIST_WORDS = GRAM_OFF + (1u << GRAM_BITS);  // digit histograms of one sort: pass p at p << rb (rb = 8 or 9 bits)
-// Words per look-back status row: 256 (8-bit digits), 512 when the 9-bit digit passes are enabled (BWTC_RADIX9=1).
-inline uint32_t status_row_words_for(int use_radix9) { return use_radix9 ? 512u : 256u; }
-inline int env_radix9() { const char* e = getenv("BWTC_RADIX9"); return e ? atoi(e) : 0; }
+constexpr uint32_t GRAM_OFF = MAX_PASSES * 256;    // the gram histogram of k_pack_round0 sits behind the digit histograms
+constexpr uint32_t HIST_WORDS = GRAM_OFF + (1u << GRAM_BITS);  // digit histograms of one sort: pass p at p << 8
 constexpr uint32_t TEXT_PAD = 64;
 
 thread_local char g_err[512] = "";
@@ -93,7 +90,7 @@ struct bwtc_cuda_ctx {
   uint8_t* d_aux[2] = {nullptr, nullptr};    // ping-pong one-byte payload of the round-0 sort (predecessor codes), N each
   uint32_t* d_scat = nullptr;     // u32[N]: staged ranks of the bucketed scatter (the ids go to the idle id buffer)
   uint32_t* d_zero = nullptr;     // [ctrl CTR_WORDS][hist HIST_WORDS][tstate rows of max_aux_tiles] zeroed per round
-  uint32_t* d_status = nullptr;   // [MAX_PASSES][LB_PAD_ROWS + max_rs_tiles][status_row_words] radix look-back words; the pad rows in
+  uint32_t* d_status = nullptr;   // [MAX_PASSES][LB_PAD_ROWS + max_rs_tiles][256] radix look-back words; the pad rows in
                                   // front of every pass hold "prefix 0" for ever, so a walk needs no bounds check
   uint32_t* d_tilecnt = nullptr;  // [2][max_aux_tiles]: per-tile live counts of k_rerank and their exclusive prefix,
                                   // then [max_aux_tiles][MAX_RERANK_WINDOWS+1] bucket offsets of the bucketed scatter
@@ -128,24 +125,11 @@ struct bwtc_cuda_ctx {
   int debug_corrupt_out = 0;      // test hook: one byte of the forward output is changed before it is verified
   uint32_t debug_corrupt_lf = 0;  // test hook (j >= 1): LFpowers[j] is changed on the device before it is verified
   int64_t debug_corrupt_sa = -1;  // test hook (r >= 0): SA[r] and SA[r+1] are swapped on the device before they are verified
-  int d2h_kernel = 0;             // BWTC_D2H_KERNEL=1: result copies to pinned host buffers by a copying kernel (k_copy_out)
-                                  // instead of the copy engine — measured no better (profiles/r02_experiments.md), kept as a knob
-  int d2h_ctas = 16;
   int debug_skip_copies = 0;      // timing experiments only (bit 0: no H2D of host blocks, bit 1: no D2H): results are WRONG
   int ladder_first = 2, ladder_more = 4;  // segmented rounds enqueued speculatively behind a sort round / per retry
-  int use_radix9 = 0;             // BWTC_RADIX9=1: 9-bit digits for 64-bit-key sorts whenever that saves a pass.  Measured
-                                  // slower (a 9-bit pass costs +23%, 7 of them more than 8 eight-bit ones): kept as an
-                                  // experiment, profiles/r02_experiments.md
-  uint32_t status_row_words = 256;
   int use_partial = 1;            // spare low bits of the round-0 key take the top bits of the next character (BWTC_PARTIAL=0: zeros)
   int use_gram = 1;               // round-0 digit histograms projected from one 12-bit gram histogram (6- and 3-bit codes; BWTC_GRAM=0:
                                   // counted per digit class + k_hist_derive)
-  int twopass = 0;                // BWTC_TWOPASS=1: with two L2 windows the second window is scattered by k_scatter_window from the
-                                  // rank words the first k_rerank launch stored in sorted order, instead of a second k_rerank
-                                  // launch (measured: Markov 32 MiB equal, source text -3%; the random scatter itself is the cost)
-  int hybrid2 = 0;                // BWTC_HYBRID2=1: with two L2 windows, window 0 is written directly and window 1 staged + one
-                                  // k_scatter_bucket, instead of one k_rerank launch per window (measured equal: 2.90 vs 2.88 ms)
-  uint32_t rerank_pf_tiles = 0;   // k_rerank: L2 prefetch distance in tiles (BWTC_RERANK_PF; 0 = off)
   int use_lazy = 1;               // lazy ranks after round 0 (DESIGN.md §3.9): 0 never, 1 when the key-shape policy predicts
                                   // that few suffixes stay in groups, 2 always (tests)
   uint32_t lazy_min_suffixes = 4u << 20;
@@ -185,10 +169,10 @@ struct bwtc_cuda_ctx {
 
 namespace {
 
-template <typename KeyT, int IPT, bool IOTA, bool AUX, int RB = 8>
+template <typename KeyT, int IPT, bool IOTA, bool AUX>
 int set_pass_attr(bwtc_cuda_ctx* ctx) {
-  CK(ctx, cudaFuncSetAttribute(k_radix_pass<KeyT, RS_BLOCK, IPT, IOTA, AUX, RB>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               (int)RadixPassSmem<KeyT, RS_BLOCK, IPT, AUX, RB>::bytes));
+  CK(ctx, cudaFuncSetAttribute(k_radix_pass<KeyT, RS_BLOCK, IPT, IOTA, AUX>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               (int)RadixPassSmem<KeyT, RS_BLOCK, IPT, AUX>::bytes));
   return 0;
 }
 
@@ -221,7 +205,6 @@ void ctx_free(bwtc_cuda_ctx* c) {
 
 struct Round0Plan {
   uint32_t sigma, bits, chars, keybytes, npass;
-  uint32_t rb;        // digit width of the round-0 sort: 9 when that saves a pass over 8-bit digits (64-bit keys only)
   uint32_t rbits;     // spare low key bits filled with the top bits of character c+1 (PackParams::rbits)
   PackParams pp;
   bool has_memory;    // the 8-gram sample says the source is not i.i.d.-like (text, repeats)
@@ -309,15 +292,10 @@ void plan_round0(const bwtc_cuda_ctx* ctx, const uint64_t* count, const bool* pr
   pl->chars = chars;
   pl->keybytes = keybytes;
   pl->npass = div_up((uint64_t)chars * b + blk_bits, 8);
-  pl->rb = 8;
-  if (ctx->use_radix9 && keybytes == 8 && div_up((uint64_t)chars * b + blk_bits, 9) < pl->npass) {
-    pl->rb = 9;
-    pl->npass = div_up((uint64_t)chars * b + blk_bits, 9);
-  }
   {
-    // the digit passes cover rb * npass bits (at most the key width): what the c characters leave over takes the top bits
+    // the digit passes cover 8 npass bits (at most the key width): what the c characters leave over takes the top bits
     // of the next character (never a whole one: the chooser above already uses every whole character that fits)
-    const uint32_t covered = std::min<uint32_t>(pl->rb * pl->npass, keybytes * 8u);
+    const uint32_t covered = std::min<uint32_t>(8u * pl->npass, keybytes * 8u);
     const uint32_t used = chars * b + blk_bits;
     uint32_t r = (ctx->use_partial && blk_bits == 0 && covered > used) ? covered - used : 0u;
     if (r >= b) r = b - 1u;
@@ -355,10 +333,9 @@ inline uint32_t tile_slot(const bwtc_cuda_ctx* ctx, uint32_t ticket_word) {
   return ctx->debug_reverse_tiles ? CTR_STATIC_REV : CTR_STATIC;
 }
 
-// Row 0 of the look-back status words of digit pass p (LB_PAD_ROWS rows of "prefix 0" words sit in front of it, for
-// either row width).
+// Row 0 of the look-back status words of digit pass p (LB_PAD_ROWS rows of "prefix 0" words sit in front of it).
 inline uint32_t* status_rows(const bwtc_cuda_ctx* ctx, int p) {
-  return ctx->d_status + ((size_t)p * (ctx->max_rs_tiles + LB_PAD_ROWS) + LB_PAD_ROWS) * ctx->status_row_words;
+  return ctx->d_status + ((size_t)p * (ctx->max_rs_tiles + LB_PAD_ROWS) + LB_PAD_ROWS) * 256;
 }
 
 struct PassTimer {
@@ -381,12 +358,12 @@ struct PassTimer {
 
 // One LSD radix sort of m records: executes the digit passes whose bit is set in pass_mask, ping-ponging
 // between buffer 0 and 1.  Records start in buffer `cur` (0); returns the buffer holding the result.
-template <typename KeyT, int IPT, bool AUX, int RB = 8>
+template <typename KeyT, int IPT, bool AUX>
 int run_sort_impl(bwtc_cuda_ctx* ctx, uint32_t m, uint32_t pass_mask, bool first_iota, uint32_t iota_top, int* cur_io,
                   PassTimer* pt, uint32_t* passes_done, uint32_t pack_bits, uint32_t topshift, uint32_t pred_mask) {
   constexpr uint32_t TILE = RS_BLOCK * IPT;
   const uint32_t tiles = div_up(m, TILE);
-  const size_t smem = RadixPassSmem<KeyT, RS_BLOCK, IPT, AUX, RB>::bytes;
+  const size_t smem = RadixPassSmem<KeyT, RS_BLOCK, IPT, AUX>::bytes;
   int cur = *cur_io;
   bool iota = first_iota;
   uint32_t done = 0;
@@ -397,13 +374,13 @@ int run_sort_impl(bwtc_cuda_ctx* ctx, uint32_t m, uint32_t pass_mask, bool first
     uint32_t* status = status_rows(ctx, p);
     if (pt->begin()) return BWTC_CUDA_ECUDA;
     if (iota)
-      k_radix_pass<KeyT, RS_BLOCK, IPT, true, AUX, RB><<<tiles, RS_BLOCK, smem, ctx->stream>>>(
-          kin, nullptr, kout, ctx->d_idx[cur ^ 1], m, (uint32_t)RB * p, ctx->d_hist() + ((size_t)p << RB), status, ctx->d_ctrl(),
+      k_radix_pass<KeyT, RS_BLOCK, IPT, true, AUX><<<tiles, RS_BLOCK, smem, ctx->stream>>>(
+          kin, nullptr, kout, ctx->d_idx[cur ^ 1], m, 8u * p, ctx->d_hist() + ((size_t)p << 8), status, ctx->d_ctrl(),
           tile_slot(ctx, (uint32_t)(CTR_PASS0 + p)), iota_top, pack_bits, topshift, pred_mask, nullptr,
           ctx->d_aux[cur ^ 1]);
     else
-      k_radix_pass<KeyT, RS_BLOCK, IPT, false, AUX, RB><<<tiles, RS_BLOCK, smem, ctx->stream>>>(
-          kin, ctx->d_idx[cur], kout, ctx->d_idx[cur ^ 1], m, (uint32_t)RB * p, ctx->d_hist() + ((size_t)p << RB), status,
+      k_radix_pass<KeyT, RS_BLOCK, IPT, false, AUX><<<tiles, RS_BLOCK, smem, ctx->stream>>>(
+          kin, ctx->d_idx[cur], kout, ctx->d_idx[cur ^ 1], m, 8u * p, ctx->d_hist() + ((size_t)p << 8), status,
           ctx->d_ctrl(), tile_slot(ctx, (uint32_t)(CTR_PASS0 + p)), iota_top, 0u, 0u, 0u, ctx->d_aux[cur], ctx->d_aux[cur ^ 1]);
     CK(ctx, cudaGetLastError());
     if (pt->end()) return BWTC_CUDA_ECUDA;
@@ -424,21 +401,11 @@ int run_sort_impl(bwtc_cuda_ctx* ctx, uint32_t m, uint32_t pass_mask, bool first
 // One LSD radix sort of m records: executes the digit passes whose bit is set in pass_mask, ping-ponging
 // between buffer 0 and 1.  Records start in buffer `cur` (0); returns the buffer holding the result.
 // aux: a one-byte payload (predecessor character code) is produced by the first pass and carried along.
-// rb: digit width, 8 or 9 bits (9 only for 64-bit keys); pass p sorts on bits [rb*p, rb*p + rb).
+// Pass p sorts on bits [8p, 8p + 8).
 template <typename KeyT, int IPT>
 int run_sort(bwtc_cuda_ctx* ctx, uint32_t m, uint32_t pass_mask, bool first_iota, uint32_t iota_top, int* cur_io,
              PassTimer* pt, uint32_t* passes_done, uint32_t pack_bits = 0, uint32_t topshift = 0,
-             uint32_t pred_mask = 0xFFFFFFFFu, bool aux = false, uint32_t rb = 8) {
-  if constexpr (sizeof(KeyT) == 8) {
-    if (rb == 9) {
-      if (aux)
-        return run_sort_impl<KeyT, IPT, true, 9>(ctx, m, pass_mask, first_iota, iota_top, cur_io, pt, passes_done, pack_bits,
-                                                 topshift, pred_mask);
-      return run_sort_impl<KeyT, IPT, false, 9>(ctx, m, pass_mask, first_iota, iota_top, cur_io, pt, passes_done, pack_bits,
-                                                topshift, pred_mask);
-    }
-  }
-  if (rb != 8) { set_err(ctx->err, "run_sort: %u-bit digits are not built for this key type", rb); return BWTC_CUDA_EINTERNAL; }
+             uint32_t pred_mask = 0xFFFFFFFFu, bool aux = false) {
   if (aux)
     return run_sort_impl<KeyT, IPT, true>(ctx, m, pass_mask, first_iota, iota_top, cur_io, pt, passes_done, pack_bits, topshift,
                                           pred_mask);
@@ -446,7 +413,7 @@ int run_sort(bwtc_cuda_ctx* ctx, uint32_t m, uint32_t pass_mask, bool first_iota
                                          pred_mask);
 }
 
-int zero_round_state(bwtc_cuda_ctx* ctx, uint32_t N, uint32_t m, uint32_t rs_tile, uint32_t pass_mask, uint32_t rb = 8) {
+int zero_round_state(bwtc_cuda_ctx* ctx, uint32_t N, uint32_t m, uint32_t rs_tile, uint32_t pass_mask) {
   const uint32_t aux_tiles = div_up(m, AUX_TILE);
   CK(ctx, cudaMemsetAsync(ctx->d_zero + CTR_STICKY, 0,
                           (size_t)(CTR_WORDS - CTR_STICKY + HIST_WORDS) * 4 + (size_t)rerank_launches(ctx, N, m) * ctx->max_aux_tiles * 8,
@@ -454,7 +421,7 @@ int zero_round_state(bwtc_cuda_ctx* ctx, uint32_t N, uint32_t m, uint32_t rs_til
   const uint32_t tiles = div_up(m, rs_tile);
   for (int p = 0; p < MAX_PASSES; ++p)
     if ((pass_mask >> p) & 1u)
-      CK(ctx, cudaMemsetAsync(status_rows(ctx, p), 0, ((size_t)tiles * 4u) << rb, ctx->stream));
+      CK(ctx, cudaMemsetAsync(status_rows(ctx, p), 0, (size_t)tiles * 256 * 4, ctx->stream));
   return 0;
 }
 
@@ -480,51 +447,31 @@ int launch_rerank(bwtc_cuda_ctx* ctx, int cur, uint32_t m, uint32_t N, RerankPar
       else k_rerank<KeyT, ROUND0><<<tiles, 256, 0, st>>>(keys, ctx->d_idx[cur], ctx->d_rank, rp, tstate, ctx->d_ctrl(), ep, sp);
     }
   };
-  const bool hybrid2 = ctx->hybrid2 && nwin == 2u && !(ROUND0 && rp.lazy);
-  if ((ctx->bucket_min_windows && nwin >= (uint32_t)ctx->bucket_min_windows) || hybrid2) {
+  if (ctx->bucket_min_windows && nwin >= (uint32_t)ctx->bucket_min_windows) {
     const uint32_t win_ids = div_up(N, nwin);
     rp.win_lo = 0;
     rp.win_hi = 0xFFFFFFFFu;
     rp.emit = 1;
-    rp.pf_tiles = ctx->rerank_pf_tiles;
     rp.ctr_slot = tile_slot(ctx, (uint32_t)CTR_RERANK);
     rp.nbuckets = nwin;
-    rp.nr_out = nullptr;
-    rp.direct0 = hybrid2 ? 1u : 0u;
     rp.bucket_magic = (uint32_t)(((1ull << 32) + win_ids - 1) / win_ids);
     StageParams sp{stage_nr, stage_id, ctx->d_tilecnt, no_stage ? 0 : 1, ctx->d_idx[cur ^ 1], ctx->d_scat, woff};
     rerank(ctx->d_tstate(), sp);
     const uint32_t grid = std::min<uint32_t>(div_up(tiles, 8), (uint32_t)ctx->sm_count * 8u);
-    for (uint32_t b = hybrid2 ? 1u : 0u; b < nwin; ++b)
+    for (uint32_t b = 0; b < nwin; ++b)
       k_scatter_bucket<<<grid, 256, 0, st>>>(ctx->d_idx[cur ^ 1], ctx->d_scat, woff, tiles, nwin, b, AUX_TILE, ctx->d_rank, ctx->d_ctrl());
     CK(ctx, cudaGetLastError());
-    ctx->stats.kernel_launches += 1 + nwin - (hybrid2 ? 1u : 0u);
-    ctx->stats.algorithmic_bytes += (uint64_t)m * (hybrid2 ? 8 : 16);  // staged (id, rank) pairs: written once, read once
+    ctx->stats.kernel_launches += 1 + nwin;
+    ctx->stats.algorithmic_bytes += (uint64_t)m * 16;  // staged (id, rank) pairs: written once, read once
     return 0;
   }
-  // Two windows: the first launch also leaves every record's new rank word beside its id (d_scat, idle here), and the
-  // second window is served by the light k_scatter_window instead of a second full re-rank.
-  const bool twopass = ctx->twopass && nwin == 2u && !(ROUND0 && rp.lazy);
   for (uint32_t w = 0; w < nwin; ++w) {
     rp.win_lo = (uint32_t)((uint64_t)N * w / nwin);
     rp.win_hi = (w + 1 == nwin) ? 0xFFFFFFFFu : (uint32_t)((uint64_t)N * (w + 1) / nwin);
-    rp.nr_out = (twopass && w == 0) ? ctx->d_scat : nullptr;
-    if (twopass && w == 1) {
-      const uint32_t grid = std::min<uint32_t>(div_up(m, 1024u), (uint32_t)ctx->sm_count * 8u);
-      const uint32_t mask = ROUND0 ? rp.id_mask : 0x7FFFFFFFu;
-      k_scatter_window<<<grid, 256, 0, st>>>(ctx->d_idx[cur], ctx->d_scat, m, mask, rp.win_lo, rp.win_hi, ctx->d_rank, ctx->d_ctrl());
-      CK(ctx, cudaGetLastError());
-      ctx->stats.kernel_launches++;
-      ctx->stats.algorithmic_bytes += (uint64_t)m * 12;  // rank words written once, ids + rank words read once
-      break;
-    }
-    // round 0: the first window launch emits every BWT byte (whole words); so does the only k_rerank launch of a two-pass
-    // scatter in any round; otherwise every window launch emits for its own ids
-    rp.emit = (ROUND0 || twopass) ? (w == 0 ? 1u : 2u) : 0u;
-    rp.pf_tiles = ctx->rerank_pf_tiles;
+    // round 0: the first window launch emits every BWT byte (whole words); otherwise every window launch emits for its own ids
+    rp.emit = ROUND0 ? (w == 0 ? 1u : 2u) : 0u;
     rp.ctr_slot = tile_slot(ctx, (uint32_t)(CTR_RERANK + w));
     rp.nbuckets = 0;
-    rp.direct0 = 0;
     rp.bucket_magic = 0;
     StageParams sp{stage_nr, stage_id, ctx->d_tilecnt, (w == 0 && !no_stage) ? 1 : 0, nullptr, nullptr, nullptr};
     rerank(ctx->d_tstate() + (size_t)w * ctx->max_aux_tiles, sp);
@@ -619,18 +566,6 @@ bool is_pinned_host(const void* p) {
     return false;
   }
   return a.type == cudaMemoryTypeHost || a.type == cudaMemoryTypeManaged;
-}
-
-// Device-side alias of a pinned host buffer (unified addressing), or nullptr if it is not mapped into the device's
-// address space — then the copy engine is used.
-uint8_t* mapped_alias(void* p) {
-  cudaPointerAttributes a;
-  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
-    cudaGetLastError();
-    return nullptr;
-  }
-  if (a.type != cudaMemoryTypeHost) return nullptr;
-  return static_cast<uint8_t*>(a.devicePointer);
 }
 
 int ensure_ring(bwtc_cuda_ctx* ctx) {
@@ -880,7 +815,7 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
   // ---- round 0: pack keys (+ all digit histograms), sort, re-rank
   const uint32_t rs_tile0 = pl.keybytes == 4 ? RS_TILE32 : RS_TILE64;
   const uint32_t all0 = (1u << pl.npass) - 1u;
-  if (zero_round_state(ctx, N, N, rs_tile0, all0, pl.rb)) return BWTC_CUDA_ECUDA;
+  if (zero_round_state(ctx, N, N, rs_tile0, all0)) return BWTC_CUDA_ECUDA;
   {
     const uint32_t ptiles = div_up(N, AUX_TILE);
     const int grid = (int)(ptiles < (uint32_t)(ctx->sm_count * 4) ? ptiles : (uint32_t)(ctx->sm_count * 4));
@@ -894,18 +829,17 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
     uint32_t regular_mask = 0;  // digits that lie entirely inside the exact characters
     for (uint32_t p = 0; p < pl.npass; ++p) {
       int rep = -1;
-      const uint32_t rb = pl.rb;
-      const bool full_p = (rb * p >= rbits) && (rb * p - rbits + rb <= keybits);
+      const bool full_p = (8u * p >= rbits) && (8u * p - rbits + 8u <= keybits);
       if (full_p) regular_mask |= 1u << p;
       if (full_p && N > 64 && !bs)  // (a batch counts every digit directly: block numbers sit above the characters)
         for (uint32_t r = 0; r < p; ++r)
-          if (((hist_mask >> r) & (regular_mask >> r) & 1u) && (rb * (p - r)) % pl.bits == 0) { rep = (int)r; break; }
+          if (((hist_mask >> r) & (regular_mask >> r) & 1u) && (8u * (p - r)) % pl.bits == 0) { rep = (int)r; break; }
       if (rep < 0) {
         hist_mask |= 1u << p;
       } else {
         dp.p[dp.count] = (uint8_t)p;
         dp.r[dp.count] = (uint8_t)rep;
-        dp.t[dp.count] = (uint8_t)(pl.rb * (p - (uint32_t)rep) / pl.bits);
+        dp.t[dp.count] = (uint8_t)(8u * (p - (uint32_t)rep) / pl.bits);
         dp.count++;
       }
     }
@@ -919,18 +853,18 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
       for (uint32_t p = 0; p < pl.npass && use_gram; ++p) {
         uint32_t u, sft;
         gp.next[p] = 0;
-        if (pl.rb * p < rbits) {  // the lowest digit reaches into the partial character: window of the following suffix
+        if (8u * p < rbits) {  // the lowest digit reaches into the partial character: window of the following suffix
           if (p != 0) use_gram = false;
           u = 0;
           sft = pl.bits - rbits;
           gp.next[p] = 1;
-          if (sft + pl.rb > (uint32_t)GRAM_BITS) use_gram = false;
+          if (sft + 8u > (uint32_t)GRAM_BITS) use_gram = false;
         } else {
-          const uint32_t lo = pl.rb * p - rbits;
+          const uint32_t lo = 8u * p - rbits;
           u = std::min<uint32_t>(lo / pl.bits, pl.chars - W);
           sft = lo - pl.bits * u;
           // the digit must lie inside the 12 bits above bit (bits * u), or run past the top of the key (zeros there)
-          if (sft + pl.rb > (uint32_t)GRAM_BITS && lo + pl.rb <= keybits) use_gram = false;
+          if (sft + 8u > (uint32_t)GRAM_BITS && lo + 8u <= keybits) use_gram = false;
         }
         if (sft >= 32u) use_gram = false;
         gp.u[p] = (uint8_t)u;
@@ -942,15 +876,14 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
     if (use_gram) { hist_mask = 0; dp.count = 0; }
     if (pl.keybytes == 4) {
       k_pack_round0<uint32_t><<<grid, 256, 0, st>>>(d_text, N, static_cast<uint32_t*>(ctx->d_keys[0]), pl.pp,
-                                                     ctx->d_hist(), hist_mask, ptiles, pl.rb, gram);
-      if (dp.count) k_hist_derive<uint32_t><<<dp.count, 256, 0, st>>>(d_text, N, pl.pp, dp, ctx->d_hist(), pl.rb);
-      if (use_gram) k_hist_from_gram<uint32_t><<<gp.npass, 256, 0, st>>>(d_text, N, pl.pp, gp, gram, ctx->d_hist(), pl.rb);
+                                                     ctx->d_hist(), hist_mask, ptiles, gram);
+      if (dp.count) k_hist_derive<uint32_t><<<dp.count, 256, 0, st>>>(d_text, N, pl.pp, dp, ctx->d_hist());
+      if (use_gram) k_hist_from_gram<uint32_t><<<gp.npass, 256, 0, st>>>(d_text, N, pl.pp, gp, gram, ctx->d_hist());
     } else {
       k_pack_round0<unsigned long long><<<grid, 256, 0, st>>>(d_text, N, static_cast<unsigned long long*>(ctx->d_keys[0]),
-                                                               pl.pp, ctx->d_hist(), hist_mask, ptiles, pl.rb, gram);
-      if (dp.count) k_hist_derive<unsigned long long><<<dp.count, 256, 0, st>>>(d_text, N, pl.pp, dp, ctx->d_hist(), pl.rb);
-      if (use_gram)
-        k_hist_from_gram<unsigned long long><<<gp.npass, 256, 0, st>>>(d_text, N, pl.pp, gp, gram, ctx->d_hist(), pl.rb);
+                                                               pl.pp, ctx->d_hist(), hist_mask, ptiles, gram);
+      if (dp.count) k_hist_derive<unsigned long long><<<dp.count, 256, 0, st>>>(d_text, N, pl.pp, dp, ctx->d_hist());
+      if (use_gram) k_hist_from_gram<unsigned long long><<<gp.npass, 256, 0, st>>>(d_text, N, pl.pp, gp, gram, ctx->d_hist());
     }
     if (dp.count || use_gram) S.kernel_launches++;
     CK(ctx, cudaGetLastError());
@@ -978,7 +911,7 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
                                       pred_mask, aux_pred);
   else
     rc = run_sort<unsigned long long, RS_IPT64>(ctx, N, mask0, true, N - 1, &cur, &pt, &pdone, pack_pred ? id_bits : 0u,
-                                                topshift, pred_mask, aux_pred, pl.rb);
+                                                topshift, pred_mask, aux_pred);
   if (rc) return rc;
   const size_t round0_events = pt.used;
   S.sort0_launches = S.sort_launches;
@@ -1120,14 +1053,7 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
                                 bs->on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, st));
       }
     } else if (!J.out_dev && !(ctx->debug_skip_copies & 2)) {
-      uint8_t* alias = ctx->d2h_kernel ? mapped_alias(J.h_out) : nullptr;
-      if (alias) {
-        k_copy_out<<<ctx->d2h_ctas, 256, 0, st>>>(ctx->d_out, alias, n, ctx->d_state, ctx->d_ctrl());
-        CK(ctx, cudaGetLastError());
-        S.kernel_launches++;
-      } else {
-        CK(ctx, cudaMemcpyAsync(J.h_out, ctx->d_out, n, cudaMemcpyDeviceToHost, st));
-      }
+      CK(ctx, cudaMemcpyAsync(J.h_out, ctx->d_out, n, cudaMemcpyDeviceToHost, st));
     }
     return 0;
   };
@@ -1135,11 +1061,7 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
   const int lo_bits = (int)ceil_log2_u64((uint64_t)N + 1);  // rank[i+h] + 1 in [0, N]
   // high part = (rank of the group head) >> 1 (k_build_keys): heads of live groups are <= N - 2
   const int hi_bits = N > 3 ? (int)ceil_log2_u64((((uint64_t)N - 2) >> 1) + 1) : 1;
-  uint32_t npassd = div_up((uint64_t)(lo_bits + hi_bits), 8), rbd = 8;
-  if (ctx->use_radix9 && div_up((uint64_t)(lo_bits + hi_bits), 9) < npassd) {  // 9-bit digits when they save a pass
-    npassd = div_up((uint64_t)(lo_bits + hi_bits), 9);
-    rbd = 9;
-  }
+  const uint32_t npassd = div_up((uint64_t)(lo_bits + hi_bits), 8);
   const uint32_t maskd = (1u << npassd) - 1u;
   bool lists_pending = true, first_chunk = true, out_enqueued = false, finished = false;
   // lean chunk: behind a global radix round whose groups were still far above the segmented-round limit nothing sort-free
@@ -1301,7 +1223,7 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
       set_err(ctx->err, "internal: global sort requested after a segmented round (maxgroup %u)", H.maxgroup);
       return BWTC_CUDA_EINTERNAL;
     }
-    if (zero_round_state(ctx, N, m, RS_TILE64, maskd, rbd)) return BWTC_CUDA_ECUDA;
+    if (zero_round_state(ctx, N, m, RS_TILE64, maskd)) return BWTC_CUDA_ECUDA;
     uint32_t expect_cursor = 0xFFFFFFFFu;
     if (from_list) {
       if (!have_lists) {
@@ -1314,7 +1236,7 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
       const int grid = (int)(bt < (uint32_t)(ctx->sm_count * 8) ? bt : (uint32_t)(ctx->sm_count * 8));
       k_build_from_list<<<grid, 256, 0, st>>>(pool.p[2 * cur + 1], m, ctx->d_rank, N, h32, lo_bits,
                                               static_cast<unsigned long long*>(ctx->d_keys[tb]), ctx->d_idx[tb],
-                                              ctx->d_hist(), (int)npassd, ctx->d_ctrl(), rbd);
+                                              ctx->d_hist(), (int)npassd, ctx->d_ctrl());
       CK(ctx, cudaGetLastError());
       S.kernel_launches++;
       S.algorithmic_bytes += (uint64_t)m * (4 + 8 + 12);
@@ -1323,14 +1245,14 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
       const uint32_t btiles = div_up(N, AUX_TILE);
       const int grid = (int)(btiles < (uint32_t)(ctx->sm_count * 8) ? btiles : (uint32_t)(ctx->sm_count * 8));
       k_build_keys<<<grid, 256, 0, st>>>(ctx->d_rank, N, h32, lo_bits, static_cast<unsigned long long*>(ctx->d_keys[0]),
-                                         ctx->d_idx[0], ctx->d_ctrl(), ctx->d_hist(), (int)npassd, btiles, rbd);
+                                         ctx->d_idx[0], ctx->d_ctrl(), ctx->d_hist(), (int)npassd, btiles);
       CK(ctx, cudaGetLastError());
       S.kernel_launches++;
       S.algorithmic_bytes += (uint64_t)N * 4 + (uint64_t)m * 12;
       cur = 0;
       expect_cursor = m;
     }
-    rc = run_sort<unsigned long long, RS_IPT64>(ctx, m, maskd, false, 0, &cur, &pt, &pdone, 0, 0, 0xFFFFFFFFu, false, rbd);
+    rc = run_sort<unsigned long long, RS_IPT64>(ctx, m, maskd, false, 0, &cur, &pt, &pdone);
     if (rc) return rc;
     {
       RerankParams rp;
@@ -1993,8 +1915,6 @@ int bwtc_cuda_ctx_create(bwtc_cuda_ctx** out, int device, uint32_t max_block_byt
   if (const char* e = getenv("BWTC_DEBUG_CORRUPT_LF")) c->debug_corrupt_lf = (uint32_t)std::max(0, atoi(e));
   if (const char* e = getenv("BWTC_DEBUG_CORRUPT_SA")) c->debug_corrupt_sa = std::max(-1L, atol(e));
   if (const char* e = getenv("BWTC_DEBUG_SKIP_COPIES")) c->debug_skip_copies = atoi(e);
-  if (const char* e = getenv("BWTC_D2H_KERNEL")) c->d2h_kernel = atoi(e);
-  if (const char* e = getenv("BWTC_D2H_CTAS")) c->d2h_ctas = std::max(1, atoi(e));
   if (const char* e = getenv("BWTC_SPIN_WAIT")) c->wait_mode = atoi(e) ? 1 : 0;
   if (const char* e = getenv("BWTC_WAIT_MODE")) c->wait_mode = atoi(e);
   if (const char* e = getenv("BWTC_POLL_SPIN_US")) c->poll_spin_us = std::max(0, atoi(e));
@@ -2002,13 +1922,8 @@ int bwtc_cuda_ctx_create(bwtc_cuda_ctx** out, int device, uint32_t max_block_byt
   if (const char* e = getenv("BWTC_LADDER_FIRST")) c->ladder_first = std::max(0, atoi(e));
   if (const char* e = getenv("BWTC_LADDER_MORE")) c->ladder_more = std::max(1, atoi(e));
   if (const char* e = getenv("BWTC_LAZY")) c->use_lazy = atoi(e);
-  if (const char* e = getenv("BWTC_HYBRID2")) c->hybrid2 = atoi(e);
-  if (const char* e = getenv("BWTC_TWOPASS")) c->twopass = atoi(e);
   if (const char* e = getenv("BWTC_GRAM")) c->use_gram = atoi(e);
   if (const char* e = getenv("BWTC_PARTIAL")) c->use_partial = atoi(e);
-  if (const char* e = getenv("BWTC_RERANK_PF")) c->rerank_pf_tiles = (uint32_t)std::max(0, atoi(e));
-  c->use_radix9 = env_radix9();
-  c->status_row_words = status_row_words_for(c->use_radix9);
   if (const char* e = getenv("BWTC_LAZY_MIN_MIB")) c->lazy_min_suffixes = (uint32_t)std::max(0L, atol(e)) << 20;
   if (const char* e = getenv("BWTC_LAZY_MAX_LIVE")) c->lazy_max_live = atof(e);
   if (const char* e = getenv("BWTC_LAZY_MAX_REPEATS")) c->lazy_max_repeats = atof(e);
@@ -2059,7 +1974,7 @@ int bwtc_cuda_ctx_create(bwtc_cuda_ctx** out, int device, uint32_t max_block_byt
   ALLOC(c->d_idx[0], N * 4);
   ALLOC(c->d_idx[1], N * 4);
   ALLOC(c->d_zero, (size_t)(CTR_WORDS + HIST_WORDS) * 4 + (size_t)MAX_RERANK_WINDOWS * c->max_aux_tiles * 8 + 64);
-  ALLOC(c->d_status, (size_t)MAX_PASSES * (c->max_rs_tiles + LB_PAD_ROWS) * c->status_row_words * 4u);
+  ALLOC(c->d_status, (size_t)MAX_PASSES * (c->max_rs_tiles + LB_PAD_ROWS) * 256 * 4u);
   ALLOC(c->d_LF, (size_t)LF_WORDS * 4);
   ALLOC(c->d_state, sizeof(LadderState));
   ALLOC(c->d_livebits, (N / 32 + 4) * 4);
@@ -2074,7 +1989,7 @@ int bwtc_cuda_ctx_create(bwtc_cuda_ctx** out, int device, uint32_t max_block_byt
   ALLOC(c->d_aux[1], padded);
 #undef ALLOC
   if (!rc) {  // pad rows of the look-back status: "inclusive prefix = 0", never overwritten
-    std::vector<uint32_t> pad((size_t)LB_PAD_ROWS * c->status_row_words, LB_PAD_WORD);
+    std::vector<uint32_t> pad((size_t)LB_PAD_ROWS * 256, LB_PAD_WORD);
     for (int p = 0; p < MAX_PASSES && !rc; ++p) {
       e = cudaMemcpy(status_rows(c, p) - pad.size(), pad.data(), pad.size() * 4, cudaMemcpyHostToDevice);
       if (e != cudaSuccess) { set_err(g_err, "cudaMemcpy(status pad): %s", cudaGetErrorString(e)); rc = BWTC_CUDA_ECUDA; }
@@ -2110,10 +2025,6 @@ int bwtc_cuda_ctx_create(bwtc_cuda_ctx** out, int device, uint32_t max_block_byt
     r2 |= set_pass_attr<uint32_t, RS_IPT32, false, true>(c);
     r2 |= set_pass_attr<unsigned long long, RS_IPT64, true, true>(c);
     r2 |= set_pass_attr<unsigned long long, RS_IPT64, false, true>(c);
-    r2 |= set_pass_attr<unsigned long long, RS_IPT64, true, false, 9>(c);
-    r2 |= set_pass_attr<unsigned long long, RS_IPT64, false, false, 9>(c);
-    r2 |= set_pass_attr<unsigned long long, RS_IPT64, true, true, 9>(c);
-    r2 |= set_pass_attr<unsigned long long, RS_IPT64, false, true, 9>(c);
     if (r2) { set_err(g_err, "%s", c->err); rc = BWTC_CUDA_ECUDA; }
   }
   if (rc) { ctx_free(c); return rc; }
@@ -2142,7 +2053,7 @@ uint64_t bwtc_cuda_scratch_bytes(uint32_t max_block_bytes) {
   b += 2 * (N * 8 + 64) + 2 * N * 4;                        // d_keys[2], d_idx[2]
   b += N * 4 + 64;                                          // d_scat
   b += (uint64_t)(CTR_WORDS + HIST_WORDS) * 4 + (uint64_t)MAX_RERANK_WINDOWS * aux_tiles * 8 + 64;  // d_zero
-  b += (uint64_t)MAX_PASSES * (rs_tiles + LB_PAD_ROWS) * status_row_words_for(env_radix9()) * 4u;     // d_status
+  b += (uint64_t)MAX_PASSES * (rs_tiles + LB_PAD_ROWS) * 256 * 4u;                         // d_status
   b += (uint64_t)LF_WORDS * 4 + sizeof(LadderState) + (uint64_t)MAX_BATCH * 256 * 4 + (uint64_t)MAX_BATCH * sizeof(void*);
   b += (uint64_t)WS_SLOTS * 12 + 64;                        // d_wtab
   b += aux_tiles * (2 + MAX_RERANK_WINDOWS + 1) * 4 + 64;   // d_tilecnt

@@ -62,11 +62,6 @@ constexpr int LB_PAD_ROWS = 8;  // rows of "prefix 0" in front of tile 0 (>= LB_
 // and a round trip of RT cycles the look-back settles at L = RT / (1 - RT / (dt * BATCH)): the batch must
 // satisfy dt * BATCH >> RT or the walk chases an ever longer chain of aggregate-only predecessors.
 constexpr int LB_BATCH = BWTC_LB_BATCH;
-#ifndef BWTC_LB_BATCH9
-#define BWTC_LB_BATCH9 2
-#endif
-constexpr int LB_BATCH9 = BWTC_LB_BATCH9;  // per digit in the 9-bit pass (two digits per thread); measured 2/4/6/8: 1.894/1.905/1.935/1.990 ms per sort
-static_assert(LB_BATCH9 <= LB_PAD_ROWS, "the look-back batch must not read past the pad rows");
 static_assert(LB_BATCH <= LB_PAD_ROWS, "the look-back batch must not read past the pad rows");
 
 // Record streams of k_radix_pass: plain loads, streaming (evict-first) stores.  Measured on the 32 MiB Markov block:
@@ -151,27 +146,6 @@ __device__ __forceinline__ uint32_t match_digit8(uint32_t d) {
   return m;
 }
 
-// The same with 9 ballots (9-bit digits, BWTC radix-9 passes).
-__device__ __forceinline__ uint32_t match_digit9(uint32_t d) {
-  uint32_t m = 0xFFFFFFFFu;
-#pragma unroll
-  for (int b = 0; b < 9; ++b) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        ".reg .b32 t;\n"
-        "and.b32 t, %1, %2;\n"
-        "setp.ne.u32 p, t, 0;\n"
-        "vote.sync.ballot.b32 t, p, 0xffffffff;\n"
-        "@p and.b32 %0, %0, t;\n"
-        "@!p lop3.b32 %0, %0, t, 0, 0x30;\n"
-        "}\n"
-        : "+r"(m)
-        : "r"(d), "r"(1u << b));
-  }
-  return m;
-}
-
 // Exclusive sum-scan over the first 256 threads of the CTA (value of threads >= 256 is ignored).
 // Every thread of the CTA must call it (contains __syncthreads). s_tot: 8 words of shared memory.
 __device__ __forceinline__ uint32_t scan256_excl(uint32_t v, uint32_t* s_tot) {
@@ -192,34 +166,6 @@ __device__ __forceinline__ uint32_t scan256_excl(uint32_t v, uint32_t* s_tot) {
   }
   __syncthreads();
   return base + inc - v;
-}
-
-// Two exclusive sum-scans over the 256 threads of the CTA at once (same barriers); tot0 / tot1 receive the totals.
-// s_tot: 16 words of shared memory.
-__device__ __forceinline__ void scan256_excl2(uint32_t v0, uint32_t v1, uint32_t* s_tot, uint32_t& e0, uint32_t& e1,
-                                              uint32_t& tot0, uint32_t& tot1) {
-  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
-  uint32_t i0 = v0, i1 = v1;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const uint32_t t0 = __shfl_up_sync(0xFFFFFFFFu, i0, o);
-    const uint32_t t1 = __shfl_up_sync(0xFFFFFFFFu, i1, o);
-    if (lane >= o) { i0 += t0; i1 += t1; }
-  }
-  if (w < 8 && lane == 31) { s_tot[w] = i0; s_tot[8 + w] = i1; }
-  __syncthreads();
-  uint32_t b0 = 0, b1 = 0, a0 = 0, a1 = 0;
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    const uint32_t t0 = s_tot[i], t1 = s_tot[8 + i];
-    a0 += t0; a1 += t1;
-    if (i < w) { b0 += t0; b1 += t1; }
-  }
-  __syncthreads();
-  e0 = b0 + i0 - v0;
-  e1 = b1 + i1 - v1;
-  tot0 = a0;
-  tot1 = a1;
 }
 
 // =====================================================================================================
@@ -387,18 +333,17 @@ template <typename KeyT>
 __global__ void __launch_bounds__(256) k_pack_round0(const uint8_t* __restrict__ text, uint32_t N,
                                                      KeyT* __restrict__ keys, PackParams pp,
                                                      uint32_t* __restrict__ hist, uint32_t hist_mask, uint32_t ntiles,
-                                                     uint32_t rb, uint32_t* __restrict__ gram) {
-  // rb: digit width of the sort that follows (8 or 9); digit p = (key >> rb*p) & (2^rb - 1), histogram p at hist + p * 2^rb
+                                                     uint32_t* __restrict__ gram) {
+  // digit p = (key >> 8p) & 255, histogram p at hist + 256 p
   // gram != nullptr (hist_mask == 0): instead of digit histograms, ONE histogram of the low GRAM_BITS bits of every key —
   // the last 2 (6-bit codes) or 4 (3-bit codes) characters of its window; every digit histogram is a projection of it
   // (k_hist_from_gram).  One shared-memory atomic per key into 4096 bins instead of four into 256-bin histograms.
   constexpr int BLOCK = 256, IPT = 8, TILE = BLOCK * IPT;
   __shared__ uint8_t s_lut[256];
   __shared__ uint8_t s_code[TILE + 64];
-  __shared__ uint32_t s_hist[8 * 512];  // digit histograms, or the gram histogram (1 << GRAM_BITS bins)
-  static_assert((1 << GRAM_BITS) <= 8 * 512, "the gram histogram shares the digit histograms' shared memory");
+  __shared__ uint32_t s_hist[1 << GRAM_BITS];  // the gram histogram, or the 8 digit histograms in its first 8 * 256 words
+  static_assert(8 * 256 <= (1 << GRAM_BITS), "the digit histograms share the gram histogram's shared memory");
   const int tid = threadIdx.x;
-  const uint32_t dmask = (1u << rb) - 1u;
   s_lut[tid] = pp.lut[tid];
 #pragma unroll
   for (int p = 0; p < 16; ++p) s_hist[p * 256 + tid] = 0;
@@ -478,7 +423,7 @@ __global__ void __launch_bounds__(256) k_pack_round0(const uint8_t* __restrict__
           if (t + k < N) {
 #pragma unroll
             for (int p = 0; p < (int)(sizeof(KeyT)); ++p)
-              if ((hist_mask >> p) & 1u) atomicAdd(&s_hist[(p << rb) + ((uint32_t)(out[k] >> (rb * p)) & dmask)], 1u);
+              if ((hist_mask >> p) & 1u) atomicAdd(&s_hist[(p << 8) + ((uint32_t)(out[k] >> (8 * p)) & 0xFFu)], 1u);
           }
         }
       }
@@ -495,10 +440,8 @@ __global__ void __launch_bounds__(256) k_pack_round0(const uint8_t* __restrict__
 #pragma unroll
   for (int p = 0; p < (int)(sizeof(KeyT)); ++p) {
     if (!((hist_mask >> p) & 1u)) continue;
-    for (uint32_t e = tid; e <= dmask; e += BLOCK) {
-      const uint32_t v = s_hist[(p << rb) + e];
-      if (v) atomicAdd(&hist[(p << rb) + e], v);
-    }
+    const uint32_t v = s_hist[(p << 8) + tid];
+    if (v) atomicAdd(&hist[(p << 8) + tid], v);
   }
 }
 
@@ -520,11 +463,11 @@ struct DeriveParams {
 // characters (W * b = 12).  Digit p of key(i) lies inside the W characters that start u_p characters above the key's low
 // end, and those are the LAST W characters of key(i - u_p) — the window slid by u_p positions, zero padding included, since
 // padding depends on the text position only.  So
-//   H_p[d] = sum_g G[g] [(g >> s_p) & dmask == d]  -  sum_{i = N-u_p}^{N-1} e((low12(key(i)) >> s_p) & dmask)   (no partner)
+//   H_p[d] = sum_g G[g] [(g >> s_p) & 255 == d]  -  sum_{i = N-u_p}^{N-1} e((low12(key(i)) >> s_p) & 255)   (no partner)
 //                                                  +  sum_{i = 0}^{u_p - 1} e(digit_p(key(i)))                    (not covered)
-// with 8p (or 9p) = b u_p + s_p, u_p capped so the W characters stay inside the key.  Block p of the grid builds H_p.
+// with 8p = b u_p + s_p, u_p capped so the W characters stay inside the key.  Block p of the grid builds H_p.
 // With partial bits (PackParams::rbits) everything above is in the coordinates of E = key >> rbits, the c exact characters:
-// G counts the low 12 bits of E, digit p is E bits [rb p - rbits, ...).  The lowest digit then reaches below E into the
+// G counts the low 12 bits of E, digit p is E bits [8p - rbits, ...).  The lowest digit then reaches below E into the
 // partial character: its 12-bit window is the low window of E(i + 1) (u = -1, flag below) and
 //   H_0 = projection(G) - e(window of suffix 0) + e(window of the all-padding "suffix N" = 0).
 struct GramParams {
@@ -550,60 +493,57 @@ __device__ __forceinline__ KeyT pack_key_at(const uint8_t* __restrict__ text, ui
 
 template <typename KeyT>
 __global__ void __launch_bounds__(256) k_hist_derive(const uint8_t* __restrict__ text, uint32_t N, PackParams pp,
-                                                     DeriveParams dp, uint32_t* __restrict__ hist, uint32_t rb) {
+                                                     DeriveParams dp, uint32_t* __restrict__ hist) {
   __shared__ uint8_t s_lut[256];
-  __shared__ uint32_t s_h[512];
+  __shared__ uint32_t s_h[256];
   const int tid = threadIdx.x;
   const uint32_t p = dp.p[blockIdx.x], r = dp.r[blockIdx.x], t = dp.t[blockIdx.x];
-  const uint32_t dmask = (1u << rb) - 1u;
   s_lut[tid] = pp.lut[tid];
-  for (uint32_t e = tid; e <= dmask; e += 256) s_h[e] = hist[(r << rb) + e];
+  s_h[tid] = hist[(r << 8) + tid];
   __syncthreads();
   if ((uint32_t)tid < t) {
     if ((uint32_t)tid < N) {  // head term: suffix i = tid counted for digit p
       const KeyT kh = pack_key_at<KeyT>(text, N, (uint32_t)tid, s_lut, pp.bits, pp.chars, pp.rbits);
-      atomicAdd(&s_h[(uint32_t)(kh >> (rb * p)) & dmask], 1u);
+      atomicAdd(&s_h[(uint32_t)(kh >> (8 * p)) & 0xFFu], 1u);
     }
     if ((uint32_t)tid < N) {  // tail term: suffix i = N-1-tid was counted for digit r but has no partner
       const KeyT kt = pack_key_at<KeyT>(text, N, N - 1u - (uint32_t)tid, s_lut, pp.bits, pp.chars, pp.rbits);
-      atomicSub(&s_h[(uint32_t)(kt >> (rb * r)) & dmask], 1u);
+      atomicSub(&s_h[(uint32_t)(kt >> (8 * r)) & 0xFFu], 1u);
     }
   }
   __syncthreads();
-  for (uint32_t e = tid; e <= dmask; e += 256) hist[(p << rb) + e] = s_h[e];
+  hist[(p << 8) + tid] = s_h[tid];
 }
 
 template <typename KeyT>
 __global__ void __launch_bounds__(256) k_hist_from_gram(const uint8_t* __restrict__ text, uint32_t N, PackParams pp,
                                                         GramParams gp, const uint32_t* __restrict__ gram,
-                                                        uint32_t* __restrict__ hist, uint32_t rb) {
+                                                        uint32_t* __restrict__ hist) {
   __shared__ uint8_t s_lut[256];
-  __shared__ uint32_t s_h[512];
+  __shared__ uint32_t s_h[256];
   const int tid = threadIdx.x;
   const uint32_t p = blockIdx.x, u = gp.u[p], sh = gp.s[p];
-  const uint32_t dmask = (1u << rb) - 1u;
   s_lut[tid] = pp.lut[tid];
   s_h[tid] = 0;
-  s_h[tid + 256] = 0;
   __syncthreads();
   for (uint32_t g = tid; g < (1u << GRAM_BITS); g += 256) {
     const uint32_t v = gram[g];
-    if (v) atomicAdd(&s_h[(g >> sh) & dmask], v);
+    if (v) atomicAdd(&s_h[(g >> sh) & 0xFFu], v);
   }
   if (gp.next[p]) {
     if (tid == 0) {
       const KeyT k0 = pack_key_at<KeyT>(text, N, 0u, s_lut, pp.bits, pp.chars, pp.rbits);
-      atomicSub(&s_h[(((uint32_t)(k0 >> pp.rbits) & ((1u << GRAM_BITS) - 1u)) >> sh) & dmask], 1u);
+      atomicSub(&s_h[(((uint32_t)(k0 >> pp.rbits) & ((1u << GRAM_BITS) - 1u)) >> sh) & 0xFFu], 1u);
       atomicAdd(&s_h[0], 1u);
     }
   } else if ((uint32_t)tid < u && (uint32_t)tid < N) {
     const KeyT kh = pack_key_at<KeyT>(text, N, (uint32_t)tid, s_lut, pp.bits, pp.chars, pp.rbits);  // head: suffix tid, digit p directly
-    atomicAdd(&s_h[(uint32_t)(kh >> (rb * p)) & dmask], 1u);
+    atomicAdd(&s_h[(uint32_t)(kh >> (8 * p)) & 0xFFu], 1u);
     const KeyT kt = pack_key_at<KeyT>(text, N, N - 1u - (uint32_t)tid, s_lut, pp.bits, pp.chars, pp.rbits);  // tail: counted, no partner
-    atomicSub(&s_h[(((uint32_t)(kt >> pp.rbits) & ((1u << GRAM_BITS) - 1u)) >> sh) & dmask], 1u);
+    atomicSub(&s_h[(((uint32_t)(kt >> pp.rbits) & ((1u << GRAM_BITS) - 1u)) >> sh) & 0xFFu], 1u);
   }
   __syncthreads();
-  for (uint32_t e = tid; e <= dmask; e += 256) hist[(p << rb) + e] = s_h[e];
+  hist[(p << 8) + tid] = s_h[tid];
 }
 
 // =====================================================================================================
@@ -617,17 +557,15 @@ __global__ void __launch_bounds__(256) k_hist_from_gram(const uint8_t* __restric
 __global__ void __launch_bounds__(256) k_build_keys(const uint32_t* __restrict__ rank, uint32_t N, uint32_t h,
                                                     int lo_bits, unsigned long long* __restrict__ keys,
                                                     uint32_t* __restrict__ idx, uint32_t* __restrict__ ctrl,
-                                                    uint32_t* __restrict__ hist, int npass, uint32_t ntiles,
-                                                    uint32_t rb) {
+                                                    uint32_t* __restrict__ hist, int npass, uint32_t ntiles) {
   constexpr int BLOCK = 256, IPT = 8, TILE = BLOCK * IPT, WARPS = BLOCK / 32;
-  __shared__ uint32_t s_hist[8 * 512];
+  __shared__ uint32_t s_hist[8 * 256];
   __shared__ uint32_t s_wtot[WARPS];
   __shared__ uint32_t s_base;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const uint32_t dmask = (1u << rb) - 1u;
   if (ctrl[CTR_ERR]) return;
 #pragma unroll
-  for (int p = 0; p < 16; ++p) s_hist[p * 256 + tid] = 0;
+  for (int p = 0; p < 8; ++p) s_hist[p * 256 + tid] = 0;
   __syncthreads();
   for (uint32_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
     // thread-blocked: 8 consecutive suffixes per thread, two 128-bit loads issued back to back (rank[] is
@@ -686,16 +624,15 @@ __global__ void __launch_bounds__(256) k_build_keys(const uint32_t* __restrict__
         keys[pos] = key;
         idx[pos] = (i0 + k) | ((r[k] & 1u) << 31);
         ++pos;
-        for (int p = 0; p < npass; ++p) atomicAdd(&s_hist[(p << rb) + ((uint32_t)(key >> (rb * p)) & dmask)], 1u);
+        for (int p = 0; p < npass; ++p) atomicAdd(&s_hist[(p << 8) + ((uint32_t)(key >> (8 * p)) & 0xFFu)], 1u);
       }
     }
   }
   __syncthreads();
-  for (int p = 0; p < npass; ++p)
-    for (uint32_t e = tid; e <= dmask; e += BLOCK) {
-      const uint32_t v = s_hist[(p << rb) + e];
-      if (v) atomicAdd(&hist[(p << rb) + e], v);
-    }
+  for (int p = 0; p < npass; ++p) {
+    const uint32_t v = s_hist[(p << 8) + tid];
+    if (v) atomicAdd(&hist[(p << 8) + tid], v);
+  }
 }
 
 // =====================================================================================================
@@ -720,25 +657,18 @@ __device__ unsigned long long* g_prof_buf = nullptr;  // [tiles][16] SM-clock st
 #define BWTC_PROF(k) do { } while (0)
 #endif
 
-template <typename KeyT, int BLOCK, int IPT, bool AUX = false, int RB = 8>
+template <typename KeyT, int BLOCK, int IPT, bool AUX = false>
 struct RadixPassSmem {
   static constexpr int TILE = BLOCK * IPT;
   static constexpr int WARPS = BLOCK / 32;
   static constexpr size_t bytes =
-      (sizeof(KeyT) + 4) * TILE + sizeof(uint32_t) * (WARPS * 256 + (1 << RB) + 32) + (AUX ? TILE : 0);
+      (sizeof(KeyT) + 4) * TILE + sizeof(uint32_t) * (WARPS * 256 + 256 + 32) + (AUX ? TILE : 0);
 };
 
 // AUX: a third, one-byte payload travels with every record — the dense code of the character preceding the
 // suffix, for blocks whose id has no spare bits for it (pack_bits) and whose text is too large for an L2-resident
 // gather at emission time.  The IOTA pass produces it (top character of the next key), later passes carry it.
-// RB = 9 (experiment, BWTC_RADIX9=1; MEASURED SLOWER: one 9-bit pass over the 32 MiB block's records takes 0.272 ms against
-// 0.220 ms, so 7 of them lose to 8 eight-bit passes — profiles/r02_experiments.md): nine-bit digits (512 bins; a
-// 55..63-bit key then takes 7 passes instead of 8).  The CTA keeps its shape: every
-// thread owns digits tid and tid + 256 — two status words per tile row of 512, two look-back walks interleaved in one
-// loop (LB_BATCH9 words each in flight) — and the per-warp histograms hold the two digits of a thread as the 16-bit
-// halves of one word (a tile has 4096 records, so neither the counts nor the tile-local offsets overflow a half):
-// zeroing, the scan over warps and the offset fold cost what they cost with 256 bins.
-template <typename KeyT, int BLOCK, int IPT, bool IOTA, bool AUX = false, int RB = 8>
+template <typename KeyT, int BLOCK, int IPT, bool IOTA, bool AUX = false>
 __global__ void __launch_bounds__(BLOCK, (sizeof(KeyT) == 4 && !AUX) ? BWTC_RS_MINB32 : BWTC_RS_MINB) k_radix_pass(const KeyT* __restrict__ keys_in,
                                                       const uint32_t* __restrict__ vals_in,
                                                       KeyT* __restrict__ keys_out, uint32_t* __restrict__ vals_out,
@@ -753,17 +683,14 @@ __global__ void __launch_bounds__(BLOCK, (sizeof(KeyT) == 4 && !AUX) ? BWTC_RS_M
   // bit pack_bits of the id, the dense code of the character PRECEDING the suffix — the top character of the
   // next key in the array — so the BWT emission of k_rerank needs no text gather at all.
   static_assert(BLOCK >= 256 && BLOCK % 32 == 0, "BLOCK must cover the 256 digit bins");
-  static_assert(RB == 8 || (RB == 9 && BLOCK == 256), "9-bit digits: two digits per thread of a 256-thread CTA");
   constexpr int TILE = BLOCK * IPT, WARPS = BLOCK / 32;
-  constexpr uint32_t BINS = 1u << RB, DMASK = BINS - 1u;
   static_assert(TILE <= 65536, "local positions are kept as uint16");
-  static_assert(RB == 8 || 2 * TILE < 65536, "9-bit digits: tile-local offsets live in 16-bit halves");
   extern __shared__ __align__(16) unsigned char smem_raw[];
   KeyT* s_keys = reinterpret_cast<KeyT*>(smem_raw);
   uint32_t* s_vals = reinterpret_cast<uint32_t*>(smem_raw + sizeof(KeyT) * TILE);  // ids staged beside the keys
   uint32_t* s_whist = s_vals + TILE;
   uint32_t* s_binbase = s_whist + WARPS * 256;
-  uint32_t* s_misc = s_binbase + BINS;  // [0] tile id, [8..23] scan scratch
+  uint32_t* s_misc = s_binbase + 256;  // [0] tile id, [8..15] scan scratch
   uint8_t* s_aux = reinterpret_cast<uint8_t*>(s_misc + 32);  // AUX: bytes staged beside keys and ids
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -858,145 +785,24 @@ __global__ void __launch_bounds__(BLOCK, (sizeof(KeyT) == 4 && !AUX) ? BWTC_RS_M
   }
 #endif
   uint32_t cnt = 0, pub = 0;
-  uint32_t* my_status = status + (size_t)tile * BINS + (tid & 255);
+  uint32_t* my_status = status + (size_t)tile * 256 + (tid & 255);
   // ---- rank inside the warp
   uint16_t lpos[IPT];
   uint32_t* my_hist = s_whist + warp * 256;
   const uint32_t lt = lanemask_lt();
 #pragma unroll
   for (int k = 0; k < IPT; ++k) {
-    const uint32_t d = (uint32_t)(key[k] >> shift) & DMASK;
-    uint32_t m;
-    if constexpr (RB == 9) m = match_digit9(d);
-    else m = match_digit8(d);
+    const uint32_t d = (uint32_t)(key[k] >> shift) & 0xFFu;
+    const uint32_t m = match_digit8(d);
     const int leader = __ffs(m) - 1;
     uint32_t old = 0;
-    if constexpr (RB == 9) {
-      const uint32_t hs = (d >> 8) * 16u;  // digit d lives in half d >> 8 of word d & 255
-      if (lane == leader) old = atomicAdd(&my_hist[d & 255u], (uint32_t)__popc(m) << hs);
-      old = (__shfl_sync(0xFFFFFFFFu, old, leader) >> hs) & 0xFFFFu;
-    } else {
-      if (lane == leader) old = atomicAdd(&my_hist[d], (uint32_t)__popc(m));  // one shared-memory RMW, not LDS+STS
-      old = __shfl_sync(0xFFFFFFFFu, old, leader);
-    }
+    if (lane == leader) old = atomicAdd(&my_hist[d], (uint32_t)__popc(m));  // one shared-memory RMW, not LDS+STS
+    old = __shfl_sync(0xFFFFFFFFu, old, leader);
     lpos[k] = (uint16_t)(old + __popc(m & lt));
     __syncwarp();
   }
   __syncthreads();
   BWTC_PROF(4);
-  if constexpr (RB == 9) {
-    // ---- two digits per thread (tid -> low half, tid + 256 -> high half of every packed word)
-    uint32_t run = 0;
-#pragma unroll
-    for (int w = 0; w < WARPS; ++w) {
-      const uint32_t t = s_whist[w * 256 + tid];
-      s_whist[w * 256 + tid] = run;
-      run += t;
-    }
-    const uint32_t cnt0 = run & 0xFFFFu, cnt1 = run >> 16;
-    const uint32_t pub0 = cnt0;
-    const uint32_t pub1 = cnt1 - ((tid == 255) ? ((uint32_t)TILE - valid) : 0u);  // pads (digit 511) are not records
-    const uint32_t first_flag = (tile == 0 ? LB_PREFIX : 0u);
-    st_relaxed_u32(my_status, first_flag | (pub0 + 1u));
-    st_relaxed_u32(my_status + 256, first_flag | (pub1 + 1u));
-    // tile-local exclusive offsets of both halves with ONE packed scan (every partial sum is <= TILE)
-    uint32_t tot_pk = 0, dummy0, dummy1;
-    uint32_t pk_excl;
-    scan256_excl2(run, 0u, s_misc + 8, pk_excl, dummy0, tot_pk, dummy1);
-    const uint32_t texcl0 = pk_excl & 0xFFFFu;
-    const uint32_t texcl1 = (pk_excl >> 16) + (tot_pk & 0xFFFFu);
-    uint32_t gexcl0, gexcl1, gtot0, gtot1;
-    scan256_excl2(ghist[tid], ghist[tid + 256], s_misc + 8, gexcl0, gexcl1, gtot0, gtot1);
-    gexcl1 += gtot0;
-    {
-      const uint32_t fold = texcl0 | (texcl1 << 16);
-#pragma unroll
-      for (int w = 0; w < WARPS; ++w) s_whist[w * 256 + tid] += fold;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int k = 0; k < IPT; ++k) {
-      const uint32_t d = (uint32_t)(key[k] >> shift) & DMASK;
-      const uint32_t p = ((my_hist[d & 255u] >> ((d >> 8) * 16u)) & 0xFFFFu) + lpos[k];
-      s_keys[p] = key[k];
-      s_vals[p] = val[k];
-      if (AUX) s_aux[p] = (uint8_t)(aux[k / 4] >> (8 * (k % 4)));
-    }
-    BWTC_PROF(5);
-    // ---- decoupled look-back of both digits, interleaved: LB_BATCH9 words of each in flight per round trip
-    uint32_t excl0 = 0, excl1 = 0;
-    if (tile != 0) {
-      long long t0 = (long long)tile - 1, t1 = t0;
-      uint32_t spins = 0;
-      uint32_t live0 = 0xFFFFFFFFu, live1 = 0xFFFFFFFFu;  // all-ones while the digit's walk is not finished
-      while (live0 | live1) {
-        uint32_t v0[LB_BATCH9], v1[LB_BATCH9];
-        const uint32_t* row0 = status + t0 * (long long)BINS + tid;
-        const uint32_t* row1 = status + t1 * (long long)BINS + 256 + tid;
-#pragma unroll
-        for (int i = 0; i < LB_BATCH9; ++i) v0[i] = ld_relaxed_u32(row0 - i * (int)BINS);
-#pragma unroll
-        for (int i = 0; i < LB_BATCH9; ++i) v1[i] = ld_relaxed_u32(row1 - i * (int)BINS);
-        uint32_t alive0 = live0, alive1 = live1, fin0 = 0, fin1 = 0;
-        int c0 = 0, c1 = 0;
-#pragma unroll
-        for (int i = 0; i < LB_BATCH9; ++i) {
-          {
-            const uint32_t pubd = (uint32_t)((int32_t)(v0[i] | (0u - v0[i])) >> 31);
-            const uint32_t ispre = (uint32_t)((int32_t)v0[i] >> 31);
-            const uint32_t isagg = pubd & ~ispre;
-            excl0 += ((v0[i] & LB_VALUE) - 1u) & alive0 & pubd;
-            fin0 |= alive0 & ispre;
-            c0 += (int)(alive0 & isagg & 1u);
-            alive0 &= isagg;
-          }
-          {
-            const uint32_t pubd = (uint32_t)((int32_t)(v1[i] | (0u - v1[i])) >> 31);
-            const uint32_t ispre = (uint32_t)((int32_t)v1[i] >> 31);
-            const uint32_t isagg = pubd & ~ispre;
-            excl1 += ((v1[i] & LB_VALUE) - 1u) & alive1 & pubd;
-            fin1 |= alive1 & ispre;
-            c1 += (int)(alive1 & isagg & 1u);
-            alive1 &= isagg;
-          }
-        }
-        live0 &= ~fin0;  // fin is all-ones once the walk met an inclusive prefix
-        live1 &= ~fin1;
-        t0 -= c0;
-        t1 -= c1;
-        if ((live0 | live1) && c0 + c1 == 0) {
-          ++spins;
-          if (spins > g_lb_spin_limit || ((spins & 255u) == 0u && ld_relaxed_u32(ctrl + CTR_ERR))) {
-            atomicExch(&ctrl[CTR_ERR], 1u);
-            break;
-          }
-          __nanosleep(20);
-        }
-      }
-      st_relaxed_u32(my_status, LB_PREFIX | ((excl0 + pub0 + 1u) & LB_VALUE));
-      st_relaxed_u32(my_status + 256, LB_PREFIX | ((excl1 + pub1 + 1u) & LB_VALUE));
-    }
-    s_binbase[tid] = gexcl0 + excl0 - texcl0;
-    s_binbase[tid + 256] = gexcl1 + excl1 - texcl1;
-    __syncthreads();
-    BWTC_PROF(6);
-#pragma unroll
-    for (int k = 0; k < IPT; ++k) {
-      const uint32_t p = tid + k * BLOCK;
-      const KeyT kk = s_keys[p];
-      const uint32_t vv = s_vals[p];
-      const uint32_t d = (uint32_t)(kk >> shift) & DMASK;
-      const uint32_t g = s_binbase[d] + p;
-      if (p < valid) {
-        BWTC_ST(keys_out + g, kk);
-        BWTC_ST(vals_out + g, vv);
-        if (AUX) aux_out[g] = s_aux[p];
-      }
-    }
-    BWTC_PROF(8);
-    return;
-  }
-
   // ---- per-digit: exclusive scan over warps; tile-local and global exclusive digit offsets
   if (tid < 256) {
     uint32_t run = 0;
@@ -1135,24 +941,14 @@ struct RerankParams {
   uint8_t decode[256];      // dense code -> byte (packed emission)
   uint32_t nbuckets;        // > 1: bucketed scatter — instead of writing rank[] the tile stages its (id, rank) pairs
   uint32_t bucket_magic;    //      grouped by id bucket (bucket = min(umulhi(id, magic), nbuckets-1)); see k_scatter_bucket
-  uint32_t* nr_out;         // != nullptr: additionally store every record's new rank word at its SORTED position (0xFFFFFFFF =
-                            // "rank unchanged"), coalesced; k_scatter_window then serves the other id windows from
-                            // (idx[], nr_out[]) without repeating the re-rank
-  uint32_t direct0;         // bucketed: ids of bucket 0 are written to rank[] directly (its window stays L2-resident during
-                            // this launch), only the other buckets are staged — the two-window case: one pass over the
-                            // records + one k_scatter_bucket over half of the pairs, instead of two passes over the records
   // ROUND0, lazy ranks (DESIGN.md §3.9): 1 = rank[] is written only for suffixes that stay in a group (and the few "short"
   // ones), their bit is set in livebits, and the first sorted position of every key prefix goes to ktab; a singleton's
   // rank is its sorted position and is looked up in the retained sorted keys when somebody needs it (rank_lookup).
   // 2 = materialise: write rank[] for the singletons only (the fallback out of lazy mode; nothing else is touched).
   uint32_t lazy;
   // Which records this launch emits BWT bytes for — 0: those whose id is in [win_lo, win_hi); 1: all (round 0: the first
-  // launch of a windowed scatter, so a thread's eight consecutive output bytes leave as one store; any round: the only
-  // k_rerank launch when k_scatter_window serves the other window); 2: none.
+  // launch of a windowed scatter, so a thread's eight consecutive output bytes leave as one store); 2: none.
   uint32_t emit;
-  // > 0: every CTA first asks L2 for the records of tile (mine + pf_tiles) — the tile a CTA launched about one wave later
-  // will load; the kernel is bound by the latency of its up-front record loads (ncu: 49% of stall samples on their first use)
-  uint32_t pf_tiles;
   uint32_t* livebits;
   uint32_t* ktab;
   uint32_t tshift;          // key >> tshift = table index
@@ -1437,21 +1233,6 @@ __global__ void __launch_bounds__(256, (ROUND0 && !LAZY) ? 5 : 4) k_rerank(const
     }
   }
   if (err_at_entry) return;
-  // (issued once my own record loads have landed: the DRAM queue is idle while the resident CTAs scan)
-  if (rp.pf_tiles) {
-    const unsigned long long pbase = ((unsigned long long)tile + rp.pf_tiles) * (unsigned long long)TILE;
-    if (pbase + TILE <= (unsigned long long)m) {
-      constexpr int KLINES = TILE * (int)sizeof(KeyT) / 128, ILINES = TILE * 4 / 128;  // 128 / 64 (u64) or 64 / 64 lines
-      const char* p = nullptr;
-      if (tid < KLINES) p = reinterpret_cast<const char*>(keys + pbase) + (size_t)tid * 128;
-      else if (tid < KLINES + ILINES) p = reinterpret_cast<const char*>(idx + pbase) + (size_t)(tid - KLINES) * 128;
-      else if (ROUND0 && rp.packed == 2u && tid < KLINES + ILINES + TILE / 128) p = reinterpret_cast<const char*>(rp.pred_aux + pbase) + (size_t)(tid - KLINES - ILINES) * 128;
-      // the address is made to depend on my last loaded record (an opaque "and 0"), so the prefetch issues behind the loads
-      uint32_t zero;
-      asm volatile("and.b32 %0, %1, 0;" : "=r"(zero) : "r"((uint32_t)key[IPT - 1] ^ id[IPT - 1]));
-      if (p) asm volatile("prefetch.global.L2 [%0];" ::"l"(p + zero));
-    }
-  }
 
   uint32_t pc0 = 0, pc1 = 0;  // packed predecessor codes of the 8 records (one byte each)
   if (ROUND0 && rp.packed == 2u) {
@@ -1625,7 +1406,6 @@ __global__ void __launch_bounds__(256, (ROUND0 && !LAZY) ? 5 : 4) k_rerank(const
   const bool bucketed = rp.nbuckets > 1;
   uint32_t live = 0, livemask = 0, gmax = 0, nrv[IPT];
   uint32_t wrmask = 0, bpos[IPT];
-  uint32_t anymask = 0;  // records whose rank word changed or became final (whatever their id window)
   uint32_t embits = 0, ew0 = 0, ew1 = 0;  // ROUND0: the BWT bytes of my eight (consecutive) sorted positions
   uint32_t sabits = 0;                    // SA && ROUND0: which of them are final (their SA entries leave as whole words)
 #pragma unroll
@@ -1669,7 +1449,6 @@ __global__ void __launch_bounds__(256, (ROUND0 && !LAZY) ? 5 : 4) k_rerank(const
       if (single) nr |= RANK_DONE;
       else if (sp.enable) { ++live; livemask |= 1u << k; gmax = max(gmax, j - HF + 1u); }
       nrv[k] = nr;
-      if (!ROUND0 && (changed || single)) anymask |= 1u << k;  // (round 0: every rank is new)
       bool wr = in_win && (changed || single);
       if (LAZY && rp.lazy) {
         const bool isshort = id[k] >= rp.short_thresh;
@@ -1688,12 +1467,8 @@ __global__ void __launch_bounds__(256, (ROUND0 && !LAZY) ? 5 : 4) k_rerank(const
       if (wr) {
         if (bucketed) {
           const uint32_t b = min(__umulhi(id[k], rp.bucket_magic), rp.nbuckets - 1u);
-          if (rp.direct0 && b == 0u) {
-            rank[id[k]] = nr;
-          } else {
-            bpos[k] = atomicAdd(&s_bcnt[b], 1u);
-            wrmask |= 1u << k;
-          }
+          bpos[k] = atomicAdd(&s_bcnt[b], 1u);
+          wrmask |= 1u << k;
         } else {
           rank[id[k]] = nr;
         }
@@ -1747,20 +1522,6 @@ __global__ void __launch_bounds__(256, (ROUND0 && !LAZY) ? 5 : 4) k_rerank(const
 #pragma unroll
       for (int k = 4; k < 8; ++k)
         if ((sabits >> k) & 1u) ps[k] = (int32_t)id[k];
-    }
-  }
-  if (rp.nr_out) {
-    uint32_t v[IPT];
-#pragma unroll
-    for (int k = 0; k < IPT; ++k) v[k] = (ROUND0 || ((anymask >> k) & 1u)) ? nrv[k] : 0xFFFFFFFFu;
-    if (tile_base + TILE <= m) {
-      uint4* po = reinterpret_cast<uint4*>(rp.nr_out + j0);  // j0 % 8 == 0, buffer 256-byte aligned
-      __stcs(po, make_uint4(v[0], v[1], v[2], v[3]));
-      __stcs(po + 1, make_uint4(v[4], v[5], v[6], v[7]));
-    } else {
-#pragma unroll
-      for (int k = 0; k < IPT; ++k)
-        if (j0 + k < m) rp.nr_out[j0 + k] = v[k];
     }
   }
   if (bucketed) {
@@ -1828,29 +1589,6 @@ __global__ void __launch_bounds__(256, (ROUND0 && !LAZY) ? 5 : 4) k_rerank(const
 // k_scatter_bucket — rank[id] = nr for the staged records of ONE id bucket (all tiles).  One warp per tile
 // segment; the bucket's slice of rank[] (<= ~72 MB) stays L2-resident, so the random 4-byte writes never pay a
 // DRAM sector fill + write-back, and — unlike re-running k_rerank once per window — every record is read once.
-// k_scatter_window — rank[id] = new rank for the records whose id lies in [win_lo, win_hi), from the sorted ids and the
-// rank words k_rerank left beside them (RerankParams::nr_out).  Sequential 128-bit reads, L2-resident random writes.
-__global__ void __launch_bounds__(256) k_scatter_window(const uint32_t* __restrict__ idx, const uint32_t* __restrict__ nrw,
-                                                        uint32_t m, uint32_t id_mask, uint32_t win_lo, uint32_t win_hi,
-                                                        uint32_t* __restrict__ rank, const uint32_t* __restrict__ ctrl) {
-  if (ctrl[CTR_ERR]) return;  // sticky error: the rank words may be incomplete
-  const uint32_t quads = m >> 2;
-  for (uint32_t q = blockIdx.x * blockDim.x + threadIdx.x; q < quads; q += gridDim.x * blockDim.x) {
-    const uint4 i4 = __ldcs(reinterpret_cast<const uint4*>(idx) + q);
-    const uint4 n4 = __ldcs(reinterpret_cast<const uint4*>(nrw) + q);
-    const uint32_t ii[4] = {i4.x & id_mask, i4.y & id_mask, i4.z & id_mask, i4.w & id_mask};
-    const uint32_t nn[4] = {n4.x, n4.y, n4.z, n4.w};
-#pragma unroll
-    for (int k = 0; k < 4; ++k)
-      if (nn[k] != 0xFFFFFFFFu && ii[k] >= win_lo && ii[k] < win_hi) rank[ii[k]] = nn[k];
-  }
-  if (blockIdx.x == 0 && threadIdx.x < (m & 3u)) {
-    const uint32_t j = (m & ~3u) + threadIdx.x;
-    const uint32_t i = idx[j] & id_mask, n = nrw[j];
-    if (n != 0xFFFFFFFFu && i >= win_lo && i < win_hi) rank[i] = n;
-  }
-}
-
 __global__ void __launch_bounds__(256) k_scatter_bucket(const uint32_t* __restrict__ sc_id, const uint32_t* __restrict__ sc_nr,
                                                         const uint32_t* __restrict__ tile_woff, uint32_t ntiles,
                                                         uint32_t nbuckets, uint32_t b, uint32_t tile_records,
@@ -2024,13 +1762,12 @@ __global__ void __launch_bounds__(256) k_build_from_list(const uint32_t* __restr
                                                          const uint32_t* __restrict__ rank, uint32_t N, uint32_t h,
                                                          int lo_bits, unsigned long long* __restrict__ keys,
                                                          uint32_t* __restrict__ idx, uint32_t* __restrict__ hist,
-                                                         int npass, const uint32_t* __restrict__ ctrl, uint32_t rb) {
-  __shared__ uint32_t s_hist[8 * 512];
+                                                         int npass, const uint32_t* __restrict__ ctrl) {
+  __shared__ uint32_t s_hist[8 * 256];
   const int tid = threadIdx.x;
-  const uint32_t dmask = (1u << rb) - 1u;
   if (ctrl[CTR_ERR]) return;
 #pragma unroll
-  for (int p = 0; p < 16; ++p) s_hist[p * 256 + tid] = 0;
+  for (int p = 0; p < 8; ++p) s_hist[p * 256 + tid] = 0;
   __syncthreads();
   for (uint32_t j = blockIdx.x * blockDim.x + tid; j < m; j += gridDim.x * blockDim.x) {
     const uint32_t i = list[j];
@@ -2039,14 +1776,13 @@ __global__ void __launch_bounds__(256) k_build_from_list(const uint32_t* __restr
     const unsigned long long key = ((unsigned long long)(r >> 1) << lo_bits) | (unsigned long long)r2;  // see k_build_keys
     keys[j] = key;
     idx[j] = i | ((r & 1u) << 31);
-    for (int p = 0; p < npass; ++p) atomicAdd(&s_hist[(p << rb) + ((uint32_t)(key >> (rb * p)) & dmask)], 1u);
+    for (int p = 0; p < npass; ++p) atomicAdd(&s_hist[(p << 8) + ((uint32_t)(key >> (8 * p)) & 0xFFu)], 1u);
   }
   __syncthreads();
-  for (int p = 0; p < npass; ++p)
-    for (uint32_t e = tid; e <= dmask; e += 256) {
-      const uint32_t v = s_hist[(p << rb) + e];
-      if (v) atomicAdd(&hist[(p << rb) + e], v);
-    }
+  for (int p = 0; p < npass; ++p) {
+    const uint32_t v = s_hist[(p << 8) + tid];
+    if (v) atomicAdd(&hist[(p << 8) + tid], v);
+  }
 }
 
 // =====================================================================================================
@@ -2528,40 +2264,6 @@ __global__ void __launch_bounds__(1024) k_small_rounds(LadderState* st, PoolPtrs
   }
 }
 
-
-// =====================================================================================================
-// k_copy_out — OPTIONAL (BWTC_D2H_KERNEL=1): the result copy to a PINNED host buffer done by SMs (plain stores through the
-// unified address space) instead of the copy engine.  Background: device-to-host traffic at the rate the end-to-end path
-// needs slows the kernels of all other streams by 12% (tests/gpu_dma_interference.py: 12.6 -> 11.0 GB/s device-resident;
-// host-to-device copies: -1%).  This kernel was built to see whether the copy ENGINE is to blame: it is not — the same
-// bytes written by 16 CTAs cost the same (e2e 10.76 vs 10.70 GB/s), more CTAs cost more.  Not the default.
-// 16-byte accesses where both pointers allow it, bytes at the ragged ends.  Skips an unfinished block (st->m != 0).
-// =====================================================================================================
-__global__ void __launch_bounds__(256) k_copy_out(const uint8_t* __restrict__ src, uint8_t* __restrict__ dst, uint32_t n,
-                                                  const LadderState* __restrict__ st, const uint32_t* __restrict__ ctrl) {
-  if (st->m != 0u || ctrl[CTR_ERR]) return;
-  const uintptr_t mis = (16u - (reinterpret_cast<uintptr_t>(dst) & 15u)) & 15u;  // bytes until dst is 16-byte aligned
-  const uint32_t head = mis < n ? (uint32_t)mis : n;
-  const uint32_t tidg = blockIdx.x * blockDim.x + threadIdx.x, nthr = gridDim.x * blockDim.x;
-  if (tidg < head) dst[tidg] = src[tidg];
-  const uint32_t body = (n - head) / 16u;
-  uint4* d4 = reinterpret_cast<uint4*>(dst + head);
-  if (((reinterpret_cast<uintptr_t>(src) + head) & 15u) == 0) {
-    const uint4* s4 = reinterpret_cast<const uint4*>(src + head);
-    for (uint32_t i = tidg; i < body; i += nthr) d4[i] = s4[i];
-  } else {
-    for (uint32_t i = tidg; i < body; i += nthr) {
-      const uint8_t* sp = src + head + (size_t)i * 16u;
-      uint32_t w[4];
-#pragma unroll
-      for (int k = 0; k < 4; ++k)
-        w[k] = (uint32_t)sp[4 * k] | ((uint32_t)sp[4 * k + 1] << 8) | ((uint32_t)sp[4 * k + 2] << 16) | ((uint32_t)sp[4 * k + 3] << 24);
-      d4[i] = make_uint4(w[0], w[1], w[2], w[3]);
-    }
-  }
-  const uint32_t done = head + body * 16u;
-  if (tidg < n - done) dst[done + tidg] = src[done + tidg];
-}
 
 // =====================================================================================================
 // k_finish — primary index + LFpowers + hole fill (the BWT bytes themselves are emitted by k_rerank as soon

@@ -136,16 +136,12 @@ def test_round0_histograms_from_the_gram_histogram(oracle, monkeypatch, gram, si
         assert (got[0] == want[0]).all() and (got[1] == want[1]).all() and (got[2] == want[2]).all(), (n, tail)
 
 
-@pytest.mark.parametrize("radix9", ["1", "0"])
 @pytest.mark.parametrize("kind,chars", [("markov", 6), ("markov", 7), ("markov", 8), ("markov", 9), ("markov", 10),
                                         ("dna", 17), ("dna", 22), ("dna", 27), ("dna", 31), ("dna", 32),
                                         ("random", 5), ("random", 8)])
-def test_digit_width_of_the_radix_passes(oracle, monkeypatch, radix9, kind, chars):
-    """64-bit keys of 34..64 used bits: with BWTC_RADIX9=1 (an experiment, measured slower, default off) 9-bit digits are
-    chosen whenever they save a pass over 8-bit digits (36 bits: 4 instead of 5 passes, ... 60 bits: 7 instead of 8; 48 and
-    64 bits: 8-bit digits stay).  Same bytes either way, and
-    the pass count of round 0 shows which width ran.  A size with a ragged last tile and >= 2 tiles per CTA wave."""
-    monkeypatch.setenv("BWTC_RADIX9", radix9)
+def test_digit_width_of_the_radix_passes(oracle, kind, chars):
+    """64-bit keys of 34..64 used bits take ceil(bits / 8) 8-bit digit passes in round 0, and give the oracle's bytes.
+    A size with a ragged last tile and >= 2 tiles per CTA wave."""
     n = 700001
     x = bw.generate(kind, n, seed=29)
     want = oracle.block(x, 8)
@@ -158,8 +154,7 @@ def test_digit_width_of_the_radix_passes(oracle, monkeypatch, radix9, kind, char
         c.close()
     assert (got[0] == want[0]).all() and (got[1] == want[1]).all() and (got[2] == want[2]).all()
     bits = {"markov": 6, "dna": 2, "random": 8}[kind] * chars
-    p8, p9 = -(-bits // 8), -(-bits // 9)
-    assert st["passes"][0] == (p9 if (radix9 == "1" and p9 < p8) else p8), (bits, st["passes"][:2])
+    assert st["passes"][0] == -(-bits // 8), (bits, st["passes"][:2])
 
 
 @pytest.mark.parametrize("force", [(0, 0), (1, 4), (3, 4), (2, 8), (5, 8), (64, 8)])
@@ -326,11 +321,7 @@ ENGINE_KNOBS = [
     {"BWTC_RERANK_WINDOW_MB": "4", "BWTC_BUCKET_MIN_WINDOWS": "2"},  # bucketed scatter from two windows on
     {"BWTC_RERANK_WINDOW_MB": "6"},                                  # exactly two windows: one k_rerank launch per window
     {"BWTC_RERANK_WINDOW_MB": "6", "BWTC_SEG": "0"},                 # ... in doubling rounds too
-    {"BWTC_RERANK_WINDOW_MB": "6", "BWTC_TWOPASS": "1"},             # exactly two windows: k_rerank + k_scatter_window (experiment, off)
-    {"BWTC_RERANK_WINDOW_MB": "6", "BWTC_TWOPASS": "1", "BWTC_SEG": "0"},
-    {"BWTC_RERANK_WINDOW_MB": "6", "BWTC_TWOPASS": "1", "BWTC_PACK_PRED": "0", "BWTC_AUX_MIN_MIB": "0"},
-    {"BWTC_RERANK_WINDOW_MB": "6", "BWTC_HYBRID2": "1"},             # ... or window 0 direct, window 1 staged (experiment, off)
-    {"BWTC_RERANK_WINDOW_MB": "6", "BWTC_HYBRID2": "1", "BWTC_SEG": "0"},  # the hybrid scatter in doubling rounds too
+    {"BWTC_RERANK_WINDOW_MB": "6", "BWTC_PACK_PRED": "0", "BWTC_AUX_MIN_MIB": "0"},  # ... carrying the one-byte payload
     {"BWTC_PACK_PRED": "0"},                                         # BWT characters gathered from the text
     {"BWTC_PACK_PRED": "0", "BWTC_AUX_MIN_MIB": "0"},                # predecessor codes as a one-byte payload array
     {"BWTC_PACK_PRED": "0", "BWTC_AUX_MIN_MIB": "0", "BWTC_RERANK_WINDOW_MB": "1"},  # ... with the bucketed scatter
@@ -348,10 +339,6 @@ ENGINE_KNOBS = [
     {"BWTC_PARTIAL": "0"},                                           # no partial character in the spare low key bits
     {"BWTC_PARTIAL": "0", "BWTC_GRAM": "0"},
     {"BWTC_GRAM": "0"},                                              # round-0 histograms counted per digit class (default: gram)
-    {"BWTC_RADIX9": "1"},                                            # 9-bit digit passes where they save a pass (experiment, default off)
-    {"BWTC_RADIX9": "1", "BWTC_SEG": "0"},                           # ... in the doubling rounds too
-    {"BWTC_RADIX9": "1", "BWTC_SEG": "0", "BWTC_STATIC_TILES": "0"},  # ... with tile tickets
-    {"BWTC_RADIX9": "1", "BWTC_PACK_PRED": "0", "BWTC_AUX_MIN_MIB": "0"},  # ... carrying the one-byte payload
 ]
 
 
