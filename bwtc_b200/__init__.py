@@ -15,7 +15,7 @@ from __future__ import annotations
 
 import ctypes
 import os
-from typing import List, Optional, Sequence
+from typing import List, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -33,6 +33,7 @@ EVERIFY = -7                      # BWTC_CUDA_EVERIFY: a verified forward output
 FLAG_VERIFIED = 1 << 6            # stats flags bit 6: the forward output was verified on the device
 FLAG_CORRUPT = 1 << 7             # stats flags bit 7: this inverse block is corrupt
 FLAG_SA = 1 << 8                  # stats flags bit 8: this call produced a suffix array (divsufsort)
+FLAG_LCP = 1 << 9                 # stats flags bit 9: this call produced an LCP array (divsufsort_lcp)
 
 
 class BwtcCudaUnavailable(RuntimeError):
@@ -121,6 +122,8 @@ C_ABI = [
     ("bwtc_cuda_divsufsort", ctypes.c_int, [_vp, _vp, _vp, ctypes.c_uint32]),
     ("bwtc_cuda_divsufsort_device", ctypes.c_int, [_vp, _vp, _vp, ctypes.c_uint32]),
     ("bwtc_cuda_sufcheck", ctypes.c_int, [_vp, _vp, _vp, ctypes.c_uint32]),
+    ("bwtc_cuda_divsufsort_lcp", ctypes.c_int, [_vp, _vp, _vp, _vp, ctypes.c_uint32]),
+    ("bwtc_cuda_divsufsort_lcp_device", ctypes.c_int, [_vp, _vp, _vp, _vp, ctypes.c_uint32]),
     ("bwtc_cuda_bwt_block", ctypes.c_int64, [_vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp]),
     ("bwtc_cuda_bwt_block_device", ctypes.c_int64, [_vp, _vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp]),
     ("bwtc_cuda_bwt_block_runs", ctypes.c_int64, [_vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp, _vp]),
@@ -262,6 +265,26 @@ class CudaContext:
     def divsufsort_device(self, d_T: int, d_SA: int, n: int) -> None:
         """divsufsort with T (n bytes) and SA (n int32, 4-byte aligned) in device memory (e.g. torch data_ptr())."""
         self._check(self._lib.bwtc_cuda_divsufsort_device(self._h, d_T, d_SA, n))
+
+    def divsufsort_lcp(self, T: np.ndarray, SA: Optional[np.ndarray] = None,
+                       LCP: Optional[np.ndarray] = None) -> Tuple[np.ndarray, np.ndarray]:
+        """(SA, LCP) of T (uint8): the suffix array as divsufsort returns it and its LCP array (LCP[0] = 0, LCP[r] = the
+        longest common prefix of suffixes SA[r-1] and SA[r]), int32[T.size] each, or written into SA / LCP (int32,
+        pageable or pinned) when given.  Raises BwtcCudaError on failure (EVERIFY with verification on: both untouched)."""
+        assert T.dtype == np.uint8 and T.flags.c_contiguous
+        if SA is None:
+            SA = np.empty(T.size, dtype=np.int32)
+        if LCP is None:
+            LCP = np.empty(T.size, dtype=np.int32)
+        for a in (SA, LCP):
+            assert a.dtype == np.int32 and a.size >= T.size and a.flags.c_contiguous
+        self._check(self._lib.bwtc_cuda_divsufsort_lcp(self._h, T.ctypes.data, SA.ctypes.data, LCP.ctypes.data, T.size))
+        return SA, LCP
+
+    def divsufsort_lcp_device(self, d_T: int, d_SA: int, d_LCP: int, n: int) -> None:
+        """divsufsort_lcp with T (n bytes, any alignment), SA and LCP (n int32 each, 4-byte aligned, not overlapping) in
+        device memory (e.g. torch data_ptr())."""
+        self._check(self._lib.bwtc_cuda_divsufsort_lcp_device(self._h, d_T, d_SA, d_LCP, n))
 
     def sufcheck(self, T: np.ndarray, SA: np.ndarray) -> bool:
         """True if SA (int32) is the suffix array of T (uint8); False if not (last_error() names the first offending row).

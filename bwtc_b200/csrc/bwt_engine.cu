@@ -509,6 +509,8 @@ struct Job {
   bwtc_cuda_runs* runs = nullptr;  // run statistics wanted (single block, block contract)
   int32_t* sa = nullptr;           // raw contract: the suffix array is emitted here (device; bwtc_cuda_divsufsort) ...
   int32_t* h_sa = nullptr;         // ... and copied to this host array once the block is finished (and verified)
+  int32_t* lcp = nullptr;          // bwtc_cuda_divsufsort_lcp: the LCP array is built here (device) behind the sort ...
+  int32_t* h_lcp = nullptr;        // ... and copied to this host array
   // ---- phase A
   uint32_t N = 0, bstride = 0, blk_bits = 0;
   bool sentinel_outside_alphabet = false;
@@ -785,6 +787,7 @@ int64_t phase_input(bwtc_cuda_ctx* ctx, Job& J) {
 
 int verify_forward(bwtc_cuda_ctx* ctx, const Job& J);
 int verify_sa(bwtc_cuda_ctx* ctx, const Job& J);
+int enqueue_lcp(bwtc_cuda_ctx* ctx, const Job& J);
 
 // ---- phase B: round 0, the device-controlled ladder of sort-free rounds, host-driven global radix rounds where
 // groups are large, final extraction, result copies.  Works from ctx->d_text only, so it can be repeated (with ticket
@@ -1301,16 +1304,26 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
     rc = J.sa ? verify_sa(ctx, J) : verify_forward(ctx, J);
     if (rc) return rc;
   }
+  // ---- the LCP array, from the (verified) suffix array
+  if (finished && J.lcp) {
+    if (enqueue_lcp(ctx, J)) return BWTC_CUDA_ECUDA;
+    CK(ctx, cudaEventRecord(ctx->ev_end, st));
+    if (!J.h_lcp && host_wait(ctx, st)) return BWTC_CUDA_ECUDA;  // (the host variant waits for its copies below)
+  }
   // ---- result copies that could not be enqueued speculatively
   if (finished) {
     if (J.sa) {
-      // the suffix array (its BWT bytes stay on the device): 4 bytes per suffix, direct from pinned memory, else staged
-      if (J.h_sa && is_pinned_host(J.h_sa)) {
-        CK(ctx, cudaMemcpyAsync(J.h_sa, J.sa, (size_t)N * 4, cudaMemcpyDeviceToHost, st));
-        if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
-      } else if (J.h_sa && download_staged(ctx, reinterpret_cast<uint8_t*>(J.h_sa), reinterpret_cast<const uint8_t*>(J.sa), (size_t)N * 4)) {
-        return BWTC_CUDA_ECUDA;
-      }
+      // the suffix array (its BWT bytes stay on the device) and the LCP array: 4 bytes per suffix each, direct to pinned
+      // memory, else staged
+      auto copy_out = [&](int32_t* h, const int32_t* d) -> int {
+        if (!h) return 0;
+        if (is_pinned_host(h)) {
+          CK(ctx, cudaMemcpyAsync(h, d, (size_t)N * 4, cudaMemcpyDeviceToHost, st));
+          return host_wait(ctx, st);
+        }
+        return download_staged(ctx, reinterpret_cast<uint8_t*>(h), reinterpret_cast<const uint8_t*>(d), (size_t)N * 4);
+      };
+      if (copy_out(J.h_sa, J.sa) || copy_out(J.h_lcp, J.lcp)) return BWTC_CUDA_ECUDA;
     } else if (bs) {
       if (!out_enqueued || !direct_out) {
         if (direct_out) {
@@ -1672,8 +1685,48 @@ int verify_sa(bwtc_cuda_ctx* ctx, const Job& J) {
   return sufcheck_failed(ctx, J.N, "verification failed: the suffix array") ? BWTC_CUDA_EVERIFY : 0;
 }
 
-// bwtc_cuda_divsufsort(_device): the raw transform with SA emission into d_sa; h_sa receives a copy.
-int run_divsufsort(bwtc_cuda_ctx* ctx, const uint8_t* h_T, const uint8_t* d_T, int32_t* h_SA, int32_t* d_SA, uint32_t n) {
+// The LCP stage of bwtc_cuda_divsufsort_lcp (DESIGN.md §3.12; kernels k_lcp_* in bwt_kernels.cuh), enqueued behind a
+// finished (and verified) suffix array J.sa of the text J.d_text; writes J.lcp.  Scratch, all idle once the sort is done:
+// X / PLCP in d_idx[0]; the window lists in d_keys[1] (rows, both slots) and d_idx[1] / d_scat (segment counters);
+// tile maxima in d_tilecnt; the control block in d_wtab.  The host variant's J.lcp is d_keys[0].  Nothing is waited for.
+int enqueue_lcp(bwtc_cuda_ctx* ctx, const Job& J) {
+  cudaStream_t st = ctx->stream;
+  bwtc_cuda_stats& S = ctx->stats;
+  const uint32_t n = J.N;
+  uint32_t* x = ctx->d_idx[0];
+  uint32_t* tiles = ctx->d_tilecnt;
+  LcpCtl* lc = reinterpret_cast<LcpCtl*>(ctx->d_wtab);
+  uint32_t* rows = static_cast<uint32_t*>(ctx->d_keys[1]);
+  const LcpLists L{{rows, rows + n}, {ctx->d_idx[1], ctx->d_scat}};
+  const uint32_t* ctrl = ctx->d_ctrl();
+  const uint32_t grid = std::max<uint32_t>(1u, std::min<uint32_t>(div_up(n, 256), (uint32_t)ctx->sm_count * 8u));
+  CK(ctx, cudaMemsetAsync(lc, 0, sizeof(LcpCtl), st));
+  CK(ctx, cudaMemsetAsync(x, 0, (size_t)n * 4, st));
+  k_lcp_short<<<grid, 256, 0, st>>>(J.d_text, J.sa, n, x, L, lc, ctrl);
+  S.kernel_launches++;
+  // one launch per window that a pair could still need (each returns at once when its list is empty)
+  for (uint32_t w = 0; w < (uint32_t)LCP_MAX_WINDOWS && ((uint64_t)LCP_SHORT_BYTES << w) + 1 < n; ++w) {
+    k_lcp_window<<<(uint32_t)ctx->sm_count * 8u, 256, 0, st>>>(J.d_text, J.sa, n, x, L, lc, w, ctrl);
+    S.kernel_launches++;
+  }
+  const uint32_t ntiles = div_up(n, LCP_SCAN_TILE);
+  k_lcp_tile_max<<<ntiles, 256, 0, st>>>(x, n, tiles, ctrl);
+  k_lcp_tile_scan<<<1, 1024, 0, st>>>(tiles, ntiles, ctrl);
+  k_lcp_apply<<<ntiles, 256, 0, st>>>(x, n, tiles, ctrl);
+  k_lcp_gather<<<grid, 256, 0, st>>>(J.sa, x, n, J.lcp, ctrl);
+  CK(ctx, cudaGetLastError());
+  S.kernel_launches += 4;
+  // X zeroed, SA read twice (rows, gather), predecessor bytes, X scattered, scanned (read twice, written), PLCP gathered,
+  // LCP written; the bytes the comparisons read depend on the text (LcpCtl counts them on the device)
+  S.algorithmic_bytes += (uint64_t)n * (4 + 8 + 2 + 4 + 12 + 8);
+  S.flags |= 512u;
+  return 0;
+}
+
+// bwtc_cuda_divsufsort(_device): the raw transform with SA emission into d_sa; h_sa receives a copy.  With d_lcp
+// (bwtc_cuda_divsufsort_lcp): the LCP array is built into d_lcp behind it, h_lcp receives a copy.
+int run_divsufsort(bwtc_cuda_ctx* ctx, const uint8_t* h_T, const uint8_t* d_T, int32_t* h_SA, int32_t* d_SA, uint32_t n,
+                   int32_t* h_LCP = nullptr, int32_t* d_LCP = nullptr) {
   uint32_t pidx = 0;
   Job J;
   J.block_mode = false;
@@ -1684,6 +1737,8 @@ int run_divsufsort(bwtc_cuda_ctx* ctx, const uint8_t* h_T, const uint8_t* d_T, i
   J.nLF = 1;
   J.sa = d_SA;
   J.h_sa = h_SA;
+  J.lcp = d_LCP;
+  J.h_lcp = h_LCP;
   const int64_t rc = run_job(ctx, J);
   return rc < 0 ? (int)rc : 0;
 }
@@ -2115,6 +2170,7 @@ int bwtc_cuda_debug_read(bwtc_cuda_ctx* ctx, int which, uint64_t offset_bytes, v
     case 5: src = reinterpret_cast<const uint8_t*>(ctx->d_idx[ctx->last_cur ^ 1]); break;
     case 6: src = reinterpret_cast<const uint8_t*>(ctx->d_zero); break;
     case 7: src = ctx->d_in; break;
+    case 9: src = reinterpret_cast<const uint8_t*>(ctx->d_wtab); break;  // LcpCtl of the last bwtc_cuda_divsufsort_lcp
 #ifdef BWTC_PROFILE_STAGES
     case 8: {
       unsigned long long* pbuf = nullptr;
@@ -2145,6 +2201,21 @@ int64_t bwtc_cuda_divbwt(bwtc_cuda_ctx* ctx, const uint8_t* T, uint8_t* U, uint3
   return bwtc_cuda_divbwtf(ctx, T, U, n, LFpowers, nLFpowers, nullptr);
 }
 
+// The host variants' device SA: 4 (cap + 1) bytes, allocated by the first call that needs it.
+static int ensure_sa(bwtc_cuda_ctx* ctx) {
+  if (ctx->d_sa) return 0;
+  if (cudaSetDevice(ctx->device) != cudaSuccess) { set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device); return BWTC_CUDA_ECUDA; }
+  const size_t bytes = ((size_t)ctx->cap + 1) * 4;
+  const cudaError_t e = cudaMalloc((void**)&ctx->d_sa, bytes);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    ctx->d_sa = nullptr;
+    set_err(ctx->err, "cudaMalloc(%zu bytes) for the suffix array: %s", bytes, cudaGetErrorString(e));
+    return BWTC_CUDA_EALLOC;
+  }
+  return 0;
+}
+
 int bwtc_cuda_divsufsort(bwtc_cuda_ctx* ctx, const uint8_t* T, int32_t* SA, uint32_t n) {
   if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
   ctx->err[0] = 0;
@@ -2157,17 +2228,7 @@ int bwtc_cuda_divsufsort(bwtc_cuda_ctx* ctx, const uint8_t* T, int32_t* SA, uint
     set_err(ctx->err, "raw text of %u bytes exceeds context capacity %u", n, ctx->cap);
     return BWTC_CUDA_ETOOBIG;
   }
-  if (!ctx->d_sa) {
-    if (cudaSetDevice(ctx->device) != cudaSuccess) { set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device); return BWTC_CUDA_ECUDA; }
-    const size_t bytes = ((size_t)ctx->cap + 1) * 4;
-    const cudaError_t e = cudaMalloc((void**)&ctx->d_sa, bytes);
-    if (e != cudaSuccess) {
-      cudaGetLastError();
-      ctx->d_sa = nullptr;
-      set_err(ctx->err, "cudaMalloc(%zu bytes) for the suffix array: %s", bytes, cudaGetErrorString(e));
-      return BWTC_CUDA_EALLOC;
-    }
-  }
+  if (const int rc = ensure_sa(ctx)) return rc;
   return run_divsufsort(ctx, T, nullptr, SA, ctx->d_sa, n);
 }
 
@@ -2182,6 +2243,42 @@ int bwtc_cuda_divsufsort_device(bwtc_cuda_ctx* ctx, const void* d_T, void* d_SA,
     return host_wait(ctx, ctx->stream) ? BWTC_CUDA_ECUDA : 0;
   }
   return run_divsufsort(ctx, nullptr, static_cast<const uint8_t*>(d_T), nullptr, static_cast<int32_t*>(d_SA), n);
+}
+
+int bwtc_cuda_divsufsort_lcp(bwtc_cuda_ctx* ctx, const uint8_t* T, int32_t* SA, int32_t* LCP, uint32_t n) {
+  if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
+  ctx->err[0] = 0;
+  if (!T || !SA || !LCP) { set_err(ctx->err, "null T, SA or LCP"); return BWTC_CUDA_EARG; }
+  if (n <= 1) {
+    if (n == 1) SA[0] = LCP[0] = 0;
+    return 0;
+  }
+  if ((uint64_t)n > (uint64_t)ctx->cap + 1) {
+    set_err(ctx->err, "raw text of %u bytes exceeds context capacity %u", n, ctx->cap);
+    return BWTC_CUDA_ETOOBIG;
+  }
+  if (const int rc = ensure_sa(ctx)) return rc;
+  return run_divsufsort(ctx, T, nullptr, SA, ctx->d_sa, n, LCP, static_cast<int32_t*>(ctx->d_keys[0]));
+}
+
+int bwtc_cuda_divsufsort_lcp_device(bwtc_cuda_ctx* ctx, const void* d_T, void* d_SA, void* d_LCP, uint32_t n) {
+  if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
+  ctx->err[0] = 0;
+  const uintptr_t a = reinterpret_cast<uintptr_t>(d_SA), b = reinterpret_cast<uintptr_t>(d_LCP);
+  if (!d_T || !d_SA || !d_LCP || ((a | b) & 3u)) {
+    set_err(ctx->err, "null d_T / d_SA / d_LCP, or d_SA / d_LCP not 4-byte aligned");
+    return BWTC_CUDA_EARG;
+  }
+  if (a < b + (uint64_t)n * 4 && b < a + (uint64_t)n * 4) { set_err(ctx->err, "d_SA and d_LCP overlap"); return BWTC_CUDA_EARG; }
+  if (n == 0) return 0;
+  if (n == 1) {
+    if (cudaSetDevice(ctx->device) != cudaSuccess) { set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device); return BWTC_CUDA_ECUDA; }
+    CK(ctx, cudaMemsetAsync(d_SA, 0, 4, ctx->stream));
+    CK(ctx, cudaMemsetAsync(d_LCP, 0, 4, ctx->stream));
+    return host_wait(ctx, ctx->stream) ? BWTC_CUDA_ECUDA : 0;
+  }
+  return run_divsufsort(ctx, nullptr, static_cast<const uint8_t*>(d_T), nullptr, static_cast<int32_t*>(d_SA), n, nullptr,
+                        static_cast<int32_t*>(d_LCP));
 }
 
 int bwtc_cuda_sufcheck(bwtc_cuda_ctx* ctx, const uint8_t* T, const int32_t* SA, uint32_t n) {

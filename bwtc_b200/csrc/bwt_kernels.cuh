@@ -2391,4 +2391,278 @@ __global__ void k_debug_swap_sa(int32_t* sa, uint32_t r) {
   sa[r + 1u] = a;
 }
 
+// =====================================================================================================
+// LCP array of a finished suffix array (bwtc_cuda_divsufsort_lcp, DESIGN.md §3.12).  No Φ and no rank array:
+//   (1) k_lcp_short, rank order: row r >= 1 with i = SA[r], j = SA[r-1] is IRREDUCIBLE when i == 0 || j == 0 ||
+//       T[i-1] != T[j-1]; only those compare T[i..] with T[j..] and store X[i] = i + lcp (row 0: X[SA[0]] = SA[0]); every
+//       other X[i] stays 0.  The irreducible LCP values sum to at most 2 n log n (Kärkkäinen, Manzini & Puglisi, CPM 2009).
+//   (2) a thread compares LCP_SHORT_BYTES bytes of its pair; a pair still equal there goes to a list and is finished in
+//       windows [K 2^w, K 2^(w+1)) (k_lcp_window, one launch per w), each split into LCP_SEG_BYTES-byte segments that
+//       warps compare independently, meeting in atomicMin(X[i]).  The warp finishing a pair's last segment appends the
+//       pair to the next window's list if the window held no mismatch.  Work per pair: at most ~3x its LCP + K.
+//   (3) PLCP[i] + i never decreases and is constant over reducible runs, so PLCP[i] = maxscan(X)[i] - i
+//       (k_lcp_tile_max, k_lcp_tile_scan, k_lcp_apply: reduce-then-scan, no inter-CTA waiting).
+//   (4) LCP[r] = PLCP[SA[r]] (k_lcp_gather).
+// Text reads never leave T[0, n): the device variant's T is the caller's unpadded buffer at any alignment.
+// =====================================================================================================
+constexpr uint32_t LCP_SHORT_BYTES = 32;     // K: bytes one thread compares before a pair goes to the window lists
+constexpr uint32_t LCP_SEG_BYTES = 1024;     // bytes of one window segment (one warp, 128 bytes per step)
+constexpr uint32_t LCP_SCAN_TILE = 4096;     // X entries per CTA of the max-scan (256 threads x 16)
+constexpr int LCP_MAX_WINDOWS = 32;          // K 2^w < 2^32
+
+struct LcpCtl {                              // zeroed per call; 64-bit work counters
+  unsigned long long irreducible;            // rows that compared bytes
+  unsigned long long short_bytes;            // bytes the short tier compared (up to and including the mismatch)
+  unsigned long long window_bytes;           // bytes the window segments compared
+  unsigned long long segments;               // window segments processed
+  uint32_t count[LCP_MAX_WINDOWS + 1];       // pairs in the list of window w (count[0]: pairs that left the short tier)
+};
+struct LcpLists {                            // the lists of windows w (slot w & 1): row r of the pair, segments done
+  uint32_t* row[2];
+  uint32_t* done[2];
+};
+
+// T[p..p+3] as a little-endian word, bytes at or past n read as 0.  Interior: two aligned loads and a funnel shift.
+__device__ __forceinline__ uint32_t lcp_word(const uint8_t* __restrict__ t, uint32_t n, uint32_t p) {
+  const uint32_t mis = (uint32_t)(reinterpret_cast<uintptr_t>(t + p) & 3u);
+  if (p >= mis && (uint64_t)p - mis + 8u <= n) {
+    const uint32_t* w = reinterpret_cast<const uint32_t*>(t + (p - mis));
+    return __funnelshift_r(__ldg(w), __ldg(w + 1), mis * 8u);
+  }
+  uint32_t v = 0;
+#pragma unroll
+  for (uint32_t k = 0; k < 4u; ++k)
+    if ((uint64_t)p + k < n) v |= (uint32_t)t[p + k] << (8u * k);
+  return v;
+}
+
+__device__ __forceinline__ void lcp_count(unsigned long long* dst, unsigned long long v) {  // one atomic per warp
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xFFFFFFFFu, v, o);
+  if ((threadIdx.x & 31u) == 0u && v) atomicAdd(dst, v);
+}
+
+// (1) + the short tier of (2).  x[0..n) must be zero.
+__global__ void __launch_bounds__(256) k_lcp_short(const uint8_t* __restrict__ t, const int32_t* __restrict__ sa, uint32_t n,
+                                                   uint32_t* __restrict__ x, LcpLists L, LcpCtl* __restrict__ lc,
+                                                   const uint32_t* __restrict__ ctrl) {
+  if (ctrl[CTR_ERR]) return;
+  unsigned long long irr = 0, bytes = 0;
+  const uint32_t stride = gridDim.x * blockDim.x;
+  for (uint32_t base = blockIdx.x * blockDim.x; base < n; base += stride) {  // (warp-uniform trip count: lcp_count)
+    const uint32_t r = base + threadIdx.x;
+    if (r >= n) continue;
+    const uint32_t i = (uint32_t)sa[r];
+    if (r == 0u) { x[i] = i; continue; }
+    const uint32_t j = (uint32_t)sa[r - 1u];
+    if (i != 0u && j != 0u && t[i - 1u] == t[j - 1u]) continue;
+    ++irr;
+    const uint32_t limit = n - max(i, j);
+    const uint32_t len = min(limit, LCP_SHORT_BYTES);
+    uint32_t l = len;
+    for (uint32_t k = 0; k < len; k += 4u) {
+      const uint32_t d = lcp_word(t, n, i + k) ^ lcp_word(t, n, j + k);
+      if (d) { l = min(len, k + ((uint32_t)(__ffs((int)d) - 1) >> 3)); break; }
+    }
+    bytes += min(l + 1u, len);
+    x[i] = i + (l < len ? l : limit);  // (a pair that goes on starts at "equal to the end"; the windows lower it)
+    if (l == len && limit > LCP_SHORT_BYTES) {
+      const uint32_t m = __activemask(), lane = threadIdx.x & 31u, lead = __ffs((int)m) - 1;
+      uint32_t pos = 0;
+      if (lane == lead) pos = atomicAdd(&lc->count[0], (uint32_t)__popc(m));
+      pos = __shfl_sync(m, pos, lead) + (uint32_t)__popc(m & ((1u << lane) - 1u));
+      L.row[0][pos] = r;
+      L.done[0][pos] = 0u;
+    }
+  }
+  __syncwarp();
+  lcp_count(&lc->irreducible, irr);
+  lcp_count(&lc->short_bytes, bytes);
+}
+
+// (2) window w = [K 2^w, K 2^(w+1)) of every pair in its list.  One warp per (pair, segment).
+__global__ void __launch_bounds__(256) k_lcp_window(const uint8_t* __restrict__ t, const int32_t* __restrict__ sa, uint32_t n,
+                                                    uint32_t* __restrict__ x, LcpLists L, LcpCtl* __restrict__ lc, uint32_t w,
+                                                    const uint32_t* __restrict__ ctrl) {
+  if (ctrl[CTR_ERR]) return;
+  const uint32_t cnt = *reinterpret_cast<volatile uint32_t*>(&lc->count[w]);
+  if (!cnt) return;
+  const uint32_t lane = threadIdx.x & 31u;
+  const uint64_t lo = (uint64_t)LCP_SHORT_BYTES << w, hi = lo << 1;
+  const uint32_t seg_len = lo < LCP_SEG_BYTES ? (uint32_t)lo : LCP_SEG_BYTES;
+  const uint32_t segs = (uint32_t)(lo / seg_len);
+  const uint64_t total = (uint64_t)cnt * segs;
+  const bool odd = (w & 1u) != 0u;  // (selects, not indexes, the slots: no local copy of L)
+  const uint32_t* rows = odd ? L.row[1] : L.row[0];
+  uint32_t* done = odd ? L.done[1] : L.done[0];
+  uint32_t* next_rows = odd ? L.row[0] : L.row[1];
+  uint32_t* next_done = odd ? L.done[0] : L.done[1];
+  unsigned long long bytes = 0, nseg = 0;
+  const uint64_t nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
+  for (uint64_t q = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; q < total; q += nwarps) {
+    const uint32_t e = (uint32_t)(q / segs), s = (uint32_t)(q % segs);
+    const uint32_t r = rows[e];
+    const uint32_t i = (uint32_t)sa[r], j = (uint32_t)sa[r - 1u];
+    const uint64_t limit = n - max(i, j);
+    const uint64_t a = lo + (uint64_t)s * seg_len;
+    uint64_t b = a + seg_len < hi ? a + seg_len : hi;
+    if (b > limit) b = limit;
+    ++nseg;
+    // skipped when an earlier segment already found a mismatch below this one
+    uint32_t found = 0;
+    if (lane == 0u) found = *reinterpret_cast<volatile uint32_t*>(&x[i]) - i;
+    found = __shfl_sync(0xFFFFFFFFu, found, 0);
+    if (a < b && (uint64_t)found > a) {
+      for (uint64_t o = a; o < b; o += 128u) {
+        const uint64_t p = o + 4u * lane;
+        uint32_t mm = 0xFFFFFFFFu;
+        if (p < b) {
+          const uint32_t d = lcp_word(t, n, (uint32_t)(i + p)) ^ lcp_word(t, n, (uint32_t)(j + p));
+          if (d) {
+            const uint64_t at = p + ((uint32_t)(__ffs((int)d) - 1) >> 3);
+            if (at < b) mm = (uint32_t)at;
+          }
+        }
+        const uint32_t hit = __ballot_sync(0xFFFFFFFFu, mm != 0xFFFFFFFFu);
+        if (hit) {
+          const uint32_t first = __shfl_sync(0xFFFFFFFFu, mm, __ffs((int)hit) - 1);
+          if (lane == 0u) atomicMin(&x[i], i + first);
+          bytes += first + 1u - o;
+          break;
+        }
+        bytes += (b - o < 128u) ? b - o : 128u;
+      }
+    }
+    if (lane == 0u) {
+      __threadfence();
+      if (atomicAdd(&done[e], 1u) == segs - 1u) {  // the last segment of this pair: does it need the next window?
+        __threadfence();
+        const uint32_t v = atomicAdd(&x[i], 0u) - i;
+        if ((uint64_t)v >= hi && hi < limit && w + 1u < (uint32_t)LCP_MAX_WINDOWS) {
+          const uint32_t pos = atomicAdd(&lc->count[w + 1u], 1u);
+          next_rows[pos] = r;
+          next_done[pos] = 0u;
+        }
+      }
+    }
+    __syncwarp();
+  }
+  if (lane == 0u) {
+    if (bytes) atomicAdd(&lc->window_bytes, bytes);
+    if (nseg) atomicAdd(&lc->segments, nseg);
+  }
+}
+
+// (3) reduce-then-scan of max(X): tile maxima, their exclusive scan (one CTA), then each tile rescanned.
+__global__ void __launch_bounds__(256) k_lcp_tile_max(const uint32_t* __restrict__ x, uint32_t n, uint32_t* __restrict__ tmax,
+                                                      const uint32_t* __restrict__ ctrl) {
+  if (ctrl[CTR_ERR]) return;
+  __shared__ uint32_t wm[8];
+  const uint64_t base = (uint64_t)blockIdx.x * LCP_SCAN_TILE;
+  uint32_t m = 0;
+  for (uint32_t k = threadIdx.x; k < LCP_SCAN_TILE; k += 256u)
+    if (base + k < n) m = max(m, x[base + k]);
+  for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(0xFFFFFFFFu, m, o));
+  if ((threadIdx.x & 31u) == 0u) wm[threadIdx.x >> 5] = m;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int k = 1; k < 8; ++k) m = max(m, wm[k]);
+    tmax[blockIdx.x] = max(m, wm[0]);
+  }
+}
+
+__global__ void __launch_bounds__(1024) k_lcp_tile_scan(uint32_t* __restrict__ tmax, uint32_t ntiles, const uint32_t* __restrict__ ctrl) {
+  if (ctrl[CTR_ERR]) return;
+  __shared__ uint32_t wm[32];
+  __shared__ uint32_t carry_s;
+  const uint32_t lane = threadIdx.x & 31u, wid = threadIdx.x >> 5;
+  uint32_t carry = 0;
+  for (uint32_t base = 0; base < ntiles; base += 1024u) {
+    const uint32_t k = base + threadIdx.x;
+    const uint32_t v = k < ntiles ? tmax[k] : 0u;
+    uint32_t inc = v;
+    for (int o = 1; o < 32; o <<= 1) {
+      const uint32_t u = __shfl_up_sync(0xFFFFFFFFu, inc, o);
+      if ((int)lane >= o) inc = max(inc, u);
+    }
+    if (lane == 31u) wm[wid] = inc;
+    __syncthreads();
+    if (wid == 0) {
+      uint32_t s = wm[lane];
+      for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t u = __shfl_up_sync(0xFFFFFFFFu, s, o);
+        if ((int)lane >= o) s = max(s, u);
+      }
+      wm[lane] = s;
+    }
+    __syncthreads();
+    const uint32_t up = __shfl_up_sync(0xFFFFFFFFu, inc, 1);
+    uint32_t excl = max(carry, wid ? wm[wid - 1] : 0u);
+    if (lane) excl = max(excl, up);
+    if (k < ntiles) tmax[k] = excl;
+    if (threadIdx.x == 1023u) carry_s = max(carry, wm[31]);
+    __syncthreads();
+    carry = carry_s;
+    __syncthreads();
+  }
+}
+
+// PLCP[i] = max(tile prefix, X[tile start .. i]) - i, in place.  Each thread owns 16 consecutive entries.
+__global__ void __launch_bounds__(256) k_lcp_apply(uint32_t* __restrict__ x, uint32_t n, const uint32_t* __restrict__ tpre,
+                                                   const uint32_t* __restrict__ ctrl) {
+  if (ctrl[CTR_ERR]) return;
+  __shared__ uint32_t wm[8];
+  const uint32_t lane = threadIdx.x & 31u, wid = threadIdx.x >> 5;
+  const uint64_t p0 = (uint64_t)blockIdx.x * LCP_SCAN_TILE + (uint64_t)threadIdx.x * 16u;
+  uint32_t v[16];
+  const bool full = p0 + 16u <= n;
+  if (full) {
+    const uint4* s = reinterpret_cast<const uint4*>(x + p0);
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const uint4 u = s[q];
+      v[4 * q] = u.x; v[4 * q + 1] = u.y; v[4 * q + 2] = u.z; v[4 * q + 3] = u.w;
+    }
+  } else {
+#pragma unroll
+    for (int q = 0; q < 16; ++q) v[q] = (p0 + q < n) ? x[p0 + q] : 0u;
+  }
+  uint32_t m = 0;
+#pragma unroll
+  for (int q = 0; q < 16; ++q) m = max(m, v[q]);
+  uint32_t inc = m;
+  for (int o = 1; o < 32; o <<= 1) {
+    const uint32_t u = __shfl_up_sync(0xFFFFFFFFu, inc, o);
+    if ((int)lane >= o) inc = max(inc, u);
+  }
+  if (lane == 31u) wm[wid] = inc;
+  __syncthreads();
+  uint32_t run = tpre[blockIdx.x];
+  for (uint32_t k = 0; k < wid; ++k) run = max(run, wm[k]);
+  const uint32_t up = __shfl_up_sync(0xFFFFFFFFu, inc, 1);
+  if (lane) run = max(run, up);
+#pragma unroll
+  for (int q = 0; q < 16; ++q) {
+    run = max(run, v[q]);
+    v[q] = run - (uint32_t)(p0 + q);
+  }
+  if (full) {
+    uint4* d = reinterpret_cast<uint4*>(x + p0);
+#pragma unroll
+    for (int q = 0; q < 4; ++q) d[q] = make_uint4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
+  } else {
+#pragma unroll
+    for (int q = 0; q < 16; ++q)
+      if (p0 + q < n) x[p0 + q] = v[q];
+  }
+}
+
+// (4) LCP[r] = PLCP[SA[r]].
+__global__ void __launch_bounds__(256) k_lcp_gather(const int32_t* __restrict__ sa, const uint32_t* __restrict__ plcp, uint32_t n,
+                                                    int32_t* __restrict__ lcp, const uint32_t* __restrict__ ctrl) {
+  if (ctrl[CTR_ERR]) return;
+  const uint32_t stride = gridDim.x * blockDim.x;
+  for (uint32_t r = blockIdx.x * blockDim.x + threadIdx.x; r < n; r += stride) lcp[r] = (int32_t)plcp[(uint32_t)sa[r]];
+}
+
 }  // namespace bwtc_b200

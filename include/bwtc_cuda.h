@@ -13,6 +13,8 @@
  *   bwtc_cuda_divsufsort / _device /       <-  divsufsort / sufcheck                  bwtransforms/divsufsort.h (the
  *   bwtc_cuda_sufcheck                         library's suffix-array entry point and its checker, beside the BWT
  *                                              entry points above)
+ *   bwtc_cuda_divsufsort_lcp / _device     <-  no counterpart in bwtc's divsufsort: the SA and its LCP array, in the
+ *                                              convention of libsais's libsais_plcp / libsais_lcp
  *   bwtc_cuda_bwt_block                    <-  BWTransform::doTransform(BWTBlock&, uint32 freqs[256])
  *                                              bwtransforms/BWTransform.cpp:39-64 (reverse / sentinel /
  *                                              hole-fill fused on the device)
@@ -88,7 +90,8 @@ typedef struct bwtc_cuda_stats {
                               * contract) and its LFpowers were verified by a device-side inversion (bwtc_cuda_ctx_set_verify,
                               * BWTC_VERIFY; for bwtc_cuda_divsufsort: its suffix array passed the device-side sufcheck); bit 7:
                               * inverse only, this block is corrupt (BWTC_CUDA_ECORRUPT); bit 8: this call produced a suffix
-                              * array (bwtc_cuda_divsufsort, _device) */
+                              * array (bwtc_cuda_divsufsort, _device, and the _lcp variants); bit 9: this call produced an
+                              * LCP array (bwtc_cuda_divsufsort_lcp, _lcp_device) */
   uint32_t batch_blocks;     /* blocks this record describes: 1, or the size of the batch that was sorted as one text (every
                               * block of the batch then carries the SAME record — count it once; flags bit 7 is the one field
                               * in which the records of one inverse batch may differ) */
@@ -132,7 +135,8 @@ int         bwtc_cuda_ctx_set_verify(bwtc_cuda_ctx* ctx, int on);
 /* Debug / test hooks: max_rounds != 0 stops the refinement after that many sort rounds (the output is
  * then deliberately incomplete); bwtc_cuda_debug_read copies an engine buffer to the host
  * (which: 0 text, 1 rank[], 2/3 sorted keys/ids of the last round, 4/5 the other sort buffer,
- * 6 control+histogram words, 7 staged input). */
+ * 6 control+histogram words, 7 staged input, 9 the work counters of the last LCP stage: irreducible rows, bytes
+ * compared by the short tier and by the windows, window segments (4 x u64), then the pairs in each window's list, u32). */
 int         bwtc_cuda_ctx_set_debug(bwtc_cuda_ctx* ctx, uint32_t max_rounds);
 int         bwtc_cuda_debug_read(bwtc_cuda_ctx* ctx, int which, uint64_t offset_bytes, void* dst, uint64_t bytes);
 
@@ -163,6 +167,22 @@ int64_t bwtc_cuda_divbwt(bwtc_cuda_ctx* ctx, const uint8_t* T, uint8_t* U, uint3
  * stats.flags bit 8 is set (bit 6 too when verified); no other entry point sets bit 8. */
 int bwtc_cuda_divsufsort(bwtc_cuda_ctx* ctx, const uint8_t* T, int32_t* SA, uint32_t n);
 int bwtc_cuda_divsufsort_device(bwtc_cuda_ctx* ctx, const void* d_T, void* d_SA, uint32_t n);  /* d_SA 4-byte aligned */
+/* divsufsort_lcp(T, SA, LCP, n): SA as bwtc_cuda_divsufsort returns it, and its longest-common-prefix array: LCP[0] = 0,
+ * LCP[r] (r >= 1) = the length of the longest common prefix of suffixes SA[r-1] and SA[r], a comparison stopping at the
+ * end of the text.  No counterpart in bwtc's divsufsort; the convention is libsais's (libsais_plcp / libsais_lcp).
+ * Returns 0 or a negative error.  n == 0: nothing is written; n == 1: SA[0] = LCP[0] = 0 (the host variant does not touch
+ * the device).  n <= max_block_bytes + 1 (else BWTC_CUDA_ETOOBIG); null pointers are BWTC_CUDA_EARG.  The LCP is built
+ * on the device behind the sort, from the text and SA already there (irreducible rows compared, a max-scan in text order,
+ * a gather into rank order; DESIGN.md §3.12), in scratch that is idle by then: the host variant allocates nothing beyond
+ * the device SA of bwtc_cuda_divsufsort, and bwtc_cuda_scratch_bytes is unchanged.  SA and LCP may each be pageable or
+ * pinned host memory (pinned: copied directly, pageable: through the staging ring).  _lcp_device writes d_SA and d_LCP
+ * (n int32 entries each, 4-byte aligned, not overlapping, else BWTC_CUDA_EARG; d_T may have any alignment and is read
+ * only within its n bytes).  With verification on, the SA is sufchecked on the device before the LCP stage runs: on a
+ * failure the call returns BWTC_CUDA_EVERIFY and host SA / LCP are untouched.  The LCP itself is not re-checked: a
+ * complete check costs as much as computing it.  stats.flags bits 8 and 9 are set (bit 6 too when verified); gpu_ms,
+ * kernel_launches and algorithmic_bytes include the LCP stage. */
+int bwtc_cuda_divsufsort_lcp(bwtc_cuda_ctx* ctx, const uint8_t* T, int32_t* SA, int32_t* LCP, uint32_t n);
+int bwtc_cuda_divsufsort_lcp_device(bwtc_cuda_ctx* ctx, const void* d_T, void* d_SA, void* d_LCP, uint32_t n);
 /* sufcheck(T, SA, n): 0 if SA (host, pageable or pinned) is the suffix array of T, BWTC_CUDA_ECORRUPT if not -- the message
  * names the first offending row and why: out of range / duplicate (of an earlier row) / out of order; range and duplicate
  * failures are reported before order failures.  Other negatives as usual (BWTC_CUDA_ETOOBIG above max_block_bytes + 1).
