@@ -34,6 +34,7 @@ FLAG_VERIFIED = 1 << 6            # stats flags bit 6: the forward output was ve
 FLAG_CORRUPT = 1 << 7             # stats flags bit 7: this inverse block is corrupt
 FLAG_SA = 1 << 8                  # stats flags bit 8: this call produced a suffix array (divsufsort)
 FLAG_LCP = 1 << 9                 # stats flags bit 9: this call produced an LCP array (divsufsort_lcp)
+FLAG_ROUND0_BUCKETS = 1 << 10     # stats flags bit 10: round 0 sorted its low key digits bucket by bucket (k_bucket_sort)
 
 
 class BwtcCudaUnavailable(RuntimeError):
@@ -71,6 +72,7 @@ class Stats(ctypes.Structure):
         ("sort0_ms", ctypes.c_float),
         ("flags", ctypes.c_uint32),
         ("batch_blocks", ctypes.c_uint32),
+        ("round0_big_buckets", ctypes.c_uint32),
     ]
 
     def as_dict(self) -> dict:
@@ -84,7 +86,7 @@ class Stats(ctypes.Structure):
             "gpu_ms": float(self.gpu_ms), "sort_ms": float(self.sort_ms), "sort_bytes": int(self.sort_bytes),
             "sort_launches": int(self.sort_launches), "sort0_launches": int(self.sort0_launches),
             "sort0_bytes": int(self.sort0_bytes), "sort0_ms": float(self.sort0_ms), "flags": int(self.flags),
-            "batch_blocks": int(self.batch_blocks),
+            "batch_blocks": int(self.batch_blocks), "round0_big_buckets": int(self.round0_big_buckets),
         }
 
 

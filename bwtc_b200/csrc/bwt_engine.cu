@@ -138,6 +138,8 @@ struct bwtc_cuda_ctx {
   double lazy_max_repeats = 32.0; // blocks with memory: at most this many other positions share a position's 8-gram (Markov
                                   // 16 / 32 / 64 MiB: 1.3 / 3.0 / 5.2; repetitive 16 MiB: ~3800, source text ~1.5e5)
   int use_seg = 1;                // segmented (sort-free) doubling rounds when every group is small
+  int round0_top = -1;            // round-0 digit passes over the top digits only, then k_bucket_sort (DESIGN.md §3.2):
+                                  // -1 policy, 0 never (all digit passes), 2..7 always with this many top passes
   int use_batch = 1;              // small equal-sized blocks of one call are sorted as one text
   int use_pack_pred = 1;          // carry code(T[id-1]) above the id through the round-0 sort when it fits
   uint32_t aux_min_suffixes = 96u << 20;  // ... else, from this many suffixes on, as a one-byte payload array (0 = never)
@@ -307,6 +309,20 @@ void plan_round0(const bwtc_cuda_ctx* ctx, const uint64_t* count, const bool* pr
   pl->pp.chars = chars;
   pl->pp.nblocks = 1;
   pl->pp.stride = 0;
+}
+
+// Round-0 digit passes over the top digits only, the low ones sorted bucket by bucket on chip (k_bucket_sort;
+// DESIGN.md §3.2): the number of top passes, 0 = every digit pass.  64-bit keys only, not for batches and not with the
+// one-byte payload (k_bucket_sort moves keys and ids).  The policy takes it for sources with memory whose 8-gram sample
+// shows few repeats (the lazy-rank statistic, §3.9): their buckets after 40 key bits are small (Markov 32 MiB: at most
+// 1194 records, 13.6 per record on average), while repeats and source text leave buckets too large for one CTA.
+constexpr uint32_t ROUND0_TOP_DEFAULT = 5;
+uint32_t plan_round0_top(const bwtc_cuda_ctx* ctx, const Round0Plan& pl, bool batch, bool aux) {
+  if (pl.keybytes != 8 || batch || aux || ctx->round0_top == 0) return 0;
+  uint32_t top = ROUND0_TOP_DEFAULT;
+  if (ctx->round0_top > 0) top = (uint32_t)ctx->round0_top;
+  else if (!(pl.has_memory && pl.repeats <= ctx->lazy_max_repeats)) return 0;
+  return (top >= 2 && top < pl.npass) ? top : 0u;
 }
 
 // Number of id windows the rank scatter of a round is split into (k_rerank RerankParams::win_lo/hi).
@@ -818,7 +834,20 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
   // ---- round 0: pack keys (+ all digit histograms), sort, re-rank
   const uint32_t rs_tile0 = pl.keybytes == 4 ? RS_TILE32 : RS_TILE64;
   const uint32_t all0 = (1u << pl.npass) - 1u;
-  if (zero_round_state(ctx, N, N, rs_tile0, all0)) return BWTC_CUDA_ECUDA;
+  // When the id and one character code fit a 32-bit payload together, the first pass stores the code of the
+  // character preceding each suffix above the id: the round-0 BWT emission then needs no text gather.
+  uint32_t id_bits = (uint32_t)ceil_log2_u64((uint64_t)N);
+  if (id_bits < 1) id_bits = 1;
+  const bool pack_pred = ctx->use_pack_pred && (id_bits + pl.bits <= 32);
+  // No spare id bits (byte alphabets above 16 MiB) and a text too large for an L2-resident gather at emission time:
+  // the predecessor codes travel as a one-byte payload array instead.
+  const bool aux_pred = !pack_pred && ctx->aux_min_suffixes && N >= ctx->aux_min_suffixes && !bs;
+  // every digit pass of the round runs (a constant digit makes its pass a stable identity permutation, and finding that
+  // out would cost a host synchronisation per block) — or only the top0 upper ones, and k_bucket_sort does the rest
+  const uint32_t top0 = plan_round0_top(ctx, pl, bs != nullptr, aux_pred);
+  const uint32_t low0 = top0 ? pl.npass - top0 : 0u;
+  const uint32_t mask0 = all0 & ~((1u << low0) - 1u);
+  if (zero_round_state(ctx, N, N, rs_tile0, mask0)) return BWTC_CUDA_ECUDA;
   {
     const uint32_t ptiles = div_up(N, AUX_TILE);
     const int grid = (int)(ptiles < (uint32_t)(ctx->sm_count * 4) ? ptiles : (uint32_t)(ctx->sm_count * 4));
@@ -893,22 +922,11 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
     S.kernel_launches++;
     S.algorithmic_bytes += (uint64_t)N + (uint64_t)N * pl.keybytes;
   }
-  // every digit pass of the round runs: a constant digit makes its pass a (stable) identity permutation, and
-  // finding that out would cost a host synchronisation per block
-  const uint32_t mask0 = all0;
   int cur = 0;
   uint32_t pdone = 0;
   int rc;
-  // When the id and one character code fit a 32-bit payload together, the first pass stores the code of the
-  // character preceding each suffix above the id: the round-0 BWT emission then needs no text gather.
-  uint32_t id_bits = (uint32_t)ceil_log2_u64((uint64_t)N);
-  if (id_bits < 1) id_bits = 1;
-  const bool pack_pred = ctx->use_pack_pred && (id_bits + pl.bits <= 32) && (mask0 & 1u);
   const uint32_t topshift = (pl.chars - 1) * pl.bits + pl.rbits;
   const uint32_t pred_mask = (1u << pl.bits) - 1u;  // (a batch key carries the block number above the characters)
-  // No spare id bits (byte alphabets above 16 MiB) and a text too large for an L2-resident gather at emission time:
-  // the predecessor codes travel as a one-byte payload array instead.
-  const bool aux_pred = !pack_pred && ctx->aux_min_suffixes && N >= ctx->aux_min_suffixes && (mask0 & 1u) && !bs;
   if (pl.keybytes == 4)
     rc = run_sort<uint32_t, RS_IPT32>(ctx, N, mask0, true, N - 1, &cur, &pt, &pdone, pack_pred ? id_bits : 0u, topshift,
                                       pred_mask, aux_pred);
@@ -916,6 +934,16 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
     rc = run_sort<unsigned long long, RS_IPT64>(ctx, N, mask0, true, N - 1, &cur, &pt, &pdone, pack_pred ? id_bits : 0u,
                                                 topshift, pred_mask, aux_pred);
   if (rc) return rc;
+  if (top0) {
+    // the passes left every bucket of equal top bits contiguous and in input order: sort each by its low 8·low0 key bits
+    k_bucket_sort<<<div_up(N, BK_T), BK_BLOCK, 0, st>>>(static_cast<unsigned long long*>(ctx->d_keys[cur]), ctx->d_idx[cur],
+                                                        static_cast<unsigned long long*>(ctx->d_keys[cur ^ 1]), ctx->d_idx[cur ^ 1],
+                                                        N, 8u * low0, ctx->d_ctrl(), &ctx->d_state->big_buckets);
+    CK(ctx, cudaGetLastError());
+    S.kernel_launches++;
+    S.algorithmic_bytes += (uint64_t)N * 24;  // keys and ids read and written once (in place)
+    ++pdone;
+  }
   const size_t round0_events = pt.used;
   S.sort0_launches = S.sort_launches;
   S.sort0_bytes = S.sort_bytes;
@@ -980,7 +1008,7 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
       CK(ctx, cudaMemcpyAsync(ctx->d_lookup, ctx->h_lookup, sizeof(LookupParams), cudaMemcpyHostToDevice, st));
     }
     S.flags = (ctx->static_tiles ? 0u : 1u) | (bs ? 2u : 0u) | (pack_pred ? 4u : 0u) | (aux_pred ? 8u : 0u) | (lazy ? 16u : 0u) |
-              (J.sa ? 256u : 0u);
+              (J.sa ? 256u : 0u) | (top0 ? 1024u : 0u);
     rp.packed = pack_pred ? 1u : (aux_pred ? 2u : 0u);
     rp.pred_aux = ctx->d_aux[cur];
     rp.id_bits = pack_pred ? id_bits : 31u;
@@ -1137,6 +1165,7 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
     }
     if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
     const LadderState& H = *ctx->h_state;
+    S.round0_big_buckets = H.big_buckets;
     if (H.err == 4u) {
       set_err(ctx->err, "segmented round met a group above its limit (internal error)");
       return BWTC_CUDA_EINTERNAL;
@@ -1983,6 +2012,7 @@ int bwtc_cuda_ctx_create(bwtc_cuda_ctx** out, int device, uint32_t max_block_byt
   if (const char* e = getenv("BWTC_LAZY_MAX_LIVE")) c->lazy_max_live = atof(e);
   if (const char* e = getenv("BWTC_LAZY_MAX_REPEATS")) c->lazy_max_repeats = atof(e);
   if (const char* e = getenv("BWTC_SEG")) c->use_seg = atoi(e);
+  if (const char* e = getenv("BWTC_ROUND0_TOP")) c->round0_top = atoi(e);
   if (const char* e = getenv("BWTC_BATCH")) c->use_batch = atoi(e);
   if (const char* e = getenv("BWTC_PACK_PRED")) c->use_pack_pred = atoi(e);
   if (const char* e = getenv("BWTC_AUX_MIN_MIB")) { const long v = atol(e); c->aux_min_suffixes = v > 0 ? (uint32_t)v << 20 : (v == 0 ? 1u : 0u); }

@@ -913,6 +913,182 @@ __global__ void __launch_bounds__(BLOCK, (sizeof(KeyT) == 4 && !AUX) ? BWTC_RS_M
 }
 
 // =====================================================================================================
+// k_bucket_sort — the low digits of the round-0 sort, bucket by bucket (DESIGN.md §3.2).  The digit passes
+// have ordered the records stably by the key bits above `lowbits`; every bucket (records with equal top bits)
+// is contiguous and still in input order.  The kernel sorts each bucket in place by its full key, ties by input
+// position: the order all 8 passes would have produced.
+// A CTA owns the buckets that START in [blockIdx.x * BK_T, + BK_T); the last one may run past that range.  It
+// loads a window of up to BK_CAP records, marks bucket heads (top bits differ from the predecessor's) in a
+// bitmap and ranks every record of its buckets by counting the members with a smaller (low key bits, window
+// offset) composite — consecutive lanes take consecutive records, so a bucket's members read the same
+// shared-memory word at the same time (broadcast).  A bucket longer than BK_CAP takes a slow single-CTA stable
+// LSD sort through the idle ping-pong buffers (`tkeys` / `tids`, same positions) and is counted in *nbig.
+// =====================================================================================================
+constexpr uint32_t BK_BLOCK = 256, BK_IPT = 16, BK_CAP = BK_BLOCK * BK_IPT;  // window capacity 4096
+constexpr uint32_t BK_T = BK_CAP - 512;  // records per CTA: a bucket that starts in range may run 512 past it in one window
+
+__global__ void __launch_bounds__(BK_BLOCK, 3) k_bucket_sort(unsigned long long* __restrict__ keys, uint32_t* __restrict__ ids,
+                                                             unsigned long long* __restrict__ tkeys, uint32_t* __restrict__ tids,
+                                                             uint32_t N, uint32_t lowbits, const uint32_t* __restrict__ ctrl,
+                                                             uint32_t* __restrict__ nbig) {
+  __shared__ unsigned long long s_cmp[BK_CAP];  // (low key bits << (64 - lowbits)) | window offset
+  __shared__ uint32_t s_head[BK_CAP / 32 + 1];  // bit r: window record r starts a bucket; bit Lw: the window's end does
+  __shared__ uint32_t s_sel[4];
+  __shared__ uint32_t s_hist[256 + 8 * 256];    // slow path: digit bases, per-warp digit counts
+  const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const uint32_t lo = blockIdx.x * BK_T;
+  if (lo >= N || ctrl[CTR_ERR]) return;
+  const uint32_t hi = min(N, lo + BK_T);
+  const uint32_t cshift = 64u - lowbits;
+  uint32_t pos = lo;
+  bool first = true;
+  for (;;) {
+    const uint32_t wend = min(N, pos + BK_CAP), Lw = wend - pos;
+    unsigned long long key[BK_IPT];
+    uint32_t id[BK_IPT];
+#pragma unroll
+    for (int k = 0; k < (int)BK_IPT; ++k) {
+      const uint32_t g = pos + tid + k * BK_BLOCK;
+      key[k] = g < wend ? keys[g] : 0ull;
+      id[k] = g < wend ? ids[g] : 0u;
+    }
+    if (tid == 0) {
+      s_head[BK_CAP / 32] = 0;
+      s_sel[0] = s_sel[1] = 0xFFFFFFFFu;
+      s_sel[2] = 0;
+    }
+#pragma unroll
+    for (int k = 0; k < (int)BK_IPT; ++k) {
+      const uint32_t r = tid + k * BK_BLOCK, g = pos + r;
+      unsigned long long prev = __shfl_up_sync(0xFFFFFFFFu, key[k], 1);
+      if (lane == 0 && g > 0 && g < wend) prev = keys[g - 1];
+      const bool head = g < wend && (g == 0 || (key[k] >> lowbits) != (prev >> lowbits));
+      const uint32_t b = __ballot_sync(0xFFFFFFFFu, head);
+      if (lane == 0) s_head[r >> 5] = b;
+    }
+    __syncthreads();
+    if (tid == 0 && (wend == N || (keys[wend] >> lowbits) != (keys[wend - 1] >> lowbits))) s_head[Lw >> 5] |= 1u << (Lw & 31);
+    __syncthreads();
+    // chunk [c0, c1) of the window: c0 = first head (at pos itself after the first window), c1 = the first head at or
+    // past hi (the CTA's last chunk), else the last head in the window (more chunks follow)
+    const uint32_t nw = (Lw >> 5) + 1;
+    if (first) {
+      if (tid < nw && s_head[tid]) atomicMin(&s_sel[0], tid * 32 + __ffs(s_head[tid]) - 1);
+      __syncthreads();
+    } else if (tid == 0) {
+      s_sel[0] = 0;
+    }
+    const uint32_t c0 = first ? s_sel[0] : 0u;
+    if (c0 == 0xFFFFFFFFu || pos + c0 >= hi) return;  // (uniform) no bucket starts in range: the window lies inside one
+    const uint32_t from = max(c0 + 1, hi - pos);
+    if (tid < nw) {
+      const uint32_t w = s_head[tid];
+      const uint32_t wlo = tid * 32;
+      const uint32_t mf = from >= wlo + 32 ? 0u : (from <= wlo ? w : w & (0xFFFFFFFFu << (from - wlo)));
+      if (mf) atomicMin(&s_sel[1], wlo + __ffs(mf) - 1);
+      const uint32_t mh = c0 + 1 >= wlo + 32 ? 0u : (c0 + 1 <= wlo ? w : w & (0xFFFFFFFFu << (c0 + 1 - wlo)));
+      if (mh) atomicMax(&s_sel[2], wlo + 32 - __clz(mh));  // last head + 1
+    }
+    __syncthreads();
+    const uint32_t fmin = s_sel[1], hmax1 = s_sel[2];
+    if (fmin == 0xFFFFFFFFu && hmax1 == 0) {
+      if (c0 > 0) {  // the first bucket in range runs past the window: start a window at it
+        pos += c0;
+        first = false;
+        __syncthreads();
+        continue;
+      }
+      break;  // the bucket at pos is longer than the window (oversized: slow path below)
+    }
+    const uint32_t c1 = fmin != 0xFFFFFFFFu ? fmin : hmax1 - 1u;
+#pragma unroll
+    for (int k = 0; k < (int)BK_IPT; ++k) {
+      const uint32_t r = tid + k * BK_BLOCK;
+      if (r < Lw) s_cmp[r] = (key[k] << cshift) | r;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int k = 0; k < (int)BK_IPT; ++k) {
+      const uint32_t r = tid + k * BK_BLOCK;
+      if (r < c0 || r >= c1) continue;
+      uint32_t w = r >> 5, m = s_head[w] & (0xFFFFFFFFu >> (31 - (r & 31)));
+      while (!m) m = s_head[--w];
+      const uint32_t bst = w * 32 + 31 - __clz(m);
+      w = (r + 1) >> 5;
+      m = s_head[w] & (0xFFFFFFFFu << ((r + 1) & 31));
+      while (!m) m = s_head[++w];
+      const uint32_t ben = w * 32 + __ffs(m) - 1;
+      const unsigned long long c = s_cmp[r];
+      uint32_t cnt = 0;
+      for (uint32_t q = bst; q < ben; ++q) cnt += s_cmp[q] < c ? 1u : 0u;
+      const uint32_t dst = pos + bst + cnt;
+      keys[dst] = key[k];
+      ids[dst] = id[k];
+    }
+    if (fmin != 0xFFFFFFFFu) return;
+    pos += c1;
+    first = false;
+    __syncthreads();
+  }
+
+  // ---- oversized bucket [pos, bend): find its end, then a stable LSD sort of its low digits by this CTA alone
+  if (tid == 0) s_sel[3] = N;
+  __syncthreads();
+  for (uint32_t base = pos + BK_CAP; base < N; base += BK_BLOCK) {
+    const uint32_t g = base + tid;
+    if (g < N && (keys[g] >> lowbits) != (keys[g - 1] >> lowbits)) atomicMin(&s_sel[3], g);
+    if (__syncthreads_or(s_sel[3] != N)) break;
+  }
+  const uint32_t bend = s_sel[3];
+  const uint32_t ndig = lowbits / 8;
+  unsigned long long* ksrc = keys;
+  uint32_t* isrc = ids;
+  unsigned long long* kdst = tkeys;
+  uint32_t* idst = tids;
+  for (uint32_t d = 0; d < ndig; ++d) {
+    const uint32_t sh = 8 * d;
+    for (uint32_t i = tid; i < 256 + 8 * 256; i += BK_BLOCK) s_hist[i] = 0;
+    __syncthreads();
+    for (uint32_t g = pos + tid; g < bend; g += BK_BLOCK) atomicAdd(&s_hist[(uint32_t)(ksrc[g] >> sh) & 0xFFu], 1u);
+    __syncthreads();
+    if (tid == 0) {
+      uint32_t run = pos;
+      for (int b = 0; b < 256; ++b) { const uint32_t t = s_hist[b]; s_hist[b] = run; run += t; }
+    }
+    __syncthreads();
+    uint32_t* wcnt = s_hist + 256;
+    for (uint32_t t0 = pos; t0 < bend; t0 += BK_BLOCK) {
+      const uint32_t g = t0 + tid;
+      const bool valid = g < bend;
+      const unsigned long long kk = valid ? ksrc[g] : 0ull;
+      const uint32_t vv = valid ? isrc[g] : 0u;
+      const uint32_t dg = valid ? (uint32_t)(kk >> sh) & 0xFFu : 256u;
+      const uint32_t peers = __match_any_sync(0xFFFFFFFFu, dg);
+      if (valid && lane == (uint32_t)(__ffs(peers) - 1)) wcnt[warp * 256 + dg] = __popc(peers);
+      __syncthreads();
+      if (valid) {
+        uint32_t off = s_hist[dg] + __popc(peers & lanemask_lt());
+        for (uint32_t w = 0; w < warp; ++w) off += wcnt[w * 256 + dg];
+        kdst[off] = kk;
+        idst[off] = vv;
+      }
+      __syncthreads();
+      uint32_t tot = 0;
+      for (int w = 0; w < 8; ++w) { tot += wcnt[w * 256 + tid]; wcnt[w * 256 + tid] = 0; }
+      s_hist[tid] += tot;
+      __syncthreads();
+    }
+    unsigned long long* kt = ksrc; ksrc = kdst; kdst = kt;
+    uint32_t* it = isrc; isrc = idst; idst = it;
+  }
+  if (ksrc != keys) {
+    __syncthreads();
+    for (uint32_t g = pos + tid; g < bend; g += BK_BLOCK) { keys[g] = ksrc[g]; ids[g] = isrc[g]; }
+  }
+  if (tid == 0) atomicAdd(nbig, 1u);
+}
+
+// =====================================================================================================
 // k_rerank — segmented re-ranking after a sort round.  Over the sorted records j = 0..m-1:
 //   headfull(j): the full key differs from its predecessor's (ROUND0: or the predecessor's window ran past
 //                the end of the text — such a suffix is unique and precedes its equal-key neighbours);
@@ -1626,7 +1802,8 @@ struct LadderState {
   uint32_t lists;     // != 0: the lists at `sel` are valid
   uint32_t err;       // copy of ctrl[CTR_ERR] taken by k_finish (so one D2H brings everything back)
   uint32_t nruns;     // run statistics (k_run_emit): maximal runs of equal bytes in the finished output
-  uint32_t pad2[4];
+  uint32_t big_buckets;  // round-0 buckets k_bucket_sort sorted on its slow path (longer than BK_CAP)
+  uint32_t pad2[3];
   uint32_t log_m[LADDER_LOG];     // records processed by ladder round i
   uint32_t log_kind[LADDER_LOG];  // 1 = segmented round, 2 = tail (k_small_rounds: all remaining rounds)
   uint32_t log_h[LADDER_LOG];

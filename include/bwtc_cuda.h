@@ -91,10 +91,12 @@ typedef struct bwtc_cuda_stats {
                               * BWTC_VERIFY; for bwtc_cuda_divsufsort: its suffix array passed the device-side sufcheck); bit 7:
                               * inverse only, this block is corrupt (BWTC_CUDA_ECORRUPT); bit 8: this call produced a suffix
                               * array (bwtc_cuda_divsufsort, _device, and the _lcp variants); bit 9: this call produced an
-                              * LCP array (bwtc_cuda_divsufsort_lcp, _lcp_device) */
+                              * LCP array (bwtc_cuda_divsufsort_lcp, _lcp_device); bit 10: round 0 ran its digit passes over the
+                              * top key digits only and sorted the low digits bucket by bucket (k_bucket_sort, BWTC_ROUND0_TOP) */
   uint32_t batch_blocks;     /* blocks this record describes: 1, or the size of the batch that was sorted as one text (every
                               * block of the batch then carries the SAME record — count it once; flags bit 7 is the one field
                               * in which the records of one inverse batch may differ) */
+  uint32_t round0_big_buckets; /* round-0 buckets too long for k_bucket_sort's on-chip path (flags bit 10), sorted on its slow path */
 } bwtc_cuda_stats;
 
 /* ---- library / device ------------------------------------------------------------------------ */
