@@ -171,6 +171,32 @@ struct bwtc_cuda_ctx {
 
 namespace {
 
+// Makes the context's device current on the calling thread.
+int select_device(bwtc_cuda_ctx* ctx) {
+  if (cudaSetDevice(ctx->device) == cudaSuccess) return 0;
+  set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device);
+  return BWTC_CUDA_ECUDA;
+}
+
+// A context holds N = cap + 1 suffixes: a block of cap bytes plus its sentinel, or a raw text of cap + 1 bytes.
+int check_capacity(bwtc_cuda_ctx* ctx, uint32_t n, bool block_mode) {
+  if ((uint64_t)n <= (uint64_t)ctx->cap + (block_mode ? 0u : 1u)) return 0;
+  set_err(ctx->err, "%s of %u bytes exceeds context capacity %u", block_mode ? "block" : "raw text", n, ctx->cap);
+  return BWTC_CUDA_ETOOBIG;
+}
+
+// The look-back watchdog fired (see k_radix_pass): the context switches to ticket tile ids for good and the caller repeats
+// its work once.  false if it already ran with tickets (a watchdog cannot fire twice): the error is `msg` (nullptr: the one
+// already set) and the caller returns BWTC_CUDA_EINTERNAL.
+bool retry_with_tickets(bwtc_cuda_ctx* ctx, const char* msg) {
+  if (ctx->static_tiles) {
+    ctx->static_tiles = 0;
+    return true;
+  }
+  if (msg) set_err(ctx->err, "%s", msg);
+  return false;
+}
+
 template <typename KeyT, int IPT, bool IOTA, bool AUX>
 int set_pass_attr(bwtc_cuda_ctx* ctx) {
   CK(ctx, cudaFuncSetAttribute(k_radix_pass<KeyT, RS_BLOCK, IPT, IOTA, AUX>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -652,14 +678,26 @@ int download_staged(bwtc_cuda_ctx* ctx, uint8_t* h_dst, const uint8_t* d_src, si
   return 0;
 }
 
+// What a caller's result buffer is, decided once per buffer: device memory, pinned (or managed) host memory, or pageable.
+enum class Dst { device, pinned, pageable };
+Dst dst_kind(const void* p, bool on_device) {
+  return on_device ? Dst::device : is_pinned_host(p) ? Dst::pinned : Dst::pageable;
+}
+
+// n result bytes from device scratch to a caller buffer.  Device and pinned buffers: one async copy on the kernel stream,
+// which the caller waits for once after all its copies.  Pageable: staged through the ring, done when this returns.
+int copy_result(bwtc_cuda_ctx* ctx, Dst kind, void* dst, const void* d_src, size_t n) {
+  if (!n) return 0;
+  if (kind == Dst::pageable) return download_staged(ctx, static_cast<uint8_t*>(dst), static_cast<const uint8_t*>(d_src), n);
+  CK(ctx, cudaMemcpyAsync(dst, d_src, n, kind == Dst::device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, ctx->stream));
+  return 0;
+}
+
 // ---- phase A: input upload, reversed text + byte histogram, key-shape policy.  ONE host synchronisation (the plan
 // needs the block's alphabet).  Nothing is written to the caller's arrays.
 int64_t phase_input(bwtc_cuda_ctx* ctx, Job& J) {
   ctx->err[0] = 0;
-  if (cudaSetDevice(ctx->device) != cudaSuccess) {
-    set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device);
-    return BWTC_CUDA_ECUDA;
-  }
+  if (select_device(ctx)) return BWTC_CUDA_ECUDA;
   const BatchSpec* bs = J.bs;
   J.bstride = bs ? bs->n0 + 1u : 0u;
   if (bs) {
@@ -671,11 +709,7 @@ int64_t phase_input(bwtc_cuda_ctx* ctx, Job& J) {
   const uint32_t n = J.n;
   const uint32_t N = J.block_mode ? n + 1 : n;
   J.N = N;
-  // a context holds N = cap + 1 suffixes: a block of cap bytes plus its sentinel, or a raw text of cap + 1 bytes
-  if (n > (J.block_mode ? (uint64_t)ctx->cap : (uint64_t)ctx->cap + 1)) {
-    set_err(ctx->err, "%s of %u bytes exceeds context capacity %u", J.block_mode ? "block" : "raw text", n, ctx->cap);
-    return BWTC_CUDA_ETOOBIG;
-  }
+  if (const int rc = check_capacity(ctx, n, J.block_mode)) return rc;
   if (J.nLF < 1 || J.nLF > 256 || J.nLF > N || !J.LF) {
     set_err(ctx->err, "bad nLFpowers %u for %u suffixes", J.nLF, N);
     return BWTC_CUDA_EARG;
@@ -810,10 +844,7 @@ int enqueue_lcp(bwtc_cuda_ctx* ctx, const Job& J);
 // tile ids) after a look-back watchdog without the caller's input.
 int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
   ctx->lb_watchdog = 0;
-  if (cudaSetDevice(ctx->device) != cudaSuccess) {
-    set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device);
-    return BWTC_CUDA_ECUDA;
-  }
+  if (select_device(ctx)) return BWTC_CUDA_ECUDA;
   cudaStream_t st = ctx->stream;
   bwtc_cuda_stats& S = ctx->stats;
   const BatchSpec* bs = J.bs;
@@ -1068,26 +1099,33 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
     return 0;
   };
 
-  // Result copies that need no host staging: pinned host buffers and device buffers.  Enqueued speculatively behind the
-  // first ladder chunk (a block whose later rounds are all sort-free then completes with one host wait); repeated at
-  // the end if the block was not finished by then.
-  const bool direct_out = bs ? (bs->on_device || is_pinned_host(bs->out[0]))
-                             : (J.out_dev != nullptr || (J.block_mode && J.h_out && is_pinned_host(J.h_out)));
-  // verification (DESIGN.md §3.10): the caller's host and batch outputs are written only after the check word is read
-  const bool verify = ctx->verify && !ctx->debug_max_rounds;
-  uint32_t* h_bLF = reinterpret_cast<uint32_t*>(ctx->h_batch + MAX_BATCH * sizeof(void*)) + MAX_BATCH * 256;
-  auto enqueue_direct_out = [&]() -> int {
+  // The BWT bytes for the caller: a batch's blocks from d_out at stride n0 + 1, a single block's from d_out unless they
+  // are already in the caller's device buffer (J.d_dst).  A raw output leaves U[pidx] untouched (divsufsort.c:506-512):
+  // two ranges around it.  A suffix-array job's BWT bytes stay on the device.
+  const Dst out_kind = bs ? dst_kind(bs->out[0], bs->on_device) : dst_kind(J.h_out, J.out_dev || !J.h_out);
+  auto copy_out = [&]() -> int {
     if (bs) {
-      for (uint32_t k = 0; k < bs->nblocks; ++k) {  // block k's BWT bytes are out[k*stride .. k*stride + n_k)
+      for (uint32_t k = 0; k < bs->nblocks; ++k) {
         const uint32_t nk = (k + 1 == bs->nblocks) ? bs->n_last : bs->n0;
-        CK(ctx, cudaMemcpyAsync(bs->out[k], ctx->d_out + (size_t)k * J.bstride, nk,
-                                bs->on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, st));
+        if (copy_result(ctx, out_kind, bs->out[k], ctx->d_out + (size_t)k * J.bstride, nk)) return BWTC_CUDA_ECUDA;
       }
-    } else if (!J.out_dev && !(ctx->debug_skip_copies & 2)) {
-      CK(ctx, cudaMemcpyAsync(J.h_out, ctx->d_out, n, cudaMemcpyDeviceToHost, st));
+    } else if (!J.block_mode) {
+      const uint32_t pidx = ctx->h_LF()[0];
+      if (copy_result(ctx, out_kind, J.h_out, ctx->d_out, pidx) ||
+          (pidx + 1 < n && copy_result(ctx, out_kind, J.h_out + pidx + 1, ctx->d_out + pidx + 1, n - pidx - 1)))
+        return BWTC_CUDA_ECUDA;
+    } else if (out_kind != Dst::device && !(out_kind == Dst::pinned && (ctx->debug_skip_copies & 2))) {
+      return copy_result(ctx, out_kind, J.h_out, ctx->d_out, n);
     }
     return 0;
   };
+  // Copies that need no host staging (device and pinned buffers) are waited for once.  In block mode they are enqueued
+  // speculatively behind the first ladder chunk (a block whose later rounds are all sort-free then completes with one host
+  // wait), and repeated at the end if the block was not finished by then.
+  const bool direct_out = bs ? out_kind != Dst::pageable : out_kind == Dst::pinned;
+  // verification (DESIGN.md §3.10): the caller's host and batch outputs are written only after the check word is read
+  const bool verify = ctx->verify && !ctx->debug_max_rounds;
+  uint32_t* h_bLF = reinterpret_cast<uint32_t*>(ctx->h_batch + MAX_BATCH * sizeof(void*)) + MAX_BATCH * 256;
 
   const int lo_bits = (int)ceil_log2_u64((uint64_t)N + 1);  // rank[i+h] + 1 in [0, N]
   // high part = (rank of the group head) >> 1 (k_build_keys): heads of live groups are <= N - 2
@@ -1159,8 +1197,8 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
     CK(ctx, cudaMemcpyAsync(ctx->h_state, ctx->d_state, sizeof(LadderState), cudaMemcpyDeviceToHost, st));
     if (bs) CK(ctx, cudaMemcpyAsync(h_bLF, ctx->d_LF, (size_t)bs->nblocks * 256 * 4, cudaMemcpyDeviceToHost, st));
     else CK(ctx, cudaMemcpyAsync(ctx->h_LF(), ctx->d_LF, J.nLF * 4, cudaMemcpyDeviceToHost, st));
-    if (first_chunk && direct_out && !dbg && !verify) {
-      if (enqueue_direct_out()) return BWTC_CUDA_ECUDA;
+    if (first_chunk && direct_out && J.block_mode && !dbg && !verify) {
+      if (copy_out()) return BWTC_CUDA_ECUDA;
       out_enqueued = true;
     }
     if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
@@ -1342,47 +1380,17 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
   // ---- result copies that could not be enqueued speculatively
   if (finished) {
     if (J.sa) {
-      // the suffix array (its BWT bytes stay on the device) and the LCP array: 4 bytes per suffix each, direct to pinned
-      // memory, else staged
-      auto copy_out = [&](int32_t* h, const int32_t* d) -> int {
+      // the suffix array and the LCP array of the host variants: 4 bytes per suffix each
+      bool pending = false;
+      auto copy_host = [&](int32_t* h, const int32_t* d) -> int {
         if (!h) return 0;
-        if (is_pinned_host(h)) {
-          CK(ctx, cudaMemcpyAsync(h, d, (size_t)N * 4, cudaMemcpyDeviceToHost, st));
-          return host_wait(ctx, st);
-        }
-        return download_staged(ctx, reinterpret_cast<uint8_t*>(h), reinterpret_cast<const uint8_t*>(d), (size_t)N * 4);
+        const Dst kind = dst_kind(h, false);
+        pending |= kind == Dst::pinned;
+        return copy_result(ctx, kind, h, d, (size_t)N * 4);
       };
-      if (copy_out(J.h_sa, J.sa) || copy_out(J.h_lcp, J.lcp)) return BWTC_CUDA_ECUDA;
-    } else if (bs) {
-      if (!out_enqueued || !direct_out) {
-        if (direct_out) {
-          if (enqueue_direct_out() || host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
-        } else {
-          for (uint32_t k = 0; k < bs->nblocks; ++k) {
-            const uint32_t nk = (k + 1 == bs->nblocks) ? bs->n_last : bs->n0;
-            if (download_staged(ctx, static_cast<uint8_t*>(bs->out[k]), ctx->d_out + (size_t)k * J.bstride, nk)) return BWTC_CUDA_ECUDA;
-          }
-        }
-      }
-    } else if (!J.out_dev) {
-      if (!J.block_mode) {
-        // raw contract: U[pidx] stays untouched (divsufsort.c:506-512) — two ranges around it
-        const uint32_t pidx = ctx->h_LF()[0];
-        if (is_pinned_host(J.h_out)) {
-          if (pidx > 0) CK(ctx, cudaMemcpyAsync(J.h_out, ctx->d_out, pidx, cudaMemcpyDeviceToHost, st));
-          if (pidx + 1 < n) CK(ctx, cudaMemcpyAsync(J.h_out + pidx + 1, ctx->d_out + pidx + 1, n - pidx - 1, cudaMemcpyDeviceToHost, st));
-          if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
-        } else {
-          if (download_staged(ctx, J.h_out, ctx->d_out, pidx)) return BWTC_CUDA_ECUDA;
-          if (pidx + 1 < n && download_staged(ctx, J.h_out + pidx + 1, ctx->d_out + pidx + 1, n - pidx - 1)) return BWTC_CUDA_ECUDA;
-        }
-      } else if (!out_enqueued) {
-        if (direct_out) {
-          if (enqueue_direct_out() || host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
-        } else if (download_staged(ctx, J.h_out, ctx->d_out, n)) {
-          return BWTC_CUDA_ECUDA;
-        }
-      }
+      if (copy_host(J.h_sa, J.sa) || copy_host(J.h_lcp, J.lcp) || (pending && host_wait(ctx, st))) return BWTC_CUDA_ECUDA;
+    } else if (!out_enqueued) {
+      if (copy_out() || (direct_out && host_wait(ctx, st))) return BWTC_CUDA_ECUDA;
     }
   }
   // ---- results for the caller: LFpowers, freqs (incremented only now that the block has succeeded)
@@ -1419,36 +1427,15 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
 // Phase A, phase B, and the fallback of the static tile ids (see k_radix_pass): if the look-back watchdog fired, the
 // context switches to ticket counters for good and repeats phase B.  The reversed, sentinel-terminated text is still
 // intact on the device, so this works for in-place device buffers too; nothing was written to LFpowers / freqs.
+// J.runs->count is BWTC_CUDA_RUNS_OVERFLOW unless the block succeeds: the entry points set it before any check, and a
+// failure after the runs were downloaded (EVERIFY, or an error in a later copy) sets it again.
 int64_t run_job(bwtc_cuda_ctx* ctx, Job& J) {
   int64_t rc = phase_input(ctx, J);
-  if (rc < 0) return rc;
-  rc = phase_sort(ctx, J);
-  if (rc == BWTC_CUDA_EINTERNAL && ctx->lb_watchdog && ctx->static_tiles) {
-    ctx->static_tiles = 0;
+  if (rc >= 0) {
     rc = phase_sort(ctx, J);
+    if (rc == BWTC_CUDA_EINTERNAL && ctx->lb_watchdog && retry_with_tickets(ctx, nullptr)) rc = phase_sort(ctx, J);
   }
-  return rc;
-}
-
-int64_t run_transform(bwtc_cuda_ctx* ctx, bool block_mode, const uint8_t* h_in, uint8_t* h_out, const uint8_t* in_dev,
-                      uint8_t* out_dev, uint32_t n, uint32_t* LF, uint32_t nLF, uint32_t* freqs,
-                      const BatchSpec* bs = nullptr, bwtc_cuda_runs* runs = nullptr) {
-  Job J;
-  J.runs = runs;
-  if (runs) runs->count = BWTC_CUDA_RUNS_OVERFLOW;
-  J.block_mode = block_mode;
-  J.h_in = h_in;
-  J.h_out = h_out;
-  J.in_dev = in_dev;
-  J.out_dev = out_dev;
-  J.n = n;
-  J.LF = LF;
-  J.nLF = nLF;
-  J.freqs = freqs;
-  J.bs = bs;
-  const int64_t rc = run_job(ctx, J);
-  // a failure after the runs were downloaded (EVERIFY, or an error in a later copy) must not leave a valid-looking count
-  if (rc < 0 && runs) runs->count = BWTC_CUDA_RUNS_OVERFLOW;
+  if (rc < 0 && J.runs) J.runs->count = BWTC_CUDA_RUNS_OVERFLOW;
   return rc;
 }
 
@@ -1524,81 +1511,99 @@ int enqueue_inverse(bwtc_cuda_ctx* ctx, const InvShape& sh, bool block_mode, con
   return 0;
 }
 
-// spec (the single-block entry points): pinned host and device outputs are written without waiting for the check, so a
-// valid block costs one host wait; a corrupt one leaves them unspecified.  !spec (a block of bwtc_cuda_inverse_blocks):
-// restored into d_out, copied to the caller only if valid.  After a look-back watchdog the device part is repeated with
-// ticket tile ids from the device copy of the input (d_in, or in_dev, which walk2 left untouched) — never from h_in, which
-// the speculative copy may already have overwritten with stale bytes when it aliases a pinned h_out.
-int64_t run_inverse(bwtc_cuda_ctx* ctx, bool block_mode, const uint8_t* h_in, uint8_t* h_out, const uint8_t* in_dev, uint8_t* out_dev,
-                    uint32_t n_in, uint32_t eob, bool spec = true) {
-  ctx->err[0] = 0;
-  if (cudaSetDevice(ctx->device) != cudaSuccess) {
-    set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device);
-    return BWTC_CUDA_ECUDA;
-  }
-  const uint32_t N = block_mode ? n_in + 1u : n_in, n = N - 1u;
-  if (n_in == 0 || n > ctx->cap || N < 2) {
-    set_err(ctx->err, "inverse: block of %u bytes exceeds context capacity %u (or is empty)", n, ctx->cap);
-    return n > ctx->cap ? BWTC_CUDA_ETOOBIG : BWTC_CUDA_EARG;
-  }
-  if (eob >= N) {
-    set_err(ctx->err, "inverse: end-of-block position %u outside [0, %u)", eob, N);
-    return BWTC_CUDA_EARG;
-  }
+// The inversion of sh's blocks from d_src into d_dst: enqueue it, read the control words back, wait, and after a look-back
+// watchdog (the only look-back kernels here are the two digit passes) once more with ticket tile ids.  fwd (the verification
+// of that forward transform): the VERIFY variant, then k_inv_verify compares d_dst with fwd->d_text; launches and bytes are
+// added to the forward's record.  Otherwise the record is the inversion's own, started over on every attempt.  spec_out: a
+// pinned buffer that receives block 0's restored bytes before the wait.  *bad: bit k = block k is corrupt (or differs).
+int invert(bwtc_cuda_ctx* ctx, const InvShape& sh, bool block_mode, const uint8_t* d_src, uint8_t* d_dst, const Job* fwd,
+           void* spec_out, uint64_t* bad) {
   cudaStream_t st = ctx->stream;
   bwtc_cuda_stats& S = ctx->stats;
-  const uint8_t* d_src = in_dev;
-  if (!in_dev) {
-    if (upload(ctx, ctx->d_in, h_in, n_in)) return BWTC_CUDA_ECUDA;
-    d_src = ctx->d_in;
-  }
-  uint8_t* d_dst = (out_dev && spec) ? out_dev : ctx->d_out;
-  const bool pinned_out = !out_dev && is_pinned_host(h_out);
-  InvShape sh;
-  sh.nblocks = 1;
-  sh.R = sh.N_last = N;
-  sh.n0 = sh.istride = n;
-  sh.S0 = sh.S_last = div_up(N, INV_K);
-  sh.eob[0] = eob;
-  sh.d_eob = nullptr;
   uint32_t rounds = 0, pdone = 0;
   for (;;) {
-    memset(&S, 0, sizeof(S));
-    S.n_suffixes = N;
-    S.batch_blocks = 1;
-    if (const int rc = enqueue_inverse(ctx, sh, block_mode, d_src, d_dst, &rounds, &pdone)) return rc;
+    if (!fwd) {
+      memset(&S, 0, sizeof(S));
+      S.n_suffixes = inv_rows(sh);
+      S.batch_blocks = sh.nblocks;
+    }
+    if (const int rc = enqueue_inverse(ctx, sh, block_mode, d_src, d_dst, &rounds, &pdone, fwd != nullptr)) return rc;
+    if (fwd) {
+      const dim3 vgrid(std::max<uint32_t>(1u, div_up((uint32_t)ctx->sm_count * 8u, sh.nblocks)), sh.nblocks);
+      k_inv_verify<<<vgrid, 256, 0, st>>>(d_dst, fwd->d_text, sh, ctx->d_ctrl());
+      CK(ctx, cudaGetLastError());
+      S.kernel_launches++;
+      S.algorithmic_bytes += 2ull * fwd->n;
+      CK(ctx, cudaEventRecord(ctx->ev_end, st));
+    }
     CK(ctx, cudaMemcpyAsync(ctx->h_ctrl(), ctx->d_ctrl(), CTR_STICKY * 4, cudaMemcpyDeviceToHost, st));
-    if (pinned_out && spec) CK(ctx, cudaMemcpyAsync(h_out, ctx->d_out, n, cudaMemcpyDeviceToHost, st));
+    if (spec_out && copy_result(ctx, Dst::pinned, spec_out, d_dst, sh.n0)) return BWTC_CUDA_ECUDA;
     if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
     if (!ctx->h_ctrl()[CTR_ERR]) break;
-    // the only look-back kernels here are the two digit passes; repeat with tickets (cannot happen twice)
-    if (!ctx->static_tiles) {
-      set_err(ctx->err, "inverse: look-back watchdog fired");
+    if (!retry_with_tickets(ctx, fwd ? "verification: look-back watchdog fired in the inverse" : "inverse: look-back watchdog fired"))
       return BWTC_CUDA_EINTERNAL;
+  }
+  *bad = (uint64_t)ctx->h_ctrl()[CTR_INV_BAD] | ((uint64_t)ctx->h_ctrl()[CTR_INV_BAD + 1] << 32);
+  if (!fwd) {
+    float ms = 0;
+    CK(ctx, cudaEventElapsedTime(&ms, ctx->ev_begin, ctx->ev_end));
+    S.gpu_ms = ms;
+    S.rounds = rounds;
+    S.passes[0] = pdone;
+    S.live[0] = S.n_suffixes;
+    // bit 1: a batch; bit 7: the one block is corrupt (a batch reports its blocks in *bad)
+    S.flags = (sh.nblocks > 1 ? 2u : 0u) | (ctx->static_tiles ? 0u : 1u) | (sh.nblocks == 1 && *bad ? 128u : 0u);
+  }
+  return 0;
+}
+
+// count >= 1 blocks (block contract, or one raw text: !block_mode) of sizes[k] restored bytes each; the caller has checked
+// the arguments.  The inputs are staged in d_in at stride n0 (one block on the device is read in place) and restored into
+// d_out.  A retry after a look-back watchdog reads the same device input, which walk 2 has not touched, never a host
+// buffer: it may alias an output that a speculative copy has already overwritten.  spec (the single-block entry points): a
+// device output is written directly and a pinned one is copied before the one host wait, so a valid block costs one wait;
+// a corrupt block leaves them unspecified.  Otherwise a block's buffer is written only after the host has read the check
+// words, and not at all if the block is corrupt.
+// *bad: bit k = block k is corrupt; the call then returns BWTC_CUDA_ECORRUPT.
+int run_inverse(bwtc_cuda_ctx* ctx, bool block_mode, const void* const* in, void* const* out, const uint32_t* sizes,
+                uint32_t count, bool on_device, const uint32_t* eobs, bool spec, uint64_t* bad) {
+  ctx->err[0] = 0;
+  if (select_device(ctx)) return BWTC_CUDA_ECUDA;
+  static_assert(INV_MAX_BLOCKS == MAX_BATCH, "InvShape holds one end-of-block row per block of a batch");
+  InvShape sh;
+  sh.nblocks = count;
+  sh.n0 = sh.istride = sizes[0];
+  sh.R = sizes[0] + 1u;
+  sh.N_last = sizes[count - 1] + 1u;
+  sh.S0 = div_up(sh.R, INV_K);
+  sh.S_last = div_up(sh.N_last, INV_K);
+  sh.d_eob = nullptr;
+  for (uint32_t k = 0; k < count; ++k) sh.eob[k] = eobs[k];
+  const uint8_t* d_src = ctx->d_in;
+  if (count == 1 && on_device) {
+    d_src = static_cast<const uint8_t*>(in[0]);
+  } else {
+    for (uint32_t k = 0; k < count; ++k) {
+      uint8_t* d = ctx->d_in + (size_t)k * sh.n0;
+      const size_t nk = sizes[k] + (block_mode ? 0u : 1u);  // (a raw text has one byte more than its result)
+      if (on_device) CK(ctx, cudaMemcpyAsync(d, in[k], nk, cudaMemcpyDeviceToDevice, ctx->stream));
+      else if (upload(ctx, d, static_cast<const uint8_t*>(in[k]), nk)) return BWTC_CUDA_ECUDA;
     }
-    ctx->static_tiles = 0;
   }
-  const bool corrupt = (ctx->h_ctrl()[CTR_INV_BAD] & 1u) != 0u;
-  if (!corrupt) {
-    if (!spec && (out_dev || pinned_out)) {
-      CK(ctx, cudaMemcpyAsync(out_dev ? out_dev : h_out, ctx->d_out, n, out_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, st));
-      if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
-    } else if (!out_dev && !pinned_out && download_staged(ctx, h_out, ctx->d_out, n)) {
-      return BWTC_CUDA_ECUDA;
-    }
+  Dst kind[INV_MAX_BLOCKS];
+  for (uint32_t k = 0; k < count; ++k) kind[k] = dst_kind(out[k], on_device);
+  const bool written = spec && kind[0] != Dst::pageable;
+  uint8_t* d_dst = spec && kind[0] == Dst::device ? static_cast<uint8_t*>(out[0]) : ctx->d_out;
+  if (const int rc = invert(ctx, sh, block_mode, d_src, d_dst, nullptr, spec && kind[0] == Dst::pinned ? out[0] : nullptr, bad))
+    return rc;
+  bool pending = false;
+  for (uint32_t k = 0; k < count && !written; ++k) {
+    if ((*bad >> k) & 1u) continue;
+    if (copy_result(ctx, kind[k], out[k], ctx->d_out + (size_t)k * sh.n0, sizes[k])) return BWTC_CUDA_ECUDA;
+    pending |= kind[k] != Dst::pageable;
   }
-  float ms = 0;
-  CK(ctx, cudaEventElapsedTime(&ms, ctx->ev_begin, ctx->ev_end));
-  S.gpu_ms = ms;
-  S.rounds = rounds;
-  S.passes[0] = pdone;
-  S.live[0] = N;
-  S.flags = (ctx->static_tiles ? 0u : 1u) | (corrupt ? 128u : 0u);
-  if (corrupt) {
-    set_err(ctx->err, "inverse: block 0 is not the BWT of any text (with end-of-block row %u)", eob);
-    return BWTC_CUDA_ECORRUPT;
-  }
-  return (int64_t)n;
+  if (pending && host_wait(ctx, ctx->stream)) return BWTC_CUDA_ECUDA;
+  return *bad ? BWTC_CUDA_ECORRUPT : 0;
 }
 
 // Verification of a finished forward transform (DESIGN.md §3.10): its device-resident output (J.d_dst, a batch at stride
@@ -1634,26 +1639,9 @@ int verify_forward(bwtc_cuda_ctx* ctx, const Job& J) {
     CK(ctx, cudaGetLastError());
     S.kernel_launches++;
   }
-  for (;;) {
-    uint32_t rounds = 0, pdone = 0;
-    if (const int rc = enqueue_inverse(ctx, sh, J.block_mode, J.d_dst, ctx->d_aux[1], &rounds, &pdone, true)) return rc;
-    const dim3 vgrid(std::max<uint32_t>(1u, div_up((uint32_t)ctx->sm_count * 8u, sh.nblocks)), sh.nblocks);
-    k_inv_verify<<<vgrid, 256, 0, st>>>(ctx->d_aux[1], J.d_text, sh, ctx->d_ctrl());
-    CK(ctx, cudaGetLastError());
-    S.kernel_launches++;
-    S.algorithmic_bytes += 2ull * J.n;
-    CK(ctx, cudaEventRecord(ctx->ev_end, st));
-    CK(ctx, cudaMemcpyAsync(ctx->h_ctrl(), ctx->d_ctrl(), CTR_STICKY * 4, cudaMemcpyDeviceToHost, st));
-    if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
-    if (!ctx->h_ctrl()[CTR_ERR]) break;
-    if (!ctx->static_tiles) {
-      set_err(ctx->err, "verification: look-back watchdog fired in the inverse");
-      return BWTC_CUDA_EINTERNAL;
-    }
-    ctx->static_tiles = 0;  // the inverse's two digit passes again with ticket tile ids (cannot fire twice)
-  }
+  uint64_t mask = 0;
+  if (const int rc = invert(ctx, sh, J.block_mode, J.d_dst, ctx->d_aux[1], &J, nullptr, &mask)) return rc;
   S.flags |= 64u;
-  const uint64_t mask = (uint64_t)ctx->h_ctrl()[CTR_INV_BAD] | ((uint64_t)ctx->h_ctrl()[CTR_INV_BAD + 1] << 32);
   if (!mask) return 0;
   if (!bs && J.block_mode && J.out_dev && J.out_dev == J.in_dev) {
     k_text_unreverse<<<ctx->sm_count * 4, 256, 0, st>>>(J.d_text, J.n, J.out_dev);
@@ -1806,7 +1794,9 @@ int transform_batch(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out,
     bs.nLF = nLF[0];
     bs.nLF_last = nLF[count - 1];
     bs.freqs = freqs;
-    const int64_t rc = run_transform(ctx, true, nullptr, nullptr, nullptr, nullptr, 0, nullptr, 0, nullptr, &bs);
+    Job J;
+    J.bs = &bs;
+    const int64_t rc = run_job(ctx, J);
     if (rc != BATCH_NEEDS_SINGLE) {
       ctx->stats.batch_blocks = count;  // the record describes the whole batch: count it once, not per block
       if (stats) for (uint32_t k = 0; k < count; ++k) stats[k] = ctx->stats;
@@ -1814,14 +1804,20 @@ int transform_batch(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out,
     }
   }
   for (uint32_t k = 0; k < count; ++k) {
-    uint32_t* fr = freqs ? freqs + (size_t)k * 256 : nullptr;
-    int64_t rc;
-    if (on_device)
-      rc = run_transform(ctx, true, nullptr, nullptr, static_cast<const uint8_t*>(in[k]), static_cast<uint8_t*>(out[k]), sizes[k],
-                         LF + (size_t)k * 256, nLF[k], fr);
-    else
-      rc = run_transform(ctx, true, static_cast<const uint8_t*>(in[k]), static_cast<uint8_t*>(out[k]), nullptr, nullptr, sizes[k],
-                         LF + (size_t)k * 256, nLF[k], fr, nullptr, count == 1 ? runs : nullptr);
+    Job J;
+    if (on_device) {
+      J.in_dev = static_cast<const uint8_t*>(in[k]);
+      J.out_dev = static_cast<uint8_t*>(out[k]);
+    } else {
+      J.h_in = static_cast<const uint8_t*>(in[k]);
+      J.h_out = static_cast<uint8_t*>(out[k]);
+      J.runs = count == 1 ? runs : nullptr;
+    }
+    J.n = sizes[k];
+    J.LF = LF + (size_t)k * 256;
+    J.nLF = nLF[k];
+    J.freqs = freqs ? freqs + (size_t)k * 256 : nullptr;
+    const int64_t rc = run_job(ctx, J);
     ctx->stats.batch_blocks = 1;
     if (stats) stats[k] = ctx->stats;
     if (rc < 0) return (int)rc;
@@ -1829,83 +1825,9 @@ int transform_batch(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out,
   return 0;
 }
 
-// 2..MAX_BATCH blocks (block contract) that batchable() accepts, inverted as ONE device-side problem (DESIGN.md §3.7).  The
-// caller has checked the arguments.  The blocks are staged in d_in (stride n0) and restored into d_out; the caller's
-// buffers are written only after the host has read CTR_ERR.  After a look-back watchdog the device part is repeated with
-// ticket tile ids from the staged input — never from the caller's buffers, which may alias the outputs.
-// *bad: bit k set = block k is corrupt; its buffer is not written, and the call returns BWTC_CUDA_ECORRUPT.
-int run_inverse_batch(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out, const uint32_t* sizes, uint32_t count,
-                      bool on_device, const uint32_t* eobs, uint64_t* bad) {
-  *bad = 0;
-  ctx->err[0] = 0;
-  if (cudaSetDevice(ctx->device) != cudaSuccess) {
-    set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device);
-    return BWTC_CUDA_ECUDA;
-  }
-  static_assert(INV_MAX_BLOCKS == MAX_BATCH, "InvShape holds one end-of-block row per block of a batch");
-  cudaStream_t st = ctx->stream;
-  InvShape sh;
-  sh.nblocks = count;
-  sh.n0 = sh.istride = sizes[0];
-  sh.R = sizes[0] + 1u;
-  sh.d_eob = nullptr;
-  sh.N_last = sizes[count - 1] + 1u;
-  sh.S0 = div_up(sh.R, INV_K);
-  sh.S_last = div_up(sh.N_last, INV_K);
-  for (uint32_t k = 0; k < count; ++k) sh.eob[k] = eobs[k];
-  for (uint32_t k = 0; k < count; ++k) {
-    uint8_t* d = ctx->d_in + (size_t)k * sh.n0;
-    if (on_device) CK(ctx, cudaMemcpyAsync(d, in[k], sizes[k], cudaMemcpyDeviceToDevice, st));
-    else if (upload(ctx, d, static_cast<const uint8_t*>(in[k]), sizes[k])) return BWTC_CUDA_ECUDA;
-  }
-  bwtc_cuda_stats& S = ctx->stats;
-  uint32_t rounds = 0, pdone = 0;
-  for (;;) {
-    memset(&S, 0, sizeof(S));
-    if (const int rc = enqueue_inverse(ctx, sh, true, ctx->d_in, ctx->d_out, &rounds, &pdone)) return rc;
-    CK(ctx, cudaMemcpyAsync(ctx->h_ctrl(), ctx->d_ctrl(), CTR_STICKY * 4, cudaMemcpyDeviceToHost, st));
-    if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
-    if (!ctx->h_ctrl()[CTR_ERR]) break;
-    if (!ctx->static_tiles) {
-      set_err(ctx->err, "inverse: look-back watchdog fired");
-      return BWTC_CUDA_EINTERNAL;
-    }
-    ctx->static_tiles = 0;  // the two digit passes again with ticket tile ids (cannot fire twice)
-  }
-  const uint64_t mask = (uint64_t)ctx->h_ctrl()[CTR_INV_BAD] | ((uint64_t)ctx->h_ctrl()[CTR_INV_BAD + 1] << 32);
-  bool pending = false;
-  for (uint32_t k = 0; k < count; ++k) {
-    if ((mask >> k) & 1u) continue;  // a corrupt block's buffer stays as it was
-    const uint8_t* d = ctx->d_out + (size_t)k * sh.n0;
-    uint8_t* o = static_cast<uint8_t*>(out[k]);
-    if (on_device) {
-      CK(ctx, cudaMemcpyAsync(o, d, sizes[k], cudaMemcpyDeviceToDevice, st));
-      pending = true;
-    } else if (is_pinned_host(o)) {
-      CK(ctx, cudaMemcpyAsync(o, d, sizes[k], cudaMemcpyDeviceToHost, st));
-      pending = true;
-    } else if (download_staged(ctx, o, d, sizes[k])) {
-      return BWTC_CUDA_ECUDA;
-    }
-  }
-  if (pending && host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
-  float ms = 0;
-  CK(ctx, cudaEventElapsedTime(&ms, ctx->ev_begin, ctx->ev_end));
-  S.n_suffixes = inv_rows(sh);
-  S.batch_blocks = count;
-  S.gpu_ms = ms;
-  S.rounds = rounds;
-  S.passes[0] = pdone;
-  S.live[0] = S.n_suffixes;
-  S.flags = 2u | (ctx->static_tiles ? 0u : 1u);
-  *bad = mask;
-  return mask ? BWTC_CUDA_ECORRUPT : 0;
-}
-
-// count blocks (block contract) through one context, each restored as run_inverse would: runs are formed greedily as in
-// bwtc_cuda_bwt_blocks, a run that batchable() accepts is inverted as one problem, any other block on its own.  Every
-// argument is checked before any work, so a bad block leaves all caller buffers untouched.  stats: count records (the
-// blocks of a batch share one) or nullptr.
+// count blocks (block contract) through one context: runs are formed greedily as in bwtc_cuda_bwt_blocks, a run that
+// batchable() accepts is inverted as one problem, any other block on its own.  Every argument is checked before any work,
+// so a bad block leaves all caller buffers untouched.  stats: count records (the blocks of a batch share one) or nullptr.
 int inverse_blocks(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out, const uint32_t* sizes, uint32_t count,
                    bool on_device, const uint32_t* eobs, bwtc_cuda_stats* stats) {
   for (uint32_t k = 0; k < count; ++k) {
@@ -1923,18 +1845,9 @@ int inverse_blocks(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out, 
   for (uint32_t k0 = 0; k0 < count;) {
     uint32_t k1 = std::min<uint32_t>(count, k0 + MAX_BATCH);
     while (k1 > k0 + 1 && !batchable(ctx, sizes + k0, k1 - k0)) --k1;
-    int64_t rc;
     uint64_t bad = 0;
-    if (k1 - k0 >= 2)
-      rc = run_inverse_batch(ctx, in + k0, out + k0, sizes + k0, k1 - k0, on_device, eobs + k0, &bad);
-    else if (on_device)
-      rc = run_inverse(ctx, true, nullptr, nullptr, static_cast<const uint8_t*>(in[k0]), static_cast<uint8_t*>(out[k0]), sizes[k0],
-                       eobs[k0], false);
-    else
-      rc = run_inverse(ctx, true, static_cast<const uint8_t*>(in[k0]), static_cast<uint8_t*>(out[k0]), nullptr, nullptr, sizes[k0],
-                       eobs[k0], false);
-    if (rc == BWTC_CUDA_ECORRUPT && k1 - k0 == 1) bad = 1u;
-    else if (rc < 0 && rc != BWTC_CUDA_ECORRUPT) return (int)rc;
+    const int rc = run_inverse(ctx, true, in + k0, out + k0, sizes + k0, k1 - k0, on_device, eobs + k0, false, &bad);
+    if (rc < 0 && rc != BWTC_CUDA_ECORRUPT) return rc;
     for (uint32_t k = k0; k < k1; ++k) {
       const bool b = (bad >> (k - k0)) & 1u;
       if (b && !ncorrupt++) first_corrupt = k;
@@ -1951,6 +1864,24 @@ int inverse_blocks(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out, 
     return BWTC_CUDA_ECORRUPT;
   }
   return 0;
+}
+
+// One block (block contract: n_in bytes, restored in place of n_in) or raw text (n_in bytes, n_in - 1 restored) through
+// run_inverse with speculative result copies.  Returns the number of restored bytes.
+int64_t inverse_one(bwtc_cuda_ctx* ctx, bool block_mode, const void* in, void* out, bool on_device, uint32_t n_in, uint32_t eob) {
+  const uint32_t N = block_mode ? n_in + 1u : n_in, n = N - 1u;
+  if (n_in == 0 || n > ctx->cap || N < 2) {
+    set_err(ctx->err, "inverse: block of %u bytes exceeds context capacity %u (or is empty)", n, ctx->cap);
+    return n > ctx->cap ? BWTC_CUDA_ETOOBIG : BWTC_CUDA_EARG;
+  }
+  if (eob >= N) {
+    set_err(ctx->err, "inverse: end-of-block position %u outside [0, %u)", eob, N);
+    return BWTC_CUDA_EARG;
+  }
+  uint64_t bad = 0;
+  const int rc = run_inverse(ctx, block_mode, &in, &out, &n, 1, on_device, &eob, true, &bad);
+  if (rc == BWTC_CUDA_ECORRUPT) set_err(ctx->err, "inverse: block 0 is not the BWT of any text (with end-of-block row %u)", eob);
+  return rc < 0 ? rc : (int64_t)n;
 }
 
 }  // namespace
@@ -2223,7 +2154,15 @@ int64_t bwtc_cuda_divbwtf(bwtc_cuda_ctx* ctx, const uint8_t* T, uint8_t* U, uint
     if (n == 1) U[0] = T[0];
     return n;
   }
-  return run_transform(ctx, false, T, U, nullptr, nullptr, n, LFpowers, nLFpowers, freqs);
+  Job J;
+  J.block_mode = false;
+  J.h_in = T;
+  J.h_out = U;
+  J.n = n;
+  J.LF = LFpowers;
+  J.nLF = nLFpowers;
+  J.freqs = freqs;
+  return run_job(ctx, J);
 }
 
 int64_t bwtc_cuda_divbwt(bwtc_cuda_ctx* ctx, const uint8_t* T, uint8_t* U, uint32_t n, uint32_t* LFpowers,
@@ -2234,7 +2173,7 @@ int64_t bwtc_cuda_divbwt(bwtc_cuda_ctx* ctx, const uint8_t* T, uint8_t* U, uint3
 // The host variants' device SA: 4 (cap + 1) bytes, allocated by the first call that needs it.
 static int ensure_sa(bwtc_cuda_ctx* ctx) {
   if (ctx->d_sa) return 0;
-  if (cudaSetDevice(ctx->device) != cudaSuccess) { set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device); return BWTC_CUDA_ECUDA; }
+  if (select_device(ctx)) return BWTC_CUDA_ECUDA;
   const size_t bytes = ((size_t)ctx->cap + 1) * 4;
   const cudaError_t e = cudaMalloc((void**)&ctx->d_sa, bytes);
   if (e != cudaSuccess) {
@@ -2254,10 +2193,7 @@ int bwtc_cuda_divsufsort(bwtc_cuda_ctx* ctx, const uint8_t* T, int32_t* SA, uint
     if (n == 1) SA[0] = 0;
     return 0;
   }
-  if ((uint64_t)n > (uint64_t)ctx->cap + 1) {
-    set_err(ctx->err, "raw text of %u bytes exceeds context capacity %u", n, ctx->cap);
-    return BWTC_CUDA_ETOOBIG;
-  }
+  if (const int rc = check_capacity(ctx, n, false)) return rc;
   if (const int rc = ensure_sa(ctx)) return rc;
   return run_divsufsort(ctx, T, nullptr, SA, ctx->d_sa, n);
 }
@@ -2268,7 +2204,7 @@ int bwtc_cuda_divsufsort_device(bwtc_cuda_ctx* ctx, const void* d_T, void* d_SA,
   if (!d_T || !d_SA || (reinterpret_cast<uintptr_t>(d_SA) & 3u)) { set_err(ctx->err, "null d_T / d_SA, or d_SA not 4-byte aligned"); return BWTC_CUDA_EARG; }
   if (n == 0) return 0;
   if (n == 1) {
-    if (cudaSetDevice(ctx->device) != cudaSuccess) { set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device); return BWTC_CUDA_ECUDA; }
+    if (select_device(ctx)) return BWTC_CUDA_ECUDA;
     CK(ctx, cudaMemsetAsync(d_SA, 0, 4, ctx->stream));
     return host_wait(ctx, ctx->stream) ? BWTC_CUDA_ECUDA : 0;
   }
@@ -2283,10 +2219,7 @@ int bwtc_cuda_divsufsort_lcp(bwtc_cuda_ctx* ctx, const uint8_t* T, int32_t* SA, 
     if (n == 1) SA[0] = LCP[0] = 0;
     return 0;
   }
-  if ((uint64_t)n > (uint64_t)ctx->cap + 1) {
-    set_err(ctx->err, "raw text of %u bytes exceeds context capacity %u", n, ctx->cap);
-    return BWTC_CUDA_ETOOBIG;
-  }
+  if (const int rc = check_capacity(ctx, n, false)) return rc;
   if (const int rc = ensure_sa(ctx)) return rc;
   return run_divsufsort(ctx, T, nullptr, SA, ctx->d_sa, n, LCP, static_cast<int32_t*>(ctx->d_keys[0]));
 }
@@ -2302,7 +2235,7 @@ int bwtc_cuda_divsufsort_lcp_device(bwtc_cuda_ctx* ctx, const void* d_T, void* d
   if (a < b + (uint64_t)n * 4 && b < a + (uint64_t)n * 4) { set_err(ctx->err, "d_SA and d_LCP overlap"); return BWTC_CUDA_EARG; }
   if (n == 0) return 0;
   if (n == 1) {
-    if (cudaSetDevice(ctx->device) != cudaSuccess) { set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device); return BWTC_CUDA_ECUDA; }
+    if (select_device(ctx)) return BWTC_CUDA_ECUDA;
     CK(ctx, cudaMemsetAsync(d_SA, 0, 4, ctx->stream));
     CK(ctx, cudaMemsetAsync(d_LCP, 0, 4, ctx->stream));
     return host_wait(ctx, ctx->stream) ? BWTC_CUDA_ECUDA : 0;
@@ -2316,16 +2249,13 @@ int bwtc_cuda_sufcheck(bwtc_cuda_ctx* ctx, const uint8_t* T, const int32_t* SA, 
   ctx->err[0] = 0;
   if (!T || !SA) { set_err(ctx->err, "null T or SA"); return BWTC_CUDA_EARG; }
   if (n == 0) return 0;
-  if ((uint64_t)n > (uint64_t)ctx->cap + 1) {
-    set_err(ctx->err, "raw text of %u bytes exceeds context capacity %u", n, ctx->cap);
-    return BWTC_CUDA_ETOOBIG;
-  }
+  if (const int rc = check_capacity(ctx, n, false)) return rc;
   if (n == 1) {
     if (SA[0] == 0) return 0;
     set_err(ctx->err, "sufcheck: row 0 of 1: value out of range");
     return BWTC_CUDA_ECORRUPT;
   }
-  if (cudaSetDevice(ctx->device) != cudaSuccess) { set_err(ctx->err, "cudaSetDevice(%d) failed", ctx->device); return BWTC_CUDA_ECUDA; }
+  if (select_device(ctx)) return BWTC_CUDA_ECUDA;
   cudaStream_t st = ctx->stream;
   bwtc_cuda_stats& S = ctx->stats;
   memset(&S, 0, sizeof(S));
@@ -2345,9 +2275,7 @@ int bwtc_cuda_sufcheck(bwtc_cuda_ctx* ctx, const uint8_t* T, const int32_t* SA, 
 
 int64_t bwtc_cuda_bwt_block(bwtc_cuda_ctx* ctx, uint8_t* block, uint32_t n, uint32_t* LFpowers, uint32_t nLFpowers,
                             uint32_t* freqs) {
-  if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
-  if (!block || n == 0) { set_err(ctx->err, "null or empty block"); return BWTC_CUDA_EARG; }
-  return run_transform(ctx, true, block, block, nullptr, nullptr, n, LFpowers, nLFpowers, freqs);
+  return bwtc_cuda_bwt_block_runs(ctx, block, n, LFpowers, nLFpowers, freqs, nullptr);
 }
 
 int64_t bwtc_cuda_bwt_block_runs(bwtc_cuda_ctx* ctx, uint8_t* block, uint32_t n, uint32_t* LFpowers, uint32_t nLFpowers,
@@ -2355,7 +2283,14 @@ int64_t bwtc_cuda_bwt_block_runs(bwtc_cuda_ctx* ctx, uint8_t* block, uint32_t n,
   if (runs) runs->count = BWTC_CUDA_RUNS_OVERFLOW;  // (every negative return leaves it so)
   if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
   if (!block || n == 0) { set_err(ctx->err, "null or empty block"); return BWTC_CUDA_EARG; }
-  return run_transform(ctx, true, block, block, nullptr, nullptr, n, LFpowers, nLFpowers, freqs, nullptr, runs);
+  Job J;
+  J.h_in = J.h_out = block;
+  J.n = n;
+  J.LF = LFpowers;
+  J.nLF = nLFpowers;
+  J.freqs = freqs;
+  J.runs = runs;
+  return run_job(ctx, J);
 }
 
 int bwtc_cuda_bwt_blocks(bwtc_cuda_ctx* ctx, void* const* blocks, const uint32_t* sizes, uint32_t count, uint32_t starts,
@@ -2378,20 +2313,26 @@ int64_t bwtc_cuda_bwt_block_device(bwtc_cuda_ctx* ctx, const void* d_in, void* d
                                    uint32_t nLFpowers, uint32_t* freqs) {
   if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
   if (!d_in || !d_out || n == 0) { set_err(ctx->err, "null or empty block"); return BWTC_CUDA_EARG; }
-  return run_transform(ctx, true, nullptr, nullptr, static_cast<const uint8_t*>(d_in), static_cast<uint8_t*>(d_out), n,
-                       LFpowers, nLFpowers, freqs);
+  Job J;
+  J.in_dev = static_cast<const uint8_t*>(d_in);
+  J.out_dev = static_cast<uint8_t*>(d_out);
+  J.n = n;
+  J.LF = LFpowers;
+  J.nLF = nLFpowers;
+  J.freqs = freqs;
+  return run_job(ctx, J);
 }
 
 int64_t bwtc_cuda_inverse_block(bwtc_cuda_ctx* ctx, uint8_t* block, uint32_t n, const uint32_t* LFpowers, uint32_t nLFpowers) {
   if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
   if (!block || n == 0 || !LFpowers || nLFpowers < 1) { set_err(ctx->err, "null or empty block / no starting point"); return BWTC_CUDA_EARG; }
-  return run_inverse(ctx, true, block, block, nullptr, nullptr, n, LFpowers[0]);
+  return inverse_one(ctx, true, block, block, false, n, LFpowers[0]);
 }
 
 int64_t bwtc_cuda_inverse_block_device(bwtc_cuda_ctx* ctx, const void* d_in, void* d_out, uint32_t n, uint32_t eob) {
   if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
   if (!d_in || !d_out || n == 0) { set_err(ctx->err, "null or empty block"); return BWTC_CUDA_EARG; }
-  return run_inverse(ctx, true, nullptr, nullptr, static_cast<const uint8_t*>(d_in), static_cast<uint8_t*>(d_out), n, eob);
+  return inverse_one(ctx, true, d_in, d_out, true, n, eob);
 }
 
 int bwtc_cuda_inverse_blocks(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out, const uint32_t* sizes, uint32_t count,
@@ -2406,7 +2347,7 @@ int bwtc_cuda_inverse_blocks(bwtc_cuda_ctx* ctx, const void* const* in, void* co
 int64_t bwtc_cuda_inverse_raw(bwtc_cuda_ctx* ctx, uint8_t* bwt, uint32_t N, const uint32_t* LFpowers, uint32_t nLFpowers) {
   if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
   if (!bwt || N < 2 || !LFpowers || nLFpowers < 1) { set_err(ctx->err, "null / too short input or no starting point"); return BWTC_CUDA_EARG; }
-  return run_inverse(ctx, false, bwt, bwt, nullptr, nullptr, N, LFpowers[0]);
+  return inverse_one(ctx, false, bwt, bwt, false, N, LFpowers[0]);
 }
 
 uint32_t bwtc_cuda_num_starting_points(uint32_t block_bytes, uint32_t starts) {
