@@ -108,8 +108,8 @@ struct bwtc_cuda_ctx {
   int32_t* d_sa = nullptr;        // suffix array of bwtc_cuda_divsufsort (host variant): 4 (cap + 1) bytes, allocated by its
                                   // first call, not counted by bwtc_cuda_scratch_bytes
   // ---- pinned host memory
-  uint32_t* h_small = nullptr;    // [ctrl CTR_WORDS][hist HIST_WORDS][LF 256 + pair statistics]
-  uint8_t* h_batch = nullptr;     // [MAX_BATCH] pointers, [MAX_BATCH][256] histograms, [MAX_BATCH][256] LFpowers
+  uint32_t* h_small = nullptr;    // [ctrl CTR_WORDS][pair statistics 4][raw text's last byte]
+  uint8_t* h_batch = nullptr;     // per block: [MAX_BATCH] pointers, [MAX_BATCH][256] histograms, [MAX_BATCH][256] LFpowers
   // ---- timing
   cudaEvent_t ev_begin = nullptr, ev_end = nullptr;
   std::vector<cudaEvent_t> ev_pool;
@@ -148,15 +148,17 @@ struct bwtc_cuda_ctx {
   uint32_t force_chars = 0, force_keybytes = 0;
   uint32_t debug_max_rounds = 0;  // != 0: stop refining after this many rounds (results are then wrong on purpose)
   int last_cur = 0;               // sort buffer holding the last round's sorted records
-  RerankParams rr0;               // round-0 re-rank parameters of the block in flight (fallback out of lazy ranks)
   bwtc_cuda_stats stats;
   char err[512];
   uint32_t* d_ctrl() const { return d_zero; }
   uint32_t* d_hist() const { return d_zero + CTR_WORDS; }
   unsigned long long* d_tstate() const { return reinterpret_cast<unsigned long long*>(d_zero + CTR_WORDS + HIST_WORDS); }
   uint32_t* h_ctrl() const { return h_small; }
-  uint32_t* h_hist() const { return h_small + CTR_WORDS; }
-  uint32_t* h_LF() const { return h_small + CTR_WORDS + HIST_WORDS; }
+  uint32_t* h_pairs() const { return h_small + CTR_WORDS; }  // 2 doubles, then the raw text's last byte (h_last)
+  uint8_t* h_last() const { return reinterpret_cast<uint8_t*>(h_small + CTR_WORDS + 4); }
+  const void** h_bptr() const { return reinterpret_cast<const void**>(h_batch); }
+  uint32_t* h_bhist() const { return reinterpret_cast<uint32_t*>(h_batch + MAX_BATCH * sizeof(void*)); }
+  uint32_t* h_bLF() const { return h_bhist() + MAX_BATCH * 256; }
 };
 
 #define CK(ctx, call)                                                                              \
@@ -256,27 +258,28 @@ void plan_round0(const bwtc_cuda_ctx* ctx, const uint64_t* count, const bool* pr
     if (present[c] && count[c]) { double p = (double)count[c] / total; H0 -= p * std::log2(p); }
   const uint32_t b = sigma <= 2 ? 1 : ceil_log2_u64(sigma);
   const uint32_t cmax64 = (64 - blk_bits) / b, cmax32 = blk_bits >= 32 - b ? 0u : (32 - blk_bits) / b;
+  const bool forced = ctx->force_chars || ctx->force_keybytes;
+  // Does the source have memory?  Compare the MEASURED collision rate of sampled 8-byte windows with the rate
+  // an i.i.d. source with this byte histogram would show, (sum q^2)^8.  Text and repeats exceed it by orders
+  // of magnitude: they keep many suffixes tied whatever the order-0 statistics say, and every extra character
+  // ordered in round 0 is far cheaper than a doubling round over the suffixes it would leave live (measured:
+  // profiles/r01_experiments.md), so their 64-bit key is filled completely.  A forced key shape takes none of this.
+  double q2 = 0.0;
+  for (int c = 0; c < 256; ++c)
+    if (present[c] && count[c]) { const double q = (double)count[c] / total; q2 += q * q; }
+  const double samples = pair_stats[1];
+  const double all_pairs = samples * (samples - 1.0) * 0.5;
+  const double expected = all_pairs * std::pow(q2, 8.0);
+  pl->has_memory = forced || (H0 < 1e-3) || samples < 64.0 || (pair_stats[0] > 8.0 * expected + 16.0);
   uint32_t chars, keybytes;
-  if (ctx->force_chars || ctx->force_keybytes) {
+  if (forced) {
     keybytes = (ctx->force_keybytes == 4 && cmax32 >= 1) ? 4 : 8;
     const uint32_t cmax = keybytes == 4 ? cmax32 : cmax64;
     chars = ctx->force_chars ? ctx->force_chars : cmax;
     if (chars > cmax) chars = cmax;
     if (chars < 1) chars = 1;
   } else {
-    // Does the source have memory?  Compare the MEASURED collision rate of sampled 8-byte windows with the rate
-    // an i.i.d. source with this byte histogram would show, (sum q^2)^8.  Text and repeats exceed it by orders
-    // of magnitude: they keep many suffixes tied whatever the order-0 statistics say, and every extra character
-    // ordered in round 0 is far cheaper than a doubling round over the suffixes it would leave live (measured:
-    // profiles/r01_experiments.md), so their 64-bit key is filled completely.
-    double q2 = 0.0;
-    for (int c = 0; c < 256; ++c)
-      if (present[c] && count[c]) { const double q = (double)count[c] / total; q2 += q * q; }
-    const double samples = pair_stats[1];
-    const double all_pairs = samples * (samples - 1.0) * 0.5;
-    const double expected = all_pairs * std::pow(q2, 8.0);
-    const bool has_memory = (H0 < 1e-3) || samples < 64.0 || (pair_stats[0] > 8.0 * expected + 16.0);
-    if (has_memory) {
+    if (pl->has_memory) {
       keybytes = 8;
       chars = cmax64;
     } else {
@@ -301,20 +304,8 @@ void plan_round0(const bwtc_cuda_ctx* ctx, const uint64_t* count, const bool* pr
       keybytes = ((uint64_t)chars * b + blk_bits <= 32) ? 4 : 8;
     }
   }
-  pl->has_memory = true;
-  pl->live_pred = 1.0;
-  pl->repeats = HUGE_VAL;
-  if (!(ctx->force_chars || ctx->force_keybytes)) {
-    double q2 = 0.0;
-    for (int c = 0; c < 256; ++c)
-      if (present[c] && count[c]) { const double q = (double)count[c] / total; q2 += q * q; }
-    const double samples = pair_stats[1];
-    const double all_pairs = samples * (samples - 1.0) * 0.5;
-    const double expected = all_pairs * std::pow(q2, 8.0);
-    pl->has_memory = (H0 < 1e-3) || samples < 64.0 || (pair_stats[0] > 8.0 * expected + 16.0);
-    if (!pl->has_memory) pl->live_pred = 1.0 - std::exp(-(double)N * std::exp2(-H0 * (double)chars));
-    if (samples >= 64.0) pl->repeats = pair_stats[0] / all_pairs * (double)N;
-  }
+  pl->live_pred = pl->has_memory ? 1.0 : 1.0 - std::exp(-(double)N * std::exp2(-H0 * (double)chars));
+  pl->repeats = (!forced && samples >= 64.0) ? pair_stats[0] / all_pairs * (double)N : HUGE_VAL;
   pl->sigma = sigma;
   pl->bits = b;
   pl->chars = chars;
@@ -523,38 +514,27 @@ int launch_rerank(bwtc_cuda_ctx* ctx, int cur, uint32_t m, uint32_t N, RerankPar
   return 0;
 }
 
-// A batch of small blocks transformed as ONE suffix-sorting problem (DESIGN.md §3.6): text = T'_0 T'_1 ... with
-// T'_k = reverse(X_k) . 0x00 at offset k * (n0 + 1).  All blocks have n0 bytes, the last one n_last <= n0.
-struct BatchSpec {
-  uint32_t nblocks, n0, n_last;
-  const void* const* in;  // per block: host pointers, or device pointers when on_device
-  void* const* out;
-  bool on_device;
-  uint32_t* LF;           // [nblocks][256]
-  uint32_t nLF, nLF_last; // LFpowers per full block / for the last block
-  uint32_t* freqs;        // [nblocks][256] incremented, or nullptr
-};
 constexpr int64_t BATCH_NEEDS_SINGLE = -1000;  // all 256 byte values present: no code left for the reserved sentinel
 
-// One transform call: what the caller handed in, and what phase A (input + policy) learnt about it.
+// One forward call of nblocks >= 1 blocks: what the caller handed in, and what phase A (input + policy) learnt about it.
+// A batch (nblocks > 1, block contract) is ONE suffix-sorting problem (DESIGN.md §3.6): text = T'_0 T'_1 ... with
+// T'_k = reverse(X_k) . 0x00 at offset k * (n0 + 1).  All blocks have n0 bytes, the last one n_last <= n0.
 struct Job {
-  bool block_mode = true;          // in = X (n block bytes), result n bytes;  false (raw): in = T (n bytes)
-  const uint8_t* h_in = nullptr;   // host buffers of a single block ...
-  uint8_t* h_out = nullptr;
-  const uint8_t* in_dev = nullptr; // ... or the caller's device buffers
-  uint8_t* out_dev = nullptr;
-  uint32_t n = 0;
-  uint32_t* LF = nullptr;
-  uint32_t nLF = 0;
-  uint32_t* freqs = nullptr;
-  const BatchSpec* bs = nullptr;   // batch of blocks (block contract): the fields above come from *bs
-  bwtc_cuda_runs* runs = nullptr;  // run statistics wanted (single block, block contract)
+  bool block_mode = true;          // in = X (n block bytes), result n bytes;  false (raw, one block): in = T (n bytes)
+  uint32_t nblocks = 1, n0 = 0, n_last = 0;
+  const void* const* in = nullptr; // per block: the caller's input and output, host buffers ...
+  void* const* out = nullptr;      // (a suffix-array job has out[0] == nullptr: its BWT bytes stay on the device)
+  bool on_device = false;          // ... or device buffers
+  uint32_t* LF = nullptr;          // per block: a row of 256 LFpowers, nLF of them (nLF_last in the last block)
+  uint32_t nLF = 0, nLF_last = 0;
+  uint32_t* freqs = nullptr;       // per block: a row of 256 byte counts, incremented; or nullptr
+  bwtc_cuda_runs* runs = nullptr;  // run statistics wanted (one host block, block contract)
   int32_t* sa = nullptr;           // raw contract: the suffix array is emitted here (device; bwtc_cuda_divsufsort) ...
   int32_t* h_sa = nullptr;         // ... and copied to this host array once the block is finished (and verified)
   int32_t* lcp = nullptr;          // bwtc_cuda_divsufsort_lcp: the LCP array is built here (device) behind the sort ...
   int32_t* h_lcp = nullptr;        // ... and copied to this host array
   // ---- phase A
-  uint32_t N = 0, bstride = 0, blk_bits = 0;
+  uint32_t n = 0, N = 0, bstride = 0, blk_bits = 0;  // n: result bytes of all blocks; bstride: n0 + 1 in a batch, else 0
   bool sentinel_outside_alphabet = false;
   uint8_t last = 0;                // raw: T[N-1], the byte of the end-of-text row
   bool present[256];
@@ -563,7 +543,26 @@ struct Job {
   uint8_t* d_dst = nullptr;
   EmitParams ep;
   uint64_t a_launches = 0, a_bytes = 0;  // kernel launches / algorithmic bytes of phase A
+  bool batch() const { return nblocks > 1; }
+  uint32_t bytes(uint32_t k) const { return k + 1 == nblocks ? n_last : n0; }
 };
+
+// A job over count blocks of sizes[k] bytes (a batch: all but the last of sizes[0] bytes) with nLF[k] LFpowers each.
+Job forward_job(const void* const* in, void* const* out, bool on_device, const uint32_t* sizes, uint32_t count, uint32_t* LF,
+                const uint32_t* nLF, uint32_t* freqs) {
+  Job J;
+  J.nblocks = count;
+  J.n0 = sizes[0];
+  J.n_last = sizes[count - 1];
+  J.in = in;
+  J.out = out;
+  J.on_device = on_device;
+  J.LF = LF;
+  J.nLF = nLF[0];
+  J.nLF_last = nLF[count - 1];
+  J.freqs = freqs;
+  return J;
+}
 
 // Host wait for everything enqueued on `st` so far.  Default: sleep on a blocking-sync event — a waiting worker
 // costs no host core, so `depth` workers per GPU times 8 ranks do not oversubscribe the box.  BWTC_SPIN_WAIT=1 spins.
@@ -694,19 +693,13 @@ int copy_result(bwtc_cuda_ctx* ctx, Dst kind, void* dst, const void* d_src, size
 }
 
 // ---- phase A: input upload, reversed text + byte histogram, key-shape policy.  ONE host synchronisation (the plan
-// needs the block's alphabet).  Nothing is written to the caller's arrays.
+// needs the blocks' alphabet).  Nothing is written to the caller's arrays.
 int64_t phase_input(bwtc_cuda_ctx* ctx, Job& J) {
   ctx->err[0] = 0;
   if (select_device(ctx)) return BWTC_CUDA_ECUDA;
-  const BatchSpec* bs = J.bs;
-  J.bstride = bs ? bs->n0 + 1u : 0u;
-  if (bs) {
-    J.n = (bs->nblocks - 1u) * J.bstride + bs->n_last;  // N - 1
-    J.nLF = bs->nLF;
-    J.LF = bs->LF;
-    J.freqs = bs->freqs;
-  }
-  const uint32_t n = J.n;
+  const bool batch = J.batch();
+  J.bstride = batch ? J.n0 + 1u : 0u;
+  const uint32_t n = J.n = (J.nblocks - 1u) * (J.n0 + 1u) + J.n_last;
   const uint32_t N = J.block_mode ? n + 1 : n;
   J.N = N;
   if (const int rc = check_capacity(ctx, n, J.block_mode)) return rc;
@@ -719,37 +712,30 @@ int64_t phase_input(bwtc_cuda_ctx* ctx, Job& J) {
   memset(&S, 0, sizeof(S));
   S.n_suffixes = N;
 
-  // ---- input
-  const uint8_t* d_src = J.in_dev;
-  const void** h_bptr = reinterpret_cast<const void**>(ctx->h_batch);
-  uint32_t* h_bhist = reinterpret_cast<uint32_t*>(ctx->h_batch + MAX_BATCH * sizeof(void*));
-  if (bs) {
-    for (uint32_t k = 0; k < bs->nblocks; ++k) {
-      const uint32_t nk = (k + 1 == bs->nblocks) ? bs->n_last : bs->n0;
-      if (bs->on_device) {
-        h_bptr[k] = bs->in[k];
-      } else {
-        if (upload(ctx, ctx->d_in + (size_t)k * bs->n0, static_cast<const uint8_t*>(bs->in[k]), nk)) return BWTC_CUDA_ECUDA;
-        h_bptr[k] = ctx->d_in + (size_t)k * bs->n0;
-      }
+  // ---- input: a device block is read where it is, a host block is uploaded to d_in at stride n0
+  const void** h_bptr = ctx->h_bptr();
+  for (uint32_t k = 0; k < J.nblocks; ++k) {
+    if (J.on_device) {
+      h_bptr[k] = J.in[k];
+    } else {
+      if (upload(ctx, ctx->d_in + (size_t)k * J.n0, static_cast<const uint8_t*>(J.in[k]), J.bytes(k))) return BWTC_CUDA_ECUDA;
+      h_bptr[k] = ctx->d_in + (size_t)k * J.n0;
     }
-    CK(ctx, cudaMemcpyAsync(ctx->d_bptr, h_bptr, bs->nblocks * sizeof(void*), cudaMemcpyHostToDevice, st));
-    d_src = ctx->d_text;  // the policy sample reads the (reversed) concatenation
-  } else if (!J.in_dev) {
-    if (upload(ctx, ctx->d_in, J.h_in, n)) return BWTC_CUDA_ECUDA;
-    d_src = ctx->d_in;
   }
-  J.d_dst = (J.out_dev && !bs) ? J.out_dev : ctx->d_out;
+  if (batch) CK(ctx, cudaMemcpyAsync(ctx->d_bptr, h_bptr, J.nblocks * sizeof(void*), cudaMemcpyHostToDevice, st));
+  // (the policy sample of a batch reads the reversed concatenation)
+  const uint8_t* d_src = batch ? ctx->d_text : static_cast<const uint8_t*>(h_bptr[0]);
+  J.d_dst = (J.on_device && !batch && J.out[0]) ? static_cast<uint8_t*>(J.out[0]) : ctx->d_out;
   CK(ctx, cudaEventRecord(ctx->ev_begin, st));
 
   // ---- byte histogram (+ reversed, sentinel-terminated text in block mode)
   CK(ctx, cudaMemsetAsync(ctx->d_zero, 0, (size_t)(CTR_WORDS + HIST_WORDS) * 4, st));
   const int pgrid = ctx->sm_count * 8;
-  if (bs) {
+  if (batch) {
     const uint32_t padded_words = div_up((uint64_t)N + TEXT_PAD, 4);
-    CK(ctx, cudaMemsetAsync(ctx->d_bhist, 0, (size_t)bs->nblocks * 256 * 4, st));
-    const dim3 grid(std::max<uint32_t>(1u, div_up((uint32_t)pgrid, bs->nblocks)), bs->nblocks);
-    k_prep_batch<<<grid, 256, 0, st>>>(reinterpret_cast<const uint8_t* const*>(ctx->d_bptr), bs->n0, bs->n_last, bs->nblocks,
+    CK(ctx, cudaMemsetAsync(ctx->d_bhist, 0, (size_t)J.nblocks * 256 * 4, st));
+    const dim3 grid(std::max<uint32_t>(1u, div_up((uint32_t)pgrid, J.nblocks)), J.nblocks);
+    k_prep_batch<<<grid, 256, 0, st>>>(reinterpret_cast<const uint8_t* const*>(ctx->d_bptr), J.n0, J.n_last, J.nblocks,
                                        ctx->d_text, N, padded_words, ctx->d_bhist);
     J.d_text = ctx->d_text;
     S.algorithmic_bytes += 2ull * n + N;
@@ -780,45 +766,43 @@ int64_t phase_input(bwtc_cuda_ctx* ctx, Job& J) {
       CK(ctx, cudaGetLastError());
       S.kernel_launches += 2;
     }
-    CK(ctx, cudaMemcpyAsync(ctx->h_LF() + 256, d_pairs, 16, cudaMemcpyDeviceToHost, st));
+    CK(ctx, cudaMemcpyAsync(ctx->h_pairs(), d_pairs, 16, cudaMemcpyDeviceToHost, st));
   }
-  if (bs) CK(ctx, cudaMemcpyAsync(h_bhist, ctx->d_bhist, (size_t)bs->nblocks * 256 * 4, cudaMemcpyDeviceToHost, st));
-  else CK(ctx, cudaMemcpyAsync(ctx->h_hist(), ctx->d_hist(), 256 * 4, cudaMemcpyDeviceToHost, st));
-  uint8_t* h_last = reinterpret_cast<uint8_t*>(ctx->h_LF() + 260);  // (behind the 16 bytes of pair statistics)
-  if (!J.block_mode && !J.h_in) CK(ctx, cudaMemcpyAsync(h_last, d_src + (N - 1), 1, cudaMemcpyDeviceToHost, st));
+  uint32_t* h_bhist = ctx->h_bhist();
+  CK(ctx, cudaMemcpyAsync(h_bhist, batch ? ctx->d_bhist : ctx->d_hist(), (size_t)J.nblocks * 256 * 4, cudaMemcpyDeviceToHost, st));
+  if (!J.block_mode && J.on_device) CK(ctx, cudaMemcpyAsync(ctx->h_last(), d_src + (N - 1), 1, cudaMemcpyDeviceToHost, st));
   if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
 
   uint64_t count[256];
   uint32_t npresent = 0;
   for (int c = 0; c < 256; ++c) {
     count[c] = 0;
-    if (bs) for (uint32_t k = 0; k < bs->nblocks; ++k) count[c] += h_bhist[k * 256 + c];
-    else count[c] = ctx->h_hist()[c];
+    for (uint32_t k = 0; k < J.nblocks; ++k) count[c] += h_bhist[k * 256 + c];
     J.present[c] = count[c] != 0;
     npresent += J.present[c] ? 1u : 0u;
   }
-  if (bs && npresent >= 256) return BATCH_NEEDS_SINGLE;
+  if (batch && npresent >= 256) return BATCH_NEEDS_SINGLE;
   // Block contract: the appended 0x00 only enters the alphabet if the block itself contains 0x00.  Otherwise
   // it is a true sentinel: it gets code 0 like the padding past the end, and the "window ran past the end"
   // rule of the round-0 re-rank starts one position earlier (DESIGN.md §3.2) — a 4-letter alphabet then packs
   // into 2 bits per character instead of 3.  A batch reserves code 0 for its sentinels instead (§3.6).
   J.sentinel_outside_alphabet = false;
   J.blk_bits = 0;
-  if (bs) {
-    J.blk_bits = std::max<uint32_t>(1u, (uint32_t)ceil_log2_u64(bs->nblocks));
+  if (batch) {
+    J.blk_bits = std::max<uint32_t>(1u, (uint32_t)ceil_log2_u64(J.nblocks));
   } else if (J.block_mode) {
     if (!J.present[0]) J.sentinel_outside_alphabet = true;
   } else {
-    const uint8_t last = J.h_in ? J.h_in[N - 1] : *h_last;
+    const uint8_t last = J.on_device ? *ctx->h_last() : static_cast<const uint8_t*>(J.in[0])[N - 1];
     J.last = last;
     J.present[last] = true;
     count[last] += 1;
   }
   double pair_stats[2];  // [0] colliding pairs among the sampled 8-byte windows, [1] samples
-  memcpy(pair_stats, ctx->h_LF() + 256, 16);
+  memcpy(pair_stats, ctx->h_pairs(), 16);
   plan_round0(ctx, count, J.present, N, pair_stats, &J.pl, J.blk_bits);
-  if (bs) { J.pl.pp.nblocks = bs->nblocks; J.pl.pp.stride = J.bstride; }
-  J.ep.nblocks = bs ? bs->nblocks : 1u;
+  if (batch) { J.pl.pp.nblocks = J.nblocks; J.pl.pp.stride = J.bstride; }
+  J.ep.nblocks = J.nblocks;
   J.ep.stride = J.bstride;
   J.ep.text = J.d_text;
   J.ep.out = J.d_dst;
@@ -839,31 +823,144 @@ int verify_forward(bwtc_cuda_ctx* ctx, const Job& J);
 int verify_sa(bwtc_cuda_ctx* ctx, const Job& J);
 int enqueue_lcp(bwtc_cuda_ctx* ctx, const Job& J);
 
-// ---- phase B: round 0, the device-controlled ladder of sort-free rounds, host-driven global radix rounds where
-// groups are large, final extraction, result copies.  Works from ctx->d_text only, so it can be repeated (with ticket
-// tile ids) after a look-back watchdog without the caller's input.
-int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
-  ctx->lb_watchdog = 0;
-  if (select_device(ctx)) return BWTC_CUDA_ECUDA;
+// One attempt of phase B: the state its steps share.  A repeated phase B (after a look-back watchdog) starts from a
+// fresh one.
+struct SortState {
+  SortState(bwtc_cuda_ctx* ctx, const Job& J)
+      : pt{ctx},
+        out_kind(dst_kind(J.out[0], J.on_device || !J.out[0])),
+        direct_out(out_kind == Dst::pinned || (J.batch() && out_kind == Dst::device)),
+        verify(ctx->verify && !ctx->debug_max_rounds) {}
+  int cur = 0;                       // sort buffer holding the last sorted records
+  bool lazy = false;                 // lazy ranks (DESIGN.md §3.9), until the ladder leaves them
+  PoolPtrs pool, norm;               // the ladder's six work arrays; norm: their full-rank layout
+  const LookupParams* lkp = nullptr; // (lazy ranks)
+  RerankParams rr0;                  // round 0's re-rank and its key type: the fallback out of lazy ranks repeats it
+  int (*rerank0)(bwtc_cuda_ctx*, int, uint32_t, uint32_t, RerankParams, const EmitParams&, uint32_t*, uint32_t*, bool,
+                 bool) = nullptr;
+  uint32_t m_prev = 0;               // records of the last global sort = extent of the k_rerank staging slots
+  uint32_t m_bound = 0;              // upper bound of the live count (it never grows)
+  uint64_t h_next = 0;
+  uint32_t pdone = 0;                // digit passes of the last sort
+  PassTimer pt;
+  size_t round0_events = 0;
+  bool lists_pending = true, first_chunk = true, out_enqueued = false, chunk_built_lists = false;
+  // lean chunk: behind a global radix round whose groups were still far above the segmented-round limit nothing sort-free
+  // is enqueued speculatively (it would only be skipped on the device): commit, k_finish (error word), state copy, wait
+  bool lean = false;
+  uint32_t nlog_seen = 0;            // ladder rounds already logged
+  // The BWT bytes for the caller.  Copies that need no host staging (device and pinned buffers) are waited for once.  In
+  // block mode they are enqueued speculatively behind the first ladder chunk (a block whose later rounds are all sort-free
+  // then completes with one host wait), and repeated at the end if the block was not finished by then.
+  const Dst out_kind;
+  const bool direct_out;
+  // verification (DESIGN.md §3.10): the caller's host and batch outputs are written only after the check word is read
+  const bool verify;
+  uint32_t sel(int c) const { return lazy ? 0x10u : ((uint32_t)(2 * c) | ((uint32_t)(2 * c + 1) << 4)); }
+};
+
+// One row of the per-round statistics (rounds past BWTC_CUDA_MAX_ROUNDS are not recorded).
+void log_round(bwtc_cuda_stats& S, uint32_t live, uint32_t passes, uint32_t prefix_len) {
+  const uint32_t r = S.rounds;
+  if (r >= BWTC_CUDA_MAX_ROUNDS) return;
+  S.live[r] = live;
+  S.passes[r] = passes;
+  S.prefix_len[r] = prefix_len;
+  S.rounds = r + 1;
+}
+
+// Round-0 digit histograms: one representative digit per phase class is counted by k_pack_round0 (*hist_mask), the others
+// are derived (k_hist_derive, *dp).  Returns true for gram mode (6- and 3-bit codes): one 4096-bin histogram of the keys'
+// low 12 bits, every digit histogram projected from it (k_hist_from_gram, *gp) — one shared-memory atomic per key instead
+// of one per counted digit.
+bool plan_histograms(const bwtc_cuda_ctx* ctx, const Round0Plan& pl, uint32_t N, bool batch, uint32_t* hist_mask,
+                     DeriveParams* dp, GramParams* gp) {
+  *hist_mask = 0;
+  dp->count = 0;
+  // (digit positions in the coordinates of the c exact characters: the key carries pl.rbits partial bits below them)
+  const uint32_t keybits = pl.chars * pl.bits;
+  const uint32_t rbits = pl.rbits;
+  uint32_t regular_mask = 0;  // digits that lie entirely inside the exact characters
+  for (uint32_t p = 0; p < pl.npass; ++p) {
+    int rep = -1;
+    const bool full_p = (8u * p >= rbits) && (8u * p - rbits + 8u <= keybits);
+    if (full_p) regular_mask |= 1u << p;
+    if (full_p && N > 64 && !batch)  // (a batch counts every digit directly: block numbers sit above the characters)
+      for (uint32_t r = 0; r < p; ++r)
+        if (((*hist_mask >> r) & (regular_mask >> r) & 1u) && (8u * (p - r)) % pl.bits == 0) { rep = (int)r; break; }
+    if (rep < 0) {
+      *hist_mask |= 1u << p;
+    } else {
+      dp->p[dp->count] = (uint8_t)p;
+      dp->r[dp->count] = (uint8_t)rep;
+      dp->t[dp->count] = (uint8_t)(8u * (p - (uint32_t)rep) / pl.bits);
+      dp->count++;
+    }
+  }
+  // Gram mode
+  gp->npass = 0;
+  bool use_gram = ctx->use_gram && !batch && N > 64 && (pl.bits == 6 || pl.bits == 3) && keybits >= (uint32_t)GRAM_BITS;
+  if (use_gram) {
+    const uint32_t W = (uint32_t)GRAM_BITS / pl.bits;
+    for (uint32_t p = 0; p < pl.npass && use_gram; ++p) {
+      uint32_t u, sft;
+      gp->next[p] = 0;
+      if (8u * p < rbits) {  // the lowest digit reaches into the partial character: window of the following suffix
+        if (p != 0) use_gram = false;
+        u = 0;
+        sft = pl.bits - rbits;
+        gp->next[p] = 1;
+        if (sft + 8u > (uint32_t)GRAM_BITS) use_gram = false;
+      } else {
+        const uint32_t lo = 8u * p - rbits;
+        u = std::min<uint32_t>(lo / pl.bits, pl.chars - W);
+        sft = lo - pl.bits * u;
+        // the digit must lie inside the 12 bits above bit (bits * u), or run past the top of the key (zeros there)
+        if (sft + 8u > (uint32_t)GRAM_BITS && lo + 8u <= keybits) use_gram = false;
+      }
+      if (sft >= 32u) use_gram = false;
+      gp->u[p] = (uint8_t)u;
+      gp->s[p] = (uint8_t)sft;
+    }
+    gp->npass = pl.npass;
+  }
+  if (use_gram) { *hist_mask = 0; dp->count = 0; }
+  return use_gram;
+}
+
+// ---- lazy ranks? (DESIGN.md §3.9)  The rank scatter of round 0 — a random 4-byte write per suffix — is 20-35% of a block,
+// but after round 0 only the ranks of suffixes that are still in a group are ever refined, and a singleton's rank is simply
+// its position in the sorted key array.  If few suffixes will stay in groups, rank[] is written for those only; the
+// segmented rounds order group members by cmp (round-0 key, then rank where it is stored) and need no integer rank, the
+// tail (k_small_rounds, k_finish) looks the few ranks it needs up in the retained sorted keys (rank_lookup).
+bool choose_lazy(const bwtc_cuda_ctx* ctx, const Job& J) {
+  const Round0Plan& pl = J.pl;
+  const uint32_t N = J.N;
+  if (!ctx->use_lazy || J.batch() || dbg_any(ctx) || N < 64 || pl.chars * pl.bits + pl.rbits < 1) return false;
+  // The decision needs no extra measurement.  For an i.i.d.-like source (DNA, random bytes) the key-shape policy has
+  // already predicted the fraction of suffixes still tied after round 0, L(c) = 1 - exp(-N 2^(-H0 c)) — it matches the
+  // measured live fractions to three digits (DNA 64 MiB: 0.0156 / 0.0155; random 256 MiB: 0.0606 / 0.0606).  For a source
+  // with memory the 8-gram sample tells text (a few other positions share a position's 8-gram: Markov 32 MiB 3.0, 3% live
+  // after its 10.7-character keys) from repeats (thousands: the 4 KiB-seed block keeps ~all suffixes tied through global
+  // radix rounds and would only pay the materialising fallback).  The 8-gram sample says nothing about how much a key
+  // longer than 8 characters separates, so a block with memory also needs keys of at least LAZY_MIN_CHARS characters
+  // (codes of <= 6 bits): the same Markov text as a 65-symbol raw text (7-bit codes, 9-character keys) left more or
+  // larger groups after round 0 than the segmented rounds take and fell back.  Segmented rounds are what makes lazy ranks cheap, so a block with memory
+  // goes lazy only where they run.  A wrong prediction only costs time: the fallback out of lazy ranks is exact.
+  constexpr uint32_t LAZY_MIN_CHARS = 10;
+  const bool memory_ok = ctx->use_seg && pl.chars >= LAZY_MIN_CHARS && pl.repeats <= ctx->lazy_max_repeats;
+  return ctx->use_lazy >= 2 ||
+         (N >= ctx->lazy_min_suffixes && (pl.has_memory ? memory_ok : pl.live_pred <= ctx->lazy_max_live));
+}
+
+// ---- round 0: pack keys (+ all digit histograms), sort, re-rank, and the first commit of the ladder
+template <typename KeyT>
+int round0(bwtc_cuda_ctx* ctx, const Job& J, SortState& s) {
+  constexpr bool K32 = sizeof(KeyT) == 4;
   cudaStream_t st = ctx->stream;
   bwtc_cuda_stats& S = ctx->stats;
-  const BatchSpec* bs = J.bs;
-  const uint32_t N = J.N, n = J.n;
+  const uint32_t N = J.N;
   const Round0Plan& pl = J.pl;
-  const EmitParams& ep = J.ep;
-  const uint8_t* d_text = J.d_text;
-  PassTimer pt{ctx};
-  // a repeated phase B starts its statistics over (phase A's launches and bytes are kept)
-  S.kernel_launches = J.a_launches;
-  S.algorithmic_bytes = J.a_bytes;
-  S.sort_bytes = S.sort0_bytes = 0;
-  S.sort_launches = S.sort0_launches = 0;
-  CK(ctx, cudaMemsetAsync(ctx->d_zero, 0, (size_t)CTR_STICKY * 4, st));  // sticky control words (CTR_ERR)
-  CK(ctx, cudaMemsetAsync(ctx->d_state, 0, sizeof(LadderState), st));
-  CK(ctx, cudaMemsetAsync(ctx->d_LF + LF_PARK, 0, (size_t)(LF_WORDS - LF_PARK) * 4, st));  // parked hole bytes
-
-  // ---- round 0: pack keys (+ all digit histograms), sort, re-rank
-  const uint32_t rs_tile0 = pl.keybytes == 4 ? RS_TILE32 : RS_TILE64;
   const uint32_t all0 = (1u << pl.npass) - 1u;
   // When the id and one character code fit a 32-bit payload together, the first pass stores the code of the
   // character preceding each suffix above the id: the round-0 BWT emission then needs no text gather.
@@ -872,490 +969,366 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
   const bool pack_pred = ctx->use_pack_pred && (id_bits + pl.bits <= 32);
   // No spare id bits (byte alphabets above 16 MiB) and a text too large for an L2-resident gather at emission time:
   // the predecessor codes travel as a one-byte payload array instead.
-  const bool aux_pred = !pack_pred && ctx->aux_min_suffixes && N >= ctx->aux_min_suffixes && !bs;
+  const bool aux_pred = !pack_pred && ctx->aux_min_suffixes && N >= ctx->aux_min_suffixes && !J.batch();
   // every digit pass of the round runs (a constant digit makes its pass a stable identity permutation, and finding that
   // out would cost a host synchronisation per block) — or only the top0 upper ones, and k_bucket_sort does the rest
-  const uint32_t top0 = plan_round0_top(ctx, pl, bs != nullptr, aux_pred);
+  const uint32_t top0 = plan_round0_top(ctx, pl, J.batch(), aux_pred);
   const uint32_t low0 = top0 ? pl.npass - top0 : 0u;
   const uint32_t mask0 = all0 & ~((1u << low0) - 1u);
-  if (zero_round_state(ctx, N, N, rs_tile0, mask0)) return BWTC_CUDA_ECUDA;
+  if (zero_round_state(ctx, N, N, K32 ? RS_TILE32 : RS_TILE64, mask0)) return BWTC_CUDA_ECUDA;
   {
     const uint32_t ptiles = div_up(N, AUX_TILE);
     const int grid = (int)(ptiles < (uint32_t)(ctx->sm_count * 4) ? ptiles : (uint32_t)(ctx->sm_count * 4));
-    // One representative digit per phase class is counted by k_pack_round0; the others are derived (k_hist_derive).
-    uint32_t hist_mask = 0;
+    uint32_t hist_mask;
     DeriveParams dp;
-    dp.count = 0;
-    // (digit positions in the coordinates of the c exact characters: the key carries pl.rbits partial bits below them)
-    const uint32_t keybits = pl.chars * pl.bits;
-    const uint32_t rbits = pl.rbits;
-    uint32_t regular_mask = 0;  // digits that lie entirely inside the exact characters
-    for (uint32_t p = 0; p < pl.npass; ++p) {
-      int rep = -1;
-      const bool full_p = (8u * p >= rbits) && (8u * p - rbits + 8u <= keybits);
-      if (full_p) regular_mask |= 1u << p;
-      if (full_p && N > 64 && !bs)  // (a batch counts every digit directly: block numbers sit above the characters)
-        for (uint32_t r = 0; r < p; ++r)
-          if (((hist_mask >> r) & (regular_mask >> r) & 1u) && (8u * (p - r)) % pl.bits == 0) { rep = (int)r; break; }
-      if (rep < 0) {
-        hist_mask |= 1u << p;
-      } else {
-        dp.p[dp.count] = (uint8_t)p;
-        dp.r[dp.count] = (uint8_t)rep;
-        dp.t[dp.count] = (uint8_t)(8u * (p - (uint32_t)rep) / pl.bits);
-        dp.count++;
-      }
-    }
-    // Gram mode (6- and 3-bit codes): one 4096-bin histogram of the keys' low 12 bits, every digit histogram projected
-    // from it (k_hist_from_gram) — one shared-memory atomic per key instead of one per counted digit.
     GramParams gp;
-    gp.npass = 0;
-    bool use_gram = ctx->use_gram && !bs && N > 64 && (pl.bits == 6 || pl.bits == 3) && keybits >= (uint32_t)GRAM_BITS;
-    if (use_gram) {
-      const uint32_t W = (uint32_t)GRAM_BITS / pl.bits;
-      for (uint32_t p = 0; p < pl.npass && use_gram; ++p) {
-        uint32_t u, sft;
-        gp.next[p] = 0;
-        if (8u * p < rbits) {  // the lowest digit reaches into the partial character: window of the following suffix
-          if (p != 0) use_gram = false;
-          u = 0;
-          sft = pl.bits - rbits;
-          gp.next[p] = 1;
-          if (sft + 8u > (uint32_t)GRAM_BITS) use_gram = false;
-        } else {
-          const uint32_t lo = 8u * p - rbits;
-          u = std::min<uint32_t>(lo / pl.bits, pl.chars - W);
-          sft = lo - pl.bits * u;
-          // the digit must lie inside the 12 bits above bit (bits * u), or run past the top of the key (zeros there)
-          if (sft + 8u > (uint32_t)GRAM_BITS && lo + 8u <= keybits) use_gram = false;
-        }
-        if (sft >= 32u) use_gram = false;
-        gp.u[p] = (uint8_t)u;
-        gp.s[p] = (uint8_t)sft;
-      }
-      gp.npass = pl.npass;
-    }
+    const bool use_gram = plan_histograms(ctx, pl, N, J.batch(), &hist_mask, &dp, &gp);
     uint32_t* gram = use_gram ? ctx->d_hist() + GRAM_OFF : nullptr;
-    if (use_gram) { hist_mask = 0; dp.count = 0; }
-    if (pl.keybytes == 4) {
-      k_pack_round0<uint32_t><<<grid, 256, 0, st>>>(d_text, N, static_cast<uint32_t*>(ctx->d_keys[0]), pl.pp,
-                                                     ctx->d_hist(), hist_mask, ptiles, gram);
-      if (dp.count) k_hist_derive<uint32_t><<<dp.count, 256, 0, st>>>(d_text, N, pl.pp, dp, ctx->d_hist());
-      if (use_gram) k_hist_from_gram<uint32_t><<<gp.npass, 256, 0, st>>>(d_text, N, pl.pp, gp, gram, ctx->d_hist());
-    } else {
-      k_pack_round0<unsigned long long><<<grid, 256, 0, st>>>(d_text, N, static_cast<unsigned long long*>(ctx->d_keys[0]),
-                                                               pl.pp, ctx->d_hist(), hist_mask, ptiles, gram);
-      if (dp.count) k_hist_derive<unsigned long long><<<dp.count, 256, 0, st>>>(d_text, N, pl.pp, dp, ctx->d_hist());
-      if (use_gram) k_hist_from_gram<unsigned long long><<<gp.npass, 256, 0, st>>>(d_text, N, pl.pp, gp, gram, ctx->d_hist());
-    }
+    k_pack_round0<KeyT><<<grid, 256, 0, st>>>(J.d_text, N, static_cast<KeyT*>(ctx->d_keys[0]), pl.pp, ctx->d_hist(), hist_mask,
+                                              ptiles, gram);
+    if (dp.count) k_hist_derive<KeyT><<<dp.count, 256, 0, st>>>(J.d_text, N, pl.pp, dp, ctx->d_hist());
+    if (use_gram) k_hist_from_gram<KeyT><<<gp.npass, 256, 0, st>>>(J.d_text, N, pl.pp, gp, gram, ctx->d_hist());
     if (dp.count || use_gram) S.kernel_launches++;
     CK(ctx, cudaGetLastError());
     S.kernel_launches++;
     S.algorithmic_bytes += (uint64_t)N + (uint64_t)N * pl.keybytes;
   }
-  int cur = 0;
-  uint32_t pdone = 0;
-  int rc;
   const uint32_t topshift = (pl.chars - 1) * pl.bits + pl.rbits;
   const uint32_t pred_mask = (1u << pl.bits) - 1u;  // (a batch key carries the block number above the characters)
-  if (pl.keybytes == 4)
-    rc = run_sort<uint32_t, RS_IPT32>(ctx, N, mask0, true, N - 1, &cur, &pt, &pdone, pack_pred ? id_bits : 0u, topshift,
-                                      pred_mask, aux_pred);
-  else
-    rc = run_sort<unsigned long long, RS_IPT64>(ctx, N, mask0, true, N - 1, &cur, &pt, &pdone, pack_pred ? id_bits : 0u,
-                                                topshift, pred_mask, aux_pred);
-  if (rc) return rc;
+  if (const int rc = run_sort<KeyT, K32 ? RS_IPT32 : RS_IPT64>(ctx, N, mask0, true, N - 1, &s.cur, &s.pt, &s.pdone,
+                                                               pack_pred ? id_bits : 0u, topshift, pred_mask, aux_pred))
+    return rc;
   if (top0) {
     // the passes left every bucket of equal top bits contiguous and in input order: sort each by its low 8·low0 key bits
-    k_bucket_sort<<<div_up(N, BK_T), BK_BLOCK, 0, st>>>(static_cast<unsigned long long*>(ctx->d_keys[cur]), ctx->d_idx[cur],
-                                                        static_cast<unsigned long long*>(ctx->d_keys[cur ^ 1]), ctx->d_idx[cur ^ 1],
-                                                        N, 8u * low0, ctx->d_ctrl(), &ctx->d_state->big_buckets);
+    k_bucket_sort<<<div_up(N, BK_T), BK_BLOCK, 0, st>>>(static_cast<unsigned long long*>(ctx->d_keys[s.cur]), ctx->d_idx[s.cur],
+                                                        static_cast<unsigned long long*>(ctx->d_keys[s.cur ^ 1]),
+                                                        ctx->d_idx[s.cur ^ 1], N, 8u * low0, ctx->d_ctrl(),
+                                                        &ctx->d_state->big_buckets);
     CK(ctx, cudaGetLastError());
     S.kernel_launches++;
     S.algorithmic_bytes += (uint64_t)N * 24;  // keys and ids read and written once (in place)
-    ++pdone;
+    ++s.pdone;
   }
-  const size_t round0_events = pt.used;
+  s.round0_events = s.pt.used;
   S.sort0_launches = S.sort_launches;
   S.sort0_bytes = S.sort_bytes;
-  S.live[0] = N;
-  S.passes[0] = pdone;
-  S.prefix_len[0] = 0;
-  S.rounds = 1;
-  // ---- lazy ranks? (DESIGN.md §3.9)  The rank scatter of round 0 — a random 4-byte write per suffix — is 20-35% of a block,
-  // but after round 0 only the ranks of suffixes that are still in a group are ever refined, and a singleton's rank is simply
-  // its position in the sorted key array.  If few suffixes will stay in groups, rank[] is written for those only; the
-  // segmented rounds order group members by cmp (round-0 key, then rank where it is stored) and need no integer rank, the
-  // tail (k_small_rounds, k_finish) looks the few ranks it needs up in the retained sorted keys (rank_lookup).
-  bool lazy = false;
+  log_round(S, N, s.pdone, 0);
+  const bool lazy = s.lazy = choose_lazy(ctx, J);
   const uint32_t keybits0 = pl.chars * pl.bits + pl.rbits;
-  if (ctx->use_lazy && !bs && !dbg_any(ctx) && N >= 64 && keybits0 >= 1) {
-    // The decision needs no extra measurement.  For an i.i.d.-like source (DNA, random bytes) the key-shape policy has
-    // already predicted the fraction of suffixes still tied after round 0, L(c) = 1 - exp(-N 2^(-H0 c)) — it matches the
-    // measured live fractions to three digits (DNA 64 MiB: 0.0156 / 0.0155; random 256 MiB: 0.0606 / 0.0606).  For a source
-    // with memory the 8-gram sample tells text (a few other positions share a position's 8-gram: Markov 32 MiB 3.0, 3% live
-    // after its 10.7-character keys) from repeats (thousands: the 4 KiB-seed block keeps ~all suffixes tied through global
-    // radix rounds and would only pay the materialising fallback).  The 8-gram sample says nothing about how much a key
-    // longer than 8 characters separates, so a block with memory also needs keys of at least LAZY_MIN_CHARS characters
-    // (codes of <= 6 bits): the same Markov text as a 65-symbol raw text (7-bit codes, 9-character keys) left more or
-    // larger groups after round 0 than the segmented rounds take and fell back.  Segmented rounds are what makes lazy ranks cheap, so a block with memory
-    // goes lazy only where they run.  A wrong prediction only costs time: the fallback below is exact.
-    constexpr uint32_t LAZY_MIN_CHARS = 10;
-    const bool memory_ok = ctx->use_seg && pl.chars >= LAZY_MIN_CHARS && pl.repeats <= ctx->lazy_max_repeats;
-    lazy = ctx->use_lazy >= 2 ||
-           (N >= ctx->lazy_min_suffixes && (pl.has_memory ? memory_ok : pl.live_pred <= ctx->lazy_max_live));
-  }
   const uint32_t tbits = std::min<uint32_t>(KTAB_BITS, keybits0);
   const uint32_t lazy_cap = N / 6;  // the lists of lazy mode live in six slices of d_scat
+  RerankParams& rp = s.rr0;
+  rp.m = N;
   {
-    RerankParams rp;
-    rp.m = N;
-    {
-      const uint32_t text_end = J.sentinel_outside_alphabet ? N - 1 : N;  // windows reaching text_end are unique
-      const uint32_t wchars = pl.chars + (pl.rbits ? 1u : 0u);  // characters a key looks at (the partial one included)
-      rp.short_thresh = wchars > text_end ? 0u : text_end - wchars + 1u;
-    }
-    rp.lo_bits = 0;
-    rp.lazy = lazy ? 1u : 0u;
-    rp.livebits = ctx->d_livebits;
-    rp.ktab = ctx->d_ktab;
-    rp.tshift = keybits0 - tbits;
-    if (lazy) {
-      CK(ctx, cudaMemsetAsync(ctx->d_livebits, 0, ((size_t)N / 32 + 4) * 4, st));
-      CK(ctx, cudaMemsetAsync(ctx->d_ktab, 0xFF, ((size_t)(1u << tbits) + 2) * 4, st));
-      LookupParams& L = *ctx->h_lookup;
-      L.enabled = 1;
-      L.keybytes = pl.keybytes;
-      L.sorted_keys = ctx->d_keys[cur];
-      L.ktab = ctx->d_ktab;
-      L.livebits = ctx->d_livebits;
-      L.text = d_text;
-      L.N = N;
-      L.bits = pl.bits;
-      L.chars = pl.chars;
-      L.rbits = pl.rbits;
-      L.tshift = keybits0 - tbits;
-      memcpy(L.lut, pl.pp.lut, 256);
-      CK(ctx, cudaMemcpyAsync(ctx->d_lookup, ctx->h_lookup, sizeof(LookupParams), cudaMemcpyHostToDevice, st));
-    }
-    S.flags = (ctx->static_tiles ? 0u : 1u) | (bs ? 2u : 0u) | (pack_pred ? 4u : 0u) | (aux_pred ? 8u : 0u) | (lazy ? 16u : 0u) |
-              (J.sa ? 256u : 0u) | (top0 ? 1024u : 0u);
-    rp.packed = pack_pred ? 1u : (aux_pred ? 2u : 0u);
-    rp.pred_aux = ctx->d_aux[cur];
-    rp.id_bits = pack_pred ? id_bits : 31u;
-    rp.id_mask = pack_pred ? (uint32_t)((1ull << id_bits) - 1ull) : 0xFFFFFFFFu;
-    memset(rp.decode, 0, sizeof(rp.decode));
-    for (int c = 0; c < 256; ++c)
-      if (J.present[c]) rp.decode[pl.pp.lut[c]] = (uint8_t)c;
-    uint32_t* snr = reinterpret_cast<uint32_t*>(ctx->d_keys[cur ^ 1]);
-    if (pl.keybytes == 4) rc = launch_rerank<uint32_t, true>(ctx, cur, N, N, rp, ep, snr, snr + N, lazy);
-    else rc = launch_rerank<unsigned long long, true>(ctx, cur, N, N, rp, ep, snr, snr + N, lazy);
-    if (rc) return rc;
-    S.algorithmic_bytes += (uint64_t)N * (pl.keybytes + 4) + (lazy ? 0ull : (uint64_t)N * 4);
-    if (lazy) {
-      const uint32_t entries = 1u << tbits, nchunks = div_up(entries, KTAB_CHUNK);
-      uint32_t* cmin = ctx->d_bhist;  // <= 256 words of the (idle) per-block histogram area
-      k_ktab_chunkmin<<<nchunks, 256, 0, st>>>(ctx->d_ktab, entries, cmin);
-      k_ktab_fill<<<nchunks, 256, 0, st>>>(ctx->d_ktab, entries, N, cmin, nchunks);
-      CK(ctx, cudaGetLastError());
-      S.kernel_launches += 2;
-    }
-    ctx->rr0 = rp;  // (kept for the fallback out of lazy mode)
+    const uint32_t text_end = J.sentinel_outside_alphabet ? N - 1 : N;  // windows reaching text_end are unique
+    const uint32_t wchars = pl.chars + (pl.rbits ? 1u : 0u);  // characters a key looks at (the partial one included)
+    rp.short_thresh = wchars > text_end ? 0u : text_end - wchars + 1u;
   }
-  // six u32[N] work arrays: halves of the two key buffers and the two id buffers
-  PoolPtrs pool;
-  pool.p[0] = reinterpret_cast<uint32_t*>(ctx->d_keys[0]);
-  pool.p[1] = reinterpret_cast<uint32_t*>(ctx->d_keys[0]) + N;
-  pool.p[2] = reinterpret_cast<uint32_t*>(ctx->d_keys[1]);
-  pool.p[3] = reinterpret_cast<uint32_t*>(ctx->d_keys[1]) + N;
-  pool.p[4] = ctx->d_idx[0];
-  pool.p[5] = ctx->d_idx[1];
-  const PoolPtrs norm = pool;  // (the staging slots of k_rerank are always halves of the idle key buffer)
-  if (lazy) {  // the sorted keys (d_keys[cur]) must survive: lists, next lists and rank updates live in six slices of d_scat
-    for (int q = 0; q < 6; ++q) pool.p[q] = ctx->d_scat + (size_t)q * lazy_cap;
+  rp.lo_bits = 0;
+  rp.lazy = lazy ? 1u : 0u;
+  rp.livebits = ctx->d_livebits;
+  rp.ktab = ctx->d_ktab;
+  rp.tshift = keybits0 - tbits;
+  if (lazy) {
+    CK(ctx, cudaMemsetAsync(ctx->d_livebits, 0, ((size_t)N / 32 + 4) * 4, st));
+    CK(ctx, cudaMemsetAsync(ctx->d_ktab, 0xFF, ((size_t)(1u << tbits) + 2) * 4, st));
+    LookupParams& L = *ctx->h_lookup;
+    L.enabled = 1;
+    L.keybytes = pl.keybytes;
+    L.sorted_keys = ctx->d_keys[s.cur];
+    L.ktab = ctx->d_ktab;
+    L.livebits = ctx->d_livebits;
+    L.text = J.d_text;
+    L.N = N;
+    L.bits = pl.bits;
+    L.chars = pl.chars;
+    L.rbits = pl.rbits;
+    L.tshift = keybits0 - tbits;
+    memcpy(L.lut, pl.pp.lut, 256);
+    CK(ctx, cudaMemcpyAsync(ctx->d_lookup, ctx->h_lookup, sizeof(LookupParams), cudaMemcpyHostToDevice, st));
   }
-  const LookupParams* lkp = lazy ? ctx->d_lookup : nullptr;
-  ctx->last_cur = cur;
-  uint32_t m_prev = N;       // records of the last global sort = extent of the k_rerank staging slots
-  uint32_t m_bound = N;      // upper bound of the live count (it never grows)
-  uint64_t h_next = pl.chars;
-  auto sel_of = [&lazy](int c) { return lazy ? 0x10u : ((uint32_t)(2 * c) | ((uint32_t)(2 * c + 1) << 4)); };
-  k_commit_sort<<<1, 1, 0, st>>>(ctx->d_state, ctx->d_ctrl(), (uint32_t)std::min<uint64_t>(h_next, 0x7FFFFFFFull), sel_of(cur),
-                                 0xFFFFFFFFu, 1u, lazy ? lazy_cap : 0xFFFFFFFFu);
-  S.kernel_launches++;
-
-  // Concatenate the per-tile chunks k_rerank staged (in d_keys[cur^1]) into compact lists in d_keys[cur], whose
-  // sorted keys are dead by now.  Tile order is kept, so every group stays contiguous.  speculative: the gather
-  // runs only if the device-side state says the next step consumes the lists.
-  auto make_lists = [&](bool speculative) -> int {
-    const uint32_t tiles = div_up(m_prev, AUX_TILE);
-    k_scan_tile_counts<<<1, 1024, 0, st>>>(ctx->d_tilecnt, ctx->d_tilecnt + ctx->max_aux_tiles, tiles);
-    k_gather_chunks<<<tiles, 256, 0, st>>>(norm.p[2 * (cur ^ 1)], norm.p[2 * (cur ^ 1) + 1], ctx->d_tilecnt,
-                                           ctx->d_tilecnt + ctx->max_aux_tiles, AUX_TILE, lazy ? pool.p[0] : norm.p[2 * cur],
-                                           lazy ? pool.p[1] : norm.p[2 * cur + 1], speculative ? ctx->d_state : nullptr,
-                                           ctx->d_ctrl());
+  S.flags = (ctx->static_tiles ? 0u : 1u) | (J.batch() ? 2u : 0u) | (pack_pred ? 4u : 0u) | (aux_pred ? 8u : 0u) |
+            (lazy ? 16u : 0u) | (J.sa ? 256u : 0u) | (top0 ? 1024u : 0u);
+  rp.packed = pack_pred ? 1u : (aux_pred ? 2u : 0u);
+  rp.pred_aux = ctx->d_aux[s.cur];
+  rp.id_bits = pack_pred ? id_bits : 31u;
+  rp.id_mask = pack_pred ? (uint32_t)((1ull << id_bits) - 1ull) : 0xFFFFFFFFu;
+  memset(rp.decode, 0, sizeof(rp.decode));
+  for (int c = 0; c < 256; ++c)
+    if (J.present[c]) rp.decode[pl.pp.lut[c]] = (uint8_t)c;
+  s.rerank0 = launch_rerank<KeyT, true>;
+  uint32_t* snr = reinterpret_cast<uint32_t*>(ctx->d_keys[s.cur ^ 1]);
+  if (const int rc = s.rerank0(ctx, s.cur, N, N, rp, J.ep, snr, snr + N, lazy, false)) return rc;
+  S.algorithmic_bytes += (uint64_t)N * (pl.keybytes + 4) + (lazy ? 0ull : (uint64_t)N * 4);
+  if (lazy) {
+    const uint32_t entries = 1u << tbits, nchunks = div_up(entries, KTAB_CHUNK);
+    uint32_t* cmin = ctx->d_bhist;  // <= 256 words of the (idle) per-block histogram area
+    k_ktab_chunkmin<<<nchunks, 256, 0, st>>>(ctx->d_ktab, entries, cmin);
+    k_ktab_fill<<<nchunks, 256, 0, st>>>(ctx->d_ktab, entries, N, cmin, nchunks);
     CK(ctx, cudaGetLastError());
     S.kernel_launches += 2;
-    return 0;
-  };
+  }
+  // six u32[N] work arrays: halves of the two key buffers and the two id buffers
+  s.pool.p[0] = reinterpret_cast<uint32_t*>(ctx->d_keys[0]);
+  s.pool.p[1] = reinterpret_cast<uint32_t*>(ctx->d_keys[0]) + N;
+  s.pool.p[2] = reinterpret_cast<uint32_t*>(ctx->d_keys[1]);
+  s.pool.p[3] = reinterpret_cast<uint32_t*>(ctx->d_keys[1]) + N;
+  s.pool.p[4] = ctx->d_idx[0];
+  s.pool.p[5] = ctx->d_idx[1];
+  s.norm = s.pool;  // (the staging slots of k_rerank are always halves of the idle key buffer)
+  if (lazy) {  // the sorted keys (d_keys[cur]) must survive: lists, next lists and rank updates live in six slices of d_scat
+    for (int q = 0; q < 6; ++q) s.pool.p[q] = ctx->d_scat + (size_t)q * lazy_cap;
+  }
+  s.lkp = lazy ? ctx->d_lookup : nullptr;
+  ctx->last_cur = s.cur;
+  s.m_prev = s.m_bound = N;
+  s.h_next = pl.chars;
+  k_commit_sort<<<1, 1, 0, st>>>(ctx->d_state, ctx->d_ctrl(), (uint32_t)std::min<uint64_t>(s.h_next, 0x7FFFFFFFull), s.sel(s.cur),
+                                 0xFFFFFFFFu, 1u, lazy ? lazy_cap : 0xFFFFFFFFu);
+  S.kernel_launches++;
+  return 0;
+}
 
-  // The BWT bytes for the caller: a batch's blocks from d_out at stride n0 + 1, a single block's from d_out unless they
-  // are already in the caller's device buffer (J.d_dst).  A raw output leaves U[pidx] untouched (divsufsort.c:506-512):
-  // two ranges around it.  A suffix-array job's BWT bytes stay on the device.
-  const Dst out_kind = bs ? dst_kind(bs->out[0], bs->on_device) : dst_kind(J.h_out, J.out_dev || !J.h_out);
-  auto copy_out = [&]() -> int {
-    if (bs) {
-      for (uint32_t k = 0; k < bs->nblocks; ++k) {
-        const uint32_t nk = (k + 1 == bs->nblocks) ? bs->n_last : bs->n0;
-        if (copy_result(ctx, out_kind, bs->out[k], ctx->d_out + (size_t)k * J.bstride, nk)) return BWTC_CUDA_ECUDA;
-      }
-    } else if (!J.block_mode) {
-      const uint32_t pidx = ctx->h_LF()[0];
-      if (copy_result(ctx, out_kind, J.h_out, ctx->d_out, pidx) ||
-          (pidx + 1 < n && copy_result(ctx, out_kind, J.h_out + pidx + 1, ctx->d_out + pidx + 1, n - pidx - 1)))
-        return BWTC_CUDA_ECUDA;
-    } else if (out_kind != Dst::device && !(out_kind == Dst::pinned && (ctx->debug_skip_copies & 2))) {
-      return copy_result(ctx, out_kind, J.h_out, ctx->d_out, n);
+// Concatenate the per-tile chunks k_rerank staged (in d_keys[cur^1]) into compact lists in d_keys[cur], whose
+// sorted keys are dead by now.  Tile order is kept, so every group stays contiguous.  speculative: the gather
+// runs only if the device-side state says the next step consumes the lists.
+int make_lists(bwtc_cuda_ctx* ctx, const SortState& s, bool speculative) {
+  cudaStream_t st = ctx->stream;
+  const uint32_t tiles = div_up(s.m_prev, AUX_TILE);
+  const int c = s.cur;
+  k_scan_tile_counts<<<1, 1024, 0, st>>>(ctx->d_tilecnt, ctx->d_tilecnt + ctx->max_aux_tiles, tiles);
+  k_gather_chunks<<<tiles, 256, 0, st>>>(s.norm.p[2 * (c ^ 1)], s.norm.p[2 * (c ^ 1) + 1], ctx->d_tilecnt,
+                                         ctx->d_tilecnt + ctx->max_aux_tiles, AUX_TILE, s.lazy ? s.pool.p[0] : s.norm.p[2 * c],
+                                         s.lazy ? s.pool.p[1] : s.norm.p[2 * c + 1], speculative ? ctx->d_state : nullptr,
+                                         ctx->d_ctrl());
+  CK(ctx, cudaGetLastError());
+  ctx->stats.kernel_launches += 2;
+  return 0;
+}
+
+// The BWT bytes for the caller: a batch's blocks from d_out at stride n0 + 1, a single block's from d_out unless they are
+// already in the caller's device buffer (J.d_dst).  A raw output leaves U[pidx] untouched (divsufsort.c:506-512): two
+// ranges around it.
+int copy_out(bwtc_cuda_ctx* ctx, const Job& J, Dst kind) {
+  if (!J.block_mode) {
+    const uint32_t pidx = ctx->h_bLF()[0], n = J.n;
+    uint8_t* U = static_cast<uint8_t*>(J.out[0]);
+    if (copy_result(ctx, kind, U, ctx->d_out, pidx) ||
+        (pidx + 1 < n && copy_result(ctx, kind, U + pidx + 1, ctx->d_out + pidx + 1, n - pidx - 1)))
+      return BWTC_CUDA_ECUDA;
+    return 0;
+  }
+  if (!J.batch() && (kind == Dst::device || (kind == Dst::pinned && (ctx->debug_skip_copies & 2)))) return 0;
+  for (uint32_t k = 0; k < J.nblocks; ++k)
+    if (copy_result(ctx, kind, J.out[k], ctx->d_out + (size_t)k * (J.n0 + 1u), J.bytes(k))) return BWTC_CUDA_ECUDA;
+  return 0;
+}
+
+// ---- one ladder chunk: [lists] [K x (segmented round, rank update, commit)] [tail] [finish] [runs], the read-back of the
+// device-side state and the LFpowers, the speculative result copies of the first chunk, and the host wait.
+int ladder_chunk(bwtc_cuda_ctx* ctx, const Job& J, SortState& s) {
+  cudaStream_t st = ctx->stream;
+  bwtc_cuda_stats& S = ctx->stats;
+  const uint32_t N = J.N, n = J.n, dbg = ctx->debug_max_rounds;
+  const EmitParams& ep = J.ep;
+  const PoolPtrs& pool = s.pool;
+  const LookupParams* lkp = s.lkp;
+  s.chunk_built_lists = s.lists_pending && !s.lean;
+  if (!(dbg && S.rounds >= dbg) && !s.lean) {
+    if (s.lists_pending) {
+      if (make_lists(ctx, s, true)) return BWTC_CUDA_ECUDA;
+      s.lists_pending = false;
     }
-    return 0;
-  };
-  // Copies that need no host staging (device and pinned buffers) are waited for once.  In block mode they are enqueued
-  // speculatively behind the first ladder chunk (a block whose later rounds are all sort-free then completes with one host
-  // wait), and repeated at the end if the block was not finished by then.
-  const bool direct_out = bs ? out_kind != Dst::pageable : out_kind == Dst::pinned;
-  // verification (DESIGN.md §3.10): the caller's host and batch outputs are written only after the check word is read
-  const bool verify = ctx->verify && !ctx->debug_max_rounds;
-  uint32_t* h_bLF = reinterpret_cast<uint32_t*>(ctx->h_batch + MAX_BATCH * sizeof(void*)) + MAX_BATCH * 256;
+    const int K = dbg ? 1 : (s.first_chunk ? ctx->ladder_first : ctx->ladder_more);
+    for (int k = 0; k < K && ctx->use_seg; ++k) {
+      // persistent grid; the first round behind a sort is the big one, later (often skipped) ones get a leaner grid
+      const uint32_t per_sm = (k == 0) ? 12u : 4u;
+      const uint32_t seg_grid = std::max<uint32_t>(1u, std::min<uint32_t>(div_up(s.m_bound, SEG_T), (uint32_t)ctx->sm_count * per_sm));
+      if (ep.sa) {
+        if (lkp) k_seg_round<true, true><<<seg_grid, 256, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), lkp);
+        else k_seg_round<false, true><<<seg_grid, 256, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), nullptr);
+      } else {
+        if (lkp) k_seg_round<true><<<seg_grid, 256, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), lkp);
+        else k_seg_round<false><<<seg_grid, 256, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), nullptr);
+      }
+      k_apply_ranks<<<ctx->sm_count * 8, 256, 0, st>>>(ctx->d_state, pool, ctx->d_ctrl(), ctx->d_rank);
+      k_commit_seg<<<1, 1, 0, st>>>(ctx->d_state, ctx->d_ctrl());
+      S.kernel_launches += 3;
+    }
+    if (!dbg) {
+      if (ep.sa) k_small_rounds<true><<<1, 1024, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), lkp);
+      else k_small_rounds<<<1, 1024, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), lkp);
+      S.kernel_launches++;
+    }
+    CK(ctx, cudaGetLastError());
+  }
+  // final extraction: pidx, LFpowers, hole fill (returns early on the device while suffixes are still live)
+  if (J.batch())
+    k_finish_batch<<<J.nblocks, 256, 0, st>>>(ctx->d_rank, N, J.bstride, J.nblocks, J.d_dst, ctx->d_LF, J.nLF, J.nLF_last,
+                                              ctx->d_LF + LF_PARK, ctx->d_state, ctx->d_ctrl());
+  else
+    k_finish<<<1, 256, 0, st>>>(ctx->d_rank, J.d_text, N, J.d_dst, J.block_mode ? 1 : 0, ctx->d_LF, J.nLF, ctx->d_LF + LF_PARK,
+                                ctx->d_state, ctx->d_ctrl(), lkp);
+  CK(ctx, cudaGetLastError());
+  S.kernel_launches++;
+  if (J.runs) {
+    // run statistics of the (finished) output: symbols -> d_aux[0], start positions -> d_scat, both idle by now; tile
+    // counts in the look-back status area (cleared again before any later digit pass uses it)
+    const uint32_t rtiles = div_up(n, RUN_TILE);
+    uint32_t* rcnt = status_rows(ctx, 0);
+    uint32_t* rexcl = rcnt + rtiles;
+    const uint32_t cap_dev = std::min<uint32_t>(J.runs->capacity, n);
+    k_run_count<<<rtiles, 256, 0, st>>>(J.d_dst, n, rcnt, ctx->d_state);
+    k_scan_tile_counts<<<1, 1024, 0, st>>>(rcnt, rexcl, rtiles);
+    k_run_emit<<<rtiles, 256, 0, st>>>(J.d_dst, n, rcnt, rexcl, rtiles, cap_dev, ctx->d_aux[0], ctx->d_scat, &ctx->d_state->nruns,
+                                       ctx->d_state);
+    CK(ctx, cudaGetLastError());
+    S.kernel_launches += 3;  // (queued in every chunk; they return at once in all but the one that finishes the block)
+  }
+  CK(ctx, cudaEventRecord(ctx->ev_end, st));
+  CK(ctx, cudaMemcpyAsync(ctx->h_state, ctx->d_state, sizeof(LadderState), cudaMemcpyDeviceToHost, st));
+  CK(ctx, cudaMemcpyAsync(ctx->h_bLF(), ctx->d_LF, ((size_t)(J.nblocks - 1) * 256 + J.nLF_last) * 4, cudaMemcpyDeviceToHost, st));
+  if (s.first_chunk && s.direct_out && J.block_mode && !dbg && !s.verify) {
+    if (copy_out(ctx, J, s.out_kind)) return BWTC_CUDA_ECUDA;
+    s.out_enqueued = true;
+  }
+  return host_wait(ctx, st) ? BWTC_CUDA_ECUDA : 0;
+}
 
+// After a chunk's wait: the device's error word, and the rounds the device ran in the chunk.
+int read_chunk(bwtc_cuda_ctx* ctx, SortState& s) {
+  bwtc_cuda_stats& S = ctx->stats;
+  const LadderState& H = *ctx->h_state;
+  S.round0_big_buckets = H.big_buckets;
+  const char* what = H.err == 4u ? "segmented round met a group above its limit (internal error)"
+                     : H.err == 5u ? "k_build_keys emitted a record count that differs from the live count (internal error)"
+                     : H.err == 3u ? "tail refinement kernel did not converge"
+                                   : nullptr;
+  if (what) {
+    set_err(ctx->err, "%s", what);
+    return BWTC_CUDA_EINTERNAL;
+  }
+  if (H.err || (ctx->debug_fake_watchdog && ctx->static_tiles)) {
+    set_err(ctx->err, "look-back watchdog fired (code %u, round %u)", H.err, S.rounds);
+    ctx->lb_watchdog = 1;
+    return BWTC_CUDA_EINTERNAL;
+  }
+  for (uint32_t i = s.nlog_seen; i < H.nlog && i < (uint32_t)LADDER_LOG; ++i) {
+    if (s.chunk_built_lists && i == s.nlog_seen) S.algorithmic_bytes += (uint64_t)H.log_m[i] * 16;  // k_gather_chunks
+    log_round(S, H.log_m[i], 0, H.log_h[i]);
+    S.algorithmic_bytes += (uint64_t)H.log_m[i] * (H.log_kind[i] == 1u ? 32u : 24u);
+  }
+  s.nlog_seen = H.nlog;
+  s.first_chunk = false;
+  return 0;
+}
+
+// ---- out of lazy mode: more suffixes stayed in groups than the small list pool holds, or groups are large (a global
+// radix round scans rank[] in text order and needs every rank).  Materialise the singletons' ranks from the sorted
+// records of round 0 (still intact), then carry on with the full-rank path; nothing else has run in between.
+int leave_lazy(bwtc_cuda_ctx* ctx, const Job& J, SortState& s) {
+  cudaStream_t st = ctx->stream;
+  bwtc_cuda_stats& S = ctx->stats;
+  const uint32_t N = J.N;
+  RerankParams rp = s.rr0;
+  rp.lazy = 2u;
+  CK(ctx, cudaMemsetAsync(ctx->d_tstate(), 0, (size_t)rerank_launches(ctx, N, N) * ctx->max_aux_tiles * 8, st));
+  CK(ctx, cudaMemsetAsync(ctx->d_ctrl() + CTR_PASS0, 0, (size_t)(CTR_WORDS - CTR_PASS0) * 4, st));  // tile tickets
+  uint32_t* snr = reinterpret_cast<uint32_t*>(ctx->d_keys[s.cur ^ 1]);
+  s.lazy = false;  // (sel() and the pools below now mean the full-rank layout)
+  if (const int rc = s.rerank0(ctx, s.cur, N, N, rp, J.ep, snr, snr + N, false, true)) return rc;
+  S.algorithmic_bytes += (uint64_t)N * (J.pl.keybytes + 4) + (uint64_t)N * 4;
+  S.flags |= 32u;  // lazy ranks were abandoned for this block
+  s.pool = s.norm;
+  s.lkp = nullptr;
+  s.lean = true;  // the lists (if the next step wants them) are built below from the intact staging
+  s.lists_pending = true;
+  return 0;
+}
+
+// ---- one global radix round (large groups: repetitive input), host-driven, over the m = H.m live suffixes
+int global_round(bwtc_cuda_ctx* ctx, const Job& J, SortState& s) {
+  cudaStream_t st = ctx->stream;
+  bwtc_cuda_stats& S = ctx->stats;
+  const LadderState& H = *ctx->h_state;
+  const uint32_t N = J.N, m = H.m, h32 = H.h;
   const int lo_bits = (int)ceil_log2_u64((uint64_t)N + 1);  // rank[i+h] + 1 in [0, N]
   // high part = (rank of the group head) >> 1 (k_build_keys): heads of live groups are <= N - 2
   const int hi_bits = N > 3 ? (int)ceil_log2_u64((((uint64_t)N - 2) >> 1) + 1) : 1;
   const uint32_t npassd = div_up((uint64_t)(lo_bits + hi_bits), 8);
   const uint32_t maskd = (1u << npassd) - 1u;
-  bool lists_pending = true, first_chunk = true, out_enqueued = false, finished = false;
-  // lean chunk: behind a global radix round whose groups were still far above the segmented-round limit nothing sort-free
-  // is enqueued speculatively (it would only be skipped on the device): commit, k_finish (error word), state copy, wait
-  bool lean = false;
   constexpr uint32_t LEAN_MAXGROUP = 8u * SEG_MAXGROUP;
-  uint32_t nlog_seen = 0;
-  const uint32_t dbg = ctx->debug_max_rounds;
-  for (;;) {
-    // ---- one ladder chunk: [lists] [K x (segmented round, rank update, commit)] [tail] [finish] [copies]
-    const bool chunk_built_lists = lists_pending && !lean;
-    if (!(dbg && S.rounds >= dbg) && !lean) {
-      if (lists_pending) {
-        if (make_lists(true)) return BWTC_CUDA_ECUDA;
-        lists_pending = false;
-      }
-      const int K = dbg ? 1 : (first_chunk ? ctx->ladder_first : ctx->ladder_more);
-      for (int k = 0; k < K && ctx->use_seg; ++k) {
-        // persistent grid; the first round behind a sort is the big one, later (often skipped) ones get a leaner grid
-        const uint32_t per_sm = (k == 0) ? 12u : 4u;
-        const uint32_t seg_grid = std::max<uint32_t>(1u, std::min<uint32_t>(div_up(m_bound, SEG_T), (uint32_t)ctx->sm_count * per_sm));
-        if (ep.sa) {
-          if (lkp) k_seg_round<true, true><<<seg_grid, 256, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), lkp);
-          else k_seg_round<false, true><<<seg_grid, 256, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), nullptr);
-        } else {
-          if (lkp) k_seg_round<true><<<seg_grid, 256, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), lkp);
-          else k_seg_round<false><<<seg_grid, 256, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), nullptr);
-        }
-        k_apply_ranks<<<ctx->sm_count * 8, 256, 0, st>>>(ctx->d_state, pool, ctx->d_ctrl(), ctx->d_rank);
-        k_commit_seg<<<1, 1, 0, st>>>(ctx->d_state, ctx->d_ctrl());
-        S.kernel_launches += 3;
-      }
-      if (!dbg) {
-        if (ep.sa) k_small_rounds<true><<<1, 1024, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), lkp);
-        else k_small_rounds<<<1, 1024, 0, st>>>(ctx->d_state, pool, ctx->d_rank, N, ep, ctx->d_ctrl(), lkp);
-        S.kernel_launches++;
-      }
-      CK(ctx, cudaGetLastError());
-    }
-    // final extraction: pidx, LFpowers, hole fill (returns early on the device while suffixes are still live)
-    if (bs)
-      k_finish_batch<<<bs->nblocks, 256, 0, st>>>(ctx->d_rank, N, J.bstride, bs->nblocks, J.d_dst, ctx->d_LF, bs->nLF, bs->nLF_last,
-                                                  ctx->d_LF + LF_PARK, ctx->d_state, ctx->d_ctrl());
-    else
-      k_finish<<<1, 256, 0, st>>>(ctx->d_rank, d_text, N, J.d_dst, J.block_mode ? 1 : 0, ctx->d_LF, J.nLF, ctx->d_LF + LF_PARK,
-                                  ctx->d_state, ctx->d_ctrl(), lkp);
-    CK(ctx, cudaGetLastError());
-    S.kernel_launches++;
-    if (J.runs && !bs && J.block_mode) {
-      // run statistics of the (finished) output: symbols -> d_aux[0], start positions -> d_scat, both idle by now; tile
-      // counts in the look-back status area (cleared again before any later digit pass uses it)
-      const uint32_t rtiles = div_up(n, RUN_TILE);
-      uint32_t* rcnt = status_rows(ctx, 0);
-      uint32_t* rexcl = rcnt + rtiles;
-      const uint32_t cap_dev = std::min<uint32_t>(J.runs->capacity, n);
-      k_run_count<<<rtiles, 256, 0, st>>>(J.d_dst, n, rcnt, ctx->d_state);
-      k_scan_tile_counts<<<1, 1024, 0, st>>>(rcnt, rexcl, rtiles);
-      k_run_emit<<<rtiles, 256, 0, st>>>(J.d_dst, n, rcnt, rexcl, rtiles, cap_dev, ctx->d_aux[0], ctx->d_scat, &ctx->d_state->nruns,
-                                         ctx->d_state);
-      CK(ctx, cudaGetLastError());
-      S.kernel_launches += 3;  // (queued in every chunk; they return at once in all but the one that finishes the block)
-    }
-    CK(ctx, cudaEventRecord(ctx->ev_end, st));
-    CK(ctx, cudaMemcpyAsync(ctx->h_state, ctx->d_state, sizeof(LadderState), cudaMemcpyDeviceToHost, st));
-    if (bs) CK(ctx, cudaMemcpyAsync(h_bLF, ctx->d_LF, (size_t)bs->nblocks * 256 * 4, cudaMemcpyDeviceToHost, st));
-    else CK(ctx, cudaMemcpyAsync(ctx->h_LF(), ctx->d_LF, J.nLF * 4, cudaMemcpyDeviceToHost, st));
-    if (first_chunk && direct_out && J.block_mode && !dbg && !verify) {
-      if (copy_out()) return BWTC_CUDA_ECUDA;
-      out_enqueued = true;
-    }
-    if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
-    const LadderState& H = *ctx->h_state;
-    S.round0_big_buckets = H.big_buckets;
-    if (H.err == 4u) {
-      set_err(ctx->err, "segmented round met a group above its limit (internal error)");
-      return BWTC_CUDA_EINTERNAL;
-    }
-    if (H.err == 5u) {
-      set_err(ctx->err, "k_build_keys emitted a record count that differs from the live count (internal error)");
-      return BWTC_CUDA_EINTERNAL;
-    }
-    if (H.err == 3u) {
-      set_err(ctx->err, "tail refinement kernel did not converge");
-      return BWTC_CUDA_EINTERNAL;
-    }
-    if (H.err || (ctx->debug_fake_watchdog && ctx->static_tiles)) {
-      set_err(ctx->err, "look-back watchdog fired (code %u, round %u)", H.err, S.rounds);
-      ctx->lb_watchdog = 1;
-      return BWTC_CUDA_EINTERNAL;
-    }
-    // rounds the device executed in this chunk
-    for (uint32_t i = nlog_seen; i < H.nlog && i < (uint32_t)LADDER_LOG; ++i) {
-      const uint32_t r = S.rounds;
-      if (chunk_built_lists && i == nlog_seen) S.algorithmic_bytes += (uint64_t)H.log_m[i] * 16;  // k_gather_chunks
-      if (r < BWTC_CUDA_MAX_ROUNDS) {
-        S.live[r] = H.log_m[i];
-        S.passes[r] = 0;
-        S.prefix_len[r] = H.log_h[i];
-        S.rounds = r + 1;
-      }
-      S.algorithmic_bytes += (uint64_t)H.log_m[i] * (H.log_kind[i] == 1u ? 32u : 24u);
-    }
-    nlog_seen = H.nlog;
-    first_chunk = false;
-    if (H.m == 0) { finished = true; break; }
-    out_enqueued = false;  // the speculative copies ran before the block was complete: repeat them at the end
-    if (lazy && !H.lists) {
-      // Out of lazy mode: more suffixes stayed in groups than the small list pool holds, or groups are large (a global
-      // radix round scans rank[] in text order and needs every rank).  Materialise the singletons' ranks from the sorted
-      // records of round 0 (still intact), then carry on with the full-rank path; nothing else has run in between.
-      RerankParams rp = ctx->rr0;
-      rp.lazy = 2u;
-      CK(ctx, cudaMemsetAsync(ctx->d_tstate(), 0, (size_t)rerank_launches(ctx, N, N) * ctx->max_aux_tiles * 8, st));
-      CK(ctx, cudaMemsetAsync(ctx->d_ctrl() + CTR_PASS0, 0, (size_t)(CTR_WORDS - CTR_PASS0) * 4, st));  // tile tickets
-      uint32_t* snr = reinterpret_cast<uint32_t*>(ctx->d_keys[cur ^ 1]);
-      lazy = false;  // (sel_of and the pools below now mean the full-rank layout)
-      if (pl.keybytes == 4) rc = launch_rerank<uint32_t, true>(ctx, cur, N, N, rp, ep, snr, snr + N, false, true);
-      else rc = launch_rerank<unsigned long long, true>(ctx, cur, N, N, rp, ep, snr, snr + N, false, true);
-      if (rc) return rc;
-      S.algorithmic_bytes += (uint64_t)N * (pl.keybytes + 4) + (uint64_t)N * 4;
-      S.flags |= 32u;  // lazy ranks were abandoned for this block
-      pool = norm;
-      lkp = nullptr;
-      lean = true;  // the lists (if the next step wants them) are built below from the intact staging
-      lists_pending = true;
-    }
-    if (lean) {
-      lean = false;
-      if (H.m <= (uint32_t)SMALL_MAX || (ctx->use_seg && H.maxgroup <= (uint32_t)SEG_MAXGROUP)) {
-        // the groups collapsed after all: build the lists now and run a normal ladder chunk
-        if (make_lists(false)) return BWTC_CUDA_ECUDA;
-        k_mark_lists<<<1, 1, 0, st>>>(ctx->d_state, sel_of(cur));
-        CK(ctx, cudaGetLastError());
-        S.kernel_launches++;
-        S.algorithmic_bytes += (uint64_t)H.m * 16;
-        lists_pending = false;
-        m_bound = H.m;
-        continue;
-      }
-    }
-    if (dbg && S.rounds >= dbg) break;
-    const uint32_t m = H.m;
-    m_bound = m;
-    if (S.rounds >= BWTC_CUDA_MAX_ROUNDS - 1 || (uint64_t)H.h >= 2ull * N + 2) {
-      set_err(ctx->err, "prefix doubling did not converge (round %u, h %u, live %u)", S.rounds, H.h, m);
-      return BWTC_CUDA_EINTERNAL;
-    }
-    if (ctx->use_seg && H.lists && H.maxgroup <= (uint32_t)SEG_MAXGROUP) continue;  // more segmented rounds than were enqueued
-    if (m <= (uint32_t)SMALL_MAX && !dbg) {
-      set_err(ctx->err, "internal: tail kernel skipped %u live suffixes", m);
-      return BWTC_CUDA_EINTERNAL;
-    }
-
-    // ---- global radix round (large groups: repetitive input), host-driven
-    const uint32_t r = S.rounds;
-    const uint32_t h32 = H.h;
-    const bool from_list = ((uint64_t)m * 8 <= (uint64_t)N);
-    const bool have_lists = H.lists != 0;
-    if (have_lists && H.sel != sel_of(cur)) {  // group sizes never grow, so a segmented round is never followed by a global sort
-      set_err(ctx->err, "internal: global sort requested after a segmented round (maxgroup %u)", H.maxgroup);
-      return BWTC_CUDA_EINTERNAL;
-    }
-    if (zero_round_state(ctx, N, m, RS_TILE64, maskd)) return BWTC_CUDA_ECUDA;
-    uint32_t expect_cursor = 0xFFFFFFFFu;
-    if (from_list) {
-      if (!have_lists) {
-        if (make_lists(false)) return BWTC_CUDA_ECUDA;
-        S.algorithmic_bytes += (uint64_t)m * 16;
-      }
-      // few live suffixes: gather-build from the id list (in d_keys[cur]) into the other buffer pair
-      const int tb = cur ^ 1;
-      const uint32_t bt = div_up(m, 256);
-      const int grid = (int)(bt < (uint32_t)(ctx->sm_count * 8) ? bt : (uint32_t)(ctx->sm_count * 8));
-      k_build_from_list<<<grid, 256, 0, st>>>(pool.p[2 * cur + 1], m, ctx->d_rank, N, h32, lo_bits,
-                                              static_cast<unsigned long long*>(ctx->d_keys[tb]), ctx->d_idx[tb],
-                                              ctx->d_hist(), (int)npassd, ctx->d_ctrl());
-      CK(ctx, cudaGetLastError());
-      S.kernel_launches++;
-      S.algorithmic_bytes += (uint64_t)m * (4 + 8 + 12);
-      cur = tb;
-    } else {
-      const uint32_t btiles = div_up(N, AUX_TILE);
-      const int grid = (int)(btiles < (uint32_t)(ctx->sm_count * 8) ? btiles : (uint32_t)(ctx->sm_count * 8));
-      k_build_keys<<<grid, 256, 0, st>>>(ctx->d_rank, N, h32, lo_bits, static_cast<unsigned long long*>(ctx->d_keys[0]),
-                                         ctx->d_idx[0], ctx->d_ctrl(), ctx->d_hist(), (int)npassd, btiles);
-      CK(ctx, cudaGetLastError());
-      S.kernel_launches++;
-      S.algorithmic_bytes += (uint64_t)N * 4 + (uint64_t)m * 12;
-      cur = 0;
-      expect_cursor = m;
-    }
-    rc = run_sort<unsigned long long, RS_IPT64>(ctx, m, maskd, false, 0, &cur, &pt, &pdone);
-    if (rc) return rc;
-    {
-      RerankParams rp;
-      rp.m = m;
-      rp.short_thresh = 0;
-      rp.lo_bits = lo_bits;
-      rp.packed = 0;
-      rp.pred_aux = nullptr;
-      rp.id_bits = 31;
-      rp.id_mask = 0xFFFFFFFFu;
-      rc = launch_rerank<unsigned long long, false>(ctx, cur, m, N, rp, ep, pool.p[2 * (cur ^ 1)], pool.p[2 * (cur ^ 1) + 1]);
-      if (rc) return rc;
-      S.algorithmic_bytes += (uint64_t)m * 12 + (uint64_t)m * 4;
-    }
-    h_next = std::min<uint64_t>((uint64_t)h32 * 2, 0x7FFFFFFFull);
-    lean = !dbg && H.maxgroup > LEAN_MAXGROUP;  // (group sizes before this round; they rarely drop 8x in one)
-    k_commit_sort<<<1, 1, 0, st>>>(ctx->d_state, ctx->d_ctrl(), (uint32_t)h_next, sel_of(cur), expect_cursor, lean ? 0u : 1u,
-                                   0xFFFFFFFFu);
-    CK(ctx, cudaGetLastError());
-    S.kernel_launches++;
-    if (r < BWTC_CUDA_MAX_ROUNDS) {
-      S.live[r] = m;
-      S.passes[r] = pdone;
-      S.prefix_len[r] = h32;
-      S.rounds = r + 1;
-    }
-    m_prev = m;
-    ctx->last_cur = cur;
-    lists_pending = true;
+  const bool from_list = ((uint64_t)m * 8 <= (uint64_t)N);
+  const bool have_lists = H.lists != 0;
+  if (have_lists && H.sel != s.sel(s.cur)) {  // group sizes never grow, so a segmented round is never followed by a global sort
+    set_err(ctx->err, "internal: global sort requested after a segmented round (maxgroup %u)", H.maxgroup);
+    return BWTC_CUDA_EINTERNAL;
   }
+  if (zero_round_state(ctx, N, m, RS_TILE64, maskd)) return BWTC_CUDA_ECUDA;
+  uint32_t expect_cursor = 0xFFFFFFFFu;
+  if (from_list) {
+    if (!have_lists) {
+      if (make_lists(ctx, s, false)) return BWTC_CUDA_ECUDA;
+      S.algorithmic_bytes += (uint64_t)m * 16;
+    }
+    // few live suffixes: gather-build from the id list (in d_keys[cur]) into the other buffer pair
+    const int tb = s.cur ^ 1;
+    const uint32_t bt = div_up(m, 256);
+    const int grid = (int)(bt < (uint32_t)(ctx->sm_count * 8) ? bt : (uint32_t)(ctx->sm_count * 8));
+    k_build_from_list<<<grid, 256, 0, st>>>(s.pool.p[2 * s.cur + 1], m, ctx->d_rank, N, h32, lo_bits,
+                                            static_cast<unsigned long long*>(ctx->d_keys[tb]), ctx->d_idx[tb],
+                                            ctx->d_hist(), (int)npassd, ctx->d_ctrl());
+    CK(ctx, cudaGetLastError());
+    S.kernel_launches++;
+    S.algorithmic_bytes += (uint64_t)m * (4 + 8 + 12);
+    s.cur = tb;
+  } else {
+    const uint32_t btiles = div_up(N, AUX_TILE);
+    const int grid = (int)(btiles < (uint32_t)(ctx->sm_count * 8) ? btiles : (uint32_t)(ctx->sm_count * 8));
+    k_build_keys<<<grid, 256, 0, st>>>(ctx->d_rank, N, h32, lo_bits, static_cast<unsigned long long*>(ctx->d_keys[0]),
+                                       ctx->d_idx[0], ctx->d_ctrl(), ctx->d_hist(), (int)npassd, btiles);
+    CK(ctx, cudaGetLastError());
+    S.kernel_launches++;
+    S.algorithmic_bytes += (uint64_t)N * 4 + (uint64_t)m * 12;
+    s.cur = 0;
+    expect_cursor = m;
+  }
+  if (const int rc = run_sort<unsigned long long, RS_IPT64>(ctx, m, maskd, false, 0, &s.cur, &s.pt, &s.pdone)) return rc;
+  {
+    RerankParams rp;
+    rp.m = m;
+    rp.short_thresh = 0;
+    rp.lo_bits = lo_bits;
+    rp.packed = 0;
+    rp.pred_aux = nullptr;
+    rp.id_bits = 31;
+    rp.id_mask = 0xFFFFFFFFu;
+    const int c = s.cur;
+    if (const int rc = launch_rerank<unsigned long long, false>(ctx, c, m, N, rp, J.ep, s.pool.p[2 * (c ^ 1)], s.pool.p[2 * (c ^ 1) + 1]))
+      return rc;
+    S.algorithmic_bytes += (uint64_t)m * 12 + (uint64_t)m * 4;
+  }
+  s.h_next = std::min<uint64_t>((uint64_t)h32 * 2, 0x7FFFFFFFull);
+  s.lean = !ctx->debug_max_rounds && H.maxgroup > LEAN_MAXGROUP;  // (group sizes before this round; they rarely drop 8x in one)
+  k_commit_sort<<<1, 1, 0, st>>>(ctx->d_state, ctx->d_ctrl(), (uint32_t)s.h_next, s.sel(s.cur), expect_cursor, s.lean ? 0u : 1u,
+                                 0xFFFFFFFFu);
+  CK(ctx, cudaGetLastError());
+  S.kernel_launches++;
+  log_round(S, m, s.pdone, h32);
+  s.m_prev = m;
+  ctx->last_cur = s.cur;
+  s.lists_pending = true;
+  return 0;
+}
 
-  // ---- run statistics first: the verification below reuses d_scat
-  if (finished && J.runs && !bs && J.block_mode) {
+// ---- delivery.  A finished job: run statistics (first: the verification reuses d_scat), verification, the LCP array from
+// the verified suffix array, the result copies that were not enqueued speculatively.  Then LFpowers and freqs
+// (incremented only now that the job has succeeded) and the times.  Returns LFpowers[0].
+int64_t deliver(bwtc_cuda_ctx* ctx, Job& J, const SortState& s, bool finished) {
+  cudaStream_t st = ctx->stream;
+  bwtc_cuda_stats& S = ctx->stats;
+  const uint32_t N = J.N, n = J.n;
+  if (finished && J.runs) {
     S.algorithmic_bytes += 2ull * n;  // the run kernels read the output twice, once per block whatever the chunk count
     const uint32_t cnt = ctx->h_state->nruns;
     if (cnt <= J.runs->capacity && cnt <= n && J.runs->symbol && J.runs->start) {
@@ -1367,61 +1340,108 @@ int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
       J.runs->count = BWTC_CUDA_RUNS_OVERFLOW;
     }
   }
-  if (finished && verify) {
-    rc = J.sa ? verify_sa(ctx, J) : verify_forward(ctx, J);
-    if (rc) return rc;
+  if (finished && s.verify) {
+    if (const int rc = J.sa ? verify_sa(ctx, J) : verify_forward(ctx, J)) return rc;
   }
-  // ---- the LCP array, from the (verified) suffix array
   if (finished && J.lcp) {
     if (enqueue_lcp(ctx, J)) return BWTC_CUDA_ECUDA;
     CK(ctx, cudaEventRecord(ctx->ev_end, st));
     if (!J.h_lcp && host_wait(ctx, st)) return BWTC_CUDA_ECUDA;  // (the host variant waits for its copies below)
   }
-  // ---- result copies that could not be enqueued speculatively
-  if (finished) {
-    if (J.sa) {
-      // the suffix array and the LCP array of the host variants: 4 bytes per suffix each
-      bool pending = false;
-      auto copy_host = [&](int32_t* h, const int32_t* d) -> int {
-        if (!h) return 0;
-        const Dst kind = dst_kind(h, false);
-        pending |= kind == Dst::pinned;
-        return copy_result(ctx, kind, h, d, (size_t)N * 4);
-      };
-      if (copy_host(J.h_sa, J.sa) || copy_host(J.h_lcp, J.lcp) || (pending && host_wait(ctx, st))) return BWTC_CUDA_ECUDA;
-    } else if (!out_enqueued) {
-      if (copy_out() || (direct_out && host_wait(ctx, st))) return BWTC_CUDA_ECUDA;
-    }
+  if (finished && J.sa) {
+    // the suffix array and the LCP array of the host variants: 4 bytes per suffix each
+    bool pending = false;
+    auto copy_host = [&](int32_t* h, const int32_t* d) -> int {
+      if (!h) return 0;
+      const Dst kind = dst_kind(h, false);
+      pending |= kind == Dst::pinned;
+      return copy_result(ctx, kind, h, d, (size_t)N * 4);
+    };
+    if (copy_host(J.h_sa, J.sa) || copy_host(J.h_lcp, J.lcp) || (pending && host_wait(ctx, st))) return BWTC_CUDA_ECUDA;
+  } else if (finished && !s.out_enqueued) {
+    if (copy_out(ctx, J, s.out_kind) || (s.direct_out && host_wait(ctx, st))) return BWTC_CUDA_ECUDA;
   }
-  // ---- results for the caller: LFpowers, freqs (incremented only now that the block has succeeded)
-  if (bs) {
-    const uint32_t* h_bhist = reinterpret_cast<const uint32_t*>(ctx->h_batch + MAX_BATCH * sizeof(void*));
-    for (uint32_t k = 0; k < bs->nblocks; ++k) {
-      const uint32_t nl = (k + 1 == bs->nblocks) ? bs->nLF_last : bs->nLF;
-      for (uint32_t j = 0; j < nl; ++j) J.LF[k * 256 + j] = h_bLF[k * 256 + j];
-      if (J.freqs)
-        for (int c = 0; c < 256; ++c) J.freqs[k * 256 + c] += h_bhist[k * 256 + c];
-    }
-  } else {
-    for (uint32_t j = 0; j < J.nLF; ++j) J.LF[j] = ctx->h_LF()[j];
+  const uint32_t* h_bhist = ctx->h_bhist();
+  const uint32_t* h_bLF = ctx->h_bLF();
+  for (uint32_t k = 0; k < J.nblocks; ++k) {
+    const uint32_t nl = (k + 1 == J.nblocks) ? J.nLF_last : J.nLF;
+    for (uint32_t j = 0; j < nl; ++j) J.LF[k * 256 + j] = h_bLF[k * 256 + j];
     if (J.freqs)
-      for (int c = 0; c < 256; ++c) J.freqs[c] += ctx->h_hist()[c];
+      for (int c = 0; c < 256; ++c) J.freqs[k * 256 + c] += h_bhist[k * 256 + c];
   }
   float ms = 0;
   CK(ctx, cudaEventElapsedTime(&ms, ctx->ev_begin, ctx->ev_end));
   S.gpu_ms = ms;
   if (ctx->timing_detail) {
     float tot = 0, tot0 = 0;
-    for (size_t i = 0; i + 1 < pt.used; i += 2) {
+    for (size_t i = 0; i + 1 < s.pt.used; i += 2) {
       float t = 0;
       CK(ctx, cudaEventElapsedTime(&t, ctx->ev_pool[i], ctx->ev_pool[i + 1]));
       tot += t;
-      if (i < round0_events) tot0 += t;
+      if (i < s.round0_events) tot0 += t;
     }
     S.sort_ms = tot;
     S.sort0_ms = tot0;
   }
   return (int64_t)J.LF[0];
+}
+
+// ---- phase B: round 0, the device-controlled ladder of sort-free rounds, host-driven global radix rounds where
+// groups are large, final extraction, result copies.  Works from ctx->d_text only, so it can be repeated (with ticket
+// tile ids) after a look-back watchdog without the caller's input.
+int64_t phase_sort(bwtc_cuda_ctx* ctx, Job& J) {
+  ctx->lb_watchdog = 0;
+  if (select_device(ctx)) return BWTC_CUDA_ECUDA;
+  cudaStream_t st = ctx->stream;
+  bwtc_cuda_stats& S = ctx->stats;
+  // a repeated phase B starts its statistics over (phase A's launches and bytes are kept)
+  S.kernel_launches = J.a_launches;
+  S.algorithmic_bytes = J.a_bytes;
+  S.sort_bytes = S.sort0_bytes = 0;
+  S.sort_launches = S.sort0_launches = 0;
+  S.rounds = 0;
+  CK(ctx, cudaMemsetAsync(ctx->d_zero, 0, (size_t)CTR_STICKY * 4, st));  // sticky control words (CTR_ERR)
+  CK(ctx, cudaMemsetAsync(ctx->d_state, 0, sizeof(LadderState), st));
+  CK(ctx, cudaMemsetAsync(ctx->d_LF + LF_PARK, 0, (size_t)(LF_WORDS - LF_PARK) * 4, st));  // parked hole bytes
+  SortState s(ctx, J);
+  int rc = J.pl.keybytes == 4 ? round0<uint32_t>(ctx, J, s) : round0<unsigned long long>(ctx, J, s);
+  if (rc) return rc;
+  const uint32_t dbg = ctx->debug_max_rounds;
+  bool finished = false;
+  for (;;) {
+    if ((rc = ladder_chunk(ctx, J, s)) || (rc = read_chunk(ctx, s))) return rc;
+    const LadderState& H = *ctx->h_state;
+    if (H.m == 0) { finished = true; break; }
+    s.out_enqueued = false;  // the speculative copies ran before the block was complete: repeat them at the end
+    if (s.lazy && !H.lists && (rc = leave_lazy(ctx, J, s))) return rc;
+    if (s.lean) {
+      s.lean = false;
+      if (H.m <= (uint32_t)SMALL_MAX || (ctx->use_seg && H.maxgroup <= (uint32_t)SEG_MAXGROUP)) {
+        // the groups collapsed after all: build the lists now and run a normal ladder chunk
+        if (make_lists(ctx, s, false)) return BWTC_CUDA_ECUDA;
+        k_mark_lists<<<1, 1, 0, st>>>(ctx->d_state, s.sel(s.cur));
+        CK(ctx, cudaGetLastError());
+        S.kernel_launches++;
+        S.algorithmic_bytes += (uint64_t)H.m * 16;
+        s.lists_pending = false;
+        s.m_bound = H.m;
+        continue;
+      }
+    }
+    if (dbg && S.rounds >= dbg) break;
+    s.m_bound = H.m;
+    if (S.rounds >= BWTC_CUDA_MAX_ROUNDS - 1 || (uint64_t)H.h >= 2ull * J.N + 2) {
+      set_err(ctx->err, "prefix doubling did not converge (round %u, h %u, live %u)", S.rounds, H.h, H.m);
+      return BWTC_CUDA_EINTERNAL;
+    }
+    if (ctx->use_seg && H.lists && H.maxgroup <= (uint32_t)SEG_MAXGROUP) continue;  // more segmented rounds than were enqueued
+    if (H.m <= (uint32_t)SMALL_MAX && !dbg) {
+      set_err(ctx->err, "internal: tail kernel skipped %u live suffixes", H.m);
+      return BWTC_CUDA_EINTERNAL;
+    }
+    if ((rc = global_round(ctx, J, s))) return rc;
+  }
+  return deliver(ctx, J, s, finished);
 }
 
 // Phase A, phase B, and the fallback of the static tile ids (see k_radix_pass): if the look-back watchdog fired, the
@@ -1615,19 +1635,17 @@ int run_inverse(bwtc_cuda_ctx* ctx, bool block_mode, const void* const* in, void
 int verify_forward(bwtc_cuda_ctx* ctx, const Job& J) {
   cudaStream_t st = ctx->stream;
   bwtc_cuda_stats& S = ctx->stats;
-  const BatchSpec* bs = J.bs;
-  InvShape sh;
-  sh.nblocks = bs ? bs->nblocks : 1u;
-  sh.n0 = bs ? bs->n0 : J.n;
-  sh.istride = bs ? J.bstride : J.n;
-  sh.R = bs ? J.bstride : J.N;
-  sh.N_last = bs ? bs->n_last + 1u : J.N;
+  InvShape sh;  // (a raw text is one block of n0 = N rows)
+  sh.nblocks = J.nblocks;
+  sh.n0 = J.n0;
+  sh.istride = sh.R = J.n0 + (J.block_mode ? 1u : 0u);
+  sh.N_last = J.n_last + (J.block_mode ? 1u : 0u);
   sh.S0 = div_up(sh.R, INV_K);
   sh.S_last = div_up(sh.N_last, INV_K);
   sh.d_eob = ctx->d_LF;
   sh.eot[0] = J.block_mode ? 0 : J.last;
   sh.nLF = J.nLF;
-  sh.nLF_last = bs ? bs->nLF_last : J.nLF;
+  sh.nLF_last = J.nLF_last;
   if (ctx->debug_corrupt_out) {
     if (J.block_mode) k_debug_flip_byte<<<1, 1, 0, st>>>(J.d_dst + sh.n0 / 2);
     else k_debug_flip_raw<<<1, 1, 0, st>>>(J.d_dst, J.N / 2, J.N, ctx->d_LF);
@@ -1643,8 +1661,8 @@ int verify_forward(bwtc_cuda_ctx* ctx, const Job& J) {
   if (const int rc = invert(ctx, sh, J.block_mode, J.d_dst, ctx->d_aux[1], &J, nullptr, &mask)) return rc;
   S.flags |= 64u;
   if (!mask) return 0;
-  if (!bs && J.block_mode && J.out_dev && J.out_dev == J.in_dev) {
-    k_text_unreverse<<<ctx->sm_count * 4, 256, 0, st>>>(J.d_text, J.n, J.out_dev);
+  if (!J.batch() && J.block_mode && J.on_device && J.out[0] == J.in[0]) {
+    k_text_unreverse<<<ctx->sm_count * 4, 256, 0, st>>>(J.d_text, J.n, static_cast<uint8_t*>(J.out[0]));
     CK(ctx, cudaGetLastError());
     S.kernel_launches++;
     if (host_wait(ctx, st)) return BWTC_CUDA_ECUDA;
@@ -1744,14 +1762,11 @@ int enqueue_lcp(bwtc_cuda_ctx* ctx, const Job& J) {
 // (bwtc_cuda_divsufsort_lcp): the LCP array is built into d_lcp behind it, h_lcp receives a copy.
 int run_divsufsort(bwtc_cuda_ctx* ctx, const uint8_t* h_T, const uint8_t* d_T, int32_t* h_SA, int32_t* d_SA, uint32_t n,
                    int32_t* h_LCP = nullptr, int32_t* d_LCP = nullptr) {
-  uint32_t pidx = 0;
-  Job J;
+  uint32_t pidx = 0, one = 1;
+  const void* in = d_T ? d_T : h_T;
+  void* out = nullptr;
+  Job J = forward_job(&in, &out, d_T != nullptr, &n, 1, &pidx, &one, nullptr);
   J.block_mode = false;
-  J.h_in = h_T;
-  J.in_dev = d_T;
-  J.n = n;
-  J.LF = &pidx;
-  J.nLF = 1;
   J.sa = d_SA;
   J.h_sa = h_SA;
   J.lcp = d_LCP;
@@ -1783,19 +1798,7 @@ int transform_batch(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out,
     nLF[k] = bwtc_cuda_num_starting_points(sizes[k], starts);
   }
   if (batchable(ctx, sizes, count)) {
-    BatchSpec bs;
-    bs.nblocks = count;
-    bs.n0 = sizes[0];
-    bs.n_last = sizes[count - 1];
-    bs.in = in;
-    bs.out = out;
-    bs.on_device = on_device;
-    bs.LF = LF;
-    bs.nLF = nLF[0];
-    bs.nLF_last = nLF[count - 1];
-    bs.freqs = freqs;
-    Job J;
-    J.bs = &bs;
+    Job J = forward_job(in, out, on_device, sizes, count, LF, nLF, freqs);
     const int64_t rc = run_job(ctx, J);
     if (rc != BATCH_NEEDS_SINGLE) {
       ctx->stats.batch_blocks = count;  // the record describes the whole batch: count it once, not per block
@@ -1804,19 +1807,9 @@ int transform_batch(bwtc_cuda_ctx* ctx, const void* const* in, void* const* out,
     }
   }
   for (uint32_t k = 0; k < count; ++k) {
-    Job J;
-    if (on_device) {
-      J.in_dev = static_cast<const uint8_t*>(in[k]);
-      J.out_dev = static_cast<uint8_t*>(out[k]);
-    } else {
-      J.h_in = static_cast<const uint8_t*>(in[k]);
-      J.h_out = static_cast<uint8_t*>(out[k]);
-      J.runs = count == 1 ? runs : nullptr;
-    }
-    J.n = sizes[k];
-    J.LF = LF + (size_t)k * 256;
-    J.nLF = nLF[k];
-    J.freqs = freqs ? freqs + (size_t)k * 256 : nullptr;
+    Job J = forward_job(in + k, out + k, on_device, sizes + k, 1, LF + (size_t)k * 256, nLF + k,
+                        freqs ? freqs + (size_t)k * 256 : nullptr);
+    J.runs = count == 1 && !on_device ? runs : nullptr;
     const int64_t rc = run_job(ctx, J);
     ctx->stats.batch_blocks = 1;
     if (stats) stats[k] = ctx->stats;
@@ -2012,7 +2005,7 @@ int bwtc_cuda_ctx_create(bwtc_cuda_ctx** out, int device, uint32_t max_block_byt
     }
   }
   if (!rc) {
-    e = cudaMallocHost((void**)&c->h_small, (size_t)(CTR_WORDS + HIST_WORDS + 256 + 8) * 4);
+    e = cudaMallocHost((void**)&c->h_small, (size_t)(CTR_WORDS + 8) * 4);
     if (e == cudaSuccess) e = cudaMallocHost((void**)&c->h_batch, (size_t)MAX_BATCH * (sizeof(void*) + 2 * 256 * 4));
     if (e == cudaSuccess) e = cudaMallocHost((void**)&c->h_state, sizeof(LadderState));
     if (e == cudaSuccess) e = cudaMallocHost((void**)&c->h_lookup, sizeof(LookupParams));
@@ -2154,14 +2147,10 @@ int64_t bwtc_cuda_divbwtf(bwtc_cuda_ctx* ctx, const uint8_t* T, uint8_t* U, uint
     if (n == 1) U[0] = T[0];
     return n;
   }
-  Job J;
+  const void* in = T;
+  void* out = U;
+  Job J = forward_job(&in, &out, false, &n, 1, LFpowers, &nLFpowers, freqs);
   J.block_mode = false;
-  J.h_in = T;
-  J.h_out = U;
-  J.n = n;
-  J.LF = LFpowers;
-  J.nLF = nLFpowers;
-  J.freqs = freqs;
   return run_job(ctx, J);
 }
 
@@ -2283,12 +2272,9 @@ int64_t bwtc_cuda_bwt_block_runs(bwtc_cuda_ctx* ctx, uint8_t* block, uint32_t n,
   if (runs) runs->count = BWTC_CUDA_RUNS_OVERFLOW;  // (every negative return leaves it so)
   if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
   if (!block || n == 0) { set_err(ctx->err, "null or empty block"); return BWTC_CUDA_EARG; }
-  Job J;
-  J.h_in = J.h_out = block;
-  J.n = n;
-  J.LF = LFpowers;
-  J.nLF = nLFpowers;
-  J.freqs = freqs;
+  const void* in = block;
+  void* out = block;
+  Job J = forward_job(&in, &out, false, &n, 1, LFpowers, &nLFpowers, freqs);
   J.runs = runs;
   return run_job(ctx, J);
 }
@@ -2313,13 +2299,7 @@ int64_t bwtc_cuda_bwt_block_device(bwtc_cuda_ctx* ctx, const void* d_in, void* d
                                    uint32_t nLFpowers, uint32_t* freqs) {
   if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
   if (!d_in || !d_out || n == 0) { set_err(ctx->err, "null or empty block"); return BWTC_CUDA_EARG; }
-  Job J;
-  J.in_dev = static_cast<const uint8_t*>(d_in);
-  J.out_dev = static_cast<uint8_t*>(d_out);
-  J.n = n;
-  J.LF = LFpowers;
-  J.nLF = nLFpowers;
-  J.freqs = freqs;
+  Job J = forward_job(&d_in, &d_out, true, &n, 1, LFpowers, &nLFpowers, freqs);
   return run_job(ctx, J);
 }
 

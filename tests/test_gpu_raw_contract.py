@@ -71,7 +71,7 @@ def raw_alphabet(T):
 
 
 def policy_flags(T, st, iid):
-    """stats flags 4 / 8 / 16 plan_round0 and phase_sort choose at default knobs: the predecessor code packed above the id
+    """stats flags 4 / 8 / 16 plan_round0, round0 and choose_lazy choose at default knobs: the predecessor code packed above the id
     when both fit 32 bits, else a one-byte payload from 96 Mi suffixes on; lazy ranks for an i.i.d. source (no memory)
     whose predicted live fraction after round 0, 1 - exp(-N 2^(-H0 c)), is at most 0.065, from 4 Mi suffixes on."""
     N = T.size

@@ -1,5 +1,5 @@
 """GPU tests of the run statistics (bwtc_cuda_bwt_block_runs, bwtc_cuda_pipeline_submit_runs; k_run_count / k_run_emit in
-ibwt_kernels.cuh, queued behind k_finish in every ladder chunk of phase_sort) at the edges where they can go wrong: the
+ibwt_kernels.cuh, queued behind k_finish in every ladder_chunk of phase_sort) at the edges where they can go wrong: the
 16-byte thread and 4096-byte tile boundaries of run_heads16 and its scalar tail, the sweeps of k_scan_tile_counts (16384
 tiles each, a carried prefix), the capacity contract, errors, every engine path, buffer kinds, the look-back status rows
 the tile counts borrow, and the pipeline's grouping rule that keeps a runs block out of a batch.

@@ -1,6 +1,6 @@
 """CPU check of the arithmetic behind the gram mode of round 0 (DESIGN.md §3.2, bwt_kernels.cuh GramParams): for 6-bit and
 3-bit codes every digit histogram of the round-0 radix sort is a projection of ONE histogram of the keys' low 12 bits,
-plus u head terms and minus u tail terms.  The (u, s) choice below is the one phase_sort makes (bwt_engine.cu, "Gram mode");
+plus u head terms and minus u tail terms.  The (u, s) choice below is the one plan_histograms makes (bwt_engine.cu, "Gram mode");
 the kernels themselves are checked bit-exactly on the GPU (tests/test_gpu_parity.py)."""
 import numpy as np
 import pytest
