@@ -35,6 +35,7 @@ FLAG_CORRUPT = 1 << 7             # stats flags bit 7: this inverse block is cor
 FLAG_SA = 1 << 8                  # stats flags bit 8: this call produced a suffix array (divsufsort)
 FLAG_LCP = 1 << 9                 # stats flags bit 9: this call produced an LCP array (divsufsort_lcp)
 FLAG_ROUND0_BUCKETS = 1 << 10     # stats flags bit 10: round 0 sorted its low key digits bucket by bucket (k_bucket_sort)
+FLAG_SEARCH = 1 << 11             # stats flags bit 11: this call was a pattern search (sa_search)
 
 
 class BwtcCudaUnavailable(RuntimeError):
@@ -126,6 +127,10 @@ C_ABI = [
     ("bwtc_cuda_sufcheck", ctypes.c_int, [_vp, _vp, _vp, ctypes.c_uint32]),
     ("bwtc_cuda_divsufsort_lcp", ctypes.c_int, [_vp, _vp, _vp, _vp, ctypes.c_uint32]),
     ("bwtc_cuda_divsufsort_lcp_device", ctypes.c_int, [_vp, _vp, _vp, _vp, ctypes.c_uint32]),
+    ("bwtc_cuda_sa_search", ctypes.c_int,
+     [_vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp, _vp, ctypes.c_uint32, _vp, _vp]),
+    ("bwtc_cuda_sa_search_device", ctypes.c_int,
+     [_vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp, _vp, ctypes.c_uint32, _vp, _vp]),
     ("bwtc_cuda_bwt_block", ctypes.c_int64, [_vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp]),
     ("bwtc_cuda_bwt_block_device", ctypes.c_int64, [_vp, _vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp]),
     ("bwtc_cuda_bwt_block_runs", ctypes.c_int64, [_vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp, _vp]),
@@ -183,6 +188,17 @@ def load_library(path: Optional[str] = None) -> ctypes.CDLL:
 
 def _ptr(a: Optional[np.ndarray]):
     return None if a is None else a.ctypes.data
+
+
+def pack_patterns(seq) -> Tuple[np.ndarray, np.ndarray]:
+    """Patterns (bytes, str as latin-1, or uint8 arrays) as the (P, P_off) pair sa_search takes: P = their bytes one
+    after the other (uint8), P_off = len(seq) + 1 offsets (uint64), pattern i = P[P_off[i]:P_off[i+1]]."""
+    parts = [np.frombuffer(p.encode("latin-1") if isinstance(p, str) else bytes(p), np.uint8) for p in seq]
+    P_off = np.zeros(len(parts) + 1, np.uint64)
+    if parts:
+        P_off[1:] = np.cumsum([p.size for p in parts], dtype=np.uint64)
+    P = np.concatenate(parts) if parts else np.zeros(0, np.uint8)
+    return np.ascontiguousarray(P, np.uint8), P_off
 
 
 def num_starting_points(block_bytes: int, starts: int) -> int:
@@ -298,6 +314,35 @@ class CudaContext:
             return False
         self._check(rc)
         return True
+
+    # pattern search in a suffix array: libdivsufsort's sa_search(T, Tsize, P, Psize, SA, SAsize, &idx), batched
+    def sa_search(self, T: np.ndarray, SA: np.ndarray, P: np.ndarray, P_off: np.ndarray,
+                  left: Optional[np.ndarray] = None, size: Optional[np.ndarray] = None) -> Tuple[np.ndarray, np.ndarray]:
+        """(left, size), int32[count] each (or written into left / size when given): pattern i = P[P_off[i]:P_off[i+1]]
+        (see pack_patterns) matches the rows SA[left[i] : left[i] + size[i]] of SA (int32, sorted suffixes of T, entries
+        outside [0, T.size) stand for the empty suffix); with no match, left[i] is where it would be inserted.  Host arrays,
+        pageable or pinned.  Raises BwtcCudaError on failure (decreasing offsets: EARG, left / size untouched)."""
+        assert T.dtype == np.uint8 and SA.dtype == np.int32 and P.dtype == np.uint8 and P_off.dtype == np.uint64
+        for a in (T, SA, P, P_off):
+            assert a.flags.c_contiguous
+        count = P_off.size - 1
+        assert count >= 0
+        if left is None:
+            left = np.empty(count, np.int32)
+        if size is None:
+            size = np.empty(count, np.int32)
+        for a in (left, size):
+            assert a.dtype == np.int32 and a.size >= count and a.flags.c_contiguous
+        self._check(self._lib.bwtc_cuda_sa_search(self._h, T.ctypes.data, T.size, SA.ctypes.data, SA.size, P.ctypes.data,
+                                                  P_off.ctypes.data, count, left.ctypes.data, size.ctypes.data))
+        return left, size
+
+    def sa_search_device(self, d_T: int, n: int, d_SA: int, SAsize: int, d_P: int, d_P_off: int, count: int,
+                         d_left: int, d_size: int) -> None:
+        """sa_search with every array in device memory (e.g. torch data_ptr()): T (n bytes) and P at any alignment, SA,
+        left and size (int32) 4-byte aligned, P_off (count + 1 uint64) 8-byte aligned."""
+        self._check(self._lib.bwtc_cuda_sa_search_device(self._h, d_T, n, d_SA, SAsize, d_P, d_P_off, count, d_left,
+                                                         d_size))
 
     # block contract: BWTransform::doTransform(BWTBlock&, freqs) — BWTransform.cpp:52-64
     def bwt_block(self, block: np.ndarray, LFpowers: np.ndarray, freqs: Optional[np.ndarray]) -> int:

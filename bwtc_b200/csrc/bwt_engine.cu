@@ -1775,6 +1775,54 @@ int run_divsufsort(bwtc_cuda_ctx* ctx, const uint8_t* h_T, const uint8_t* d_T, i
   return rc < 0 ? (int)rc : 0;
 }
 
+// ---- pattern search (bwtc_cuda_sa_search / _device, DESIGN.md §3.13; kernels k_sa_search_* in bwt_kernels.cuh).  No
+// look-back, tickets or watchdog: no kernel waits for another CTA.
+SearchCtl* search_ctl(bwtc_cuda_ctx* ctx) {  // behind the LCP stage's LcpCtl, so a search keeps debug_read(9) intact
+  return reinterpret_cast<SearchCtl*>(reinterpret_cast<uint8_t*>(ctx->d_wtab) + SEARCH_CTL_OFFSET);
+}
+const SearchCtl* search_ctl_host(const bwtc_cuda_ctx* ctx) { return reinterpret_cast<const SearchCtl*>(ctx->h_ctrl()); }
+
+// A search's record (flags bit 11) and its zeroed counters.
+int begin_search(bwtc_cuda_ctx* ctx, uint32_t n) {
+  if (select_device(ctx)) return BWTC_CUDA_ECUDA;
+  memset(&ctx->stats, 0, sizeof(ctx->stats));
+  ctx->stats.n_suffixes = n;
+  ctx->stats.flags = 2048u;
+  CK(ctx, cudaMemsetAsync(search_ctl(ctx), 0, sizeof(SearchCtl), ctx->stream));
+  return 0;
+}
+
+// One launch pair over the a.count patterns of a host chunk or of a whole device batch, between ev_begin and ev_end.
+// Nothing is waited for.
+int enqueue_search(bwtc_cuda_ctx* ctx, const SearchArgs& a) {
+  cudaStream_t st = ctx->stream;
+  CK(ctx, cudaMemsetAsync(&a.ctl->long_count, 0, 4, st));
+  CK(ctx, cudaEventRecord(ctx->ev_begin, st));
+  const uint32_t grid = std::max<uint32_t>(1u, std::min<uint32_t>(div_up(a.count, 256), (uint32_t)ctx->sm_count * 64u));
+  k_sa_search_short<<<grid, 256, 0, st>>>(a);
+  k_sa_search_long<<<(uint32_t)ctx->sm_count * 8u, 256, 0, st>>>(a);
+  CK(ctx, cudaGetLastError());
+  CK(ctx, cudaEventRecord(ctx->ev_end, st));
+  ctx->stats.kernel_launches += 2;
+  // offsets and results; the pattern bytes are counted on the device, the bytes the probes read depend on the data
+  ctx->stats.algorithmic_bytes += ((uint64_t)a.count + 1) * 8 + (uint64_t)a.count * 8;
+  return 0;
+}
+
+// Adds the device time of the last launch pair to the record; ev_end must be complete.
+int add_search_time(bwtc_cuda_ctx* ctx) {
+  float ms = 0;
+  CK(ctx, cudaEventElapsedTime(&ms, ctx->ev_begin, ctx->ev_end));
+  ctx->stats.gpu_ms += ms;
+  return 0;
+}
+
+// The call's counters into h_ctrl (enqueued; search_ctl_host reads them after the host wait).
+int read_search_ctl(bwtc_cuda_ctx* ctx) {
+  CK(ctx, cudaMemcpyAsync(ctx->h_ctrl(), search_ctl(ctx), sizeof(SearchCtl), cudaMemcpyDeviceToHost, ctx->stream));
+  return 0;
+}
+
 // count blocks (block contract) through one context: as ONE batch when they qualify — 2..MAX_BATCH blocks, all of
 // sizes[0] bytes except the last which may be shorter, together within the context's capacity, and at least one byte
 // value unused (the batch reserves a code for its sentinels) — otherwise one after the other.  Results are
@@ -2125,6 +2173,7 @@ int bwtc_cuda_debug_read(bwtc_cuda_ctx* ctx, int which, uint64_t offset_bytes, v
     case 6: src = reinterpret_cast<const uint8_t*>(ctx->d_zero); break;
     case 7: src = ctx->d_in; break;
     case 9: src = reinterpret_cast<const uint8_t*>(ctx->d_wtab); break;  // LcpCtl of the last bwtc_cuda_divsufsort_lcp
+    case 10: src = reinterpret_cast<const uint8_t*>(search_ctl(ctx)); break;  // SearchCtl of the last bwtc_cuda_sa_search
 #ifdef BWTC_PROFILE_STAGES
     case 8: {
       unsigned long long* pbuf = nullptr;
@@ -2260,6 +2309,115 @@ int bwtc_cuda_sufcheck(bwtc_cuda_ctx* ctx, const uint8_t* T, const int32_t* SA, 
   CK(ctx, cudaEventElapsedTime(&ms, ctx->ev_begin, ctx->ev_end));
   S.gpu_ms = ms;
   return sufcheck_failed(ctx, n, "sufcheck") ? BWTC_CUDA_ECORRUPT : 0;
+}
+
+int bwtc_cuda_sa_search(bwtc_cuda_ctx* ctx, const uint8_t* T, uint32_t n, const int32_t* SA, uint32_t SAsize,
+                        const uint8_t* P, const uint64_t* P_off, uint32_t count, int32_t* left, int32_t* size) {
+  if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
+  ctx->err[0] = 0;
+  if (!T || !SA || !P || !P_off || !left || !size) { set_err(ctx->err, "null T, SA, P, P_off, left or size"); return BWTC_CUDA_EARG; }
+  if ((uint64_t)SAsize > (uint64_t)n + 1) { set_err(ctx->err, "SAsize %u exceeds n + 1 = %llu", SAsize, (unsigned long long)n + 1); return BWTC_CUDA_EARG; }
+  if (const int rc = check_capacity(ctx, n, false)) return rc;
+  if (count == 0) return 0;
+  for (uint32_t i = 0; i < count; ++i)
+    if (P_off[i + 1] < P_off[i]) {
+      set_err(ctx->err, "pattern %u of %u: P_off[%u] < P_off[%u] (offsets decrease)", i, count, i + 1, i);
+      return BWTC_CUDA_EARG;
+    }
+  if (begin_search(ctx, n)) return BWTC_CUDA_ECUDA;
+  // T in d_in and SA in d_keys[1], as for sufcheck.  A chunk of whole patterns: its pattern bytes (each cut at n + 1) in
+  // the lower half of d_keys[0], its offsets (from 0) in the upper half, its results in d_idx[0] / d_idx[1].
+  const uint64_t N = (uint64_t)ctx->cap + 1, n1 = (uint64_t)n + 1;
+  uint8_t* d_pat = static_cast<uint8_t*>(ctx->d_keys[0]);
+  const uint64_t pat_cap = (4 * N + 7) & ~7ull;  // >= n + 1: every cut pattern fits
+  const uint32_t cmax = (uint32_t)std::min<uint64_t>(N, (8 * N + 64 - pat_cap) / 8 - 1);
+  const int32_t* d_SA = static_cast<const int32_t*>(ctx->d_keys[1]);
+  SearchArgs a{ctx->d_in, n, d_SA, SAsize, d_pat, reinterpret_cast<const uint64_t*>(d_pat + pat_cap), 0,
+               reinterpret_cast<int32_t*>(ctx->d_idx[0]), reinterpret_cast<int32_t*>(ctx->d_idx[1]), search_ctl(ctx)};
+  if (upload(ctx, ctx->d_in, T, n)) return BWTC_CUDA_ECUDA;
+  if (upload(ctx, reinterpret_cast<uint8_t*>(ctx->d_keys[1]), reinterpret_cast<const uint8_t*>(SA), (size_t)SAsize * 4)) return BWTC_CUDA_ECUDA;
+  std::vector<uint64_t> off;
+  std::vector<int32_t> h_left, h_size;  // a batch of several chunks: its results until the last chunk is done
+  for (uint32_t first = 0, last = 0; first < count; first = last) {
+    off.assign(1, 0);
+    for (last = first; last < count && last - first < cmax; ++last) {
+      const uint64_t end = off.back() + std::min(P_off[last + 1] - P_off[last], n1);
+      if (end > pat_cap) break;
+      off.push_back(end);
+    }
+    for (uint32_t i = first; i < last;) {  // one upload per run of patterns that were not cut (contiguous in P)
+      uint64_t len = 0;
+      bool cut = false;
+      uint32_t j = i;
+      while (j < last && !cut) {
+        const uint64_t full = P_off[j + 1] - P_off[j];
+        len += std::min(full, n1);
+        cut = full > n1;
+        ++j;
+      }
+      if (upload(ctx, d_pat + off[i - first], P + P_off[i], len)) return BWTC_CUDA_ECUDA;
+      i = j;
+    }
+    if (upload(ctx, d_pat + pat_cap, reinterpret_cast<const uint8_t*>(off.data()), off.size() * 8)) return BWTC_CUDA_ECUDA;
+    a.count = last - first;
+    if (enqueue_search(ctx, a)) return BWTC_CUDA_ECUDA;
+    if (first == 0 && last == count) {  // one chunk: straight to the caller's buffers
+      if (read_search_ctl(ctx) || copy_result(ctx, dst_kind(left, false), left, a.left, (size_t)count * 4) ||
+          copy_result(ctx, dst_kind(size, false), size, a.size, (size_t)count * 4) || host_wait(ctx, ctx->stream))
+        return BWTC_CUDA_ECUDA;
+    } else {  // (the staged copies return when the results are on the host, so the next chunk may reuse the scratch)
+      if (h_left.empty()) {
+        h_left.resize(count);
+        h_size.resize(count);
+      }
+      if (download_staged(ctx, reinterpret_cast<uint8_t*>(h_left.data() + first), reinterpret_cast<const uint8_t*>(a.left), (size_t)a.count * 4) ||
+          download_staged(ctx, reinterpret_cast<uint8_t*>(h_size.data() + first), reinterpret_cast<const uint8_t*>(a.size), (size_t)a.count * 4))
+        return BWTC_CUDA_ECUDA;
+      CK(ctx, cudaEventSynchronize(ctx->ev_end));
+    }
+    if (add_search_time(ctx)) return BWTC_CUDA_ECUDA;
+  }
+  if (!h_left.empty()) {
+    if (read_search_ctl(ctx) || host_wait(ctx, ctx->stream)) return BWTC_CUDA_ECUDA;
+    memcpy(left, h_left.data(), (size_t)count * 4);
+    memcpy(size, h_size.data(), (size_t)count * 4);
+  }
+  ctx->stats.algorithmic_bytes += search_ctl_host(ctx)->pattern_bytes;
+  return 0;
+}
+
+int bwtc_cuda_sa_search_device(bwtc_cuda_ctx* ctx, const void* d_T, uint32_t n, const void* d_SA, uint32_t SAsize,
+                               const void* d_P, const void* d_P_off, uint32_t count, void* d_left, void* d_size) {
+  if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
+  ctx->err[0] = 0;
+  if (!d_T || !d_SA || !d_P || !d_P_off || !d_left || !d_size) {
+    set_err(ctx->err, "null d_T, d_SA, d_P, d_P_off, d_left or d_size");
+    return BWTC_CUDA_EARG;
+  }
+  if (((reinterpret_cast<uintptr_t>(d_SA) | reinterpret_cast<uintptr_t>(d_left) | reinterpret_cast<uintptr_t>(d_size)) & 3u) ||
+      (reinterpret_cast<uintptr_t>(d_P_off) & 7u)) {
+    set_err(ctx->err, "d_SA, d_left and d_size must be 4-byte aligned and d_P_off 8-byte aligned");
+    return BWTC_CUDA_EARG;
+  }
+  if ((uint64_t)SAsize > (uint64_t)n + 1) { set_err(ctx->err, "SAsize %u exceeds n + 1 = %llu", SAsize, (unsigned long long)n + 1); return BWTC_CUDA_EARG; }
+  if ((uint64_t)n > (uint64_t)BWTC_CUDA_MAX_BLOCK + 1) {  // (keeps SAsize <= n + 1 within int32)
+    set_err(ctx->err, "text of %u bytes exceeds the engine limit of %u", n, BWTC_CUDA_MAX_BLOCK + 1);
+    return BWTC_CUDA_ETOOBIG;
+  }
+  if (count == 0) return 0;
+  if (begin_search(ctx, n)) return BWTC_CUDA_ECUDA;
+  const SearchArgs a{static_cast<const uint8_t*>(d_T), n, static_cast<const int32_t*>(d_SA), SAsize,
+                     static_cast<const uint8_t*>(d_P), static_cast<const uint64_t*>(d_P_off), count,
+                     static_cast<int32_t*>(d_left), static_cast<int32_t*>(d_size), search_ctl(ctx)};
+  if (enqueue_search(ctx, a) || read_search_ctl(ctx) || host_wait(ctx, ctx->stream) || add_search_time(ctx)) return BWTC_CUDA_ECUDA;
+  const SearchCtl* c = search_ctl_host(ctx);
+  ctx->stats.algorithmic_bytes += c->pattern_bytes;
+  if (c->bad) {
+    const uint32_t i = ~c->bad;
+    set_err(ctx->err, "pattern %u of %u: P_off[%u] < P_off[%u] (offsets decrease)", i, count, i + 1, i);
+    return BWTC_CUDA_EARG;
+  }
+  return 0;
 }
 
 int64_t bwtc_cuda_bwt_block(bwtc_cuda_ctx* ctx, uint8_t* block, uint32_t n, uint32_t* LFpowers, uint32_t nLFpowers,

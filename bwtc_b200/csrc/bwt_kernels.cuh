@@ -2842,4 +2842,213 @@ __global__ void __launch_bounds__(256) k_lcp_gather(const int32_t* __restrict__ 
   for (uint32_t r = blockIdx.x * blockDim.x + threadIdx.x; r < n; r += stride) lcp[r] = (int32_t)plcp[(uint32_t)sa[r]];
 }
 
+// =====================================================================================================
+// Pattern search in a suffix array (bwtc_cuda_sa_search / _device, DESIGN.md §3.13): libdivsufsort's sa_search for a
+// batch of patterns.  Row r of SA stands for the suffix T[SA[r]..n); an entry >= n as uint32 (negative ones included) is
+// the empty suffix, which sorts below every non-empty pattern and reads no byte.  Pattern i (m bytes, cut at n + 1: a
+// longer pattern matches nothing and its first n + 1 bytes already decide where it goes) gets
+//   lower = the first row whose suffix does not sort below P (= the rows whose first m bytes sort below P), and
+//   upper = the first row after the rows that start with P; left = lower, size = upper - lower.
+// Two binary searches, the second only when row `lower` starts with P.  Each keeps the bytes that the rows at both ends
+// of its interval share with P (l, r) and starts a comparison at min(l, r): for a sorted SA every row in between shares
+// them (the match-length heuristic of libdivsufsort's sa_search).  Comparisons end where the pattern or the suffix ends:
+// lengths decide, never the zero bytes lcp_word reads past an end.  Two tiers, neither waits for another CTA:
+//   k_sa_search_short: one thread per pattern of at most SEARCH_SHORT_BYTES bytes (word compares, __ffs of the XOR); it
+//                      also writes the special cases, checks the offsets and counts the long patterns;
+//   k_sa_search_long : one warp per longer pattern, 128 bytes per step (a ballot finds the first mismatch), grid-stride
+//                      over all patterns; it returns at once when k_sa_search_short counted no long pattern.
+// An unsorted SA gives unspecified results, still within left in [-1, SAsize], size in [0, SAsize] and T[0, n).
+// =====================================================================================================
+constexpr uint32_t SEARCH_SHORT_BYTES = 32;  // patterns up to this many bytes: one thread each (LCP_SHORT_BYTES)
+constexpr uint32_t SEARCH_CTL_OFFSET = 256;  // SearchCtl's byte offset in the context's d_wtab, behind the LcpCtl
+static_assert(sizeof(LcpCtl) <= SEARCH_CTL_OFFSET, "the search counters must not overlap the LCP stage's");
+
+struct SearchCtl {                           // zeroed per call
+  unsigned long long probes;                 // SA rows compared with a pattern
+  unsigned long long bytes;                  // text bytes compared (up to and including the mismatch)
+  unsigned long long pattern_bytes;          // pattern bytes that take part (each pattern cut at n + 1 bytes)
+  uint32_t long_count;                       // long patterns of the current launch pair (zeroed before each pair)
+  uint32_t bad;                              // ~(first pattern i with P_off[i+1] < P_off[i]), 0 if none (atomicMax)
+};
+
+struct SearchArgs {
+  const uint8_t* t;                          // text, n bytes, any alignment
+  uint32_t n;
+  const int32_t* sa;                         // sa_size rows
+  uint32_t sa_size;
+  const uint8_t* p;                          // pattern bytes, any alignment
+  const uint64_t* p_off;                     // count + 1 offsets into p
+  uint32_t count;
+  int32_t* left;
+  int32_t* size;
+  SearchCtl* ctl;
+};
+
+// Bytes of pattern i that can affect its result and where they start.  Decreasing offsets give an empty pattern.
+__device__ __forceinline__ uint32_t search_len(const SearchArgs& a, uint32_t i, uint64_t& beg, bool& bad) {
+  beg = a.p_off[i];
+  const uint64_t end = a.p_off[i + 1u];
+  bad = end < beg;
+  return bad ? 0u : (uint32_t)min(end - beg, (uint64_t)a.n + 1u);
+}
+
+// Suffix T[s..n) against the pattern q[0..m) (m >= 1), from byte min(k0, its length) on.  Returns < 0, 0, > 0 as the
+// suffix sorts below P, starts with P, sorts above P (a suffix that ends first sorts below); `match` = the bytes they
+// share.  One thread.
+__device__ __forceinline__ int search_cmp_thread(const uint8_t* __restrict__ t, uint32_t n, uint32_t s,
+                                                 const uint8_t* __restrict__ q, uint32_t m, uint32_t k0, uint32_t& match,
+                                                 unsigned long long& bytes) {
+  if (s >= n) { match = 0; return -1; }
+  const uint32_t len = min(m, n - s);
+  const uint32_t k_start = min(k0, len);
+  for (uint32_t k = k_start; k < len; k += 4u) {
+    const uint32_t a = lcp_word(t, n, s + k), b = lcp_word(q, m, k), d = a ^ b;
+    if (d) {
+      const uint32_t sh = (uint32_t)(__ffs((int)d) - 1) & ~7u;
+      const uint32_t j = k + (sh >> 3);
+      if (j >= len) break;  // (a difference past the end of the suffix or of the pattern)
+      match = j;
+      bytes += j + 1u - k_start;
+      return ((a >> sh) & 0xFFu) < ((b >> sh) & 0xFFu) ? -1 : 1;
+    }
+  }
+  match = len;
+  bytes += len - k_start;
+  return len == m ? 0 : -1;
+}
+
+// The same comparison by a whole warp, 128 bytes per step; every lane returns the same values.
+__device__ __forceinline__ int search_cmp_warp(const uint8_t* __restrict__ t, uint32_t n, uint32_t s,
+                                               const uint8_t* __restrict__ q, uint32_t m, uint32_t k0, uint32_t& match,
+                                               unsigned long long& bytes) {
+  if (s >= n) { match = 0; return -1; }
+  const uint32_t lane = threadIdx.x & 31u;
+  const uint32_t len = min(m, n - s);
+  for (uint32_t o = min(k0, len); o < len; o += 128u) {
+    const uint32_t p = o + 4u * lane;
+    uint32_t mm = 0xFFFFFFFFu;
+    int c = 0;
+    if (p < len) {
+      const uint32_t a = lcp_word(t, n, s + p), b = lcp_word(q, m, p), d = a ^ b;
+      if (d) {
+        const uint32_t sh = (uint32_t)(__ffs((int)d) - 1) & ~7u;
+        if (p + (sh >> 3) < len) {
+          mm = p + (sh >> 3);
+          c = ((a >> sh) & 0xFFu) < ((b >> sh) & 0xFFu) ? -1 : 1;
+        }
+      }
+    }
+    const uint32_t hit = __ballot_sync(0xFFFFFFFFu, mm != 0xFFFFFFFFu);
+    if (hit) {
+      const int src = __ffs((int)hit) - 1;
+      match = __shfl_sync(0xFFFFFFFFu, mm, src);
+      bytes += match + 1u - o;
+      return __shfl_sync(0xFFFFFFFFu, c, src);
+    }
+    bytes += min(128u, len - o);
+  }
+  match = len;
+  return len == m ? 0 : -1;
+}
+
+// lower and upper of one pattern of m >= 1 bytes; cmp(s, k0, match) compares the suffix of row value s.  l / r: the bytes
+// that the rows at lo - 1 / hi share with P (0 for a row never compared).
+template <typename Cmp>
+__device__ __forceinline__ void search_bounds(const int32_t* __restrict__ sa, uint32_t sa_size, uint32_t m, Cmp cmp,
+                                              uint32_t& lower, uint32_t& upper, unsigned long long& probes) {
+  uint32_t lo = 0, hi = sa_size, l = 0, r = 0;
+  while (lo < hi) {
+    const uint32_t mid = lo + ((hi - lo) >> 1);
+    uint32_t mt;
+    const int c = cmp((uint32_t)sa[mid], min(l, r), mt);
+    ++probes;
+    if (c < 0) { lo = mid + 1u; l = mt; }
+    else { hi = mid; r = mt; }
+  }
+  lower = upper = lo;
+  if (r != m) return;  // row `lower` does not start with P (or does not exist): no match
+  lo = lower + 1u;
+  hi = sa_size;
+  l = m;
+  r = 0;
+  while (lo < hi) {
+    const uint32_t mid = lo + ((hi - lo) >> 1);
+    uint32_t mt;
+    const int c = cmp((uint32_t)sa[mid], min(l, r), mt);
+    ++probes;
+    if (c <= 0) { lo = mid + 1u; l = mt; }
+    else { hi = mid; r = mt; }
+  }
+  upper = lo;
+}
+
+// One thread per pattern: the special cases, the offsets check, the count of long patterns and the short tier.
+__global__ void __launch_bounds__(256) k_sa_search_short(SearchArgs a) {
+  unsigned long long probes = 0, bytes = 0, pbytes = 0, nlong = 0;
+  const uint32_t stride = gridDim.x * blockDim.x;
+  for (uint32_t base = blockIdx.x * blockDim.x; base < a.count; base += stride) {  // (warp-uniform trip count: lcp_count)
+    const uint32_t i = base + threadIdx.x;
+    if (i >= a.count) continue;
+    uint64_t beg;
+    bool bad;
+    const uint32_t m = search_len(a, i, beg, bad);
+    if (bad) atomicMax(&a.ctl->bad, ~i);
+    pbytes += m;
+    int32_t left, size;
+    if (a.n == 0u || a.sa_size == 0u) {
+      left = -1;
+      size = 0;
+    } else if (m == 0u) {
+      left = 0;
+      size = (int32_t)a.sa_size;
+    } else if (m > SEARCH_SHORT_BYTES) {
+      ++nlong;
+      continue;
+    } else {
+      const uint8_t* q = a.p + beg;
+      uint32_t lower, upper;
+      search_bounds(a.sa, a.sa_size, m,
+                    [&](uint32_t s, uint32_t k0, uint32_t& mt) { return search_cmp_thread(a.t, a.n, s, q, m, k0, mt, bytes); },
+                    lower, upper, probes);
+      left = (int32_t)lower;
+      size = (int32_t)(upper - lower);
+    }
+    a.left[i] = left;
+    a.size[i] = size;
+  }
+  __syncwarp();
+  lcp_count(&a.ctl->probes, probes);
+  lcp_count(&a.ctl->bytes, bytes);
+  lcp_count(&a.ctl->pattern_bytes, pbytes);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) nlong += __shfl_xor_sync(0xFFFFFFFFu, nlong, o);
+  if ((threadIdx.x & 31u) == 0u && nlong) atomicAdd(&a.ctl->long_count, (uint32_t)nlong);
+}
+
+// One warp per pattern of more than SEARCH_SHORT_BYTES bytes, grid-stride over all patterns.
+__global__ void __launch_bounds__(256) k_sa_search_long(SearchArgs a) {
+  if (*reinterpret_cast<volatile uint32_t*>(&a.ctl->long_count) == 0u) return;
+  unsigned long long probes = 0, bytes = 0;
+  const uint32_t nwarps = (gridDim.x * blockDim.x) >> 5;
+  for (uint32_t i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < a.count; i += nwarps) {
+    uint64_t beg;
+    bool bad;
+    const uint32_t m = search_len(a, i, beg, bad);
+    if (a.n == 0u || a.sa_size == 0u || m <= SEARCH_SHORT_BYTES) continue;
+    const uint8_t* q = a.p + beg;
+    uint32_t lower, upper;
+    search_bounds(a.sa, a.sa_size, m,
+                  [&](uint32_t s, uint32_t k0, uint32_t& mt) { return search_cmp_warp(a.t, a.n, s, q, m, k0, mt, bytes); },
+                  lower, upper, probes);
+    if ((threadIdx.x & 31u) == 0u) {
+      a.left[i] = (int32_t)lower;
+      a.size[i] = (int32_t)(upper - lower);
+    }
+  }
+  if ((threadIdx.x & 31u) == 0u) {
+    if (probes) atomicAdd(&a.ctl->probes, probes);
+    if (bytes) atomicAdd(&a.ctl->bytes, bytes);
+  }
+}
+
 }  // namespace bwtc_b200

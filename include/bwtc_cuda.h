@@ -15,6 +15,8 @@
  *                                              entry points above)
  *   bwtc_cuda_divsufsort_lcp / _device     <-  no counterpart in bwtc's divsufsort: the SA and its LCP array, in the
  *                                              convention of libsais's libsais_plcp / libsais_lcp
+ *   bwtc_cuda_sa_search / _device          <-  sa_search / sa_simplesearch                 (libdivsufsort's pattern
+ *                                              search in a suffix array, for a batch of patterns)
  *   bwtc_cuda_bwt_block                    <-  BWTransform::doTransform(BWTBlock&, uint32 freqs[256])
  *                                              bwtransforms/BWTransform.cpp:39-64 (reverse / sentinel /
  *                                              hole-fill fused on the device)
@@ -92,7 +94,8 @@ typedef struct bwtc_cuda_stats {
                               * inverse only, this block is corrupt (BWTC_CUDA_ECORRUPT); bit 8: this call produced a suffix
                               * array (bwtc_cuda_divsufsort, _device, and the _lcp variants); bit 9: this call produced an
                               * LCP array (bwtc_cuda_divsufsort_lcp, _lcp_device); bit 10: round 0 ran its digit passes over the
-                              * top key digits only and sorted the low digits bucket by bucket (k_bucket_sort, BWTC_ROUND0_TOP) */
+                              * top key digits only and sorted the low digits bucket by bucket (k_bucket_sort, BWTC_ROUND0_TOP);
+                              * bit 11: this call was a pattern search (bwtc_cuda_sa_search, _device; no other entry point sets it) */
   uint32_t batch_blocks;     /* blocks this record describes: 1, or the size of the batch that was sorted as one text (every
                               * block of the batch then carries the SAME record — count it once; flags bit 7 is the one field
                               * in which the records of one inverse batch may differ) */
@@ -138,7 +141,8 @@ int         bwtc_cuda_ctx_set_verify(bwtc_cuda_ctx* ctx, int on);
  * then deliberately incomplete); bwtc_cuda_debug_read copies an engine buffer to the host
  * (which: 0 text, 1 rank[], 2/3 sorted keys/ids of the last round, 4/5 the other sort buffer,
  * 6 control+histogram words, 7 staged input, 9 the work counters of the last LCP stage: irreducible rows, bytes
- * compared by the short tier and by the windows, window segments (4 x u64), then the pairs in each window's list, u32). */
+ * compared by the short tier and by the windows, window segments (4 x u64), then the pairs in each window's list, u32;
+ * 10 the work counters of the last pattern search: probes made and text bytes compared, 2 x u64). */
 int         bwtc_cuda_ctx_set_debug(bwtc_cuda_ctx* ctx, uint32_t max_rounds);
 int         bwtc_cuda_debug_read(bwtc_cuda_ctx* ctx, int which, uint64_t offset_bytes, void* dst, uint64_t bytes);
 
@@ -191,6 +195,37 @@ int bwtc_cuda_divsufsort_lcp_device(bwtc_cuda_ctx* ctx, const void* d_T, void* d
  * Unlike libdivsufsort's sequential sufcheck, which returns -2 / -3 / -4 for the three kinds of failure, one code is used:
  * those values are BWTC_CUDA_EALLOC / ECUDA / EINTERNAL here.  Runs in the context's scratch (stats: gpu_ms = the check). */
 int bwtc_cuda_sufcheck(bwtc_cuda_ctx* ctx, const uint8_t* T, const int32_t* SA, uint32_t n);
+/* sa_search(T, n, P, Psize, SA, SAsize, &idx) for a batch of count patterns: pattern i is P[P_off[i] .. P_off[i+1]) (m
+ * bytes; P_off holds count + 1 offsets).  Row r of SA stands for the suffix T[SA[r]..n); an entry outside [0, n) stands for
+ * the empty suffix, which sorts below every non-empty pattern and reads nothing (an SA with a sentinel row n).  Bytes
+ * compare as unsigned, and a suffix that ends before the pattern does sorts below it.  Results:
+ *   n == 0 or SAsize == 0: size[i] = 0, left[i] = -1;  otherwise m == 0: size[i] = SAsize, left[i] = 0;
+ *   otherwise size[i] = the rows whose suffix starts with the pattern, and left[i] = the first such row, or, when there
+ *   is none, the row where the pattern would be inserted (the rows whose first m bytes sort below it).
+ * The matches are SA[left .. left + size).  sa_simplesearch(T, n, SA, SAsize, c, &idx) is the search for the one-byte
+ * pattern {c}, so it has no entry point of its own.  The results are exact whenever SA lists suffixes in sorted order: the
+ * suffix array (from bwtc_cuda_divsufsort), with a sentinel row, or any sorted subsequence such as a sparse SA.  For an
+ * unsorted SA they are unspecified but within left in [-1, SAsize], size in [0, SAsize].  Only T[0, n), SA[0, SAsize) and
+ * the pattern bytes are read; only the first n + 1 bytes of a pattern can affect its result (a longer one has size 0).
+ * Returns 0 or a negative error: null pointers, SAsize > n + 1, or decreasing offsets (P_off[i+1] < P_off[i]; the message
+ * names the first such pattern) are BWTC_CUDA_EARG; count == 0 writes nothing.  Both variants wait for the search.
+ *   host: T, SA, P, P_off, left and size may each be pageable or pinned (pinned: copied directly, pageable: through the
+ *         staging ring).  n <= max_block_bytes + 1 (else BWTC_CUDA_ETOOBIG).  The offsets are checked before any work
+ *         (on an error left and size are untouched); left and size are written only after the whole search succeeded.
+ *         Runs in the context's scratch, in chunks of whole patterns (results do not depend on the chunking);
+ *         bwtc_cuda_scratch_bytes is unchanged.
+ *   _device: every array in device memory; d_SA, d_left and d_size 4-byte aligned, d_P_off 8-byte aligned (else
+ *         BWTC_CUDA_EARG), d_T and d_P at any alignment.  Needs no per-suffix scratch, so the context's capacity does not
+ *         limit it: n <= BWTC_CUDA_MAX_BLOCK + 1 (else BWTC_CUDA_ETOOBIG).  Decreasing offsets are found on the device;
+ *         d_left / d_size then hold unspecified values.
+ * stats: a new record with n_suffixes = n, gpu_ms = the search's device time (without uploads), kernel_launches,
+ * algorithmic_bytes = offsets, results and pattern bytes, flags bit 11.  Verification (bwtc_cuda_ctx_set_verify) does not
+ * apply: results are the same with it on and bit 6 stays clear (checking an SA is bwtc_cuda_sufcheck's job).
+ * bwtc_cuda_debug_read(ctx, 10, ...) returns the search's probe and byte counters.  DESIGN.md §3.13. */
+int bwtc_cuda_sa_search(bwtc_cuda_ctx* ctx, const uint8_t* T, uint32_t n, const int32_t* SA, uint32_t SAsize,
+                        const uint8_t* P, const uint64_t* P_off, uint32_t count, int32_t* left, int32_t* size);
+int bwtc_cuda_sa_search_device(bwtc_cuda_ctx* ctx, const void* d_T, uint32_t n, const void* d_SA, uint32_t SAsize,
+                               const void* d_P, const void* d_P_off, uint32_t count, void* d_left, void* d_size);
 
 /* ---- block contract: BWTransform::doTransform(BWTBlock&, freqs) (BWTransform.cpp:52-64) ---------- */
 /* block: n bytes (host), transformed IN PLACE; unlike the reference wrapper the byte after the block
