@@ -36,6 +36,7 @@ FLAG_SA = 1 << 8                  # stats flags bit 8: this call produced a suff
 FLAG_LCP = 1 << 9                 # stats flags bit 9: this call produced an LCP array (divsufsort_lcp)
 FLAG_ROUND0_BUCKETS = 1 << 10     # stats flags bit 10: round 0 sorted its low key digits bucket by bucket (k_bucket_sort)
 FLAG_SEARCH = 1 << 11             # stats flags bit 11: this call was a pattern search (sa_search)
+FLAG_LZ77 = 1 << 12               # stats flags bit 12: this call produced an LZ77 factorisation (lz77)
 
 
 class BwtcCudaUnavailable(RuntimeError):
@@ -131,6 +132,8 @@ C_ABI = [
      [_vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp, _vp, ctypes.c_uint32, _vp, _vp]),
     ("bwtc_cuda_sa_search_device", ctypes.c_int,
      [_vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp, _vp, ctypes.c_uint32, _vp, _vp]),
+    ("bwtc_cuda_lz77", ctypes.c_int64, [_vp, _vp, ctypes.c_uint32, _vp, _vp, ctypes.c_uint32]),
+    ("bwtc_cuda_lz77_device", ctypes.c_int64, [_vp, _vp, ctypes.c_uint32, _vp, _vp, ctypes.c_uint32]),
     ("bwtc_cuda_bwt_block", ctypes.c_int64, [_vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp]),
     ("bwtc_cuda_bwt_block_device", ctypes.c_int64, [_vp, _vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp]),
     ("bwtc_cuda_bwt_block_runs", ctypes.c_int64, [_vp, _vp, ctypes.c_uint32, _vp, ctypes.c_uint32, _vp, _vp]),
@@ -343,6 +346,34 @@ class CudaContext:
         left and size (int32) 4-byte aligned, P_off (count + 1 uint64) 8-byte aligned."""
         self._check(self._lib.bwtc_cuda_sa_search_device(self._h, d_T, n, d_SA, SAsize, d_P, d_P_off, count, d_left,
                                                          d_size))
+
+    # greedy LZ77 factorisation (self-reference allowed, KKP's source rule; include/bwtc_cuda.h)
+    def lz77(self, T: np.ndarray, src: Optional[np.ndarray] = None,
+             len: Optional[np.ndarray] = None) -> Tuple[np.ndarray, np.ndarray]:
+        """(src, len), int32[z] each: the greedy LZ77 phrases of T (uint8).  Phrase k is a literal when len[k] == 0 (src[k]
+        is the byte) and otherwise copies len[k] bytes from position src[k], before its start.  The call runs with capacity
+        min(src.size, len.size), T.size for fresh arrays (z <= T.size always, so no count query is needed), and returns
+        views of the first z entries.  Given arrays (int32, pageable or pinned) too small for z raise ValueError and stay
+        untouched.  Raises BwtcCudaError on failure (EVERIFY with verification on: src / len untouched)."""
+        assert T.dtype == np.uint8 and T.flags.c_contiguous
+        n = T.size
+        if src is None:
+            src = np.empty(n, np.int32)
+        if len is None:
+            len = np.empty(n, np.int32)
+        for a in (src, len):
+            assert a.dtype == np.int32 and a.flags.c_contiguous
+        cap = min(src.size, len.size)
+        z = self._check(self._lib.bwtc_cuda_lz77(self._h, T.ctypes.data, n, src.ctypes.data, len.ctypes.data, cap))
+        if z > cap:
+            raise ValueError(f"lz77: {z} phrases do not fit arrays of {cap} entries (src / len untouched)")
+        return src[:z], len[:z]
+
+    def lz77_device(self, d_T: int, n: int, d_src: int, d_len: int, capacity: int) -> int:
+        """lz77 with T (n bytes, any alignment) and the phrase arrays (capacity int32 each, 4-byte aligned, not
+        overlapping) in device memory (e.g. torch data_ptr()).  Returns z; the arrays are written only when z <= capacity
+        (capacity 0 with null arrays: a count query)."""
+        return self._check(self._lib.bwtc_cuda_lz77_device(self._h, d_T, n, d_src or None, d_len or None, capacity))
 
     # block contract: BWTransform::doTransform(BWTBlock&, freqs) — BWTransform.cpp:52-64
     def bwt_block(self, block: np.ndarray, LFpowers: np.ndarray, freqs: Optional[np.ndarray]) -> int:

@@ -533,6 +533,7 @@ struct Job {
   int32_t* h_sa = nullptr;         // ... and copied to this host array once the block is finished (and verified)
   int32_t* lcp = nullptr;          // bwtc_cuda_divsufsort_lcp: the LCP array is built here (device) behind the sort ...
   int32_t* h_lcp = nullptr;        // ... and copied to this host array
+  bool lz = false;                 // bwtc_cuda_lz77: the LZ77 stage runs behind the LCP stage (phrases left in scratch)
   // ---- phase A
   uint32_t n = 0, N = 0, bstride = 0, blk_bits = 0;  // n: result bytes of all blocks; bstride: n0 + 1 in a batch, else 0
   bool sentinel_outside_alphabet = false;
@@ -822,6 +823,7 @@ int64_t phase_input(bwtc_cuda_ctx* ctx, Job& J) {
 int verify_forward(bwtc_cuda_ctx* ctx, const Job& J);
 int verify_sa(bwtc_cuda_ctx* ctx, const Job& J);
 int enqueue_lcp(bwtc_cuda_ctx* ctx, const Job& J);
+int enqueue_lz(bwtc_cuda_ctx* ctx, const Job& J);
 
 // One attempt of phase B: the state its steps share.  A repeated phase B (after a look-back watchdog) starts from a
 // fresh one.
@@ -1322,8 +1324,8 @@ int global_round(bwtc_cuda_ctx* ctx, const Job& J, SortState& s) {
 }
 
 // ---- delivery.  A finished job: run statistics (first: the verification reuses d_scat), verification, the LCP array from
-// the verified suffix array, the result copies that were not enqueued speculatively.  Then LFpowers and freqs
-// (incremented only now that the job has succeeded) and the times.  Returns LFpowers[0].
+// the verified suffix array (then the LZ77 phrases from both), the result copies that were not enqueued speculatively.
+// Then LFpowers and freqs (incremented only now that the job has succeeded) and the times.  Returns LFpowers[0].
 int64_t deliver(bwtc_cuda_ctx* ctx, Job& J, const SortState& s, bool finished) {
   cudaStream_t st = ctx->stream;
   bwtc_cuda_stats& S = ctx->stats;
@@ -1344,7 +1346,7 @@ int64_t deliver(bwtc_cuda_ctx* ctx, Job& J, const SortState& s, bool finished) {
     if (const int rc = J.sa ? verify_sa(ctx, J) : verify_forward(ctx, J)) return rc;
   }
   if (finished && J.lcp) {
-    if (enqueue_lcp(ctx, J)) return BWTC_CUDA_ECUDA;
+    if (enqueue_lcp(ctx, J) || (J.lz && enqueue_lz(ctx, J))) return BWTC_CUDA_ECUDA;
     CK(ctx, cudaEventRecord(ctx->ev_end, st));
     if (!J.h_lcp && host_wait(ctx, st)) return BWTC_CUDA_ECUDA;  // (the host variant waits for its copies below)
   }
@@ -1758,6 +1760,22 @@ int enqueue_lcp(bwtc_cuda_ctx* ctx, const Job& J) {
   return 0;
 }
 
+// The device SA of the host divsufsort variants and of both lz77 variants: 4 (cap + 1) bytes, allocated by the first call
+// that needs it.
+int ensure_sa(bwtc_cuda_ctx* ctx) {
+  if (ctx->d_sa) return 0;
+  if (select_device(ctx)) return BWTC_CUDA_ECUDA;
+  const size_t bytes = ((size_t)ctx->cap + 1) * 4;
+  const cudaError_t e = cudaMalloc((void**)&ctx->d_sa, bytes);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    ctx->d_sa = nullptr;
+    set_err(ctx->err, "cudaMalloc(%zu bytes) for the suffix array: %s", bytes, cudaGetErrorString(e));
+    return BWTC_CUDA_EALLOC;
+  }
+  return 0;
+}
+
 // bwtc_cuda_divsufsort(_device): the raw transform with SA emission into d_sa; h_sa receives a copy.  With d_lcp
 // (bwtc_cuda_divsufsort_lcp): the LCP array is built into d_lcp behind it, h_lcp receives a copy.
 int run_divsufsort(bwtc_cuda_ctx* ctx, const uint8_t* h_T, const uint8_t* d_T, int32_t* h_SA, int32_t* d_SA, uint32_t n,
@@ -1773,6 +1791,92 @@ int run_divsufsort(bwtc_cuda_ctx* ctx, const uint8_t* h_T, const uint8_t* d_T, i
   J.h_lcp = h_LCP;
   const int64_t rc = run_job(ctx, J);
   return rc < 0 ? (int)rc : 0;
+}
+
+// ---- LZ77 factorisation (bwtc_cuda_lz77 / _device, DESIGN.md §3.14; kernels k_lz_* in bwt_kernels.cuh).  No look-back,
+// tickets or watchdog: no kernel waits for another CTA.
+LzCtl* lz_ctl(bwtc_cuda_ctx* ctx) {  // behind SearchCtl, so debug_read(9) and (10) stay intact
+  return reinterpret_cast<LzCtl*>(reinterpret_cast<uint8_t*>(ctx->d_wtab) + LZ_CTL_OFFSET);
+}
+const LzCtl* lz_ctl_host(const bwtc_cuda_ctx* ctx) { return reinterpret_cast<const LzCtl*>(ctx->h_ctrl()); }
+
+// The LZ77 stage, enqueued behind enqueue_lcp: J.sa and J.lcp (d_keys[0]) are complete.  Scratch, idle by then: LPF
+// (8 bytes per position) in d_keys[1]; the group minima and the tile tree of stage A, then the marks of stage B, in d_scat;
+// exit / jump arrays in d_idx[0] / d_idx[1], then the phrases' src / len; tile counts in d_tilecnt; LzCtl in d_wtab, read
+// back into h_ctrl.  Nothing is waited for.
+int enqueue_lz(bwtc_cuda_ctx* ctx, const Job& J) {
+  cudaStream_t st = ctx->stream;
+  bwtc_cuda_stats& S = ctx->stats;
+  const uint32_t n = J.N;
+  const uint32_t* ctrl = ctx->d_ctrl();
+  LzCtl* lc = lz_ctl(ctx);
+  uint2* lpf = static_cast<uint2*>(ctx->d_keys[1]);
+  const uint32_t ngroups = div_up(n, LZ_GROUP), rtiles = div_up(n, LZ_ROW_TILE), ttiles = div_up(n, LZ_TEXT_TILE);
+  const uint32_t L2 = 1u << ceil_log2_u64(rtiles);
+  uint2* grp = reinterpret_cast<uint2*>(ctx->d_scat);
+  uint2* top = grp + ngroups;  // 2 L2 nodes: (n / 4 + n / 64) bytes at most, within d_scat's 4 n
+  uint8_t* mark = reinterpret_cast<uint8_t*>(ctx->d_scat);
+  uint32_t* jump[2] = {ctx->d_idx[0], ctx->d_idx[1]};
+  CK(ctx, cudaMemsetAsync(lc, 0, sizeof(LzCtl), st));
+  k_lz_minima<<<rtiles, 256, 0, st>>>(J.sa, J.lcp, n, grp, top, L2, ctrl);
+  k_lz_tree<<<1, 1024, 0, st>>>(top, rtiles, L2, ctrl);
+  k_lz_lpf<<<rtiles, 256, 0, st>>>(J.d_text, J.sa, J.lcp, n, grp, top, L2, lpf, lc, ctrl);
+  k_lz_exit<<<ttiles, 256, 0, st>>>(lpf, n, jump[0], mark, ctrl);
+  const uint32_t rounds = ceil_log2_u64(ttiles);  // the path from 0 has at most one exit node per tile
+  const uint32_t grid = std::max<uint32_t>(1u, std::min<uint32_t>(div_up(n, 256), (uint32_t)ctx->sm_count * 8u));
+  for (uint32_t k = 0; k < rounds; ++k)
+    k_lz_round<<<grid, 256, 0, st>>>(jump[k & 1u], jump[(k & 1u) ^ 1u], n, mark, lc, k, k + 1u == rounds ? 1u : 0u, ctrl);
+  k_lz_mark_tile<<<ttiles, 256, 0, st>>>(lpf, n, mark, ctx->d_tilecnt, ctrl);
+  k_lz_scan<<<1, 1024, 0, st>>>(ctx->d_tilecnt, ttiles, lc, ctrl);
+  k_lz_emit<<<ttiles, 256, 0, st>>>(lpf, mark, n, ctx->d_tilecnt, reinterpret_cast<int32_t*>(jump[0]),
+                                    reinterpret_cast<int32_t*>(jump[1]), ctrl);
+  CK(ctx, cudaGetLastError());
+  CK(ctx, cudaMemcpyAsync(ctx->h_ctrl(), lc, sizeof(LzCtl), cudaMemcpyDeviceToHost, st));
+  S.kernel_launches += 7 + rounds;
+  // stage A: SA and LCP read twice, LPF scattered; stage B: LPF read twice, exit written, marks written, read and
+  // rewritten.  The marking rounds and the emitted phrases depend on the text (added after the wait, lz_account).
+  S.algorithmic_bytes += (uint64_t)n * (16 + 8) + (uint64_t)n * (16 + 4 + 1 + 2 + 1);
+  S.flags |= 4096u;
+  return 0;
+}
+
+// After the host wait: the bytes of the marking rounds that ran (mark, jump, jump of jump, next jump) and of the z phrases
+// emitted (LPF entry read, src and len written).
+void lz_account(bwtc_cuda_ctx* ctx, uint32_t n) {
+  const LzCtl* c = lz_ctl_host(ctx);
+  const uint32_t launched = ceil_log2_u64(div_up(n, LZ_TEXT_TILE));
+  const uint64_t ran = std::min<uint64_t>((uint64_t)c->rounds + 1u, launched);
+  ctx->stats.algorithmic_bytes += ran * (uint64_t)n * 13 + c->phrases * 16;
+}
+
+// bwtc_cuda_lz77(_device): sort, LCP and LZ77 stages in one job; the z phrases go to h_src / h_len (host) or d_src / d_len
+// (device) when z <= capacity.  Returns z or a negative error.
+int64_t run_lz77(bwtc_cuda_ctx* ctx, const uint8_t* h_T, const uint8_t* d_T, uint32_t n, int32_t* src, int32_t* len,
+                 uint32_t capacity) {
+  if (const int rc = ensure_sa(ctx)) return rc;
+  uint32_t pidx = 0, one = 1;
+  const void* in = d_T ? d_T : h_T;
+  void* out = nullptr;
+  Job J = forward_job(&in, &out, d_T != nullptr, &n, 1, &pidx, &one, nullptr);
+  J.block_mode = false;
+  J.sa = ctx->d_sa;
+  J.lcp = static_cast<int32_t*>(ctx->d_keys[0]);
+  J.lz = true;
+  const int64_t rc = run_job(ctx, J);
+  if (rc < 0) return rc;
+  if (!(ctx->stats.flags & 4096u)) {  // (a debug round limit stopped the sort before the stage)
+    set_err(ctx->err, "the LZ77 stage did not run: the sort was stopped early (bwtc_cuda_ctx_set_debug)");
+    return BWTC_CUDA_EINTERNAL;
+  }
+  lz_account(ctx, n);
+  const uint64_t z = lz_ctl_host(ctx)->phrases;
+  if (z > capacity) return (int64_t)z;
+  const Dst kind = dst_kind(src, d_T != nullptr);
+  const Dst kind_len = dst_kind(len, d_T != nullptr);
+  if (copy_result(ctx, kind, src, ctx->d_idx[0], (size_t)z * 4) || copy_result(ctx, kind_len, len, ctx->d_idx[1], (size_t)z * 4) ||
+      ((kind != Dst::pageable || kind_len != Dst::pageable) && host_wait(ctx, ctx->stream)))
+    return BWTC_CUDA_ECUDA;
+  return (int64_t)z;
 }
 
 // ---- pattern search (bwtc_cuda_sa_search / _device, DESIGN.md §3.13; kernels k_sa_search_* in bwt_kernels.cuh).  No
@@ -2174,6 +2278,7 @@ int bwtc_cuda_debug_read(bwtc_cuda_ctx* ctx, int which, uint64_t offset_bytes, v
     case 7: src = ctx->d_in; break;
     case 9: src = reinterpret_cast<const uint8_t*>(ctx->d_wtab); break;  // LcpCtl of the last bwtc_cuda_divsufsort_lcp
     case 10: src = reinterpret_cast<const uint8_t*>(search_ctl(ctx)); break;  // SearchCtl of the last bwtc_cuda_sa_search
+    case 11: src = reinterpret_cast<const uint8_t*>(lz_ctl(ctx)); break;  // LzCtl of the last bwtc_cuda_lz77
 #ifdef BWTC_PROFILE_STAGES
     case 8: {
       unsigned long long* pbuf = nullptr;
@@ -2206,21 +2311,6 @@ int64_t bwtc_cuda_divbwtf(bwtc_cuda_ctx* ctx, const uint8_t* T, uint8_t* U, uint
 int64_t bwtc_cuda_divbwt(bwtc_cuda_ctx* ctx, const uint8_t* T, uint8_t* U, uint32_t n, uint32_t* LFpowers,
                          uint32_t nLFpowers) {
   return bwtc_cuda_divbwtf(ctx, T, U, n, LFpowers, nLFpowers, nullptr);
-}
-
-// The host variants' device SA: 4 (cap + 1) bytes, allocated by the first call that needs it.
-static int ensure_sa(bwtc_cuda_ctx* ctx) {
-  if (ctx->d_sa) return 0;
-  if (select_device(ctx)) return BWTC_CUDA_ECUDA;
-  const size_t bytes = ((size_t)ctx->cap + 1) * 4;
-  const cudaError_t e = cudaMalloc((void**)&ctx->d_sa, bytes);
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    ctx->d_sa = nullptr;
-    set_err(ctx->err, "cudaMalloc(%zu bytes) for the suffix array: %s", bytes, cudaGetErrorString(e));
-    return BWTC_CUDA_EALLOC;
-  }
-  return 0;
 }
 
 int bwtc_cuda_divsufsort(bwtc_cuda_ctx* ctx, const uint8_t* T, int32_t* SA, uint32_t n) {
@@ -2280,6 +2370,54 @@ int bwtc_cuda_divsufsort_lcp_device(bwtc_cuda_ctx* ctx, const void* d_T, void* d
   }
   return run_divsufsort(ctx, nullptr, static_cast<const uint8_t*>(d_T), nullptr, static_cast<int32_t*>(d_SA), n, nullptr,
                         static_cast<int32_t*>(d_LCP));
+}
+
+int64_t bwtc_cuda_lz77(bwtc_cuda_ctx* ctx, const uint8_t* T, uint32_t n, int32_t* src, int32_t* len, uint32_t capacity) {
+  if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
+  ctx->err[0] = 0;
+  if (!T) { set_err(ctx->err, "null T"); return BWTC_CUDA_EARG; }
+  if (capacity && (!src || !len)) { set_err(ctx->err, "null src or len with capacity %u", capacity); return BWTC_CUDA_EARG; }
+  if (n == 0) return 0;
+  if (const int rc = check_capacity(ctx, n, false)) return rc;
+  if (n == 1) {
+    if (capacity) {
+      src[0] = T[0];
+      len[0] = 0;
+    }
+    return 1;
+  }
+  return run_lz77(ctx, T, nullptr, n, src, len, capacity);
+}
+
+int64_t bwtc_cuda_lz77_device(bwtc_cuda_ctx* ctx, const void* d_T, uint32_t n, void* d_src, void* d_len, uint32_t capacity) {
+  if (!ctx) { set_err(g_err, "null context"); return BWTC_CUDA_EARG; }
+  ctx->err[0] = 0;
+  if (!d_T) { set_err(ctx->err, "null d_T"); return BWTC_CUDA_EARG; }
+  if (capacity) {
+    const uintptr_t a = reinterpret_cast<uintptr_t>(d_src), b = reinterpret_cast<uintptr_t>(d_len);
+    if (!d_src || !d_len || ((a | b) & 3u)) {
+      set_err(ctx->err, "null d_src / d_len, or d_src / d_len not 4-byte aligned");
+      return BWTC_CUDA_EARG;
+    }
+    if (a < b + (uint64_t)capacity * 4 && b < a + (uint64_t)capacity * 4) {
+      set_err(ctx->err, "d_src and d_len overlap within %u entries", capacity);
+      return BWTC_CUDA_EARG;
+    }
+  }
+  if (n == 0) return 0;
+  if (const int rc = check_capacity(ctx, n, false)) return rc;
+  if (n == 1) {
+    if (capacity) {  // src[0] = T[0] as an int32 (little-endian: the byte, then three zero bytes), len[0] = 0
+      if (select_device(ctx)) return BWTC_CUDA_ECUDA;
+      CK(ctx, cudaMemsetAsync(d_src, 0, 4, ctx->stream));
+      CK(ctx, cudaMemcpyAsync(d_src, d_T, 1, cudaMemcpyDeviceToDevice, ctx->stream));
+      CK(ctx, cudaMemsetAsync(d_len, 0, 4, ctx->stream));
+      if (host_wait(ctx, ctx->stream)) return BWTC_CUDA_ECUDA;
+    }
+    return 1;
+  }
+  return run_lz77(ctx, nullptr, static_cast<const uint8_t*>(d_T), n, static_cast<int32_t*>(d_src), static_cast<int32_t*>(d_len),
+                  capacity);
 }
 
 int bwtc_cuda_sufcheck(bwtc_cuda_ctx* ctx, const uint8_t* T, const int32_t* SA, uint32_t n) {

@@ -3051,4 +3051,369 @@ __global__ void __launch_bounds__(256) k_sa_search_long(SearchArgs a) {
   }
 }
 
+
+// =====================================================================================================
+// Greedy LZ77 factorisation from the suffix and LCP arrays (bwtc_cuda_lz77 / _device, DESIGN.md §3.14).  Phrase k starts
+// at p_k (p_0 = 0, p_{k+1} = p_k + max(1, len_k)); len_k is the longest previous factor, its source the PSV or NSV row of
+// p_k's row r (the nearest rows above / below r whose SA value is smaller), PSV on ties; a literal (len 0) carries T[p_k].
+//   Stage A, rank order: lcp(p, SA[PSV]) = min LCP[PSV+1 .. r], lcp(p, SA[NSV]) = min LCP[r+1 .. NSV], so no text byte is
+//     compared.  k_lz_minima: (min SA, min LCP) of every LZ_GROUP rows and of every LZ_ROW_TILE-row tile; k_lz_tree: a
+//     min tree over the tiles (one CTA); k_lz_lpf: each tile's rows in a shared-memory min tree, PSV / NSV found in
+//     O(log tile) steps; a row whose PSV or NSV lies outside its tile walks the tile tree (O(log tiles) steps), then the
+//     found tile's groups and one group's rows (at most LZ_ROW_TILE / LZ_GROUP + LZ_GROUP steps).  (len, src) is
+//     scattered to text order: LPF[SA[r]], 8 bytes.
+//   Stage B, text order: next[i] = i + max(1, len[i]); the phrase starts are the path from 0.  k_lz_exit: per
+//     LZ_TEXT_TILE-position tile, pointer doubling in shared memory gives exit[i], the first path node from i past the
+//     tile.  k_lz_round (ceil(log2 tiles) launches): marking by pointer doubling on exit[] in HBM -- every marked i marks
+//     jump[i], then jump[i] = jump[jump[i]] from the previous round's array -- so the path from 0 gets its first node in
+//     every tile it enters; a round that marks nothing new means all are marked, and the later rounds return at once.
+//     k_lz_mark_tile: the same marking in shared memory from each tile's entry, then the tile's count; k_lz_scan and
+//     k_lz_emit compact the starts into (src, len) in position order (reduce-then-scan, as k_lcp_tile_*).
+// Work: O(n log n) in the worst case, no thread follows a chain, and no kernel waits for another CTA.
+// =====================================================================================================
+constexpr uint32_t LZ_ROW_TILE = 2048;       // rows per CTA of stage A (256 threads x 8), leaves of its shared-memory tree
+constexpr uint32_t LZ_GROUP = 32;            // rows per group minimum (the steps inside a tile found through the tile tree)
+constexpr uint32_t LZ_TEXT_TILE = 4096;      // positions per CTA of stage B (256 threads x 16)
+constexpr uint32_t LZ_NONE = 0xFFFFFFFFu;    // "no row" / neutral element of the minima
+constexpr uint32_t LZ_CTL_OFFSET = 320;      // LzCtl's byte offset in the context's d_wtab, behind the SearchCtl
+static_assert(SEARCH_CTL_OFFSET + sizeof(SearchCtl) <= LZ_CTL_OFFSET, "the LZ counters must not overlap the search's");
+
+struct LzCtl {                               // zeroed per call
+  unsigned long long phrases;                // z, written by k_lz_scan
+  unsigned long long outside;                // rows whose PSV or NSV lay outside their stage-A tile
+  uint32_t rounds;                           // HBM marking rounds that found a new phrase start
+  uint32_t pad;
+};
+
+__device__ __forceinline__ uint2 lz_min2(uint2 a, uint2 b) { return make_uint2(min(a.x, b.x), min(a.y, b.y)); }
+
+// In the min tree tr (heap order, L leaves at L + i, .x = min SA, .y = min LCP): the nearest leaf left of leaf i
+// (right: right of it) whose .x < p, or L if there is none; m = min(m, .y of every leaf strictly between).
+__device__ __forceinline__ uint32_t lz_tree_find(const uint2* tr, uint32_t L, uint32_t i, uint32_t p, bool right, uint32_t& m) {
+  for (uint32_t k = L + i; k > 1u; k >>= 1) {
+    if (right == !(k & 1u)) {
+      uint32_t s = right ? k + 1u : k - 1u;
+      const uint2 v = tr[s];
+      if (v.x < p) {
+        while (s < L) {
+          const uint32_t near = right ? 2u * s : 2u * s + 1u;
+          const uint2 c = tr[near];
+          if (c.x < p) { s = near; }
+          else { m = min(m, c.y); s = near ^ 1u; }
+        }
+        return s - L;
+      }
+      m = min(m, v.y);
+    }
+  }
+  return L;
+}
+
+// (min SA, min LCP) of every group and every tile of rows; leaf t of the tile tree at top[L2 + t].
+__global__ void __launch_bounds__(256) k_lz_minima(const int32_t* __restrict__ sa, const int32_t* __restrict__ lcp, uint32_t n,
+                                                   uint2* __restrict__ grp, uint2* __restrict__ top, uint32_t L2,
+                                                   const uint32_t* __restrict__ ctrl) {
+  if (ctrl[CTR_ERR]) return;
+  __shared__ uint2 wm[8];
+  const uint32_t lane = threadIdx.x & 31u, wid = threadIdx.x >> 5;
+  const uint64_t base = (uint64_t)blockIdx.x * LZ_ROW_TILE;
+  uint2 tm = make_uint2(LZ_NONE, LZ_NONE);
+  for (uint32_t g = wid; g < LZ_ROW_TILE / LZ_GROUP; g += 8u) {
+    const uint64_t r = base + g * LZ_GROUP + lane;
+    uint2 v = r < n ? make_uint2((uint32_t)sa[r], (uint32_t)lcp[r]) : make_uint2(LZ_NONE, LZ_NONE);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1)
+      v = lz_min2(v, make_uint2(__shfl_xor_sync(0xFFFFFFFFu, v.x, o), __shfl_xor_sync(0xFFFFFFFFu, v.y, o)));
+    if (lane == 0u && base + g * LZ_GROUP < n) grp[(base >> 5) + g] = v;
+    tm = lz_min2(tm, v);
+  }
+  if (lane == 0u) wm[wid] = tm;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int k = 1; k < 8; ++k) tm = lz_min2(tm, wm[k]);
+    top[L2 + blockIdx.x] = tm;
+  }
+}
+
+// The tile tree's padding leaves and inner nodes, one level after the other.  One CTA.
+__global__ void __launch_bounds__(1024) k_lz_tree(uint2* __restrict__ top, uint32_t ntiles, uint32_t L2, const uint32_t* __restrict__ ctrl) {
+  if (ctrl[CTR_ERR]) return;
+  for (uint32_t t = ntiles + threadIdx.x; t < L2; t += 1024u) top[L2 + t] = make_uint2(LZ_NONE, LZ_NONE);
+  __syncthreads();
+  for (uint32_t h = L2 >> 1; h >= 1u; h >>= 1) {
+    for (uint32_t k = h + threadIdx.x; k < 2u * h; k += 1024u) top[k] = lz_min2(top[2u * k], top[2u * k + 1u]);
+    __syncthreads();
+  }
+}
+
+// Stage A: (len, src) of every row into LPF[SA[r]] (.x = len, .y = src).
+__global__ void __launch_bounds__(256) k_lz_lpf(const uint8_t* __restrict__ t, const int32_t* __restrict__ sa,
+                                                const int32_t* __restrict__ lcp, uint32_t n, const uint2* __restrict__ grp,
+                                                const uint2* __restrict__ top, uint32_t L2, uint2* __restrict__ lpf,
+                                                LzCtl* __restrict__ ctl, const uint32_t* __restrict__ ctrl) {
+  if (ctrl[CTR_ERR]) return;
+  constexpr uint32_t T = LZ_ROW_TILE;
+  __shared__ uint2 tr[2 * T];
+  const uint32_t tile = blockIdx.x;
+  const uint64_t base = (uint64_t)tile * T;
+  for (uint32_t k = threadIdx.x; k < T; k += 256u) {
+    const uint64_t r = base + k;
+    tr[T + k] = r < n ? make_uint2((uint32_t)sa[r], (uint32_t)lcp[r]) : make_uint2(LZ_NONE, LZ_NONE);
+  }
+  __syncthreads();
+  for (uint32_t h = T >> 1; h >= 1u; h >>= 1) {
+    for (uint32_t k = h + threadIdx.x; k < 2u * h; k += 256u) tr[k] = lz_min2(tr[2u * k], tr[2u * k + 1u]);
+    __syncthreads();
+  }
+  const uint32_t ngroups = (uint32_t)(((uint64_t)n + LZ_GROUP - 1u) / LZ_GROUP);
+  unsigned long long outside = 0;
+  for (uint32_t k = threadIdx.x; k < T; k += 256u) {  // (warp-uniform trip count: lcp_count)
+    const uint64_t r = base + k;
+    if (r >= n) continue;
+    const uint2 me = tr[T + k];
+    const uint32_t p = me.x;
+    bool out = false;
+    // PSV: lcp = min LCP[PSV+1 .. r]
+    uint32_t lp = me.y, sp = 0, m = LZ_NONE;
+    uint32_t j = lz_tree_find(tr, T, k, p, false, m);
+    lp = min(lp, m);
+    if (j < T) {
+      sp = tr[T + j].x;
+    } else {
+      out = true;
+      m = LZ_NONE;
+      const uint32_t t2 = lz_tree_find(top, L2, tile, p, false, m);
+      lp = min(lp, m);
+      if (t2 < L2) {
+        for (uint32_t g = t2 * (T / LZ_GROUP) + (T / LZ_GROUP - 1u);; --g) {
+          if (g >= ngroups) continue;
+          const uint2 v = grp[g];
+          if (v.x < p) {
+            for (uint32_t q = min(g * LZ_GROUP + LZ_GROUP, n) - 1u;; --q) {
+              const uint32_t s = (uint32_t)sa[q];
+              if (s < p) { sp = s; break; }
+              lp = min(lp, (uint32_t)lcp[q]);
+            }
+            break;
+          }
+          lp = min(lp, v.y);
+        }
+      } else {
+        lp = 0;
+      }
+    }
+    // NSV: lcp = min LCP[r+1 .. NSV]
+    uint32_t ln = LZ_NONE, sn = 0;
+    j = lz_tree_find(tr, T, k, p, true, ln);
+    if (j < T) {
+      ln = min(ln, tr[T + j].y);
+      sn = tr[T + j].x;
+    } else {
+      out = true;
+      m = LZ_NONE;
+      const uint32_t t2 = lz_tree_find(top, L2, tile, p, true, m);
+      ln = min(ln, m);
+      if (t2 < L2) {
+        for (uint32_t g = t2 * (T / LZ_GROUP);; ++g) {
+          const uint2 v = grp[g];
+          if (v.x < p) {
+            for (uint32_t q = g * LZ_GROUP;; ++q) {
+              const uint32_t s = (uint32_t)sa[q];
+              ln = min(ln, (uint32_t)lcp[q]);
+              if (s < p) { sn = s; break; }
+            }
+            break;
+          }
+          ln = min(ln, v.y);
+        }
+      } else {
+        ln = 0;
+      }
+    }
+    const uint32_t len = max(lp, ln);
+    lpf[p] = make_uint2(len, len == 0u ? (uint32_t)t[p] : (lp >= ln ? sp : sn));
+    outside += out ? 1u : 0u;
+  }
+  __syncwarp();
+  lcp_count(&ctl->outside, outside);
+}
+
+// Stage B, per text tile [b0, b1): next[] in shared memory, doubled until every entry lies past the tile.  exit[i] to
+// jump[i]; mark[i] = (i == 0).
+__global__ void __launch_bounds__(256) k_lz_exit(const uint2* __restrict__ lpf, uint32_t n, uint32_t* __restrict__ jump,
+                                                 uint8_t* __restrict__ mark, const uint32_t* __restrict__ ctrl) {
+  if (ctrl[CTR_ERR]) return;
+  constexpr uint32_t T = LZ_TEXT_TILE, PER = T / 256u;
+  __shared__ uint32_t nx[T];
+  const uint32_t b0 = blockIdx.x * T, b1 = (uint32_t)min((uint64_t)b0 + T, (uint64_t)n);
+  for (uint32_t k = threadIdx.x; k < T; k += 256u) {
+    const uint32_t i = b0 + k;
+    nx[k] = i < b1 ? i + max(1u, lpf[i].x) : n;
+  }
+  __syncthreads();
+  for (;;) {
+    uint32_t v[PER];
+    bool more = false;
+#pragma unroll
+    for (uint32_t q = 0; q < PER; ++q) {
+      const uint32_t j = nx[threadIdx.x + 256u * q];
+      v[q] = j < b1 ? nx[j - b0] : j;
+      more |= v[q] < b1;
+    }
+    __syncthreads();
+#pragma unroll
+    for (uint32_t q = 0; q < PER; ++q) nx[threadIdx.x + 256u * q] = v[q];
+    if (!__syncthreads_or(more)) break;
+  }
+  for (uint32_t k = threadIdx.x; k < T; k += 256u) {
+    const uint32_t i = b0 + k;
+    if (i < b1) {
+      jump[i] = nx[k];
+      mark[i] = i == 0u ? 1u : 0u;
+    }
+  }
+}
+
+// One HBM marking round k on exit[] (jin = jump^(2^k), jout = jump^(2^(k+1)) unless last).  Runs only if round k - 1 found
+// a new start (ctl->rounds >= k); marks set by this round may be seen by it, which only marks path nodes early.
+__global__ void __launch_bounds__(256) k_lz_round(const uint32_t* __restrict__ jin, uint32_t* __restrict__ jout, uint32_t n,
+                                                  uint8_t* mark, LzCtl* ctl, uint32_t k, uint32_t last,
+                                                  const uint32_t* __restrict__ ctrl) {
+  if (ctrl[CTR_ERR] || *reinterpret_cast<volatile uint32_t*>(&ctl->rounds) < k) return;
+  bool found = false;
+  const uint32_t stride = gridDim.x * blockDim.x;
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+    const uint32_t j = jin[i];
+    if (j < n && mark[i] && !mark[j]) {
+      mark[j] = 1u;
+      found = true;
+    }
+    if (!last) jout[i] = j < n ? jin[j] : n;
+  }
+  if (found && *reinterpret_cast<volatile uint32_t*>(&ctl->rounds) == k) atomicCAS(&ctl->rounds, k, k + 1u);
+}
+
+// Marks the phrase starts of a text tile from its entry (marked by the rounds), by pointer doubling in shared memory;
+// writes the marks back and the tile's count to tcnt.
+__global__ void __launch_bounds__(256) k_lz_mark_tile(const uint2* __restrict__ lpf, uint32_t n, uint8_t* __restrict__ mark,
+                                                      uint32_t* __restrict__ tcnt, const uint32_t* __restrict__ ctrl) {
+  if (ctrl[CTR_ERR]) return;
+  constexpr uint32_t T = LZ_TEXT_TILE, PER = T / 256u;
+  __shared__ uint32_t nx[T];
+  __shared__ uint8_t mk[T];
+  __shared__ uint32_t wc[8];
+  const uint32_t b0 = blockIdx.x * T, b1 = (uint32_t)min((uint64_t)b0 + T, (uint64_t)n);
+  bool any = false;
+  for (uint32_t k = threadIdx.x; k < T; k += 256u) {
+    const uint32_t i = b0 + k;
+    nx[k] = i < b1 ? i + max(1u, lpf[i].x) : n;
+    mk[k] = i < b1 ? mark[i] : 0u;
+    any |= mk[k] != 0u;
+  }
+  if (!__syncthreads_or(any)) {  // no phrase starts here (a phrase spans the whole tile)
+    if (threadIdx.x == 0) tcnt[blockIdx.x] = 0;
+    return;
+  }
+  for (;;) {
+    uint32_t v[PER];
+    bool found = false;
+#pragma unroll
+    for (uint32_t q = 0; q < PER; ++q) {
+      const uint32_t k = threadIdx.x + 256u * q, j = nx[k];
+      if (j < b1 && mk[k] && !mk[j - b0]) {
+        mk[j - b0] = 1u;
+        found = true;
+      }
+      v[q] = j < b1 ? nx[j - b0] : j;
+    }
+    __syncthreads();
+#pragma unroll
+    for (uint32_t q = 0; q < PER; ++q) nx[threadIdx.x + 256u * q] = v[q];
+    if (!__syncthreads_or(found)) break;
+  }
+  uint32_t c = 0;
+  for (uint32_t k = threadIdx.x; k < T; k += 256u) {
+    const uint32_t i = b0 + k;
+    if (i < b1) {
+      mark[i] = mk[k];
+      c += mk[k];
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xFFFFFFFFu, c, o);
+  if ((threadIdx.x & 31u) == 0u) wc[threadIdx.x >> 5] = c;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int k = 1; k < 8; ++k) c += wc[k];
+    tcnt[blockIdx.x] = c;
+  }
+}
+
+// Exclusive sum of the tile counts, in place; the total is z.  One CTA.
+__global__ void __launch_bounds__(1024) k_lz_scan(uint32_t* __restrict__ tcnt, uint32_t ntiles, LzCtl* __restrict__ ctl,
+                                                  const uint32_t* __restrict__ ctrl) {
+  if (ctrl[CTR_ERR]) return;
+  __shared__ uint32_t ws[32];
+  __shared__ uint32_t carry_s;
+  const uint32_t lane = threadIdx.x & 31u, wid = threadIdx.x >> 5;
+  uint32_t carry = 0;
+  for (uint32_t base = 0; base < ntiles; base += 1024u) {
+    const uint32_t k = base + threadIdx.x;
+    const uint32_t v = k < ntiles ? tcnt[k] : 0u;
+    uint32_t inc = v;
+    for (int o = 1; o < 32; o <<= 1) {
+      const uint32_t u = __shfl_up_sync(0xFFFFFFFFu, inc, o);
+      if ((int)lane >= o) inc += u;
+    }
+    if (lane == 31u) ws[wid] = inc;
+    __syncthreads();
+    if (wid == 0) {
+      uint32_t s = ws[lane];
+      for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t u = __shfl_up_sync(0xFFFFFFFFu, s, o);
+        if ((int)lane >= o) s += u;
+      }
+      ws[lane] = s;
+    }
+    __syncthreads();
+    if (k < ntiles) tcnt[k] = carry + (wid ? ws[wid - 1] : 0u) + inc - v;
+    if (threadIdx.x == 1023u) carry_s = carry + ws[31];
+    __syncthreads();
+    carry = carry_s;
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) ctl->phrases = carry;
+}
+
+// The marked starts of a text tile, in position order, to src[tpre + rank] / len[tpre + rank].  Each thread owns 16
+// consecutive positions.
+__global__ void __launch_bounds__(256) k_lz_emit(const uint2* __restrict__ lpf, const uint8_t* __restrict__ mark, uint32_t n,
+                                                 const uint32_t* __restrict__ tpre, int32_t* __restrict__ src,
+                                                 int32_t* __restrict__ len, const uint32_t* __restrict__ ctrl) {
+  if (ctrl[CTR_ERR]) return;
+  constexpr uint32_t PER = LZ_TEXT_TILE / 256u;
+  __shared__ uint32_t ws[8];
+  const uint32_t lane = threadIdx.x & 31u, wid = threadIdx.x >> 5;
+  const uint64_t p0 = (uint64_t)blockIdx.x * LZ_TEXT_TILE + (uint64_t)threadIdx.x * PER;
+  uint32_t bits = 0;
+#pragma unroll
+  for (uint32_t q = 0; q < PER; ++q)
+    if (p0 + q < n && mark[p0 + q]) bits |= 1u << q;
+  const uint32_t c = (uint32_t)__popc(bits);
+  uint32_t inc = c;
+  for (int o = 1; o < 32; o <<= 1) {
+    const uint32_t u = __shfl_up_sync(0xFFFFFFFFu, inc, o);
+    if ((int)lane >= o) inc += u;
+  }
+  if (lane == 31u) ws[wid] = inc;
+  __syncthreads();
+  uint32_t o = tpre[blockIdx.x] + inc - c;
+  for (uint32_t k = 0; k < wid; ++k) o += ws[k];
+  for (; bits; bits &= bits - 1u, ++o) {
+    const uint2 v = lpf[p0 + (uint32_t)(__ffs((int)bits) - 1)];
+    len[o] = (int32_t)v.x;
+    src[o] = (int32_t)v.y;
+  }
+}
+
 }  // namespace bwtc_b200

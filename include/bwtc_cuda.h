@@ -17,6 +17,8 @@
  *                                              convention of libsais's libsais_plcp / libsais_lcp
  *   bwtc_cuda_sa_search / _device          <-  sa_search / sa_simplesearch                 (libdivsufsort's pattern
  *                                              search in a suffix array, for a batch of patterns)
+ *   bwtc_cuda_lz77 / _device               <-  no counterpart in bwtc: the greedy LZ77 factorisation from the SA and
+ *                                              LCP arrays (the KKP convention, self-reference allowed)
  *   bwtc_cuda_bwt_block                    <-  BWTransform::doTransform(BWTBlock&, uint32 freqs[256])
  *                                              bwtransforms/BWTransform.cpp:39-64 (reverse / sentinel /
  *                                              hole-fill fused on the device)
@@ -95,7 +97,9 @@ typedef struct bwtc_cuda_stats {
                               * array (bwtc_cuda_divsufsort, _device, and the _lcp variants); bit 9: this call produced an
                               * LCP array (bwtc_cuda_divsufsort_lcp, _lcp_device); bit 10: round 0 ran its digit passes over the
                               * top key digits only and sorted the low digits bucket by bucket (k_bucket_sort, BWTC_ROUND0_TOP);
-                              * bit 11: this call was a pattern search (bwtc_cuda_sa_search, _device; no other entry point sets it) */
+                              * bit 11: this call was a pattern search (bwtc_cuda_sa_search, _device; no other entry point sets it);
+                              * bit 12: this call produced an LZ77 factorisation (bwtc_cuda_lz77, _device; no other entry point
+                              * sets it) */
   uint32_t batch_blocks;     /* blocks this record describes: 1, or the size of the batch that was sorted as one text (every
                               * block of the batch then carries the SAME record — count it once; flags bit 7 is the one field
                               * in which the records of one inverse batch may differ) */
@@ -142,7 +146,9 @@ int         bwtc_cuda_ctx_set_verify(bwtc_cuda_ctx* ctx, int on);
  * (which: 0 text, 1 rank[], 2/3 sorted keys/ids of the last round, 4/5 the other sort buffer,
  * 6 control+histogram words, 7 staged input, 9 the work counters of the last LCP stage: irreducible rows, bytes
  * compared by the short tier and by the windows, window segments (4 x u64), then the pairs in each window's list, u32;
- * 10 the work counters of the last pattern search: probes made and text bytes compared, 2 x u64). */
+ * 10 the work counters of the last pattern search: probes made and text bytes compared, 2 x u64;
+ * 11 the counters of the last LZ77 factorisation: phrases z and the rows whose PSV or NSV lay outside their tile (2 x u64),
+ * then the marking rounds in HBM that found new phrase starts (u32)). */
 int         bwtc_cuda_ctx_set_debug(bwtc_cuda_ctx* ctx, uint32_t max_rounds);
 int         bwtc_cuda_debug_read(bwtc_cuda_ctx* ctx, int which, uint64_t offset_bytes, void* dst, uint64_t bytes);
 
@@ -226,6 +232,34 @@ int bwtc_cuda_sa_search(bwtc_cuda_ctx* ctx, const uint8_t* T, uint32_t n, const 
                         const uint8_t* P, const uint64_t* P_off, uint32_t count, int32_t* left, int32_t* size);
 int bwtc_cuda_sa_search_device(bwtc_cuda_ctx* ctx, const void* d_T, uint32_t n, const void* d_SA, uint32_t SAsize,
                                const void* d_P, const void* d_P_off, uint32_t count, void* d_left, void* d_size);
+
+/* lz77(T, n): the greedy LZ77 factorisation of T with self-reference allowed (the convention of Karkkainen, Kempa &
+ * Puglisi's KKP and of Shun & Zhao, "Practical Parallel Lempel-Ziv Factorization", DCC 2013).  Phrase k starts at p_k, p_0 = 0 and
+ * p_{k+1} = p_k + max(1, len_k); len_k is the longest l with T[p_k .. p_k+l) = T[j .. j+l) for some j < p_k (the source may
+ * overlap the phrase).  A literal (len_k == 0) has src_k = T[p_k], the byte value 0..255.  Otherwise the source is fixed,
+ * so that results compare bit for bit: with r the row of p_k in bwtc_cuda_divsufsort's SA, PSV = the largest row r' < r
+ * with SA[r'] < p_k and NSV = the smallest row r' > r with SA[r'] < p_k; l_P / l_N = their LCPs with p_k (0 for a missing
+ * one); len_k = max(l_P, l_N) and src_k = SA[PSV] if l_P >= l_N, else SA[NSV].  Decoding copies len_k bytes from src_k one
+ * by one (so overlapping sources work), or appends the literal.
+ * Returns the phrase count z >= 0 or a negative error, like snprintf: src[0..z) and len[0..z) are written only when
+ * z <= capacity; otherwise z is returned and both arrays are untouched.  With capacity == 0, src and len may be NULL (a
+ * count query).  n == 0 returns 0 and writes nothing; n == 1 returns 1 and writes the literal (T[0], 0) if capacity >= 1
+ * (the host variant does not touch the device).  n <= max_block_bytes + 1 (else BWTC_CUDA_ETOOBIG; both variants sort in the
+ * context).  Null T / d_T is BWTC_CUDA_EARG; so are, when capacity > 0, null phrase arrays and, for _device, d_src / d_len
+ * not 4-byte aligned or overlapping within capacity entries.
+ * The sort, the LCP stage of bwtc_cuda_divsufsort_lcp and the LZ77 stage run on the device (DESIGN.md §3.14: nearest
+ * smaller values with range minima of the LCP in rank order, then the greedy parse by pointer doubling in text order,
+ * compacted in scratch).  One host wait reads z; the z phrases are then copied: _device with one device-to-device copy
+ * each, the host variant directly into pinned arrays and through the staging ring into pageable ones.  Memory: the SA goes
+ * to the 4 (max_block_bytes + 1)-byte device array of bwtc_cuda_divsufsort, which either variant allocates on its first
+ * call (BWTC_CUDA_EALLOC if that fails); everything else runs in scratch that is idle by then, and
+ * bwtc_cuda_scratch_bytes is unchanged.  With verification on, the SA is sufchecked before the LCP and LZ77 stages: on a
+ * failure the call returns BWTC_CUDA_EVERIFY and src / len are untouched; the phrases are not re-checked.
+ * stats: a new record with n_suffixes = n, flags bits 8, 9 and 12 (bit 6 too when verified); gpu_ms, kernel_launches and
+ * algorithmic_bytes include the LCP and LZ77 stages.  bwtc_cuda_debug_read(ctx, 11, ...) returns the stage's counters. */
+int64_t bwtc_cuda_lz77(bwtc_cuda_ctx* ctx, const uint8_t* T, uint32_t n, int32_t* src, int32_t* len, uint32_t capacity);
+int64_t bwtc_cuda_lz77_device(bwtc_cuda_ctx* ctx, const void* d_T, uint32_t n, void* d_src, void* d_len,
+                              uint32_t capacity);
 
 /* ---- block contract: BWTransform::doTransform(BWTBlock&, freqs) (BWTransform.cpp:52-64) ---------- */
 /* block: n bytes (host), transformed IN PLACE; unlike the reference wrapper the byte after the block
